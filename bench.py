@@ -4,6 +4,7 @@
 as secondary lines.
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
+    python bench.py --steps K --dump-outputs DIR             # ... and the outputs of its last timed step as DIR/*.npy
     python bench.py --impl reference --gpus N --steps K ...  # the CPU arm (oracle, all host threads)
 
 A "step" is one VmapAutoResetWrapper(Connector).step over the whole batch with actions from the
@@ -179,6 +180,57 @@ def timed_samples(dd: Dist, enqueue, steps: int, min_ms: float = 60.0, samples: 
     return R, out
 
 
+def timed_window(dd: Dist, enqueue, steps: int, spin_cycles: int = 2_000_000) -> float:
+    """Device time in ms of exactly `steps` steps enqueued back to back between two CUDA events, max over ranks.
+    A spin kernel of about 1 ms ahead of the first event keeps the stream busy while the host enqueues the first
+    launches, so the window times the steps and not the host's launch latency."""
+    import torch
+
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    dd.sync()
+    torch.cuda._sleep(spin_cycles)
+    e0.record()
+    enqueue(steps)
+    e1.record()
+    dd.sync()
+    return dd.max(e0.elapsed_time(e1))
+
+
+DUMP_ENVS = 16384  # envs sampled for --dump-outputs: 45 MB at 10x10/5, under a budget of 64 MB
+
+
+def _dump_outputs(path, state, ts, act, t, B):
+    """The last timed step as a caller of rbg_connector_rollout_random receives it: TimeStep `t` of the stacked outputs, the
+    actions taken in that step and the State after it, for a fixed seeded sample of envs (all of them when B <= DUMP_ENVS).
+    Keys (uint32) as float64, everything else as float32: codes, counts and coordinates are small integers, exact in both."""
+    import numpy as np
+    import torch
+
+    idx = np.arange(B) if B <= DUMP_ENVS else np.sort(np.random.default_rng(0).choice(B, DUMP_ENVS, replace=False))
+    sel = torch.from_numpy(idx).to(state.grid.device)
+    o, a = ts.observation, state.agents
+    arrays = {
+        "env_index": (torch.from_numpy(idx), np.float64),
+        "observation_grid": (o.grid[t], np.float32), "observation_action_mask": (o.action_mask[t], np.float32), "observation_step_count": (o.step_count[t], np.float32),
+        "reward": (ts.reward[t], np.float32), "discount": (ts.discount[t], np.float32), "step_type": (ts.step_type[t], np.float32),
+        "num_connections": (ts.extras["num_connections"][t], np.float32), "ratio_connections": (ts.extras["ratio_connections"][t], np.float32),
+        "total_path_length": (ts.extras["total_path_length"][t], np.float32), "action": (act[t], np.float32),
+        "state_grid": (state.grid, np.float32), "state_step_count": (state.step_count, np.float32), "state_key": (state.key.view(torch.int32), np.float64),
+        "agent_id": (a.id, np.float32), "agent_start": (a.start, np.float32), "agent_target": (a.target, np.float32), "agent_position": (a.position, np.float32),
+    }
+    os.makedirs(path, exist_ok=True)
+    total = 0
+    for name, (x, dtype) in arrays.items():
+        x = x if name == "env_index" else x.index_select(0, sel)
+        v = x.cpu().numpy()
+        if name == "state_key":
+            v = v.view(np.uint32)
+        v = v.astype(dtype)
+        total += v.nbytes
+        np.save(os.path.join(path, f"{name}.npy"), v)
+    assert total <= 64 << 20, total
+
+
 def _stats(xs):
     return {"median": round(statistics.median(xs), 6), "min": round(min(xs), 6), "max": round(max(xs), 6)}
 
@@ -223,10 +275,13 @@ def run_ours(args):
     ts = engine.alloc_timestep(B, G, N, chunk)
     act = torch.empty((chunk, B, N), dtype=torch.int32, device=dev)
 
+    last = {}
+
     def run_steps(k):
         while k > 0:
             n = min(k, chunk)
             engine.connector_rollout_random(state, n, TIME_LIMIT, -0.03, 0.1, autoreset_kind="parallel_random_walk", out=ts, actions=act, owner=env)
+            last["t"] = n - 1  # the slot of the stacked outputs that holds the latest step
             k -= n
 
     # Burn-in to the stationary regime: right after reset() every env is at step 0, so the
@@ -236,15 +291,16 @@ def run_ours(args):
     run_steps(max(args.warmup, 3))
     dd.sync()
 
-    # ---- timed region: blocks of exactly K steps, device-timed, max over ranks
+    # ---- timed region: exactly K steps, device-timed, max over ranks
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     rbg.launch_count(reset=True)
-    R, block_ms = timed_samples(dd, run_steps, args.steps, min_ms=args.min_ms, samples=args.samples)
+    ms_window = timed_window(dd, run_steps, args.steps)
     launches = rbg.launch_count()
-    ms_block = statistics.median(block_ms)
-    value = total * args.steps / (ms_block / 1e3)
+    value = total * args.steps / (ms_window / 1e3)
+    if args.dump_outputs and rank == 0:
+        _dump_outputs(args.dump_outputs, state, ts, act, last["t"], B)
 
     # ---- the dominant kernel alone: event pairs recorded inside the library around every launch
     # (which also switches the head-to-tail chaining of consecutive launches off), over a second pass
@@ -267,13 +323,13 @@ def run_ours(args):
     # regeneration of finished envs), chained head to tail, so its average launch duration over the region is the
     # region's device time / launches.  The same launch timed ALONE (event pair around it, not chained: its ragged tail
     # and the generator warps' drain are exposed) is reported next to it.
-    launches_per_block = max(1, -(-args.steps // chunk))
-    k_ms = ms_block / launches_per_block
-    achieved = alg * (args.steps / launches_per_block / steps_per_launch) / (k_ms / 1e3) / 1e9
+    launches_timed = -(-args.steps // chunk)
+    k_ms = ms_window / launches_timed
+    achieved = alg * (args.steps / launches_timed / steps_per_launch) / (k_ms / 1e3) / 1e9
     alone_ms = ms_ro / max(n_ro, 1)
     alone = alg / (alone_ms / 1e3) / 1e9
     step_alg = B * (TS_BYTES + 4 * N + 2 * STATE_BYTES / steps_per_launch)  # algorithmic bytes of one whole step
-    step_gbs = step_alg / (ms_block / args.steps / 1e3) / 1e9
+    step_gbs = step_alg / (ms_window / args.steps / 1e3) / 1e9
     roofline = {"kernel": "rollout_persist_kernel", "bound": "hbm", "achieved": round(achieved, 1), "peak": peak, "unit": "GB/s", "frac": round(achieved / peak, 4),
                 "traffic": _profile_number("rollout_persist_kernel"), "algorithmic_bytes_per_launch": int(alg), "steps_per_launch": steps_per_launch,
                 "avg_launch_ms": round(k_ms, 5), "peak_source": peak_src, "kernel_share_of_step": round(ms_ro / max(ms_ro + ms_prw + ms_env, 1e-9), 4),
@@ -315,14 +371,15 @@ def run_ours(args):
     if rank == 0:
         line = {
             "metric": METRIC, "value": round(value, 1), "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3),
-            "ms_per_step": round(ms_block / args.steps, 5), "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "int32",
+            "ms_per_step": round(ms_window / args.steps, 5), "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "int32",
             "data": "synthetic (keys = split(PRNGKey(0), B), random-policy actions)",
             "config": {"workload": "connector_step_random_agent_autoreset_prw", "grid": G, "agents": N, "envs_per_gpu": B, "envs_total": total, "time_limit": TIME_LIMIT,
                        "generator": "ParallelRandomWalkGenerator", "parallelism": f"env-sharded x{world}", "burnin_steps": args.burnin,
                        "api": f"rbg_connector_rollout_random, {chunk} steps per call (the reference's n_steps scan), State in place, stacked TimeSteps and actions written every step",
                        "l2": f"no flush: every step writes {(TS_BYTES + 4 * N) * B / 1e6:.0f} MB per GPU into a fresh slice of the stacked [{chunk}, B, ...] outputs ({(TS_BYTES + 4 * N) * B * chunk / 1e9:.1f} GB per call), far beyond the 126 MB L2"},
-            "timing": {"what": f"a sample = {R} blocks of exactly {args.steps} steps enqueued back to back between two CUDA events (barrier + synchronize on both sides, max over ranks); value / ms_per_step from the median sample",
-                       "blocks_per_sample": R, "samples": len(block_ms), "ms_per_block": _stats(block_ms), "sample_ms": round(R * ms_block, 3)},
+            "timing": {"what": f"exactly {args.steps} steps ({launches_timed} rollout calls) enqueued back to back between two CUDA events (barrier + synchronize on both sides, max over ranks); "
+                               "the window includes the ramp of its first launch and the drain of its last, which a short window does not amortise",
+                       "window_ms": round(ms_window, 4)},
             "roofline": roofline, "cpu_baseline": cpu_baseline, "e2e": e2e, "gpu_launches": launches, "clocks": clocks, "secondary": secondary,
         }
         print(json.dumps(line), flush=True)
@@ -685,19 +742,21 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=500)
+    ap.add_argument("--steps", type=int, default=500, help="timed steps: exactly this many, in one window")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--envs", type=int, default=ENVS_PER_GPU, help="envs per GPU")
     ap.add_argument("--burnin", type=int, default=160, help="untimed steps after reset() so that episode ends are desynchronised")
     ap.add_argument("--chunk", type=int, default=20, help="env steps per rollout call (the reference's n_steps)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
-    ap.add_argument("--min-ms", type=float, default=60.0, help="a timed sample lasts at least this long (blocks of --steps steps back to back)")
-    ap.add_argument("--samples", type=int, default=5, help="timed samples (median reported)")
     ap.add_argument("--skip-e2e", action="store_true")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs (rank 0's envs, a fixed sample of at most "
+                    f"{DUMP_ENVS}) to DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,10 +1,13 @@
 """The CPU oracle against outputs of the REFERENCE'S OWN Python source.
 
 tests/golden/reference_runs.json was produced by tests/tools/make_reference_fixtures.py, which
-imports the reference's files unmodified from /root/reference and runs them on the NumPy stand-in
-for jax in tests/tools/jax_shim (jax / jumanji are not installable here).  This pins what the
+imports the reference's files unmodified from a checkout of the reference and runs them on the NumPy
+stand-in for jax in tests/tools/jax_shim (jax / jumanji are not installable here).  This pins what the
 reference's own goldens do not cover: the ParallelRandomWalk collision branch, SeedExtension with
 every option, and the three generators' States.  No GPU needed.
+
+The last two tests run the reference's own source, which this repository does not contain: they
+skip unless RBG_REFERENCE names a checkout of mwolinska/Routing-Board-Generation.
 """
 import json
 import os
@@ -15,7 +18,8 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = os.environ.get("RBG_REFERENCE", "")
+needs_reference = pytest.mark.skipif(not (REF and os.path.isdir(os.path.join(REF, "routing_board_generation"))), reason="RBG_REFERENCE does not name a checkout of the reference")
 
 
 @pytest.fixture(scope="module")
@@ -95,19 +99,19 @@ def test_dataset_generator(orc, runs):
             assert st["start"][b].tolist() == ref_st["start"] and st["target"][b].tolist() == ref_st["target"]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="/root/reference is not mounted (GPU box)")
-def test_shim_passes_the_references_own_tests():
+@needs_reference
+def test_shim_passes_the_references_own_tests(tmp_path):
     """The NumPy jax stand-in the fixtures were made with runs the reference's only test file green."""
     shim = os.path.join(ROOT, "tests", "tools", "jax_shim")
     test = os.path.join(REF, "routing_board_generation/board_generation_methods/jax_implementation/board_generation/test_parallel_random_walk_board.py")
     env = dict(os.environ, PYTHONPATH=shim + os.pathsep + REF)
-    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", test], cwd="/tmp", env=env, capture_output=True, text=True, timeout=600)
+    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", test], cwd=tmp_path, env=env, capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stdout[-2000:]
     assert "35 passed" in r.stdout
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="/root/reference is not mounted (GPU box)")
-def test_sequential_random_walk_is_not_instantiable():
+@needs_reference
+def test_sequential_random_walk_is_not_instantiable(tmp_path):
     """SURVEY 8(f).4: SequentialRandomWalkBoard subclasses the NumPy AbstractBoard without implementing
     its abstract methods, so the reference cannot construct it (nor the generator built on it) as shipped.
     The engine's mirror IS instantiable and reproduces the method bodies, which tests/tools/make_seqrw_fixtures.py
@@ -121,6 +125,6 @@ def test_sequential_random_walk_is_not_instantiable():
         "    print('TypeError:', e)\n"
     )
     env = dict(os.environ, PYTHONPATH=shim + os.pathsep + REF)
-    r = subprocess.run([sys.executable, "-c", code], cwd="/tmp", env=env, capture_output=True, text=True, timeout=300)
+    r = subprocess.run([sys.executable, "-c", code], cwd=tmp_path, env=env, capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stderr[-2000:]
     assert "TypeError" in r.stdout and "abstract" in r.stdout
