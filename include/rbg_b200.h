@@ -194,14 +194,14 @@ int rbg_connector_reset(int kind, const uint32_t *keys, int64_t B, int G, int N,
 /* bytes of device scratch rbg_connector_step needs when autoreset is on.  The
  * workspace belongs to ONE env batch for as long as that batch is stepped: besides
  * the reset lists it caches, per env, the next episode's start / target pins, which
- * the library generates ahead of time on an internal side stream (the reset key of
+ * the library generates ahead of time on the caller's stream (the reset key of
  * an episode is known when the episode starts).  16-byte aligned, need not be
  * cleared.  Call rbg_workspace_release before freeing it, and before handing it to
  * another env batch (the library re-initialises it by itself when the shape or the
  * generator kind changes, or after a SeedExtension batch has used it; a batch of the
  * same shape and kind would merely start with cache misses). */
 int64_t rbg_step_workspace_bytes(int64_t B, int G, int N);
-/* waits for the side-stream work tied to `workspace` and forgets it */
+/* waits for the work queued on `workspace` (on the stream it was last used on) and forgets it */
 int rbg_workspace_release(void *workspace);
 
 /* Connector.step(state, action) (JUM env.py step), or with
@@ -319,17 +319,17 @@ int64_t rbg_launch_count(int reset);
  * every kernel launch is bracketed by a pair of CUDA events recorded on the
  * launching stream.  rbg_kernel_time synchronises on the recorded events,
  * returns the number of launches of `kernel` (RBG_K_*) and their summed device
- * time since the last call, and clears that kernel's record.  The fused rollout
- * normally runs slices of the batch on several streams so that their kernels
- * overlap; while timing is enabled it launches everything on the caller's
- * stream, one kernel at a time, so that a pair of events times one kernel. */
+ * time since the last call, and clears that kernel's record.  Consecutive fused
+ * rollout launches, and a per-step env kernel with the cache refill of the step
+ * before it, normally overlap on the stream; while timing is enabled they run one kernel at
+ * a time, so that a pair of events times one kernel. */
 #define RBG_K_PRW 0        /* prw_kernel: ParallelRandomWalk / Uniform generator */
 #define RBG_K_ENV 1        /* env_kernel: Connector step / observe */
 #define RBG_K_RANDACT 2    /* random_actions_kernel */
 #define RBG_K_SPLIT 3      /* split_keys_kernel */
 #define RBG_K_VALIDATE 4   /* validate_kernel */
 #define RBG_K_SEEDEXT 5    /* seedext_kernel */
-#define RBG_K_ROLLOUT 6    /* rollout_warp_kernel: T fused steps */
+#define RBG_K_ROLLOUT 6    /* rollout_persist_kernel (rollout_warp_kernel for the dataset generator): T fused steps */
 #define RBG_K_SEQRW 7      /* seqrw_walk_kernel + its finish kernel */
 #define RBG_K_COUNT 8
 int rbg_kernel_timing(int enable);

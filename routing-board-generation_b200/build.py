@@ -15,7 +15,7 @@ LIBDIR = os.path.join(HERE, "lib")
 SO = os.path.join(LIBDIR, "librbg_b200.so")
 SOURCES = ["c_api.cu", "prw_kernel.cu", "connector_kernel.cu", "misc_kernels.cu", "seedext_kernel.cu", "seqrw_kernel.cu", "host_pool.cpp"]
 CXX_FLAGS = ["-O3", "-std=c++17", "-fPIC", "-pthread"]  # plain C++ sources (host threads of the transport layer): g++
-HEADERS = ["rbg_device.cuh", "connector_device.cuh", "obs_stage.cuh", "prw_warp.cuh", "gen_warp.cuh", "select.cuh", "rbg_host.h", os.path.join("..", "..", "include", "rbg_b200.h")]
+HEADERS = ["rbg_device.cuh", "connector_device.cuh", "obs_stage.cuh", "gen_warp.cuh", "select.cuh", "rbg_host.h", os.path.join("..", "..", "include", "rbg_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

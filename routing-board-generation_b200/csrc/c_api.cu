@@ -214,8 +214,8 @@ static int generator_state_impl(int kind, const uint32_t *keys, int64_t B, int G
 // ---- auto-reset workspace ------------------------------------------------------
 // VmapAutoResetWrapper regenerates a board whenever an env finishes.  The reset key
 // of an episode is known as soon as the episode starts (split(state.key)[0]), so the
-// NEXT episode of every env that just reset is generated ahead of time on a side
-// stream ("refill") into a per-env cache; when the env finishes, env_kernel swaps the
+// NEXT episode of every env that just reset is generated ahead of time ("refill")
+// into a per-env cache; when the env finishes, env_kernel swaps the
 // cached episode in.  Only envs whose cache entry is not ready (first episode, or two
 // terminations in consecutive steps) take the synchronous reset kernel.  Results are
 // identical either way: a board is a pure function of its key.
@@ -254,50 +254,18 @@ struct AutoResetCtx {
   int G = 0, N = 0, kind = -1;
   uint64_t step = 0;
   int persist_epoch = 0;  // launches of the persistent rollout on this workspace
-  int persist_groups = 0; // group size the flags were laid out for
   cudaStream_t last_stream = nullptr;  // the stream the workspace was last used on
   bool tail_valid = false;
-  cudaStream_t side = nullptr;
-  cudaEvent_t env_done = nullptr;
-  cudaEvent_t refill_done[2] = {nullptr, nullptr};
-  bool refill_pending[2] = {false, false};
-  // fused rollout: slices 1.. of the batch run on their own streams
-  cudaStream_t slice_stream[3] = {nullptr, nullptr, nullptr};
-  cudaEvent_t slice_fork = nullptr, slice_done[3] = {nullptr, nullptr, nullptr};
 };
 static std::mutex g_ar_mu;
 static std::unordered_map<void *, AutoResetCtx> g_ar;
 
 // The next speculative call on `workspace` must adopt it afresh (counters zeroed, cache warm-started):
-// its contents are no longer what the recorded context left there.  Pending refills are joined first.
-static void invalidate_workspace(void *workspace, cudaStream_t stream, bool block = false) {
+// its contents are no longer what the recorded context left there.
+static void invalidate_workspace(void *workspace) {
   std::lock_guard<std::mutex> lock(g_ar_mu);
   auto it = g_ar.find(workspace);
-  if (it == g_ar.end()) return;
-  for (int i = 0; i < 2; ++i)
-    if (it->second.refill_pending[i]) {
-      if (block)
-        cudaEventSynchronize(it->second.refill_done[i]);
-      else
-        cudaStreamWaitEvent(stream, it->second.refill_done[i], 0);
-      it->second.refill_pending[i] = false;
-    }
-  it->second.B = 0;
-}
-
-// Per-step auto-reset: where the cache refill of step t runs.  Default: on the CALLER'S stream, as a kernel that says
-// launch_dependents at once, followed (next call) by an env kernel launched with programmatic stream serialization, so
-// the refill of step t overlaps the env kernel of step t + 1 by construction and nothing else moves (the synchronous
-// reset kernel of step t + 1 is a plain launch and waits for both).  RBG_STEP_SIDE_STREAM=1: the round-1 scheme, a
-// low-priority side stream joined two steps later, whose overlap depended on which hardware queue the side stream
-// happened to share (65.6 or 84.5 us per step, DESIGN.md K2).
-static bool step_side_stream() {
-  static int v = -1;
-  if (v < 0) {
-    const char *e = getenv("RBG_STEP_SIDE_STREAM");
-    v = (e && atoi(e) != 0) ? 1 : 0;
-  }
-  return v == 1;
+  if (it != g_ar.end()) it->second.B = 0;
 }
 
 // The workspace moves to another stream (rare): its work on the old stream is awaited on the host.  Events per call
@@ -312,15 +280,11 @@ static int workspace_follow_stream(AutoResetCtx *ctx, cudaStream_t stream) {
   return RBG_OK;
 }
 
-static bool speculative_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char *e = getenv("RBG_NO_SPECULATIVE_RESET");
-    v = (e && atoi(e) != 0) ? 0 : 1;
-  }
-  return v == 1;
-}
-
+// Per-step auto-reset with the cache (ParallelRandomWalk / Uniform): everything runs on the caller's stream.  The
+// synchronous resets of step t and the cache refill are one kernel (prw_pair_kernel) that says launch_dependents
+// between the two, and the env kernel of step t + 1 is launched with programmatic stream serialization, so the refill
+// of step t overlaps the env kernel of step t + 1 by construction and nothing else moves.  While kernel timing is on,
+// the three run unchained: env kernel, synchronous reset kernel, refill kernel.
 static int connector_step_impl(const rbg_state *in, const rbg_state *out, const int32_t *action, int32_t *action_out,
                                int random_policy, int64_t B, int G, int N, const rbg_env_params *params,
                                const rbg_timestep *ts, void *workspace, cudaStream_t stream) {
@@ -358,36 +322,19 @@ static int connector_step_impl(const rbg_state *in, const rbg_state *out, const 
   if (!aligned16(ws)) return set_error(RBG_EALIGN, "workspace not 16-byte aligned");
   const WsLayout wl = ws_layout(B, N);
   const int kind = params->autoreset_kind;
-  const bool speculative = speculative_enabled() && (kind == RBG_GEN_PRW || kind == RBG_GEN_UNIFORM);
+  const bool speculative = kind == RBG_GEN_PRW || kind == RBG_GEN_UNIFORM;
   int32_t *sync_count = reinterpret_cast<int32_t *>(ws);
   int32_t *sync_list = reinterpret_cast<int32_t *>(ws + wl.sync_list);
   p.list = sync_list;
   p.list_count = sync_count;
   cudaError_t e;
   AutoResetCtx *ctx = nullptr;
-  int par = 0;
   if (speculative) {
     std::lock_guard<std::mutex> lock(g_ar_mu);
     ctx = &g_ar[workspace];
-    if (!step_side_stream()) {
-      if ((rc = workspace_follow_stream(ctx, stream))) return rc;
-    } else if (!ctx->side) {
-      // lowest priority: the refill has a whole step of slack, env_kernel's CTAs go first
-      int prio_lo = 0, prio_hi = 0;
-      cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
-      if ((e = cudaStreamCreateWithPriority(&ctx->side, cudaStreamNonBlocking, prio_lo)) != cudaSuccess) return set_cuda_error(e, "cudaStreamCreate(side)");
-      if ((e = cudaEventCreateWithFlags(&ctx->env_done, cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
-      for (int i = 0; i < 2; ++i)
-        if ((e = cudaEventCreateWithFlags(&ctx->refill_done[i], cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
-    }
+    if ((rc = workspace_follow_stream(ctx, stream))) return rc;
     if (ctx->B != B || ctx->G != G || ctx->N != N || ctx->kind != kind) {
-      // first use of this workspace (or a different batch in it): nothing cached yet.
-      // Pending refills of the previous occupant must not land after the clear.
-      for (int i = 0; i < 2; ++i)
-        if (ctx->refill_pending[i]) {
-          cudaStreamWaitEvent(stream, ctx->refill_done[i], 0);
-          ctx->refill_pending[i] = false;
-        }
+      // first use of this workspace (or a different batch in it): nothing cached yet
       if ((e = cudaMemsetAsync(ws, 0, 256, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(counters)");
       // warm start: the next episode of EVERY env, one bulk generation keyed by the
       // current State.key (a cold cache would send each env's first reset down the
@@ -413,12 +360,8 @@ static int connector_step_impl(const rbg_state *in, const rbg_state *out, const 
       ctx->step = 0;
       ctx->persist_epoch = 0;
     }
-    par = (int)(ctx->step & 1);
-    // the refill launched two steps ago used this parity's list buffers
-    if (ctx->refill_pending[par]) {
-      if ((e = cudaStreamWaitEvent(stream, ctx->refill_done[par], 0)) != cudaSuccess) return set_cuda_error(e, "cudaStreamWaitEvent");
-      ctx->refill_pending[par] = false;
-    }
+    // the refill lists alternate between two buffers: this step's env kernel runs under the previous step's refill
+    const int par = (int)(ctx->step & 1);
     p.cache_tag = reinterpret_cast<const unsigned long long *>(ws + wl.cache_tag);
     p.cache_key = reinterpret_cast<const uint2 *>(ws + wl.cache_key);
     p.cache_pins = reinterpret_cast<const uint32_t *>(ws + wl.cache_pins);
@@ -433,9 +376,9 @@ static int connector_step_impl(const rbg_state *in, const rbg_state *out, const 
     // This path leaves its reset count in the counter.  If the same workspace has served (or will
     // serve) a speculative batch, that batch must adopt it afresh: its kernels rely on counters
     // that are zero between steps.
-    invalidate_workspace(workspace, stream);
+    invalidate_workspace(workspace);
   }
-  const bool chained = speculative && !step_side_stream() && !g_timing.load(std::memory_order_relaxed);
+  const bool chained = speculative && !g_timing.load(std::memory_order_relaxed);
   if ((rc = launch_env(p, stream, chained))) return rc;
   // VmapAutoResetWrapper._auto_reset: key, _ = split(state.key); reset(key):
   // one more leading split()[0] than a plain generator call.
@@ -478,11 +421,6 @@ static int connector_step_impl(const rbg_state *in, const rbg_state *out, const 
   }
   if ((rc = generator_state_impl(kind, out->key, B, G, N, out, ts, 1, sync_list, sync_count, stream, speculative ? sync_count + 1 : nullptr))) return rc;
   if (speculative) {
-    const bool side = step_side_stream();
-    if (side) {
-      if ((e = cudaEventRecord(ctx->env_done, stream)) != cudaSuccess) return set_cuda_error(e, "cudaEventRecord");
-      if ((e = cudaStreamWaitEvent(ctx->side, ctx->env_done, 0)) != cudaSuccess) return set_cuda_error(e, "cudaStreamWaitEvent(side)");
-    }
     PrwParams q;
     memset(&q, 0, sizeof(q));
     q.keys = p.refill_keys;
@@ -500,14 +438,8 @@ static int connector_step_impl(const rbg_state *in, const rbg_state *out, const 
     q.cache_tag = reinterpret_cast<unsigned long long *>(ws + wl.cache_tag);
     q.cache_key = reinterpret_cast<uint2 *>(ws + wl.cache_key);
     q.cache_pins = reinterpret_cast<uint32_t *>(ws + wl.cache_pins);
-    if (side) {
-      if ((rc = launch_prw(q, B, env_int("RBG_PRW_M"), env_int("RBG_PRW_THREADS"), ctx->side))) return rc;
-      if ((e = cudaEventRecord(ctx->refill_done[par], ctx->side)) != cudaSuccess) return set_cuda_error(e, "cudaEventRecord(side)");
-      ctx->refill_pending[par] = true;
-    } else {
-      q.trigger_dependents = 1;
-      if ((rc = launch_prw(q, B, env_int("RBG_PRW_M"), env_int("RBG_PRW_THREADS"), stream))) return rc;
-    }
+    q.trigger_dependents = 1;
+    if ((rc = launch_prw(q, B, env_int("RBG_PRW_M"), env_int("RBG_PRW_THREADS"), stream))) return rc;
     ctx->step++;
   }
   return RBG_OK;
@@ -958,23 +890,8 @@ int rbg_workspace_release(void *workspace) {
   std::lock_guard<std::mutex> lock(g_ar_mu);
   auto it = g_ar.find(workspace);
   if (it == g_ar.end()) return RBG_OK;
-  AutoResetCtx &c = it->second;
-  if (c.side) {
-    cudaStreamSynchronize(c.side);
-    cudaStreamDestroy(c.side);
-    cudaEventDestroy(c.env_done);
-    cudaEventDestroy(c.refill_done[0]);
-    cudaEventDestroy(c.refill_done[1]);
-  }
-  for (int i = 0; i < 3; ++i)
-    if (c.slice_stream[i]) {
-      cudaStreamSynchronize(c.slice_stream[i]);
-      cudaStreamDestroy(c.slice_stream[i]);
-      cudaEventDestroy(c.slice_done[i]);
-    }
-  if (c.slice_fork) cudaEventDestroy(c.slice_fork);
-  if (c.tail_valid) {
-    cudaStreamSynchronize(c.last_stream);
+  if (it->second.tail_valid) {
+    cudaStreamSynchronize(it->second.last_stream);
     cudaGetLastError();
   }
   g_ar.erase(it);
@@ -991,8 +908,19 @@ int rbg_connector_step_random(const rbg_state *in, const rbg_state *out, int32_t
   return connector_step_impl(in, out, nullptr, action_out, 1, B, G, N, params, ts, workspace, (cudaStream_t)stream);
 }
 
-// Fused rollout (rollout_warp_kernel): one launch per chunk of steps plus one refill of
-// the next-episode cache for the envs that reset during the chunk.
+// Steps per launch of the fused rollout kernels (RBG_ROLLOUT_CHUNK; default the reference's n_steps,
+// agent_training/configs/env/connector.yaml:27)
+static int rollout_chunk() {
+  static int v = -1;
+  if (v < 0) {
+    v = env_int("RBG_ROLLOUT_CHUNK");
+    if (v <= 0) v = 20;
+  }
+  return v;
+}
+
+// Fused ParallelRandomWalk / Uniform rollout (rollout_persist_kernel): one launch per chunk of steps.  The kernel's
+// generator warps keep the next-episode cache filled; consecutive launches on the stream overlap head to tail.
 static int rollout_fused(const rbg_state *state, int32_t *action_out, int64_t T, int64_t B, int G, int N,
                          const rbg_env_params *params, const rbg_timestep *ts, void *workspace, cudaStream_t stream) {
   uint8_t *ws = reinterpret_cast<uint8_t *>(workspace);
@@ -1006,14 +934,11 @@ static int rollout_fused(const rbg_state *state, int32_t *action_out, int64_t T,
     ctx = &g_ar[workspace];
   }
   if ((rc = workspace_follow_stream(ctx, stream))) return rc;
-  // refills launched by the step-wise path on the side stream must have landed
-  for (int i = 0; i < 2; ++i)
-    if (ctx->refill_pending[i]) {
-      if ((e = cudaStreamWaitEvent(stream, ctx->refill_done[i], 0)) != cudaSuccess) return set_cuda_error(e, "cudaStreamWaitEvent");
-      ctx->refill_pending[i] = false;
-    }
-  auto cache_params = [&](PrwParams &q) {
+  if (ctx->B != B || ctx->G != G || ctx->N != N || ctx->kind != kind) {
+    if ((e = cudaMemsetAsync(ws, 0, 256, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(counters)");
+    PrwParams q;  // warm start: the next episode of every env
     memset(&q, 0, sizeof(q));
+    q.keys = state->key;
     q.B = B;
     q.G = G;
     q.N = N;
@@ -1024,33 +949,6 @@ static int rollout_fused(const rbg_state *state, int32_t *action_out, int64_t T,
     q.cache_tag = reinterpret_cast<unsigned long long *>(ws + wl.cache_tag);
     q.cache_key = reinterpret_cast<uint2 *>(ws + wl.cache_key);
     q.cache_pins = reinterpret_cast<uint32_t *>(ws + wl.cache_pins);
-  };
-  // Next-episode cache + refill kernel, or every reset generated inside the rollout kernel?  Inside,
-  // a whole warp generates one board (prw_kernel packs 32 / Np per warp), but the work hides in the
-  // kernel's idle issue slots and no refill kernel runs.  Measured: the cache wins while a step emits
-  // little per env (10x10/5: 2.10 vs 1.45 G env-steps/s, 16x16/8: 678 vs 636 M), in-kernel generation
-  // wins for large boards, where resets are rare per byte written (24x24/12: 214 vs 183 M, 32x32/16:
-  // 95 vs 84 M, 40x40/32: 26.8 vs 23.3 M); 20x20/10 (16 000 B per env-step) is the break-even.
-  static int no_cache_env = -2;
-  if (no_cache_env == -2) {
-    const char *ex = getenv("RBG_ROLLOUT_NO_CACHE");
-    no_cache_env = ex ? (atoi(ex) != 0 ? 1 : 0) : -1;
-  }
-  // RBG_ROLLOUT_IMPL=legacy: rollout_warp_kernel + refill kernel (round 1); default: the persistent kernel whose
-  // CTAs carry their own generator warps (rollout_persist_kernel), which always works from the cache
-  static int persist = -1;
-  if (persist < 0) {
-    const char *ex = getenv("RBG_ROLLOUT_IMPL");
-    persist = (ex && strcmp(ex, "legacy") == 0) ? 0 : 1;
-  }
-  const bool no_cache = persist ? false : (no_cache_env >= 0 ? no_cache_env == 1 : (size_t)N * G * G * 4 > 16384);
-  if (no_cache) {
-    ctx->B = 0;  // the cache is not maintained: a later step-wise call adopts the workspace afresh
-  } else if (ctx->B != B || ctx->G != G || ctx->N != N || ctx->kind != kind) {
-    if ((e = cudaMemsetAsync(ws, 0, 256, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(counters)");
-    PrwParams q;  // warm start: the next episode of every env
-    cache_params(q);
-    q.keys = state->key;
     if ((rc = launch_prw(q, B, env_int("RBG_PRW_M"), env_int("RBG_PRW_THREADS"), stream))) return rc;
     ctx->B = B;
     ctx->G = G;
@@ -1058,11 +956,6 @@ static int rollout_fused(const rbg_state *state, int32_t *action_out, int64_t T,
     ctx->kind = kind;
     ctx->step = 0;
     ctx->persist_epoch = 0;
-  }
-  static int chunk_env = -1;
-  if (chunk_env < 0) {
-    chunk_env = env_int("RBG_ROLLOUT_CHUNK");
-    if (chunk_env <= 0) chunk_env = 20;  // the reference's n_steps (agent_training/configs/env/connector.yaml:27)
   }
   EnvParams p;
   memset(&p, 0, sizeof(p));
@@ -1077,83 +970,22 @@ static int rollout_fused(const rbg_state *state, int32_t *action_out, int64_t T,
   p.cache_tag = reinterpret_cast<const unsigned long long *>(ws + wl.cache_tag);
   p.cache_key = reinterpret_cast<const uint2 *>(ws + wl.cache_key);
   p.cache_pins = reinterpret_cast<const uint32_t *>(ws + wl.cache_pins);
-  if (no_cache) p.cache_tag = nullptr;
-  // Slices of the batch on their own streams: each slice alternates rollout chunk -> cache
-  // refill, and while one slice's (memory-bound) rollout drains, another slice's (issue-bound)
-  // refill and the ramp of its next chunk fill the SMs.  Slices never share an env, a list or
-  // a cache entry, so the result does not depend on how they interleave.
-  static int slices_env = -1;
-  if (slices_env < 0) {
-    slices_env = env_int("RBG_ROLLOUT_SLICES");
-    if (slices_env <= 0) slices_env = 2;
-    if (slices_env > 4) slices_env = 4;
-  }
-  int nsl = persist ? 1 : slices_env;  // a persistent grid fills the machine by itself; its launches overlap head to tail instead
-  while (nsl > 1 && B < (int64_t)nsl * 2048) --nsl;
-  if (g_timing.load(std::memory_order_relaxed)) nsl = 1;  // event pairs must time one kernel at a time
-  int64_t cuts[5];
-  cuts[0] = 0;
-  for (int s = 1; s < nsl; ++s) cuts[s] = ((B * s / nsl) + 127) & ~(int64_t)127;  // whole CTAs on either side
-  cuts[nsl] = B;
-  if (nsl > 1) {
-    if (!ctx->slice_fork && (e = cudaEventCreateWithFlags(&ctx->slice_fork, cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
-    if ((e = cudaEventRecord(ctx->slice_fork, stream)) != cudaSuccess) return set_cuda_error(e, "cudaEventRecord(fork)");
-    for (int s = 1; s < nsl; ++s) {
-      if (!ctx->slice_stream[s - 1]) {
-        if ((e = cudaStreamCreateWithFlags(&ctx->slice_stream[s - 1], cudaStreamNonBlocking)) != cudaSuccess) return set_cuda_error(e, "cudaStreamCreate(slice)");
-        if ((e = cudaEventCreateWithFlags(&ctx->slice_done[s - 1], cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
-      }
-      if ((e = cudaStreamWaitEvent(ctx->slice_stream[s - 1], ctx->slice_fork, 0)) != cudaSuccess) return set_cuda_error(e, "cudaStreamWaitEvent(fork)");
-    }
-  }
-  for (int64_t t0 = 0; t0 < T; t0 += chunk_env) {
-    const int n = (int)((T - t0) < chunk_env ? (T - t0) : chunk_env);
+  const int chunk = rollout_chunk();
+  for (int64_t t0 = 0; t0 < T; t0 += chunk) {
+    const int n = (int)((T - t0) < chunk ? (T - t0) : chunk);
     p.ts = timestep_at(*ts, t0 * B, G, N);
-    for (int s = 0; s < nsl; ++s) {
-      cudaStream_t st = s == 0 ? stream : ctx->slice_stream[s - 1];
-      p.env_lo = cuts[s];
-      p.env_hi = cuts[s + 1];
-      // the slice's share of the list buffers; counter + ticket pairs 16 bytes apart from ws + 64
-      p.refill_list = reinterpret_cast<int32_t *>(ws + wl.refill_list[0]) + p.env_lo;
-      p.refill_keys = reinterpret_cast<uint32_t *>(ws + wl.refill_keys[0]) + 2 * p.env_lo;
-      p.refill_count = reinterpret_cast<int32_t *>(ws + 64 + 16 * s);
-      if (persist) {
-        static int overlap_env = -1;  // RBG_ROLLOUT_OVERLAP=0: plain stream order between launches
-        if (overlap_env < 0) {
-          const char *ex = getenv("RBG_ROLLOUT_OVERLAP");
-          overlap_env = (ex && atoi(ex) == 0) ? 0 : 1;
-        }
-        if (ctx->persist_epoch == 0 || ctx->persist_epoch > 0x3fffffff) {  // flags start at 0 = "written by launch 0"
-          if ((e = cudaMemsetAsync(ws + wl.group_done, 0, (wl.group_pending - wl.group_done) + 4 * (size_t)B, st)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(group flags)");
-          if ((e = cudaMemsetAsync(ws + 256, 0, 256, st)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(persist counters)");
-          ctx->persist_epoch = 0;
-        }
-        const int epoch = ++ctx->persist_epoch;
-        const bool overlap = overlap_env == 1 && epoch > 1 && !g_timing.load(std::memory_order_relaxed);
-        if ((rc = launch_rollout_persist(p, kind, n, action_out ? action_out + t0 * B * N : nullptr, reinterpret_cast<int32_t *>(ws + 256),
-                                         reinterpret_cast<int32_t *>(ws + wl.group_done), reinterpret_cast<int32_t *>(ws + wl.group_pending), epoch, overlap,
-                                         reinterpret_cast<uint64_t *>(ws + wl.cache_tag), reinterpret_cast<uint2 *>(ws + wl.cache_key),
-                                         reinterpret_cast<uint32_t *>(ws + wl.cache_pins), st)))
-          return rc;
-        continue;
-      }
-      if (no_cache) p.refill_list = nullptr;
-      if ((rc = launch_rollout(p, kind, n, action_out ? action_out + t0 * B * N : nullptr, st))) return rc;
-      if (no_cache) continue;
-      PrwParams q;  // refill the cache entries consumed in this chunk (the kernel clears the counter when done)
-      cache_params(q);
-      q.keys = p.refill_keys;
-      q.keys_compact = 1;
-      q.list = p.refill_list;
-      q.list_count = p.refill_count;
-      q.list_ticket = p.refill_count + 1;
-      q.bulk_list = 1;
-      if ((rc = launch_prw(q, p.env_hi - p.env_lo, env_int("RBG_PRW_M"), env_int("RBG_PRW_THREADS"), st))) return rc;
+    if (ctx->persist_epoch == 0 || ctx->persist_epoch > 0x3fffffff) {  // flags start at 0 = "written by launch 0"
+      if ((e = cudaMemsetAsync(ws + wl.group_done, 0, (wl.group_pending - wl.group_done) + 4 * (size_t)B, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(group flags)");
+      if ((e = cudaMemsetAsync(ws + 256, 0, 256, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(persist counters)");
+      ctx->persist_epoch = 0;
     }
-  }
-  for (int s = 1; s < nsl; ++s) {
-    if ((e = cudaEventRecord(ctx->slice_done[s - 1], ctx->slice_stream[s - 1])) != cudaSuccess) return set_cuda_error(e, "cudaEventRecord(join)");
-    if ((e = cudaStreamWaitEvent(stream, ctx->slice_done[s - 1], 0)) != cudaSuccess) return set_cuda_error(e, "cudaStreamWaitEvent(join)");
+    const int epoch = ++ctx->persist_epoch;
+    const bool overlap = epoch > 1 && !g_timing.load(std::memory_order_relaxed);  // event pairs must time one kernel at a time
+    if ((rc = launch_rollout_persist(p, kind, n, action_out ? action_out + t0 * B * N : nullptr, reinterpret_cast<int32_t *>(ws + 256),
+                                     reinterpret_cast<int32_t *>(ws + wl.group_done), reinterpret_cast<int32_t *>(ws + wl.group_pending), epoch, overlap,
+                                     reinterpret_cast<uint64_t *>(ws + wl.cache_tag), reinterpret_cast<uint2 *>(ws + wl.cache_key),
+                                     reinterpret_cast<uint32_t *>(ws + wl.cache_pins), stream)))
+      return rc;
   }
   return RBG_OK;
 }
@@ -1164,22 +996,17 @@ int rbg_connector_rollout_random(const rbg_state *state, int32_t *action_out, in
   if (T < 0) return set_error(RBG_EINVAL, "rollout length T=%lld", (long long)T);
   if ((rc = check_dims(B, G, N, 1))) return rc;
   if (B == 0 || T == 0) return RBG_OK;  // an empty batch has no buffers to check
+  // (when G*G % 4 == 0 every step slice of the stacked arrays keeps the 16-byte alignment the
+  // vector path needs; otherwise the kernels use scalar accesses)
   if ((rc = check_state(state, "state", G))) return rc;
   if ((rc = check_timestep(ts, G))) return rc;
   if (!params) return set_error(RBG_EINVAL, "params is NULL");
-  // (when G*G % 4 == 0 every step slice of the stacked arrays keeps the 16-byte alignment the
-  // vector path needs; otherwise the kernels use scalar accesses)
-  if (B == 0 || T == 0) return RBG_OK;
   const int kind = params->autoreset_kind;
-  static int fused = -1;
-  if (fused < 0) fused = env_int("RBG_NO_FUSED_ROLLOUT") ? 0 : 1;
   if (kind > RBG_GEN_SEQRW) return set_error(RBG_EINVAL, "unknown autoreset generator kind %d", kind);
   if (kind < 0) return set_error(RBG_EINVAL, "rollout needs an auto-reset generator kind (params->autoreset_kind >= 0)");
-  if (kind == RBG_GEN_DATASET && (rc = check_dataset(params))) return rc;
-  if (fused && kind == RBG_GEN_DATASET) {
-    // resets are a table lookup inside the kernel: no cache, no refill, no workspace
-    int chunk = env_int("RBG_ROLLOUT_CHUNK");
-    if (chunk <= 0) chunk = 20;
+  if (kind == RBG_GEN_DATASET) {
+    if ((rc = check_dataset(params))) return rc;
+    // resets are a table lookup inside rollout_warp_kernel: no cache, no workspace
     EnvParams p;
     memset(&p, 0, sizeof(p));
     p.in = *state;
@@ -1190,18 +1017,20 @@ int rbg_connector_rollout_random(const rbg_state *state, int32_t *action_out, in
     p.mode = ENV_MODE_STEP;
     p.random_policy = 1;
     p.env = *params;
+    const int chunk = rollout_chunk();
     for (int64_t t0 = 0; t0 < T; t0 += chunk) {
       const int n = (int)((T - t0) < chunk ? (T - t0) : chunk);
       p.ts = timestep_at(*ts, t0 * B, G, N);
-      if ((rc = launch_rollout(p, kind, n, action_out ? action_out + t0 * B * N : nullptr, (cudaStream_t)stream))) return rc;
+      if ((rc = launch_rollout(p, n, action_out ? action_out + t0 * B * N : nullptr, (cudaStream_t)stream))) return rc;
     }
     return RBG_OK;
   }
-  if (fused && speculative_enabled() && workspace && (kind == RBG_GEN_PRW || kind == RBG_GEN_UNIFORM)) {
+  if (kind == RBG_GEN_PRW || kind == RBG_GEN_UNIFORM) {
+    if (!workspace) return set_error(RBG_EINVAL, "auto-reset needs a workspace (rbg_step_workspace_bytes)");
     if (!aligned16(workspace)) return set_error(RBG_EALIGN, "workspace not 16-byte aligned");
     return rollout_fused(state, action_out, T, B, G, N, params, ts, workspace, (cudaStream_t)stream);
   }
-  for (int64_t t = 0; t < T; ++t) {  // step-wise: SeedExtension / SequentialRandomWalk resets, or the fused kernel switched off
+  for (int64_t t = 0; t < T; ++t) {  // step-wise: SeedExtension / SequentialRandomWalk resets
     const rbg_timestep tt = timestep_at(*ts, t * B, G, N);
     rc = connector_step_impl(state, state, nullptr, action_out ? action_out + t * B * N : nullptr, 1, B, G, N, params, &tt, workspace,
                              (cudaStream_t)stream);
@@ -1268,7 +1097,7 @@ static int use_device(int device, int *cur) {
 static void scratch_claim(const ScratchSig &sig, uint8_t *ws, size_t stride, int64_t nws) {
   if (g_scratch_sig == sig) return;
   g_scratch_sig = sig;
-  for (int64_t i = 0; i < nws; ++i) invalidate_workspace(ws + (size_t)i * stride, nullptr, true);
+  for (int64_t i = 0; i < nws; ++i) invalidate_workspace(ws + (size_t)i * stride);
 }
 
 int rbg_prw_generate_host(const uint32_t *keys, int64_t B, int G, int N, int32_t *heads, int32_t *targets,

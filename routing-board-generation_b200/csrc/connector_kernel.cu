@@ -20,7 +20,6 @@
 #include "connector_device.cuh"
 #include "gen_warp.cuh"
 #include "obs_stage.cuh"
-#include "prw_warp.cuh"
 #include "rbg_host.h"
 
 namespace rbg {
@@ -194,7 +193,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, RBG_ENV_MIN_CTAS) env_warp_kern
   const int sc = sc0 + (is_step ? 1 : 0);
   const bool terminal = is_step && env_ok && (ndone == N || sc >= p.env.time_limit);
   int tflag = terminal ? 1 : 0;
-  // The cache entry may be REPLACED by the refill kernel (side stream) while this kernel runs, e.g. when a
+  // The cache entry may be REPLACED by the previous step's refill, which this kernel runs under, e.g. when a
   // State is stepped twice (functional use, inplace=False) or two batches share a workspace.  The entry is
   // a seqlock whose version is its tag: the writer (prw_kernel, to_cache) invalidates the tag, fences,
   // writes key and pins, fences, publishes the new tag; a reader takes the entry only if the tag reads as
@@ -343,30 +342,21 @@ __global__ void __launch_bounds__(EW_WARPS * 32, RBG_ENV_MIN_CTAS) env_warp_kern
 }
 
 // ---------------------------------------------------------------------------
-// rollout_warp_kernel: T random-policy steps with auto-reset in ONE launch (the
-// reference's `n_steps` scan: generation, reset and stepping fused).  Same lane layout
-// as env_warp_kernel, but the warp keeps its K envs on chip for the whole rollout: the
-// State is read once and written once per launch, so a step only pays for what it must
-// emit (observation, mask, reward, discount, step_type, extras, action); PATH counts are
-// carried instead of recounted.  Finished envs swap in their pre-generated next episode
-// (cache, see c_api.cu "AutoReset"); an env that finishes AGAIN before the host has had
-// a chance to refill its cache entry gets its episode generated right here by the warp
-// (prw_warp.cuh).  Envs that reset are queued for one refill after the launch.
+// rollout_warp_kernel: T random-policy steps with auto-reset from a board dataset
+// (BoardDatasetGeneratorJAX) in ONE launch (the reference's `n_steps` scan: reset and
+// stepping fused).  Same lane layout as env_warp_kernel, but the warp keeps its K envs on
+// chip for the whole rollout: the State is read once and written once per launch, so a
+// step only pays for what it must emit (observation, mask, reward, discount, step_type,
+// extras, action); PATH counts are carried instead of recounted.  A finished env's next
+// episode is a table lookup in the dataset.
 struct RolloutParams {
   int T;
-  int kind;              // RBG_GEN_PRW / RBG_GEN_UNIFORM
-  int gen_off;           // smem byte offset of the per-warp generator scratch
-  int gen_stride;        // bytes per warp
-  int gen_cand_bytes;    // cand region size within the scratch
-  int gen_sel_bytes;
-  int cap;
-  uint32_t thresh;
   int32_t *action_out;   // [T,B,N] or NULL
   int ratio_off;         // smem byte offset of the n / N table
   int stage_off;         // smem byte offset of the per-warp observation staging
   int stage_bytes;       // bytes per buffer
   int stage_nbuf;        // 1: one chunk per step (a whole step passes before it is refilled); 2: alternate
-  int stage_warp;        // bytes per warp (>= stage_nbuf * stage_bytes; the generator scratch aliases it)
+  int stage_warp;        // bytes per warp (>= stage_nbuf * stage_bytes)
   int ce, cv;            // a staged chunk = ce whole envs (cv == N) or cv views of one env (ce == 1)
 };
 
@@ -389,20 +379,11 @@ __global__ void __launch_bounds__(EW_WARPS * 32, RBG_ROLLOUT_MIN_CTAS) rollout_w
   if (tid <= N) ratio_lut[tid] = __fdiv_rn((float)tid, (float)N);
   __syncthreads();  // the only CTA-wide barrier
 
-  const long long e0 = p.env_lo + ((long long)blockIdx.x * EW_WARPS + warp) * K;
-  if (e0 >= p.env_hi) return;
-  const int kc = (int)((p.env_hi - e0) < (long long)K ? (p.env_hi - e0) : (long long)K);
+  const long long e0 = ((long long)blockIdx.x * EW_WARPS + warp) * K;
+  if (e0 >= p.B) return;
+  const int kc = (int)((p.B - e0) < (long long)K ? (p.B - e0) : (long long)K);
   uint8_t *wg = smem_raw + p.so[0] + (size_t)warp * p.so[1];
   uint32_t *wg32 = reinterpret_cast<uint32_t *>(wg);
-  WarpGenScratch gs;
-  {
-    uint8_t *gb = VEC ? smem_raw + rp.stage_off + (size_t)warp * rp.stage_warp : smem_raw + rp.gen_off + (size_t)warp * rp.gen_stride;
-    gs.cand = reinterpret_cast<uint64_t *>(gb);
-    gs.sel = reinterpret_cast<uint16_t *>(gb + rp.gen_cand_bytes);
-    gs.board = gb + rp.gen_cand_bytes + rp.gen_sel_bytes;
-    gs.cap = rp.cap;
-    gs.thresh = rp.thresh;
-  }
 
   const int j = lane / Np, a = lane & (Np - 1);
   const bool env_ok = j < kc, agent = env_ok && a < N;
@@ -455,7 +436,6 @@ __global__ void __launch_bounds__(EW_WARPS * 32, RBG_ROLLOUT_MIN_CTAS) rollout_w
     }
   }
   for (int off = Np >> 1; off; off >>= 1) paths += __shfl_xor_sync(FULL, paths, off);
-  bool did_reset = false;
   // the action mask of the state an env is in: what step t emits is what step t+1's policy samples from
   uint32_t mk3 = 0;
   if (agent) mk3 = move_mask(sg, pos >> 8, pos & 255, a, pos == tgt);
@@ -509,13 +489,10 @@ __global__ void __launch_bounds__(EW_WARPS * 32, RBG_ROLLOUT_MIN_CTAS) rollout_w
     const bool terminal = env_ok && (ndone == N || sc >= p.env.time_limit);
     const int tpl = paths + N;
 
-    // ---- auto-reset: cached episode, else generate it here
-    // (the host refills the cache on this stream BEFORE the launch, so unlike the per-step
-    // kernel no acquire fence is needed and the three reads go out together)
-    bool hit = false;
+    // ---- auto-reset: the dataset board that follows
     uint32_t nk0 = 0, nk1 = 0;
     int npos = pos, ntgt = tgt;
-    if (terminal && rp.kind == RBG_GEN_DATASET) {
+    if (terminal) {
       // VmapAutoResetWrapper._auto_reset: key, _ = split(state.key); then BoardDatasetGeneratorJAX.__call__
       uint32_t a0, a1, b0, b1;
       split2(k0, k1, a0, a1, b0, b1);
@@ -525,39 +502,6 @@ __global__ void __launch_bounds__(EW_WARPS * 32, RBG_ROLLOUT_MIN_CTAS) rollout_w
         const int hi = G - 1;
         npos = (min(max(__ldg(h + a), 0), hi) << 8) | min(max(__ldg(h + N + a), 0), hi);
         ntgt = (min(max(__ldg(tt + a), 0), hi) << 8) | min(max(__ldg(tt + N + a), 0), hi);
-      }
-      hit = true;
-    } else if (terminal && p.cache_tag) {
-      const unsigned long long tag = __ldcg(p.cache_tag + e);
-      const uint2 nk = __ldcg(p.cache_key + e);
-      const uint32_t pin = a < N ? __ldcg(p.cache_pins + e * N + a) : 0u;
-      if (tag == (((unsigned long long)k1 << 32) | k0)) {
-        nk0 = nk.x;
-        nk1 = nk.y;
-        npos = (int)(pin >> 16);
-        ntgt = (int)(pin & 0xffffu);
-        hit = true;
-      }
-    }
-    uint32_t missm = __ballot_sync(FULL, terminal && !hit && a == 0);
-    while (missm) {  // warp-uniform: generate the episode of env `jj` with the whole warp
-      const int src_lane = __ffs(missm) - 1;
-      missm &= missm - 1;
-      const uint32_t gk0 = __shfl_sync(FULL, k0, src_lane), gk1 = __shfl_sync(FULL, k1, src_lane);
-      uint32_t x0, x1;
-      int gstart, gfin;
-      if (OBS == 2) os.drain(lane);  // the generator scratch aliases the observation staging
-      warp_generate_pins(rp.kind, gk0, gk1, G, N, p.divG, gs, lane, x0, x1, gstart, gfin);
-      // lane i < N holds agent i's pins; hand them to env jj's lanes
-      const int from = a < N ? a : 0;
-      const int hs = __shfl_sync(FULL, gstart, from), hf = __shfl_sync(FULL, gfin, from);
-      if (lane >= src_lane && lane < src_lane + Np) {
-        nk0 = x0;
-        nk1 = x1;
-        if (a < N) {
-          npos = hs;
-          ntgt = hf;
-        }
       }
     }
     // ---- small outputs of step t (terminal step's reward / discount / step_type / extras)
@@ -581,7 +525,6 @@ __global__ void __launch_bounds__(EW_WARPS * 32, RBG_ROLLOUT_MIN_CTAS) rollout_w
       k1 = nk1;
       sc = 0;
       paths = 0;
-      did_reset = true;
       __syncwarp(gmask);
       if (a < N) g[(pos >> 8) * G + (pos & 255)] = (uint8_t)(3 * a + POSITION);
       __syncwarp(gmask);
@@ -611,7 +554,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, RBG_ROLLOUT_MIN_CTAS) rollout_w
     __syncwarp();  // the next step's writes must not overtake these reads
   }
 
-  // ---- write the State once; queue the envs that reset for a cache refill
+  // ---- write the State once
   if (VEC) {
     if (OBS == 2) os.drain(lane);
     int4 *gdst = reinterpret_cast<int4 *>(p.out.grid) + e0 * c4;
@@ -624,12 +567,6 @@ __global__ void __launch_bounds__(EW_WARPS * 32, RBG_ROLLOUT_MIN_CTAS) rollout_w
     p.out.step_count[e] = sc;
     p.out.key[2 * e] = k0;
     p.out.key[2 * e + 1] = k1;
-    if (did_reset && p.refill_list) {
-      const int slot = atomicAdd(p.refill_count, 1);
-      p.refill_list[slot] = (int32_t)e;
-      p.refill_keys[2 * slot] = k0;
-      p.refill_keys[2 * slot + 1] = k1;
-    }
   }
   if (agent) {
     const long long ga = e * N + a;
@@ -676,7 +613,7 @@ struct PersistParams {
   int *group_done;     // [ngroups] last launch epoch that has written the group's State
   int *group_pending;  // [ngroups] episode requests in flight
   int epoch;           // this launch (> 0, +1 per launch on the workspace)
-  int ngroups;    // groups of K envs in [env_lo, env_hi)
+  int ngroups;    // groups of K envs in the batch
   int env_warps;  // env warps per CTA (1..EW_WARPS)
   int gen_warps;  // generator warps per CTA (1..2)
   int tmpl_off;   // smem byte offsets: empty padded board, queues, done flag, generator scratch
@@ -777,8 +714,8 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, RBG_PERSIST_MIN_CTAS)
 #ifdef RBG_PERSIST_TRACE
     ++tr_groups;
 #endif
-    const long long e0 = p.env_lo + (long long)grp * K;
-    const int kc = (int)((p.env_hi - e0) < (long long)K ? (p.env_hi - e0) : (long long)K);
+    const long long e0 = (long long)grp * K;
+    const int kc = (int)((p.B - e0) < (long long)K ? (p.B - e0) : (long long)K);
     const bool env_ok = j < kc, agent = env_ok && a < N;
     const long long e = e0 + (env_ok ? j : 0);
     GenQueue *myq = queues + (int)(e % pp.gen_warps);
@@ -1084,7 +1021,7 @@ static size_t balance_waves(int64_t ctas, int cmax, int cmin, size_t smem_needed
   return pad > smem_needed ? pad : smem_needed;
 }
 
-int launch_rollout(EnvParams p, int kind, int T, int32_t *action_out, cudaStream_t stream) {
+int launch_rollout(EnvParams p, int T, int32_t *action_out, cudaStream_t stream) {
   const int G = p.G, N = p.N;
   p.cells = G * G;
   const bool vec = (p.cells & 3) == 0;
@@ -1093,10 +1030,6 @@ int launch_rollout(EnvParams p, int kind, int T, int32_t *action_out, cudaStream
   p.divC4 = FastDiv::make((uint32_t)(vec ? p.cells >> 2 : 1));
   p.divCells = FastDiv::make((uint32_t)p.cells);
   if (p.B <= 0 || T <= 0) return RBG_OK;
-  if (p.env_hi <= p.env_lo) {
-    p.env_lo = 0;
-    p.env_hi = p.B;
-  }
   int Np = 1;
   while (Np < N) Np <<= 1;
   p.Np = Np;
@@ -1108,20 +1041,8 @@ int launch_rollout(EnvParams p, int kind, int T, int32_t *action_out, cudaStream
   p.so[1] = (int)wgrid;
   RolloutParams rp;
   rp.T = T;
-  rp.kind = kind;
   rp.action_out = action_out;
-  const int nsel = kind == RBG_GEN_PRW ? N : 2 * N;
-  rp.cap = 4 * nsel + 32;
-  {
-    const double frac = (2.0 * nsel + 16.0) / (double)p.cells;
-    rp.thresh = frac >= 1.0 ? 0xffffffffu : (uint32_t)(frac * 4294967296.0);
-  }
-  rp.gen_cand_bytes = (int)(((size_t)rp.cap * 8 + 15) & ~(size_t)15);
-  rp.gen_sel_bytes = (int)(((size_t)(2 * N + 2) * 2 + 15) & ~(size_t)15);
-  const size_t board = (((size_t)(G + 4) * (G + 4) + 15) / 16) * 16;
-  rp.gen_stride = (int)(rp.gen_cand_bytes + rp.gen_sel_bytes + board);
-  rp.gen_off = (int)(lutB + EW_WARPS * wgrid);
-  rp.ratio_off = rp.gen_off + (vec ? 0 : EW_WARPS * rp.gen_stride);
+  rp.ratio_off = (int)(lutB + EW_WARPS * wgrid);
   size_t smem = (((size_t)rp.ratio_off + 4 * (RBG_MAX_N + 4)) + 15) & ~(size_t)15;
   rp.stage_off = (int)smem;
   rp.stage_bytes = 0;
@@ -1135,13 +1056,11 @@ int launch_rollout(EnvParams p, int kind, int T, int32_t *action_out, cudaStream
     rp.stage_nbuf = pl.nbuf;
     rp.ce = pl.ce;
     rp.cv = pl.cv;
-    rp.stage_warp = rp.stage_nbuf * rp.stage_bytes;
-    if (rp.stage_warp < rp.gen_stride) rp.stage_warp = rp.gen_stride;
-    rp.stage_warp = (rp.stage_warp + 15) & ~15;
+    rp.stage_warp = (rp.stage_nbuf * rp.stage_bytes + 15) & ~15;
     smem += (size_t)EW_WARPS * rp.stage_warp;
   }
   if (smem > 200 * 1024) return set_error(RBG_EINVAL, "rollout: shared memory %zu too large", smem);
-  const int64_t ctas = (p.env_hi - p.env_lo + p.E - 1) / p.E;
+  const int64_t ctas = (p.B + p.E - 1) / p.E;
   {  // residency: registers allow RBG_ROLLOUT_MIN_CTAS per SM, shared memory (1 KB reserved per CTA) maybe fewer
     int cmax = (int)(device_smem_per_sm() / (smem + 1024));
     if (cmax > RBG_ROLLOUT_MIN_CTAS) cmax = RBG_ROLLOUT_MIN_CTAS;
@@ -1187,10 +1106,6 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   p.divC4 = FastDiv::make((uint32_t)(vec ? p.cells >> 2 : 1));
   p.divCells = FastDiv::make((uint32_t)p.cells);
   if (p.B <= 0 || T <= 0) return RBG_OK;
-  if (p.env_hi <= p.env_lo) {
-    p.env_lo = 0;
-    p.env_hi = p.B;
-  }
   int Np = 1;
   while (Np < N) Np <<= 1;
   p.Np = Np;
@@ -1204,7 +1119,6 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   RolloutParams rp;
   memset(&rp, 0, sizeof(rp));
   rp.T = T;
-  rp.kind = kind;
   rp.action_out = action_out;
   static int env_warps_env = -1;  // RBG_PERSIST_ENV_WARPS=n: n env warps per CTA (experiments; default EW_WARPS)
   if (env_warps_env < 0) {
@@ -1259,10 +1173,9 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   pp.group_done = group_done;
   pp.group_pending = group_pending;
   pp.epoch = epoch;
-  pp.ngroups = (int)((p.env_hi - p.env_lo + K - 1) / K);
+  pp.ngroups = (int)((p.B + K - 1) / K);
   gc.group_pending = group_pending;
   gc.seqlock = 0;  // nobody reads an entry while it is rewritten here (see gen_warp_batch)
-  gc.env_lo = p.env_lo;
   gc.kshift = 0;
   while ((1 << gc.kshift) < K) ++gc.kshift;
   static int gen_warps_env = -1;

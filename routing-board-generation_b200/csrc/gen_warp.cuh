@@ -10,7 +10,7 @@
 // agent, exactly the lane layout of prw_kernel's walk), and publishes each result into the env's
 // next-episode cache entry in global memory (the same seqlock-tagged entry the per-step path uses).
 //
-// Algorithm and key derivation as prw_kernel.cu / prw_warp.cuh (reference parallel_random_walk.py:60-447,
+// Algorithm and key derivation as prw_kernel.cu (reference parallel_random_walk.py:60-447,
 // parallel_random_walk_generator.py:46-77, uniform_generator.py:70-109; VmapAutoResetWrapper's
 // `key, _ = split(state.key)` first).
 #pragma once
@@ -85,7 +85,6 @@ struct GenWarpCfg {
   // (NULL: not counted)
   int *group_pending;
   int seqlock;         // readers may be running (per-step path): invalidate the entry's tag before rewriting it
-  long long env_lo;
   int kshift;          // log2(envs per group)
 };
 
@@ -251,9 +250,9 @@ __device__ inline void gen_warp_batch(const GenWarpCfg &c, const GenWarpScratch 
   const long long e = (long long)__shfl_sync(FULL, req_env, have ? grp : 0);
   const uint32_t tk0 = __shfl_sync(FULL, req_k0, have ? grp : 0), tk1 = __shfl_sync(FULL, req_k1, have ? grp : 0);
   const uint32_t pk0 = __shfl_sync(FULL, nk0, have ? 2 * grp : 0), pk1 = __shfl_sync(FULL, nk1, have ? 2 * grp : 0);
-  // (nobody reads this entry while it is rewritten: its env consumed it before asking for the next one, and the
-  // per-step path's side-stream refill is joined before a rollout launch; so no invalidation round, and one
-  // release store instead of fences.  bar.warp.sync orders the other lanes' pin stores before lane 0's release.)
+  // (nobody reads this entry while it is rewritten: its env consumed it before asking for the next one, and a
+  // per-step refill that may still be running under a rollout launch writes the same episode, a board being a pure
+  // function of its key; so no invalidation round, and one release store instead of fences.  bar.warp.sync orders the other lanes' pin stores before lane 0's release.)
   if (c.seqlock) {  // (warp-uniform) the tag is the version: invalidate, fence, write, publish
     if (have && a == 0) *reinterpret_cast<volatile unsigned long long *>(c.cache_tag + e) = 0ull;
     __threadfence();
@@ -267,7 +266,7 @@ __device__ inline void gen_warp_batch(const GenWarpCfg &c, const GenWarpScratch 
     st_release_u64(c.cache_tag + e, ((unsigned long long)tk1 << 32) | tk0);
     if (c.group_pending) {
       __threadfence();  // the entry is visible before the group's count drops
-      atomicSub(c.group_pending + ((e - c.env_lo) >> c.kshift), 1);
+      atomicSub(c.group_pending + (e >> c.kshift), 1);
     }
   }
 }

@@ -512,11 +512,10 @@ static int prw_prepare(PrwParams &p, int64_t max_boards, int force_M, int force_
     threads = 64;
     M = 2 * gpw * 2;  // one board per group + one refill
   }
-  if (p.list && !p.bulk_list) {  // per-step lists: a few percent of the batch, latency matters
+  if (p.list) {  // per-step lists: a few percent of the batch, latency matters
     threads = 64;
     M = 2 * gpw;
   }
-  if (p.bulk_list) M = 32;  // a rollout chunk's refill is ~0.8 x the batch: smaller pools balance the CTA waves (measured)
   if (force_threads > 0) threads = force_threads;
   if (force_M > 0) M = force_M;
   // keep shared memory per CTA moderate so several CTAs share an SM
@@ -530,7 +529,7 @@ static int prw_prepare(PrwParams &p, int64_t max_boards, int force_M, int force_
   const size_t smem = prw_carve(p, threads / 32, nullptr, nullptr);
   if (smem > 200 * 1024) return set_error(RBG_EINVAL, "prw_kernel: %zu bytes of shared memory per CTA", smem);
   int64_t ctas = (max_boards + M - 1) / M;
-  if (p.list && !p.bulk_list && ctas > sms * (p.to_cache ? 4 : 2)) ctas = sms * (p.to_cache ? 4 : 2);  // per-step lists hold a few percent of the batch and the kernel strides over them
+  if (p.list && ctas > sms * (p.to_cache ? 4 : 2)) ctas = sms * (p.to_cache ? 4 : 2);  // per-step lists hold a few percent of the batch and the kernel strides over them
   *threads_out = threads;
   *smem_out = smem;
   *ctas_out = ctas;

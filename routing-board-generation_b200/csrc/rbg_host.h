@@ -48,7 +48,6 @@ struct PrwParams {
   // auto-reset cache refill: keys[] is indexed by list slot (not env id) and the
   // result goes to the env's cache entry instead of State / TimeStep
   int keys_compact, to_cache;
-  int bulk_list;  // the list is large (a rollout chunk's resets): use the bulk launch shape
   int trigger_dependents;  // griddepcontrol.launch_dependents at the start: the next kernel of the stream, if it was launched
                            // with programmatic stream serialization, need not wait for this one (per-step cache refill)
   unsigned long long *cache_tag;  // [B]   state.key this entry succeeds (k0 | k1 << 32)
@@ -74,7 +73,6 @@ struct EnvParams {
   const int32_t *action;  // [B,N] (STEP)
   int32_t *action_out;    // optional (random policy)
   long long B;
-  long long env_lo, env_hi;  // rollout: the slice [env_lo, env_hi) of the batch this launch covers (0, 0 = all)
   int G, N;
   int mode;           // ENV_MODE_*
   int random_policy;  // sample actions in-kernel
@@ -98,9 +96,10 @@ struct EnvParams {
 // pdl: launch with programmatic stream serialization (the kernel may begin while a preceding kernel that has said
 // launch_dependents is still running; any other predecessor completes first)
 int launch_env(EnvParams p, cudaStream_t stream, bool pdl = false);
-// T random-policy auto-reset steps in one launch (kind: RBG_GEN_PRW / RBG_GEN_UNIFORM); ts fields stacked [T,B,...]
-int launch_rollout(EnvParams p, int kind, int T, int32_t *action_out, cudaStream_t stream);
-// the same as a persistent kernel whose CTAs carry their own generator warps (no refill kernel); needs the cache
+// T random-policy steps in one launch, auto-reset from the board dataset of p.env; ts fields stacked [T,B,...]
+int launch_rollout(EnvParams p, int T, int32_t *action_out, cudaStream_t stream);
+// T random-policy steps with ParallelRandomWalk / Uniform auto-reset (kind) as a persistent kernel whose CTAs carry
+// their own generator warps; needs the cache
 // `counter`: 8 zeroed ints (two sets, recycled by the kernel); group_done / group_pending: zeroed int[groups];
 // epoch: 1, 2, ... per launch on those arrays; overlap: chain to the previous launch of the stream (PDL)
 int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, int32_t *counter, int32_t *group_done, int32_t *group_pending,

@@ -311,7 +311,7 @@ _ws_tokens = itertools.count(1)
 def _workspace(B: int, G: int, N: int, owner=None) -> torch.Tensor:
     """Auto-reset scratch (reset lists + the next-episode cache) of one env batch.  Keyed by the
     owning wrapper when there is one, so two batches of the same shape do not evict each other's
-    cache entries; kept alive for the process (the library's side stream may still be filling it
+    cache entries; kept alive for the process (kernels queued on the stream may still be filling it
     when the caller drops its last State)."""
     dev = _device()
     token = None
@@ -333,7 +333,7 @@ def _workspace(B: int, G: int, N: int, owner=None) -> torch.Tensor:
 
 
 def _drop_workspace(k) -> None:
-    """The owning env is gone: let the library forget the workspace (waits for its side stream) and free it."""
+    """The owning env is gone: let the library forget the workspace (waits for the work queued on it) and free it."""
     ws = _workspaces.pop(k, None)
     if ws is not None:
         try:

@@ -515,21 +515,21 @@ def test_fused_random_step_matches_two_calls(rbg, orc):
 
 
 @pytest.mark.parametrize("kind,G,N,B,T,time_limit", [
-    ("parallel_random_walk", 10, 5, 3000, 45, 9),     # resets inside every chunk, some envs twice (in-kernel generation)
+    ("parallel_random_walk", 10, 5, 3000, 45, 9),     # resets inside every chunk, some envs twice (generator warps)
     ("parallel_random_walk", 32, 16, 96, 12, 9),      # BASELINE configs[4] shape
-    ("parallel_random_walk", 10, 5, 1000, 25, 1),     # every step is terminal: the in-kernel generator runs constantly
+    ("parallel_random_walk", 10, 5, 1000, 25, 1),     # every step is terminal: the generator warps run constantly
     ("parallel_random_walk", 10, 5, 1000, 25, 2),
     ("parallel_random_walk", 5, 3, 777, 23, 6),       # cells % 4 != 0: scalar path, ragged last warp
     ("parallel_random_walk", 9, 9, 301, 14, 5),       # N > 8: two envs per warp
     ("parallel_random_walk", 12, 20, 130, 14, 7),     # N > 16: one env per warp
     ("parallel_random_walk", 40, 32, 40, 8, 5),       # largest supported shape
-    ("parallel_random_walk", 8, 4, 4611, 24, 6),      # two batch slices on two streams, ragged cut and ragged last warp
-    ("parallel_random_walk", 12, 10, 4099, 22, 7),    # staged views in two alternating buffers (5.7 KB per env), two slices
+    ("parallel_random_walk", 8, 4, 4611, 24, 6),      # ragged last group and ragged last warp
+    ("parallel_random_walk", 12, 10, 4099, 22, 7),    # staged views in two alternating buffers (5.7 KB per env)
     ("parallel_random_walk", 6, 12, 310, 21, 4),      # c4 = 9 < 32 lanes, one env per warp
     ("parallel_random_walk", 4, 2, 1300, 21, 3),      # 16 envs per warp, 2 KB of views per step
     ("uniform", 10, 5, 2000, 30, 7),
     ("uniform", 7, 6, 500, 21, 3),
-    ("uniform", 8, 8, 4200, 21, 5),                   # two slices, Uniform in-kernel generation
+    ("uniform", 8, 8, 4200, 21, 5),                   # Uniform generation in the generator warps
     ("seed_extension", 10, 5, 300, 12, 5),            # no fused kernel for this generator: step-wise path
 ])
 def test_rollout_matches_stepwise_oracle(rbg, orc, kind, G, N, B, T, time_limit):
@@ -555,58 +555,36 @@ def test_rollout_matches_stepwise_oracle(rbg, orc, kind, G, N, B, T, time_limit)
     _assert_state(st, rst, "after the second rollout")
 
 
-def _rollout_in_subprocess(env_vars, G, N, B, T, time_limit=6):
-    """A fused rollout against the oracle in a fresh process (the library reads its switches once)."""
-    import os
-    import subprocess
-    import sys
+@pytest.mark.parametrize("G,N,B,time_limit", [(10, 5, 8200, 6), (10, 5, 4300, 5), (24, 12, 300, 5), (7, 3, 900, 5)])
+def test_rollout_step_rollout_matches_oracle(rbg, orc, G, N, B, time_limit):
+    """Two fused rollouts of 21 steps, each followed by a step-wise call that shares the auto-reset workspace
+    (next-episode cache and group flags) with them: every action, every leaf of every TimeStep and the State
+    against the oracle."""
+    import torch
 
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    code = (
-        "import sys, numpy as np; sys.path.insert(0, %r)\n"
-        "import routing_board_generation_b200 as rbg\n"
-        "from oracle import oracle as orc\n"
-        "G, N, B, T, TL = %d, %d, %d, %d, %d\n"
-        "k = rbg.split(rbg.PRNGKey(5), B); kr = orc.split(orc.PRNGKey(5), B)\n"
-        "env = rbg.VmapAutoResetWrapper(rbg.Connector(generator=rbg.ParallelRandomWalkGenerator(G, N), time_limit=TL))\n"
-        "st, _ = env.reset(k); rst, _ = orc.connector_reset_batch('parallel_random_walk', kr, G, N)\n"
-        "for rep in range(2):\n"
-        "    st, ts, act = env.rollout_random(st, T)\n"
-        "    obs, rew, stype = ts.observation.grid.cpu().numpy(), ts.reward.cpu().numpy(), ts.step_type.cpu().numpy()\n"
-        "    for t in range(T):\n"
-        "        a = orc.random_actions_batch(rst)\n"
-        "        assert np.array_equal(act[t].cpu().numpy(), a), t\n"
-        "        rst, rts = orc.connector_step_batch(rst, a, time_limit=TL, autoreset_kind='parallel_random_walk')\n"
-        "        assert np.array_equal(obs[t], rts['obs']) and np.array_equal(rew[t], rts['reward']) and np.array_equal(stype[t], rts['step_type']), t\n"
-        "    assert np.array_equal(st.grid.cpu().numpy(), rst['grid']) and np.array_equal(st.key.cpu().numpy(), rst['key'])\n"
-        "    st, ts1 = env.step(st, a)  # a step-wise call in between shares the workspace\n"
-        "    rst, rts = orc.connector_step_batch(rst, a, time_limit=TL, autoreset_kind='parallel_random_walk')\n"
-        "    assert np.array_equal(ts1.observation.grid.cpu().numpy(), rts['obs']) and np.array_equal(st.grid.cpu().numpy(), rst['grid'])\n"
-        "print('rollout ok')\n"
-    ) % (root, G, N, B, T, time_limit)
-    r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, **env_vars), capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "rollout ok" in r.stdout, (r.stdout[-500:], r.stderr[-2000:])
-
-
-@pytest.mark.parametrize("slices", [1, 3, 4])
-def test_rollout_slice_counts(rbg, slices):
-    """The fused rollout splits the batch into slices that run on separate streams (2 by default);
-    RBG_ROLLOUT_SLICES selects 1, 3 or 4: same results."""
-    _rollout_in_subprocess({"RBG_ROLLOUT_SLICES": str(slices)}, 10, 5, 8200, 21)
-
-
-@pytest.mark.parametrize("no_cache,G,N,B", [("1", 10, 5, 4300), ("0", 24, 12, 300), ("1", 7, 3, 900)])
-def test_rollout_generation_modes(rbg, no_cache, G, N, B):
-    """Resets served by the next-episode cache + refill kernel (default for small boards) or all generated
-    inside the rollout kernel (default for large boards): RBG_ROLLOUT_NO_CACHE forces the other one."""
-    _rollout_in_subprocess({"RBG_ROLLOUT_NO_CACHE": no_cache}, G, N, B, 21, time_limit=5)
+    T = 21
+    keys, kref = _keys(rbg, orc, 5, B)
+    env = rbg.VmapAutoResetWrapper(rbg.Connector(generator=rbg.ParallelRandomWalkGenerator(G, N), time_limit=time_limit))
+    st, _ = env.reset(keys)
+    rst, _ = orc.connector_reset_batch("parallel_random_walk", kref, G, N)
+    for rep in range(2):
+        st, ts, act = env.rollout_random(st, T)
+        for t in range(T):
+            a = orc.random_actions_batch(rst)
+            assert np.array_equal(_np(act[t]), a), f"actions differ at step {t} of rollout {rep}"
+            rst, rts = orc.connector_step_batch(rst, a, time_limit=time_limit, autoreset_kind="parallel_random_walk")
+            _assert_timestep(ts[t], rts, f"at step {t} of rollout {rep}")
+        _assert_state(st, rst, f"after rollout {rep}")
+        st, ts = env.step(st, torch.from_numpy(a).cuda())
+        rst, rts = orc.connector_step_batch(rst, a, time_limit=time_limit, autoreset_kind="parallel_random_walk")
+        _assert_state(st, rst, f"after the step that follows rollout {rep}")
+        _assert_timestep(ts, rts, f"at the step that follows rollout {rep}")
 
 
 @pytest.mark.parametrize("G,N,B,T,time_limit", [(10, 5, 65536, 45, 50), (32, 16, 8192, 22, 9)])
 def test_rollout_full_size_matches_oracle(rbg, orc, G, N, B, T, time_limit):
     """BASELINE configs[1] (65 536 envs, 10x10/5) and configs[4] (32x32/16, 8 192 envs) at FULL size against the
-    oracle: every leaf of every TimeStep of the fused rollout (rollout_warp_kernel, bulk refill, two batch slices
-    on two streams) and the final State; then the step-by-step path (env_warp_kernel, speculative + synchronous
+    oracle: every leaf of every TimeStep of the fused rollout (rollout_persist_kernel) and the final State; then the step-by-step path (env_warp_kernel, speculative + synchronous
     reset kernels) continues from that State for a few steps, also against the oracle."""
     import torch
 
@@ -811,13 +789,19 @@ def test_connector_reference_fixtures_on_gpu(rbg):
     assert term > 150 and early > 20
 
 
-@pytest.mark.parametrize("board_name,G,N,K,time_limit", [("offline_parallel_rw", 10, 5, 200, 7), ("offline_seed_extension", 8, 4, 37, 5), ("offline_parallel_rw", 5, 3, 3, 2)])
+@pytest.mark.parametrize("board_name,G,N,K,time_limit", [
+    ("offline_parallel_rw", 10, 5, 200, 7),       # rollout_warp_kernel: observation staged in one buffer
+    ("offline_seed_extension", 8, 4, 37, 5),
+    ("offline_parallel_rw", 5, 3, 3, 2),          # cells % 4 != 0: scalar stores
+    ("offline_parallel_rw", 12, 10, 40, 5),       # two alternating staging buffers
+    ("offline_parallel_rw", 32, 16, 20, 5),       # direct 128-bit stores
+])
 def test_connector_with_dataset_generator(rbg, orc, board_name, G, N, K, time_limit):
     """Connector(generator=BoardDatasetGeneratorJAX(...)) as rl_training/setup_train.py:119-133,158 builds it:
     reset, 60 auto-reset steps and a fused rollout against the oracle (the in-kernel reset is a table lookup)."""
     import torch
 
-    B = 900
+    B = 300 if G >= 32 else 900  # 32x32/16 emits 64 KB of observation per env-step
     gen = rbg.BoardDatasetGeneratorJAX(G, N, board_name=board_name, number_of_boards=K)
     heads, targets = _np(gen.heads), _np(gen.targets)
     env = rbg.VmapAutoResetWrapper(rbg.Connector(generator=gen, time_limit=time_limit))
