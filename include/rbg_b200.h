@@ -290,9 +290,9 @@ int rbg_connector_step_host(const rbg_state *in, const rbg_state *out,
  * `state` must have been produced on the device's default stream (or a stream that synchronises with it); the call
  * orders itself behind that stream with an event and waits for its own copy streams at exit.
  * Transport: the observation (96 % of a TimeStep's bytes; codes <= 3 * RBG_MAX_N) crosses the bus as one byte per
- * cell (half a byte when N <= 5: codes <= 15; RBG_HOST_IO_BITS=8 keeps bytes) into a pinned staging buffer of the library and is widened to ts->obs_grid's int32 by a pool of host threads
+ * cell (half a byte when N <= 5: codes <= 15) into a pinned staging buffer of the library and is widened to ts->obs_grid's int32 by a pool of host threads
  * (all cores of the affinity mask / LOCAL_WORLD_SIZE, or RBG_HOST_THREADS), slice by slice while later slices are
- * in flight; ts->obs_grid need not be pinned.  RBG_HOST_IO_WIDE=1: int32 over the bus, no host threads. */
+ * in flight; ts->obs_grid need not be pinned. */
 int rbg_connector_step_host_io(const rbg_state *state, const int32_t *action,
                                int64_t B, int G, int N,
                                const rbg_env_params *params,
@@ -305,7 +305,7 @@ int rbg_host_widen(const uint8_t *src, int32_t *dst, int64_t n);
  * first); n = number of int32 outputs, even */
 int rbg_host_widen4(const uint8_t *src, int32_t *dst, int64_t n);
 /* Bytes the _host_io calls moved over the bus since the last reset (counted where the copies are enqueued) and the
- * number of host threads that widen the observation (0 with RBG_HOST_IO_WIDE=1); any pointer may be NULL. */
+ * number of host threads that widen the observation; any pointer may be NULL. */
 int rbg_host_transfer_stats(int64_t *h2d_bytes, int64_t *d2h_bytes, int *host_threads, int reset);
 /* pinned host allocation helpers for the _host variants (optional) */
 void *rbg_host_alloc(int64_t bytes);

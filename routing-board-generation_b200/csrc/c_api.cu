@@ -467,67 +467,24 @@ struct ScratchSig {
 struct HostCtx {
   Scratch scratch;
   cudaStream_t streams[3] = {nullptr, nullptr, nullptr};
-  cudaEvent_t stream_ev[3] = {nullptr, nullptr, nullptr};
   cudaEvent_t slice_ev[16] = {nullptr};
   cudaEvent_t copy_ev[16] = {nullptr};
   cudaEvent_t entry_ev = nullptr;
   uint8_t *stage8 = nullptr;  // pinned host staging of the byte observation (rbg_connector_step_host_io)
   size_t stage8_bytes = 0;
-  // thread-count tuning of the packed transport: the first calls of a batch shape try 1/4, 1/2, 3/4 and all of the
+  // thread-count tuning of the byte transport: the first calls of a batch shape try 1/4, 1/2, 3/4 and all of the
   // pool's workers (four calls each, the last three timed; more threads must win by 1 %) and the fastest count stays
   int64_t tune_B = -1;
   int tune_call = 0, tune_best = 0;
   double tune_best_s = 0.0;
-  // mixed transport: how many of the step's slices cross the bus as int32 straight into the caller's (pinned) buffer
-  // instead of as bytes for the host threads to widen; moved by one slice per call towards the balance of bus and host
-  int wide_slices = 0;
-  int64_t wide_B = -1;
   ScratchSig sig;
 };
 // what the _host variants moved over the bus since the last reset (rbg_host_transfer_stats)
 static std::atomic<long long> g_h2d_bytes{0}, g_d2h_bytes{0};
-static bool host_io_wide() {  // RBG_HOST_IO_WIDE=1: the observation crosses the bus as int32 (round 1's transport)
-  static int v = -1;
-  if (v < 0) {
-    const char *e = getenv("RBG_HOST_IO_WIDE");
-    v = e && atoi(e) != 0 ? 1 : 0;
-  }
-  return v == 1;
-}
 static HostCtx g_host[kMaxDevices];
-// RBG_HOST_IO_SPLIT=k: k of a step's slices cross the bus as int32 straight into the caller's (pinned) buffer instead of as
-// bytes for the host threads; RBG_HOST_IO_SPLIT=auto: adaptive (one slice per call towards whichever of bus and host
-// finished last).  Default: none.  Measured (profiles/r02g_hostio_split.log): on the boxes of this pool the bus (38 MB of
-// bytes per step land after 0.87 ms) and 8 widening threads (1.0 ms) are already balanced, so moving slices to the bus gains
-// nothing (1 / 3 of 16 slices at the end of the step: 44.5 / 42.2 against 43.5 M env-steps/s on the same box) and a wide
-// slice at the START of the step costs 0.7 ms.
-static int host_io_split_env() {  // -2 off, -1 auto, >= 0 fixed
-  static int v = -3;
-  if (v == -3) {
-    const char *e = getenv("RBG_HOST_IO_SPLIT");
-    v = !e ? -2 : (strcmp(e, "auto") == 0 ? -1 : atoi(e));
-    if (v < -2) v = -2;
-  }
-  return v;
-}
-static bool host_io_fixed_split() { return host_io_split_env() >= 0; }
-static int host_io_split_init(int nslices) {
-  const int v = host_io_split_env();
-  if (v >= 0) return v > nslices ? nslices : v;
-  return v == -1 ? nslices / 8 : 0;
-}
-static bool host_io_blocking_sync() {  // RBG_HOST_BLOCKING_SYNC=1: the calling thread sleeps on the copy events instead of spinning
-  static int v = -1;
-  if (v < 0) {
-    const char *e = getenv("RBG_HOST_BLOCKING_SYNC");
-    v = (e && atoi(e) != 0) ? 1 : 0;
-  }
-  return v == 1;
-}
 static thread_local HostCtx *g_hc = &g_host[0];  // the device of the _host call in progress (set by use_device)
 #define g_scratch (g_hc->scratch)
 #define g_streams (g_hc->streams)
-#define g_stream_ev (g_hc->stream_ev)
 #define g_scratch_sig (g_hc->sig)
 
 static int scratch_get(size_t bytes, int device, void **out) {
@@ -548,10 +505,19 @@ static int scratch_get(size_t bytes, int device, void **out) {
     if (!g_streams[i]) {
       cudaError_t e = cudaStreamCreateWithFlags(&g_streams[i], cudaStreamNonBlocking);
       if (e != cudaSuccess) return set_cuda_error(e, "cudaStreamCreate");
-      if ((e = cudaEventCreateWithFlags(&g_stream_ev[i], cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
     }
   *out = g_scratch.ptr;
   return RBG_OK;
+}
+
+// Waits for all three streams of the _host variants, also after one of them has failed.
+static int sync_streams() {
+  int rc = RBG_OK;
+  for (int i = 0; i < 3; ++i) {
+    cudaError_t e = cudaStreamSynchronize(g_streams[i]);
+    if (e != cudaSuccess) rc = set_cuda_error(e, "cudaStreamSynchronize");
+  }
+  return rc;
 }
 
 struct Carver {
@@ -565,6 +531,19 @@ struct Carver {
     return p;
   }
 };
+
+// `layout(Carver &)` takes a call's device buffers in order.  It runs once on a null base to size the scratch and
+// once on the scratch itself, so the two passes cannot disagree.
+template <typename Layout>
+static int scratch_carve(int device, void **base, Layout &&layout) {
+  Carver size{nullptr};
+  layout(size);
+  int rc = scratch_get(size.off + 256, device, base);
+  if (rc) return rc;
+  Carver c{reinterpret_cast<uint8_t *>(*base)};
+  layout(c);
+  return RBG_OK;
+}
 
 static void carve_state(Carver &c, int64_t B, int G, int N, rbg_state *s) {
   s->grid = c.take<int32_t>((size_t)B * G * G);
@@ -605,12 +584,11 @@ static int copy_state(const rbg_state *dst, const rbg_state *src, int64_t off, i
   RBG_CPY(dst->key + dst_off * 2, src->key + off * 2, n * 8, kind, st);
   return RBG_OK;
 }
-// `parts`: 1 = observation.grid (the bulk), 2 = every other leaf, 3 = both
+// `with_obs`: false leaves observation.grid (the bulk) out
 static int copy_timestep(const rbg_timestep *dst, const rbg_timestep *src, int64_t off, int64_t n, int G, int N,
-                         cudaMemcpyKind kind, int64_t dst_off, cudaStream_t st, int parts = 3) {
+                         cudaMemcpyKind kind, int64_t dst_off, cudaStream_t st, bool with_obs = true) {
   const size_t c = (size_t)G * G * N;
-  if (parts & 1) RBG_CPY(dst->obs_grid + dst_off * c, src->obs_grid + off * c, n * c * 4, kind, st);
-  if (!(parts & 2)) return RBG_OK;
+  if (with_obs) RBG_CPY(dst->obs_grid + dst_off * c, src->obs_grid + off * c, n * c * 4, kind, st);
   RBG_CPY(dst->action_mask + dst_off * N * 5, src->action_mask + off * N * 5, n * N * 5, kind, st);
   RBG_CPY(dst->obs_step_count + dst_off, src->obs_step_count + off, n * 4, kind, st);
   RBG_CPY(dst->reward + dst_off * N, src->reward + off * N, n * N * 4, kind, st);
@@ -1108,19 +1086,17 @@ int rbg_prw_generate_host(const uint32_t *keys, int64_t B, int G, int N, int32_t
   if (!keys || !heads || !targets || !solved) return set_error(RBG_EINVAL, "rbg_prw_generate_host: NULL pointer");
   if ((rc = use_device(device, &dev))) return rc;
   std::lock_guard<std::mutex> lock(g_scratch_mu);
-  Carver size{nullptr};
-  size.take<uint32_t>((size_t)B * 2);
-  size.take<int32_t>((size_t)B * 2 * N);
-  size.take<int32_t>((size_t)B * 2 * N);
-  size.take<int32_t>((size_t)B * G * G);
+  uint32_t *dk;
+  int32_t *dh, *dt, *ds;
   void *base;
-  if ((rc = scratch_get(size.off + 256, dev, &base))) return rc;
+  rc = scratch_carve(dev, &base, [&](Carver &c) {
+    dk = c.take<uint32_t>((size_t)B * 2);
+    dh = c.take<int32_t>((size_t)B * 2 * N);
+    dt = c.take<int32_t>((size_t)B * 2 * N);
+    ds = c.take<int32_t>((size_t)B * G * G);
+  });
+  if (rc) return rc;
   scratch_claim(ScratchSig{1, B, G, N, -1, base}, nullptr, 0, 0);
-  Carver c{reinterpret_cast<uint8_t *>(base)};
-  uint32_t *dk = c.take<uint32_t>((size_t)B * 2);
-  int32_t *dh = c.take<int32_t>((size_t)B * 2 * N);
-  int32_t *dt = c.take<int32_t>((size_t)B * 2 * N);
-  int32_t *ds = c.take<int32_t>((size_t)B * G * G);
   const int nsl = B >= 4096 ? 4 : 1;
   const int64_t sl = slice_size(B, nsl);
   int si = 0;
@@ -1134,11 +1110,7 @@ int rbg_prw_generate_host(const uint32_t *keys, int64_t B, int G, int N, int32_t
     RBG_CPY(targets + off * 2 * N, dt + off * 2 * N, n * 2 * N * 4, cudaMemcpyDeviceToHost, st);
     RBG_CPY(solved + off * G * G, ds + off * G * G, n * G * G * 4, cudaMemcpyDeviceToHost, st);
   }
-  for (int i = 0; i < 3; ++i) {
-    cudaError_t e = cudaStreamSynchronize(g_streams[i]);
-    if (e != cudaSuccess) return set_cuda_error(e, "cudaStreamSynchronize");
-  }
-  return RBG_OK;
+  return sync_streams();
 }
 
 int rbg_connector_reset_host(int kind, const uint32_t *keys, int64_t B, int G, int N, const rbg_state *state,
@@ -1149,19 +1121,17 @@ int rbg_connector_reset_host(int kind, const uint32_t *keys, int64_t B, int G, i
   if (!keys || !state || !ts) return set_error(RBG_EINVAL, "rbg_connector_reset_host: NULL pointer");
   if ((rc = use_device(device, &dev))) return rc;
   std::lock_guard<std::mutex> lock(g_scratch_mu);
-  Carver size{nullptr};
+  uint32_t *dk;
   rbg_state ds;
   rbg_timestep dt;
-  size.take<uint32_t>((size_t)B * 2);
-  carve_state(size, B, G, N, &ds);
-  carve_timestep(size, B, G, N, &dt);
   void *base;
-  if ((rc = scratch_get(size.off + 256, dev, &base))) return rc;
+  rc = scratch_carve(dev, &base, [&](Carver &c) {
+    dk = c.take<uint32_t>((size_t)B * 2);
+    carve_state(c, B, G, N, &ds);
+    carve_timestep(c, B, G, N, &dt);
+  });
+  if (rc) return rc;
   scratch_claim(ScratchSig{2, B, G, N, kind, base}, nullptr, 0, 0);
-  Carver c{reinterpret_cast<uint8_t *>(base)};
-  uint32_t *dk = c.take<uint32_t>((size_t)B * 2);
-  carve_state(c, B, G, N, &ds);
-  carve_timestep(c, B, G, N, &dt);
   const int nsl = B >= 4096 ? 4 : 1;
   const int64_t sl = slice_size(B, nsl);
   int si = 0;
@@ -1175,11 +1145,7 @@ int rbg_connector_reset_host(int kind, const uint32_t *keys, int64_t B, int G, i
     if ((rc = copy_state(state, &ds, off, n, G, N, cudaMemcpyDeviceToHost, off, st))) return rc;
     if ((rc = copy_timestep(ts, &dt, off, n, G, N, cudaMemcpyDeviceToHost, off, st))) return rc;
   }
-  for (int i = 0; i < 3; ++i) {
-    cudaError_t e = cudaStreamSynchronize(g_streams[i]);
-    if (e != cudaSuccess) return set_cuda_error(e, "cudaStreamSynchronize");
-  }
-  return RBG_OK;
+  return sync_streams();
 }
 
 int rbg_connector_step_host(const rbg_state *in, const rbg_state *out, const int32_t *action, int64_t B, int G,
@@ -1193,21 +1159,19 @@ int rbg_connector_step_host(const rbg_state *in, const rbg_state *out, const int
   const int nsl = B >= 4096 ? 8 : 1;
   const int64_t sl = slice_size(B, nsl);
   const int64_t nslices = (B + sl - 1) / sl;
-  Carver size{nullptr};
+  const size_t ws_bytes = (size_t)rbg_step_workspace_bytes(sl, G, N);
   rbg_state ds;
   rbg_timestep dt;
-  carve_state(size, B, G, N, &ds);
-  carve_timestep(size, B, G, N, &dt);
-  size.take<int32_t>((size_t)B * N);
-  const size_t ws_bytes = (size_t)rbg_step_workspace_bytes(sl, G, N);
-  size.take<uint8_t>((size_t)nslices * ws_bytes);
+  int32_t *da;
+  uint8_t *ws;
   void *base;
-  if ((rc = scratch_get(size.off + 256, dev, &base))) return rc;
-  Carver c{reinterpret_cast<uint8_t *>(base)};
-  carve_state(c, B, G, N, &ds);
-  carve_timestep(c, B, G, N, &dt);
-  int32_t *da = c.take<int32_t>((size_t)B * N);
-  uint8_t *ws = c.take<uint8_t>((size_t)nslices * ws_bytes);
+  rc = scratch_carve(dev, &base, [&](Carver &c) {
+    carve_state(c, B, G, N, &ds);
+    carve_timestep(c, B, G, N, &dt);
+    da = c.take<int32_t>((size_t)B * N);
+    ws = c.take<uint8_t>((size_t)nslices * ws_bytes);
+  });
+  if (rc) return rc;
   scratch_claim(ScratchSig{3, B, G, N, params->autoreset_kind, base}, ws, ws_bytes, nslices);
   int si = 0;
   for (int64_t off = 0; off < B; off += sl, ++si) {
@@ -1222,11 +1186,7 @@ int rbg_connector_step_host(const rbg_state *in, const rbg_state *out, const int
     if ((rc = copy_state(out, &ds, off, n, G, N, cudaMemcpyDeviceToHost, off, st))) return rc;
     if ((rc = copy_timestep(ts, &dt, off, n, G, N, cudaMemcpyDeviceToHost, off, st))) return rc;
   }
-  for (int i = 0; i < 3; ++i) {
-    cudaError_t e = cudaStreamSynchronize(g_streams[i]);
-    if (e != cudaSuccess) return set_cuda_error(e, "cudaStreamSynchronize");
-  }
-  return RBG_OK;
+  return sync_streams();
 }
 
 // Env-pool style step: the State stays on the device (updated in place), the actions come from and
@@ -1241,11 +1201,9 @@ int rbg_connector_step_host_io(const rbg_state *state, const int32_t *action, in
   if ((rc = use_device(device, &dev))) return rc;
   std::lock_guard<std::mutex> lock(g_scratch_mu);
   cudaError_t e;
-  const bool packed = !host_io_wide();
   const auto t_call0 = std::chrono::steady_clock::now();
   int tune_slot = -1;  // which candidate this call measures (odd calls of the tuning phase)
-  bool in_tuning = false;  // the thread count is being tried out: the bus / host split stays put meanwhile
-  if (packed && !host_pool_fixed() && host_pool_max_threads() >= 4) {
+  if (!host_pool_fixed() && host_pool_max_threads() >= 4) {
     const int64_t key = B * 4096 + (int64_t)G * 64 + N;
     if (g_hc->tune_B != key) {
       g_hc->tune_B = key;
@@ -1260,7 +1218,6 @@ int rbg_connector_step_host_io(const rbg_state *state, const int32_t *action, in
     const bool big = host_pool_max_threads() >= 8;
     const int ncand = big ? 3 : 4;
     if (g_hc->tune_call < 4 * ncand) {
-      in_tuning = true;
       const int cand = g_hc->tune_call / 4;  // four calls each, the last three timed
       int n = big ? host_pool_max_threads() * (cand + 2) / 8 : host_pool_max_threads() * (cand + 1) / 4;
       host_pool_set_threads(n < 1 ? 1 : n);
@@ -1271,34 +1228,26 @@ int rbg_connector_step_host_io(const rbg_state *state, const int32_t *action, in
       g_hc->tune_call++;
     }
   }
-  static int nsl_env = -1;
-  if (nsl_env < 0) {
-    const char *ex = getenv("RBG_HOST_IO_SLICES");
-    nsl_env = ex ? atoi(ex) : 0;
-    if (nsl_env < 0 || nsl_env > 16) nsl_env = 0;
-  }
   // 16 slices for big batches: the host starts widening after 1/16 of the copies and ends 1/16 after them (measured at
   // 65 536 envs 10x10/5: 8 slices 1.27-1.6 ms per step, 16 slices 1.17-1.24 ms)
-  const int nsl = B >= 4096 ? (nsl_env ? nsl_env : (packed && B >= 32768 ? 16 : 8)) : 1;
+  const int nsl = B >= 32768 ? 16 : B >= 4096 ? 8 : 1;
   const int64_t sl = slice_size(B, nsl);
   const int64_t nslices = (B + sl - 1) / sl;
   const size_t obs_n = (size_t)B * N * G * G;
-  Carver size{nullptr};
-  rbg_timestep dt;
-  carve_timestep(size, B, G, N, &dt);
-  size.take<int32_t>((size_t)B * N);
   const size_t ws_bytes = (size_t)rbg_step_workspace_bytes(sl, G, N);
-  size.take<uint8_t>((size_t)nslices * ws_bytes);
-  if (packed) size.take<uint8_t>(obs_n);
+  rbg_timestep dt;
+  int32_t *da;
+  uint8_t *ws, *obs8;
   void *base;
-  if ((rc = scratch_get(size.off + 256, dev, &base))) return rc;
-  Carver c{reinterpret_cast<uint8_t *>(base)};
-  carve_timestep(c, B, G, N, &dt);
-  int32_t *da = c.take<int32_t>((size_t)B * N);
-  uint8_t *ws = c.take<uint8_t>((size_t)nslices * ws_bytes);
-  uint8_t *obs8 = packed ? c.take<uint8_t>(obs_n) : nullptr;
+  rc = scratch_carve(dev, &base, [&](Carver &c) {
+    carve_timestep(c, B, G, N, &dt);
+    da = c.take<int32_t>((size_t)B * N);
+    ws = c.take<uint8_t>((size_t)nslices * ws_bytes);
+    obs8 = c.take<uint8_t>(obs_n);
+  });
+  if (rc) return rc;
   scratch_claim(ScratchSig{4, B, G, N, params->autoreset_kind, base}, ws, ws_bytes, nslices);
-  if (packed && g_hc->stage8_bytes < obs_n) {
+  if (g_hc->stage8_bytes < obs_n) {
     if (g_hc->stage8) cudaFreeHost(g_hc->stage8);
     g_hc->stage8 = nullptr;
     g_hc->stage8_bytes = 0;
@@ -1308,9 +1257,9 @@ int rbg_connector_step_host_io(const rbg_state *state, const int32_t *action, in
   // One compute stream runs the slices' kernels back to back (the whole batch is ~0.1 ms of kernels); the two
   // copy streams take the observation (96 % of the bytes) of each slice as soon as its kernel is done, so the
   // bus is busy from the first slice on.  The small leaves go once for the whole batch: 8 copies instead of 8 per
-  // slice.  Packed transport (default): the observation's codes cross the bus as bytes into a pinned staging
-  // buffer and the host pool widens slice s into the caller's int32 buffer while slices s+1.. are in flight; the
-  // caller's observation buffer need not be pinned.
+  // slice.  The observation's codes cross the bus as bytes into a pinned staging buffer and the host pool widens
+  // slice s into the caller's int32 buffer while slices s+1.. are in flight; the caller's observation buffer need
+  // not be pinned.
   cudaEvent_t *slice_ev = g_hc->slice_ev, *copy_ev = g_hc->copy_ev;
   cudaStream_t cs = g_streams[0];
   // The State was produced by the caller on the device's default stream (or a stream that stream synchronises
@@ -1323,114 +1272,42 @@ int rbg_connector_step_host_io(const rbg_state *state, const int32_t *action, in
   const size_t per_env = (size_t)N * G * G;
   // Observation codes are <= 3 N: with at most 5 agents they fit a nibble, two cells per byte over the bus (a slice is a
   // multiple of 64 envs, so every slice starts on a whole, 16-byte aligned byte when an env has an even number of cells).
-  // RBG_HOST_IO_BITS=8 keeps a byte per cell.
-  static const int bits_env = env_int("RBG_HOST_IO_BITS");
-  const int obits = (packed && 3 * N <= 15 && (per_env & 1u) == 0 && bits_env != 8) ? 4 : 8;
+  const int obits = (3 * N <= 15 && (per_env & 1u) == 0) ? 4 : 8;
   const int oshift = obits == 4 ? 1 : 0;
-  // Mixed transport (off by default, see host_io_split_env): `nwide` of the step's slices go over the bus as int32, the
-  // rest as bytes.
-  bool mix = false;
-  if (packed && nslices > 1 && host_io_split_env() == -1) {
-    cudaPointerAttributes pa;
-    if (cudaPointerGetAttributes(&pa, ts->obs_grid) == cudaSuccess && pa.type == cudaMemoryTypeHost) mix = true;
-    (void)cudaGetLastError();
-  }
-  const int64_t mix_key = B * 4096 + (int64_t)G * 64 + N;
-  if (g_hc->wide_B != mix_key) {
-    g_hc->wide_B = mix_key;
-    g_hc->wide_slices = host_io_split_init((int)nslices);
-  }
-  const int nwide = !packed ? (int)nslices : (mix || host_io_fixed_split()) ? (g_hc->wide_slices > (int)nslices ? (int)nslices : g_hc->wide_slices) : 0;
-  // evenly spread, the first slice first and never the last one (its widening is the host's tail either way)
-  static const int split_pos = env_int("RBG_HOST_IO_SPLIT_POS");  // experiment: 1 = evenly spread from the first slice on, 2 = the first ones
-  auto slice_is_wide = [&](int i) {
-    if (!packed) return true;
-    if (split_pos == 1) return ((int64_t)i * nwide) % nslices < nwide;
-    if (split_pos == 2) return i < nwide;
-    return i >= (int)nslices - nwide;  // the last ones: the host threads get their bytes first
-  };
-  size_t packed_cells = 0, wide_cells = 0;
   int si = 0;
   for (int64_t off = 0; off < B; off += sl, ++si) {
     const int64_t n = (B - off) < sl ? (B - off) : sl;
-    const bool wide = slice_is_wide(si);
+    const size_t codes_off = ((size_t)off * per_env) >> oshift;
     rbg_state dss = state_at(*state, off, G, N);
     rbg_timestep dts = timestep_at(dt, off, G, N);
     if ((rc = rbg_connector_step(&dss, &dss, da + off * N, n, G, N, params, &dts, ws + (size_t)si * ws_bytes, cs))) return rc;
-    if (!wide && (rc = launch_narrow_codes(dts.obs_grid, obs8 + (((size_t)off * per_env) >> oshift), (int64_t)((size_t)n * per_env), cs, obits))) return rc;
+    if ((rc = launch_narrow_codes(dts.obs_grid, obs8 + codes_off, (int64_t)((size_t)n * per_env), cs, obits))) return rc;
     if (!slice_ev[si] && (e = cudaEventCreateWithFlags(&slice_ev[si], cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
     if ((e = cudaEventRecord(slice_ev[si], cs)) != cudaSuccess) return set_cuda_error(e, "cudaEventRecord");
     cudaStream_t xs = g_streams[1 + (si & 1)];
     if ((e = cudaStreamWaitEvent(xs, slice_ev[si], 0)) != cudaSuccess) return set_cuda_error(e, "cudaStreamWaitEvent");
-    (wide ? wide_cells : packed_cells) += (size_t)n * per_env;
-    if (!wide) {
-      RBG_CPY(g_hc->stage8 + (((size_t)off * per_env) >> oshift), obs8 + (((size_t)off * per_env) >> oshift), ((size_t)n * per_env) >> oshift, cudaMemcpyDeviceToHost, xs);
-      if (!copy_ev[si] && (e = cudaEventCreateWithFlags(&copy_ev[si], cudaEventDisableTiming | (host_io_blocking_sync() ? cudaEventBlockingSync : 0))) != cudaSuccess)
-        return set_cuda_error(e, "cudaEventCreate");
-      if ((e = cudaEventRecord(copy_ev[si], xs)) != cudaSuccess) return set_cuda_error(e, "cudaEventRecord(copy)");
-    } else if ((rc = copy_timestep(ts, &dt, off, n, G, N, cudaMemcpyDeviceToHost, off, xs, 1))) {
-      return rc;
+    RBG_CPY(g_hc->stage8 + codes_off, obs8 + codes_off, ((size_t)n * per_env) >> oshift, cudaMemcpyDeviceToHost, xs);
+    if (!copy_ev[si] && (e = cudaEventCreateWithFlags(&copy_ev[si], cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
+    if ((e = cudaEventRecord(copy_ev[si], xs)) != cudaSuccess) return set_cuda_error(e, "cudaEventRecord(copy)");
+  }
+  if ((rc = copy_timestep(ts, &dt, 0, B, G, N, cudaMemcpyDeviceToHost, 0, cs, false))) return rc;
+  g_d2h_bytes.fetch_add((long long)(obs_n >> oshift) + (long long)B * (N * 5 + 4 + N * 8 + 1 + 12), std::memory_order_relaxed);
+  si = 0;
+  for (int64_t off = 0; off < B; off += sl, ++si) {
+    const int64_t n = (B - off) < sl ? (B - off) : sl;
+    if ((e = cudaEventSynchronize(copy_ev[si])) != cudaSuccess) {
+      host_pool_wait();
+      return set_cuda_error(e, "cudaEventSynchronize(copy)");
     }
+    const size_t codes_off = ((size_t)off * per_env) >> oshift;
+    if (obits == 4)
+      host_pool_widen4(g_hc->stage8 + codes_off, ts->obs_grid + (size_t)off * per_env, (size_t)n * per_env);
+    else
+      host_pool_widen(g_hc->stage8 + codes_off, ts->obs_grid + (size_t)off * per_env, (size_t)n * per_env);
   }
-  if ((rc = copy_timestep(ts, &dt, 0, B, G, N, cudaMemcpyDeviceToHost, 0, cs, 2))) return rc;
-  const auto t_issued = std::chrono::steady_clock::now();
-  g_d2h_bytes.fetch_add((long long)((packed_cells >> oshift) + 4 * wide_cells) + (long long)B * (N * 5 + 4 + N * 8 + 1 + 12), std::memory_order_relaxed);
-  if (packed) {
-    si = 0;
-    for (int64_t off = 0; off < B; off += sl, ++si) {
-      const int64_t n = (B - off) < sl ? (B - off) : sl;
-      if (slice_is_wide(si)) continue;
-      if ((e = cudaEventSynchronize(copy_ev[si])) != cudaSuccess) {
-        host_pool_wait();
-        return set_cuda_error(e, "cudaEventSynchronize(copy)");
-      }
-      if (obits == 4)
-        host_pool_widen4(g_hc->stage8 + (((size_t)off * per_env) >> 1), ts->obs_grid + (size_t)off * per_env, (size_t)n * per_env);
-      else
-        host_pool_widen(g_hc->stage8 + (size_t)off * per_env, ts->obs_grid + (size_t)off * per_env, (size_t)n * per_env);
-    }
-  }
-  int rc_sync = RBG_OK;
-  for (int i = 0; i < 3; ++i) {
-    e = cudaStreamSynchronize(g_streams[i]);
-    if (e != cudaSuccess) rc_sync = set_cuda_error(e, "cudaStreamSynchronize");
-  }
-  const auto t_bus_done = std::chrono::steady_clock::now();
-  if (packed) host_pool_wait();
-  {  // RBG_HOST_IO_TRACE=1: where a call's time goes (issue of the launches and copies / until the last copy landed / until
-     // the last slice is widened), averaged over 32 calls, on stderr
-    static const int trace = env_int("RBG_HOST_IO_TRACE");
-    if (trace) {
-      static double acc[3] = {0, 0, 0};
-      static int ncalls = 0;
-      const auto t_now = std::chrono::steady_clock::now();
-      acc[0] += std::chrono::duration<double>(t_issued - t_call0).count();
-      acc[1] += std::chrono::duration<double>(t_bus_done - t_call0).count();
-      acc[2] += std::chrono::duration<double>(t_now - t_call0).count();
-      if (++ncalls == 32) {
-        fprintf(stderr, "[rbg host_io] threads %d wide slices %d/%d: issued %.3f ms, copies landed %.3f ms, widened %.3f ms\n", host_pool_threads(), nwide, (int)nslices,
-                acc[0] / 32 * 1e3, acc[1] / 32 * 1e3, acc[2] / 32 * 1e3);
-        acc[0] = acc[1] = acc[2] = 0;
-        ncalls = 0;
-      }
-    }
-  }
-  if (mix && rc_sync == RBG_OK) {
-    // who finished last?  The host threads still busy well after the last copy landed: the host is the bound, one more
-    // slice goes over the bus as int32.  The pool idle when the copies ended (their last slice is widened within a
-    // twentieth of the call): the bus is the bound, one slice fewer.
-    const auto t_end = std::chrono::steady_clock::now();
-    const double total = std::chrono::duration<double>(t_end - t_call0).count();
-    const double host_tail = std::chrono::duration<double>(t_end - t_bus_done).count();
-    // (the widening of the last byte slice always trails the copies by about 1 / nslices of the call: the dead band)
-    if (!in_tuning) {
-      if (host_tail > 1.6 / (double)nslices * total && g_hc->wide_slices < (int)nslices - 1)
-        g_hc->wide_slices++;
-      else if (host_tail < 0.6 / (double)nslices * total && g_hc->wide_slices > 0)
-        g_hc->wide_slices--;
-    }
-  }
-  if (tune_slot >= 0 && rc_sync == RBG_OK) {
+  rc = sync_streams();
+  host_pool_wait();
+  if (tune_slot >= 0 && rc == RBG_OK) {
     const double dt = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_call0).count();
     // the fastest call decides; a larger thread count must beat a smaller one by 1 % to replace it (the candidates of a
     // single-rank host stop at half of the cores, where more threads still help: 6 / 8 threads 65.4 / 68.1 M env-steps/s)
@@ -1440,7 +1317,7 @@ int rbg_connector_step_host_io(const rbg_state *state, const int32_t *action, in
       g_hc->tune_best_s = dt;
     }
   }
-  return rc_sync;
+  return rc;
 }
 
 int rbg_host_widen(const uint8_t *src, int32_t *dst, int64_t n) {
@@ -1462,7 +1339,7 @@ int rbg_host_widen4(const uint8_t *src, int32_t *dst, int64_t n) {
 int rbg_host_transfer_stats(int64_t *h2d_bytes, int64_t *d2h_bytes, int *host_threads, int reset) {
   if (h2d_bytes) *h2d_bytes = reset ? g_h2d_bytes.exchange(0) : g_h2d_bytes.load();
   if (d2h_bytes) *d2h_bytes = reset ? g_d2h_bytes.exchange(0) : g_d2h_bytes.load();
-  if (host_threads) *host_threads = host_io_wide() ? 0 : host_pool_threads();
+  if (host_threads) *host_threads = host_pool_threads();
   return RBG_OK;
 }
 

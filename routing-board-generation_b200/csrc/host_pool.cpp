@@ -62,18 +62,6 @@ __attribute__((target("avx2"))) void widen_avx2(const uint8_t *src, int32_t *dst
 #endif
 
 #if defined(__x86_64__)
-__attribute__((target("avx2"))) void widen_avx2_cached(const uint8_t *src, int32_t *dst, size_t n) {
-  size_t i = 0;
-  for (; i + 16 <= n; i += 16) {
-    const __m128i a = _mm_loadu_si128(reinterpret_cast<const __m128i *>(src + i));
-    _mm256_storeu_si256(reinterpret_cast<__m256i *>(dst + i), _mm256_cvtepu8_epi32(a));
-    _mm256_storeu_si256(reinterpret_cast<__m256i *>(dst + i + 8), _mm256_cvtepu8_epi32(_mm_srli_si128(a, 8)));
-  }
-  for (; i < n; ++i) dst[i] = src[i];
-}
-#endif
-
-#if defined(__x86_64__)
 // 16 source bytes -> 32 int32 per iteration; NT: the destination is 32-byte aligned after an EVEN number of scalar outputs
 // (the caller checks), so that the vector loop starts on a whole source byte
 template <bool NT>
@@ -111,12 +99,11 @@ __attribute__((target("avx2"))) void widen4_avx2(const uint8_t *src, int32_t *ds
 void widen4(const uint8_t *src, int32_t *dst, size_t n) {
 #if defined(__x86_64__)
   static const bool avx2 = __builtin_cpu_supports("avx2");
-  static const bool nt = !(getenv("RBG_HOST_NT") && atoi(getenv("RBG_HOST_NT")) == 0);
   if (avx2) {
     // outputs to the next 32-byte boundary of dst: odd (a destination at an odd int32 offset) would leave the vector loop
     // in the middle of a source byte: plain unaligned stores then
     const size_t head = ((32u - (reinterpret_cast<uintptr_t>(dst) & 31u)) & 31u) >> 2;
-    return (nt && (head & 1u) == 0) ? widen4_avx2<true>(src, dst, n) : widen4_avx2<false>(src, dst, n);
+    return (head & 1u) == 0 ? widen4_avx2<true>(src, dst, n) : widen4_avx2<false>(src, dst, n);
   }
 #endif
   widen4_scalar(src, dst, n);
@@ -125,8 +112,7 @@ void widen4(const uint8_t *src, int32_t *dst, size_t n) {
 void widen(const uint8_t *src, int32_t *dst, size_t n) {
 #if defined(__x86_64__)
   static const bool avx2 = __builtin_cpu_supports("avx2");
-  static const bool nt = !(getenv("RBG_HOST_NT") && atoi(getenv("RBG_HOST_NT")) == 0);
-  if (avx2) return nt ? widen_avx2(src, dst, n) : widen_avx2_cached(src, dst, n);
+  if (avx2) return widen_avx2(src, dst, n);
 #endif
   widen_scalar(src, dst, n);
 }

@@ -1,4 +1,4 @@
-"""e2e step (rbg_connector_step_host_io) under different transports / thread counts / slice counts: one subprocess per setting."""
+"""e2e step (rbg_connector_step_host_io) under different host thread counts (RBG_HOST_THREADS): one subprocess per setting."""
 import os, subprocess, sys
 root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 code = r'''
@@ -30,13 +30,9 @@ for _ in range(10): step()
 st_ = L.host_transfer_stats()
 print("%%.3f ms/step  %%.1f M env-steps/s  threads %%d  d2h MB/step %%.1f" %% (best * 1e3, B / best / 1e6, st_[2], st_[1] / 10 / 1e6))
 ''' % root
-settings = [{}, {"RBG_HOST_THREADS": "8"}, {"RBG_HOST_THREADS": "10"}, {"RBG_HOST_THREADS": "12"}, {"RBG_HOST_THREADS": "16"},
-            {"RBG_HOST_BLOCKING_SYNC": "1"}, {"RBG_HOST_BLOCKING_SYNC": "1", "RBG_HOST_THREADS": "8"}, {"RBG_HOST_BLOCKING_SYNC": "1", "RBG_HOST_THREADS": "12"},
-            {"RBG_HOST_BLOCKING_SYNC": "1", "RBG_HOST_THREADS": "16"}]
+settings = [{}, {"RBG_HOST_THREADS": "8"}, {"RBG_HOST_THREADS": "10"}, {"RBG_HOST_THREADS": "12"}, {"RBG_HOST_THREADS": "16"}]
 if len(sys.argv) > 1:
     settings = [dict(kv.split("=") for kv in a.split(",") if kv) for a in sys.argv[1:]]
 for env in settings:
     r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, **env), capture_output=True, text=True, timeout=600)
     print(env, r.stdout.strip() or r.stderr[-600:], flush=True)
-    if 'RBG_HOST_IO_TRACE' in env:
-        print('   ' + '\n   '.join([l for l in r.stderr.splitlines() if 'host_io' in l][-3:]), flush=True)
