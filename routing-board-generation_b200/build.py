@@ -42,7 +42,7 @@ def is_stale() -> bool:
 
 
 def build(force: bool = False, verbose: bool = False) -> str:
-    extra = os.environ.get("RBG_NVCC_EXTRA", "").split()  # e.g. -DRBG_TF_PLAIN_ADD for A/B builds
+    extra = os.environ.get("RBG_NVCC_EXTRA", "").split()  # extra nvcc flags, passed through as given (no source file has -D switches of its own)
     if not force and not extra and not is_stale():
         return SO
     os.makedirs(LIBDIR, exist_ok=True)

@@ -138,26 +138,73 @@ static int debug_flags() {
   }
   return v;
 }
-static int env_int(const char *name) {
-  const char *e = getenv(name);
-  return e ? atoi(e) : 0;
+
+// ---- auto-reset workspace ------------------------------------------------------
+// VmapAutoResetWrapper regenerates a board whenever an env finishes.  The reset key
+// of an episode is known as soon as the episode starts (split(state.key)[0]), so the
+// NEXT episode of every env that just reset is generated ahead of time ("refill")
+// into a per-env cache; when the env finishes, env_kernel swaps the
+// cached episode in.  Only envs whose cache entry is not ready (first episode, or two
+// terminations in consecutive steps) take the synchronous reset kernel.  Results are
+// identical either way: a board is a pure function of its key.
+struct WsLayout {
+  size_t sync_list, refill_list[2], refill_keys[2], cache_tag, cache_key, cache_pins, group_done, group_pending, total;
+};
+static WsLayout ws_layout(int64_t B, int N) {
+  auto up = [](size_t x) { return (x + 255) & ~(size_t)255; };
+  WsLayout w;
+  size_t off = 512;  // counters: sync @0, refill[0] @64, refill[1] @128; persistent rollout: 16 sets of 4 ints @256
+  const size_t b = (size_t)(B > 0 ? B : 0);
+  w.sync_list = off;
+  off = up(off + 4 * b);
+  for (int i = 0; i < 2; ++i) {
+    w.refill_list[i] = off;
+    off = up(off + 4 * b);
+    w.refill_keys[i] = off;
+    off = up(off + 8 * b);
+  }
+  w.cache_tag = off;
+  off = up(off + 8 * b);
+  w.cache_key = off;
+  off = up(off + 8 * b);
+  w.cache_pins = off;
+  off = up(off + 4 * b * (size_t)N);
+  w.group_done = off;  // persistent rollout: per env group, the last launch that wrote it / its requests in flight
+  off = up(off + 4 * b);
+  w.group_pending = off;
+  off = up(off + 4 * b);
+  w.total = off;
+  return w;
+}
+
+// A ParallelRandomWalk / Uniform generation (kind) of the boards that follow `keys`, after `extra_split` leading
+// split()[0]: PRWG:52 key, pos_key = split(key): the board uses split(key)[0]; UG:76 the uniform generator consumes the
+// split itself (both halves).  With `cache_ws` the boards go to the next-episode cache of that auto-reset workspace.
+static PrwParams prw_params(int kind, const uint32_t *keys, int64_t B, int G, int N, int extra_split, uint8_t *cache_ws = nullptr) {
+  PrwParams p;
+  memset(&p, 0, sizeof(p));
+  p.keys = keys;
+  p.B = B;
+  p.G = G;
+  p.N = N;
+  p.mode = kind == RBG_GEN_PRW ? PRW_MODE_STATE : PRW_MODE_UNIFORM;
+  p.extra_split = (kind == RBG_GEN_PRW ? 1 : 0) + extra_split;
+  p.debug = debug_flags();
+  if (cache_ws) {
+    const WsLayout wl = ws_layout(B, N);
+    p.to_cache = 1;
+    p.cache_tag = reinterpret_cast<unsigned long long *>(cache_ws + wl.cache_tag);
+    p.cache_key = reinterpret_cast<uint2 *>(cache_ws + wl.cache_key);
+    p.cache_pins = reinterpret_cast<uint32_t *>(cache_ws + wl.cache_pins);
+  }
+  return p;
 }
 
 static int generator_state_impl(int kind, const uint32_t *keys, int64_t B, int G, int N, const rbg_state *out,
                                 const rbg_timestep *ts, int extra_split, const int32_t *list,
                                 const int32_t *list_count, cudaStream_t stream, int32_t *list_ticket = nullptr) {
   if (kind == RBG_GEN_PRW || kind == RBG_GEN_UNIFORM) {
-    PrwParams p;
-    memset(&p, 0, sizeof(p));
-    p.keys = keys;
-    p.B = B;
-    p.G = G;
-    p.N = N;
-    p.mode = kind == RBG_GEN_PRW ? PRW_MODE_STATE : PRW_MODE_UNIFORM;
-    // PRWG:52 key, pos_key = split(key): the board uses split(key)[0].
-    // UG:76 the uniform generator consumes the split itself (both halves).
-    p.extra_split = (kind == RBG_GEN_PRW ? 1 : 0) + extra_split;
-    p.debug = debug_flags();
+    PrwParams p = prw_params(kind, keys, B, G, N, extra_split);
     p.st = *out;
     if (ts) {
       p.ts = *ts;
@@ -166,7 +213,7 @@ static int generator_state_impl(int kind, const uint32_t *keys, int64_t B, int G
     p.list = list;
     p.list_count = list_count;
     p.list_ticket = list_ticket;
-    return launch_prw(p, B, env_int("RBG_PRW_M"), env_int("RBG_PRW_THREADS"), stream);
+    return launch_prw(p, B, stream);
   }
   if (kind == RBG_GEN_SEEDEXT) {
     SeedExtParams p;
@@ -209,44 +256,6 @@ static int generator_state_impl(int kind, const uint32_t *keys, int64_t B, int G
     return launch_seqrw(p, B, stream);
   }
   return set_error(RBG_EINVAL, "unknown generator kind %d", kind);
-}
-
-// ---- auto-reset workspace ------------------------------------------------------
-// VmapAutoResetWrapper regenerates a board whenever an env finishes.  The reset key
-// of an episode is known as soon as the episode starts (split(state.key)[0]), so the
-// NEXT episode of every env that just reset is generated ahead of time ("refill")
-// into a per-env cache; when the env finishes, env_kernel swaps the
-// cached episode in.  Only envs whose cache entry is not ready (first episode, or two
-// terminations in consecutive steps) take the synchronous reset kernel.  Results are
-// identical either way: a board is a pure function of its key.
-struct WsLayout {
-  size_t sync_list, refill_list[2], refill_keys[2], cache_tag, cache_key, cache_pins, group_done, group_pending, total;
-};
-static WsLayout ws_layout(int64_t B, int N) {
-  auto up = [](size_t x) { return (x + 255) & ~(size_t)255; };
-  WsLayout w;
-  size_t off = 512;  // counters: sync @0, refill[0] @64, refill[1] @128; persistent rollout: 16 sets of 4 ints @256
-  const size_t b = (size_t)(B > 0 ? B : 0);
-  w.sync_list = off;
-  off = up(off + 4 * b);
-  for (int i = 0; i < 2; ++i) {
-    w.refill_list[i] = off;
-    off = up(off + 4 * b);
-    w.refill_keys[i] = off;
-    off = up(off + 8 * b);
-  }
-  w.cache_tag = off;
-  off = up(off + 8 * b);
-  w.cache_key = off;
-  off = up(off + 8 * b);
-  w.cache_pins = off;
-  off = up(off + 4 * b * (size_t)N);
-  w.group_done = off;  // persistent rollout: per env group, the last launch that wrote it / its requests in flight
-  off = up(off + 4 * b);
-  w.group_pending = off;
-  off = up(off + 4 * b);
-  w.total = off;
-  return w;
 }
 
 struct AutoResetCtx {
@@ -339,20 +348,7 @@ static int connector_step_impl(const rbg_state *in, const rbg_state *out, const 
       // warm start: the next episode of EVERY env, one bulk generation keyed by the
       // current State.key (a cold cache would send each env's first reset down the
       // synchronous path)
-      PrwParams q;
-      memset(&q, 0, sizeof(q));
-      q.keys = in->key;
-      q.B = B;
-      q.G = G;
-      q.N = N;
-      q.mode = kind == RBG_GEN_PRW ? PRW_MODE_STATE : PRW_MODE_UNIFORM;
-      q.extra_split = (kind == RBG_GEN_PRW ? 1 : 0) + 1;
-      q.debug = debug_flags();
-      q.to_cache = 1;
-      q.cache_tag = reinterpret_cast<unsigned long long *>(ws + wl.cache_tag);
-      q.cache_key = reinterpret_cast<uint2 *>(ws + wl.cache_key);
-      q.cache_pins = reinterpret_cast<uint32_t *>(ws + wl.cache_pins);
-      if ((rc = launch_prw(q, B, env_int("RBG_PRW_M"), env_int("RBG_PRW_THREADS"), stream))) return rc;
+      if ((rc = launch_prw(prw_params(kind, in->key, B, G, N, 1, ws), B, stream))) return rc;
       ctx->B = B;
       ctx->G = G;
       ctx->N = N;
@@ -384,62 +380,31 @@ static int connector_step_impl(const rbg_state *in, const rbg_state *out, const 
   // one more leading split()[0] than a plain generator call.
   if (chained) {
     // one launch: the synchronous resets (rare misses), launch_dependents, then the cache refill
-    PrwParams a, q;
-    memset(&a, 0, sizeof(a));
-    a.keys = out->key;
-    a.B = B;
-    a.G = G;
-    a.N = N;
-    a.mode = kind == RBG_GEN_PRW ? PRW_MODE_STATE : PRW_MODE_UNIFORM;
-    a.extra_split = (kind == RBG_GEN_PRW ? 1 : 0) + 1;
-    a.debug = debug_flags();
+    PrwParams a = prw_params(kind, out->key, B, G, N, 1);
     a.st = *out;
     a.ts = *ts;
     a.observe = 1;
     a.list = sync_list;
     a.list_count = sync_count;
     a.list_ticket = sync_count + 1;
-    memset(&q, 0, sizeof(q));
-    q.keys = p.refill_keys;
+    PrwParams q = prw_params(kind, p.refill_keys, B, G, N, 1, ws);
     q.keys_compact = 1;
-    q.B = B;
-    q.G = G;
-    q.N = N;
-    q.mode = a.mode;
-    q.extra_split = a.extra_split;
-    q.debug = a.debug;
     q.list = p.refill_list;
     q.list_count = p.refill_count;
     q.list_ticket = p.refill_count + 1;
-    q.to_cache = 1;
-    q.cache_tag = reinterpret_cast<unsigned long long *>(ws + wl.cache_tag);
-    q.cache_key = reinterpret_cast<uint2 *>(ws + wl.cache_key);
-    q.cache_pins = reinterpret_cast<uint32_t *>(ws + wl.cache_pins);
     if ((rc = launch_prw_pair(a, q, B, stream))) return rc;
     ctx->step++;
     return RBG_OK;
   }
   if ((rc = generator_state_impl(kind, out->key, B, G, N, out, ts, 1, sync_list, sync_count, stream, speculative ? sync_count + 1 : nullptr))) return rc;
   if (speculative) {
-    PrwParams q;
-    memset(&q, 0, sizeof(q));
-    q.keys = p.refill_keys;
+    PrwParams q = prw_params(kind, p.refill_keys, B, G, N, 1, ws);  // as the auto-reset call above
     q.keys_compact = 1;
-    q.B = B;
-    q.G = G;
-    q.N = N;
-    q.mode = kind == RBG_GEN_PRW ? PRW_MODE_STATE : PRW_MODE_UNIFORM;
-    q.extra_split = (kind == RBG_GEN_PRW ? 1 : 0) + 1;  // as the auto-reset call above
-    q.debug = debug_flags();
     q.list = p.refill_list;
     q.list_count = p.refill_count;
     q.list_ticket = p.refill_count + 1;
-    q.to_cache = 1;
-    q.cache_tag = reinterpret_cast<unsigned long long *>(ws + wl.cache_tag);
-    q.cache_key = reinterpret_cast<uint2 *>(ws + wl.cache_key);
-    q.cache_pins = reinterpret_cast<uint32_t *>(ws + wl.cache_pins);
     q.trigger_dependents = 1;
-    if ((rc = launch_prw(q, B, env_int("RBG_PRW_M"), env_int("RBG_PRW_THREADS"), stream))) return rc;
+    if ((rc = launch_prw(q, B, stream))) return rc;
     ctx->step++;
   }
   return RBG_OK;
@@ -713,7 +678,7 @@ int rbg_prw_generate(const uint32_t *keys, int64_t B, int G, int N, int32_t *hea
   p.targets = targets;
   p.solved = solved;
   p.stats = stats;
-  return launch_prw(p, B, env_int("RBG_PRW_M"), env_int("RBG_PRW_THREADS"), (cudaStream_t)stream);
+  return launch_prw(p, B, (cudaStream_t)stream);
 }
 
 int rbg_generator_state(int kind, const uint32_t *keys, int64_t B, int G, int N, const rbg_state *out, void *stream) {
@@ -886,16 +851,8 @@ int rbg_connector_step_random(const rbg_state *in, const rbg_state *out, int32_t
   return connector_step_impl(in, out, nullptr, action_out, 1, B, G, N, params, ts, workspace, (cudaStream_t)stream);
 }
 
-// Steps per launch of the fused rollout kernels (RBG_ROLLOUT_CHUNK; default the reference's n_steps,
-// agent_training/configs/env/connector.yaml:27)
-static int rollout_chunk() {
-  static int v = -1;
-  if (v < 0) {
-    v = env_int("RBG_ROLLOUT_CHUNK");
-    if (v <= 0) v = 20;
-  }
-  return v;
-}
+// Steps per launch of the fused rollout kernels: the reference's n_steps (agent_training/configs/env/connector.yaml:27)
+constexpr int kRolloutChunk = 20;
 
 // Fused ParallelRandomWalk / Uniform rollout (rollout_persist_kernel): one launch per chunk of steps.  The kernel's
 // generator warps keep the next-episode cache filled; consecutive launches on the stream overlap head to tail.
@@ -914,20 +871,8 @@ static int rollout_fused(const rbg_state *state, int32_t *action_out, int64_t T,
   if ((rc = workspace_follow_stream(ctx, stream))) return rc;
   if (ctx->B != B || ctx->G != G || ctx->N != N || ctx->kind != kind) {
     if ((e = cudaMemsetAsync(ws, 0, 256, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(counters)");
-    PrwParams q;  // warm start: the next episode of every env
-    memset(&q, 0, sizeof(q));
-    q.keys = state->key;
-    q.B = B;
-    q.G = G;
-    q.N = N;
-    q.mode = kind == RBG_GEN_PRW ? PRW_MODE_STATE : PRW_MODE_UNIFORM;
-    q.extra_split = (kind == RBG_GEN_PRW ? 1 : 0) + 1;
-    q.debug = debug_flags();
-    q.to_cache = 1;
-    q.cache_tag = reinterpret_cast<unsigned long long *>(ws + wl.cache_tag);
-    q.cache_key = reinterpret_cast<uint2 *>(ws + wl.cache_key);
-    q.cache_pins = reinterpret_cast<uint32_t *>(ws + wl.cache_pins);
-    if ((rc = launch_prw(q, B, env_int("RBG_PRW_M"), env_int("RBG_PRW_THREADS"), stream))) return rc;
+    // warm start: the next episode of every env
+    if ((rc = launch_prw(prw_params(kind, state->key, B, G, N, 1, ws), B, stream))) return rc;
     ctx->B = B;
     ctx->G = G;
     ctx->N = N;
@@ -948,9 +893,8 @@ static int rollout_fused(const rbg_state *state, int32_t *action_out, int64_t T,
   p.cache_tag = reinterpret_cast<const unsigned long long *>(ws + wl.cache_tag);
   p.cache_key = reinterpret_cast<const uint2 *>(ws + wl.cache_key);
   p.cache_pins = reinterpret_cast<const uint32_t *>(ws + wl.cache_pins);
-  const int chunk = rollout_chunk();
-  for (int64_t t0 = 0; t0 < T; t0 += chunk) {
-    const int n = (int)((T - t0) < chunk ? (T - t0) : chunk);
+  for (int64_t t0 = 0; t0 < T; t0 += kRolloutChunk) {
+    const int n = (int)((T - t0) < kRolloutChunk ? (T - t0) : kRolloutChunk);
     p.ts = timestep_at(*ts, t0 * B, G, N);
     if (ctx->persist_epoch == 0 || ctx->persist_epoch > 0x3fffffff) {  // flags start at 0 = "written by launch 0"
       if ((e = cudaMemsetAsync(ws + wl.group_done, 0, (wl.group_pending - wl.group_done) + 4 * (size_t)B, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(group flags)");
@@ -995,9 +939,8 @@ int rbg_connector_rollout_random(const rbg_state *state, int32_t *action_out, in
     p.mode = ENV_MODE_STEP;
     p.random_policy = 1;
     p.env = *params;
-    const int chunk = rollout_chunk();
-    for (int64_t t0 = 0; t0 < T; t0 += chunk) {
-      const int n = (int)((T - t0) < chunk ? (T - t0) : chunk);
+    for (int64_t t0 = 0; t0 < T; t0 += kRolloutChunk) {
+      const int n = (int)((T - t0) < kRolloutChunk ? (T - t0) : kRolloutChunk);
       p.ts = timestep_at(*ts, t0 * B, G, N);
       if ((rc = launch_rollout(p, n, action_out ? action_out + t0 * B * N : nullptr, (cudaStream_t)stream))) return rc;
     }

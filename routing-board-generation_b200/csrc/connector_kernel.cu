@@ -15,8 +15,6 @@
 // kernel reads the State once (int32 -> uint8 into shared memory) and writes State +
 // observation [N,G,G] int32 exactly once; the fused rollout kernel keeps the State on
 // chip for a whole chunk of steps.  All bulk traffic is 128-bit coalesced.
-#include <stdlib.h>
-
 #include "connector_device.cuh"
 #include "gen_warp.cuh"
 #include "obs_stage.cuh"
@@ -62,12 +60,10 @@ __device__ __forceinline__ int random_action(uint32_t k0, uint32_t k1,
 // kernel spent half of its warp-time at __syncthreads waiting for the agent phases;
 // it is in the history, profiles/r01a_env_full.csv is its ncu capture).
 constexpr int EW_WARPS = 4;
-#ifndef RBG_ENV_MIN_CTAS
-#define RBG_ENV_MIN_CTAS 12
-#endif
+constexpr int kEnvMinCtas = 12;
 
 template <bool VEC>
-__global__ void __launch_bounds__(EW_WARPS * 32, RBG_ENV_MIN_CTAS) env_warp_kernel(const EnvParams p) {
+__global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) env_warp_kernel(const EnvParams p) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int G = p.G, N = p.N, cells = p.cells;
@@ -360,12 +356,10 @@ struct RolloutParams {
   int ce, cv;            // a staged chunk = ce whole envs (cv == N) or cv views of one env (ce == 1)
 };
 
-#ifndef RBG_ROLLOUT_MIN_CTAS
-#define RBG_ROLLOUT_MIN_CTAS 6
-#endif
+constexpr int kRolloutMinCtas = 6;
 // OBS: 0 scalar stores (cells % 4 != 0), 1 direct 128-bit stores, 2 staged + bulk copies (obs_stage.cuh)
 template <int OBS>
-__global__ void __launch_bounds__(EW_WARPS * 32, RBG_ROLLOUT_MIN_CTAS) rollout_warp_kernel(const EnvParams p, const RolloutParams rp) {
+__global__ void __launch_bounds__(EW_WARPS * 32, kRolloutMinCtas) rollout_warp_kernel(const EnvParams p, const RolloutParams rp) {
   constexpr bool VEC = OBS != 0;
   extern __shared__ __align__(16) uint8_t smem_raw[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -604,9 +598,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, RBG_ROLLOUT_MIN_CTAS) rollout_w
 //    however many small launches are in flight at once they never share a counter.
 constexpr int kPersistSets = 16;
 constexpr int kPersistSetInts = 4;
-#ifndef RBG_PERSIST_MIN_CTAS
-#define RBG_PERSIST_MIN_CTAS 4
-#endif
+constexpr int kPersistMinCtas = 4;
 
 struct PersistParams {
   int *counter;   // [0] next env group, [1] env warps that have finished (the last one clears both), [2] epoch that may use the set next (0: any of the first kPersistSets)
@@ -622,7 +614,7 @@ struct PersistParams {
 };
 
 template <int OBS>
-__global__ void __launch_bounds__((EW_WARPS + 2) * 32, RBG_PERSIST_MIN_CTAS)
+__global__ void __launch_bounds__((EW_WARPS + 2) * 32, kPersistMinCtas)
     rollout_persist_kernel(const EnvParams p, const RolloutParams rp, const PersistParams pp, const GenWarpCfg gc) {
   constexpr bool VEC = OBS != 0;
   extern __shared__ __align__(16) uint8_t smem_raw[];
@@ -652,39 +644,17 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, RBG_PERSIST_MIN_CTAS)
   if (warp >= pp.env_warps) {  // ---- generator warp
     const int gw = warp - pp.env_warps;
     if (gw >= pp.gen_warps) return;
-#ifdef RBG_PERSIST_STATS
-    if (lane == 0) {
-      RBG_STAT(8, 1);  // generator warps
-    }
-#endif
     uint8_t *gb = smem_raw + pp.gscr_off + (size_t)gw * pp.gscr_stride;
     GenWarpScratch gs;
     gs.cand = reinterpret_cast<uint64_t *>(gb);
     gs.sel = reinterpret_cast<uint16_t *>(gb + pp.gcand_bytes);
     gs.board = gb + pp.gcand_bytes + pp.gsel_bytes;
     gs.tmpl = tmpl;
-#ifdef RBG_PERSIST_TRACE
-    const unsigned long long tr0 = rbg_gtime();
-#endif
     gen_warp_loop(gc, gs, queues + gw, env_done, pp.env_warps, lane);
-#ifdef RBG_PERSIST_TRACE
-    if (lane == 0) {
-      const int wi = blockIdx.x * (EW_WARPS + 2) + warp;
-      g_persist_trace[3 * wi] = tr0;
-      g_persist_trace[3 * wi + 1] = rbg_gtime();
-      g_persist_trace[3 * wi + 2] = 1000000;
-    }
-#endif
     return;
   }
 
   // ---- env warp
-#ifdef RBG_PERSIST_STATS
-  if (lane == 0) {
-    RBG_STAT(12, 1);  // env warps
-    RBG_STAT(13, clock64());  // (start stamps; the exit stamps are added below: sum(exit) - sum(start) = total env-warp time)
-  }
-#endif
   uint8_t *wg = smem_raw + p.so[0] + (size_t)warp * p.so[1];
   uint32_t *wg32 = reinterpret_cast<uint32_t *>(wg);
   const int j = lane / Np, a = lane & (Np - 1);
@@ -693,10 +663,6 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, RBG_PERSIST_MIN_CTAS)
   const SmemGrid sg{g, G, 0, G};
   ObsStager os;
   if (VEC) os.init(smem_raw + rp.stage_off + (size_t)warp * rp.stage_warp, lut, wg32, N, c4, p.divC4, lane, rp.stage_bytes, rp.stage_nbuf, rp.ce, rp.cv);
-#ifdef RBG_PERSIST_TRACE
-  const unsigned long long tr0 = rbg_gtime();
-  int tr_groups = 0;
-#endif
 
   if (lane == 0) {  // the launch that used this counter set last (kPersistSets launches ago) must have recycled it
     for (;;) {
@@ -711,9 +677,6 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, RBG_PERSIST_MIN_CTAS)
     if (lane == 0) grp = atomicAdd(pp.counter, 1);
     grp = __shfl_sync(FULL, grp, 0);
     if (grp >= pp.ngroups) break;
-#ifdef RBG_PERSIST_TRACE
-    ++tr_groups;
-#endif
     const long long e0 = (long long)grp * K;
     const int kc = (int)((p.B - e0) < (long long)K ? (p.B - e0) : (long long)K);
     const bool env_ok = j < kc, agent = env_ok && a < N;
@@ -794,12 +757,8 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, RBG_PERSIST_MIN_CTAS)
         if (action != NOOP) dest = r * G + c + (action == UP ? -G : (action == DOWN ? G : (action == RIGHT ? 1 : -1)));
       }
       const uint32_t mval = dest >= 0 ? (((uint32_t)j << 16) | (uint32_t)dest) : (0x80000000u | (uint32_t)lane);
-#ifdef RBG_ENV_SHFL_COLLISION
-      const bool win = wins_collision(mval, dest >= 0, a, j * Np, N);
-#else
       const uint32_t mm = __match_any_sync(FULL, mval);
       const bool win = dest >= 0 && lane == 31 - __clz(mm);
-#endif
       __syncwarp();
       if (win) {
         g[r * G + c] = (uint8_t)(3 * a + PATH);
@@ -835,12 +794,10 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, RBG_PERSIST_MIN_CTAS)
       }
       // ---- auto-reset: the env's cached next episode; its generator warp may still be working on it
       if (terminal) {  // group-uniform
-        if (a == 0) RBG_STAT(7, 1);  // resets
         const unsigned long long want = ((unsigned long long)k1 << 32) | k0;
         if (a == 0)
           while (ld_acquire_u64(p.cache_tag + e) != want) {
             myq->urgent = 1;
-            RBG_STAT(6, 1);  // env-warp wait polls (0.1 us)
             __nanosleep(100);
           }
         __syncwarp(gmask);
@@ -915,17 +872,6 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, RBG_PERSIST_MIN_CTAS)
     if (lane == 0) st_release_s32(pp.group_done + grp, pp.epoch);
   }
   if (OBS == 2) os.drain(lane);  // shared memory must outlive the bulk copies
-#ifdef RBG_PERSIST_STATS
-  if (lane == 0) RBG_STAT(14, clock64());
-#endif
-#ifdef RBG_PERSIST_TRACE
-  if (lane == 0) {
-    const int wi = blockIdx.x * (EW_WARPS + 2) + warp;
-    g_persist_trace[3 * wi] = tr0;
-    g_persist_trace[3 * wi + 1] = rbg_gtime();
-    g_persist_trace[3 * wi + 2] = tr_groups;
-  }
-#endif
   // this env warp is done: tell the CTA's generator warps, and the grid (the last warp recycles the counters)
   __syncwarp();
   if (lane == 0) {
@@ -1061,26 +1007,13 @@ int launch_rollout(EnvParams p, int T, int32_t *action_out, cudaStream_t stream)
   }
   if (smem > 200 * 1024) return set_error(RBG_EINVAL, "rollout: shared memory %zu too large", smem);
   const int64_t ctas = (p.B + p.E - 1) / p.E;
-  {  // residency: registers allow RBG_ROLLOUT_MIN_CTAS per SM, shared memory (1 KB reserved per CTA) maybe fewer
+  {  // residency: registers allow kRolloutMinCtas per SM, shared memory (1 KB reserved per CTA) maybe fewer
     int cmax = (int)(device_smem_per_sm() / (smem + 1024));
-    if (cmax > RBG_ROLLOUT_MIN_CTAS) cmax = RBG_ROLLOUT_MIN_CTAS;
-    static int force = -1;  // RBG_ROLLOUT_CTAS=n: n CTAs per SM instead of the wave-balanced choice (experiments)
-    if (force < 0) {
-      const char *ex = getenv("RBG_ROLLOUT_CTAS");
-      force = ex ? atoi(ex) : 0;
-    }
-    if (force > 0) {
-      const size_t pad = device_smem_per_sm() / (size_t)(force + 1) + 1024;
-      if (force < cmax && pad > smem) smem = pad;
-    } else if (cmax >= 3)
-      smem = balance_waves(ctas, cmax, cmax - 2, smem);
+    if (cmax > kRolloutMinCtas) cmax = kRolloutMinCtas;
+    if (cmax >= 3) smem = balance_waves(ctas, cmax, cmax - 2, smem);
   }
   LaunchScope scope(RBG_K_ROLLOUT, stream);
-#ifdef RBG_OBS_DIRECT
-  const bool staged = false;  // A/B build: never stage
-#else
   const bool staged = vec && rp.stage_nbuf != 0;
-#endif
   if (staged) {
     if (smem > 48 * 1024) cudaFuncSetAttribute(rollout_warp_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     rollout_warp_kernel<2><<<(unsigned)ctas, EW_WARPS * 32, smem, stream>>>(p, rp);
@@ -1120,53 +1053,17 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   memset(&rp, 0, sizeof(rp));
   rp.T = T;
   rp.action_out = action_out;
-  static int env_warps_env = -1;  // RBG_PERSIST_ENV_WARPS=n: n env warps per CTA (experiments; default EW_WARPS)
-  if (env_warps_env < 0) {
-    const char *ex = getenv("RBG_PERSIST_ENV_WARPS");
-    env_warps_env = ex ? atoi(ex) : 0;
-  }
   // CTA shape.  "Isolated": 3 env warps + 1 generator warp = 4 warps per CTA, one per SM sub-partition, so the generator
   // warps of all resident CTAs share ONE sub-partition and never compete with env warps for issue slots, at most 4 CTAs
   // per SM.  "Packed": 4 env + 2 generator warps, as many CTAs as fit.  Measured (65 536 envs, M env-steps/s, isolated /
   // packed): 10x10/5 2501 / 2338, 12x12/6 1649 / 1508, 10x10/4 2884 / 2850, 10x10/8 1598 / 1596; 8x8/4 2817 / 3432,
   // 8x8/8 1477 / 1687, 6x6/3 2623 / 2989 (issue-bound: more env warps win); 14x14/7 1013 / 1034, 16x16/8 761 / 774,
   // 20x20/10 372 / 378, 32x32/16 94.9 / 96.8 (resets are rare per byte: packed is 2 % ahead).
-  const bool isolated = env_warps_env > 0 ? env_warps_env == 3 : (G >= 9 && G <= 13 && N <= 8);
-  const int PW = env_warps_env >= 1 && env_warps_env <= EW_WARPS ? env_warps_env : (isolated ? 3 : EW_WARPS);
+  const bool isolated = G >= 9 && G <= 13 && N <= 8;
+  const int PW = isolated ? 3 : EW_WARPS;
   size_t off = lutB + PW * wgrid;
   rp.ratio_off = (int)off;
   off = up16(off + 4 * (RBG_MAX_N + 4));
-  // generator configuration: W lanes per board, N + 2 of them busy when that fits (agents + the two key-advance lanes)
-  GenWarpCfg gc;
-  memset(&gc, 0, sizeof(gc));
-  gc.kind = kind;
-  gc.G = G;
-  gc.N = N;
-  int W = 1;
-  while (W < N + 2 && W < 32) W <<= 1;
-  gc.W = W;
-  gc.S = G + 4;
-  gc.SBp = (int)up16((size_t)gc.S * gc.S);
-  gc.cells = p.cells;
-  gc.nsel = kind == RBG_GEN_PRW ? N : 2 * N;
-  gc.nselp = (gc.nsel + 1) & ~1;
-  gc.cap = 4 * gc.nsel + 32;
-  {
-    const double frac = (2.0 * gc.nsel + 16.0) / (double)p.cells;
-    gc.thresh = frac >= 1.0 ? 0xffffffffu : (uint32_t)(frac * 4294967296.0);
-  }
-  gc.divG = p.divG;
-  {
-    static int patience_env = -2;
-    if (patience_env == -2) {
-      const char *ex = getenv("RBG_GEN_PATIENCE");
-      patience_env = ex ? atoi(ex) : -1;
-    }
-    gc.patience = patience_env >= 0 ? patience_env : 20;
-  }
-  gc.cache_tag = reinterpret_cast<unsigned long long *>(cache_tag_w);
-  gc.cache_key = cache_key_w;
-  gc.cache_pins = cache_pins_w;
   PersistParams pp;
   memset(&pp, 0, sizeof(pp));
   pp.counter = counter + (epoch % kPersistSets) * kPersistSetInts;
@@ -1174,16 +1071,16 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   pp.group_pending = group_pending;
   pp.epoch = epoch;
   pp.ngroups = (int)((p.B + K - 1) / K);
+  GenWarpCfg gc = gen_warp_cfg(kind, G, N, &pp.gcand_bytes, &pp.gsel_bytes, &pp.gscr_stride);
+  gc.patience = 20;
+  gc.cache_tag = reinterpret_cast<unsigned long long *>(cache_tag_w);
+  gc.cache_key = cache_key_w;
+  gc.cache_pins = cache_pins_w;
   gc.group_pending = group_pending;
   gc.seqlock = 0;  // nobody reads an entry while it is rewritten here (see gen_warp_batch)
   gc.kshift = 0;
   while ((1 << gc.kshift) < K) ++gc.kshift;
-  static int gen_warps_env = -1;
-  if (gen_warps_env < 0) {
-    const char *ex = getenv("RBG_GEN_WARPS");
-    gen_warps_env = ex ? atoi(ex) : 0;
-  }
-  pp.gen_warps = gen_warps_env > 0 ? (gen_warps_env > 2 ? 2 : gen_warps_env) : (isolated ? 1 : 2);
+  pp.gen_warps = isolated ? 1 : 2;
   pp.env_warps = PW;
   pp.tmpl_off = (int)off;
   off = up16(off + gc.SBp);
@@ -1191,10 +1088,6 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   off = up16(off + pp.gen_warps * sizeof(GenQueue));
   pp.done_off = (int)off;
   off += 16;
-  const int gpw = 32 / W;
-  pp.gcand_bytes = (int)up16((size_t)gc.cap * 8);
-  pp.gsel_bytes = (int)up16((size_t)gpw * gc.nselp * 2);
-  pp.gscr_stride = (int)up16((size_t)pp.gcand_bytes + pp.gsel_bytes + (size_t)gpw * gc.SBp);
   pp.gscr_off = (int)off;
   off += (size_t)pp.gen_warps * pp.gscr_stride;
   rp.stage_off = (int)off;
@@ -1212,11 +1105,7 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   }
   const size_t smem = up16(off);
   if (smem > 200 * 1024) return set_error(RBG_EINVAL, "rollout: shared memory %zu too large", smem);
-#ifdef RBG_OBS_DIRECT
-  const bool staged = false;
-#else
   const bool staged = vec && rp.stage_nbuf != 0;
-#endif
   const int threads = (PW + pp.gen_warps) * 32;
   const void *fn = staged ? (const void *)rollout_persist_kernel<2> : (vec ? (const void *)rollout_persist_kernel<1> : (const void *)rollout_persist_kernel<0>);
   cudaError_t ce;
@@ -1225,13 +1114,7 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   int resident = 0;
   if ((ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, fn, threads, smem)) != cudaSuccess) return set_cuda_error(ce, "cudaOccupancyMaxActiveBlocksPerMultiprocessor");
   if (resident < 1) return set_error(RBG_EINVAL, "rollout_persist_kernel does not fit an SM (%zu bytes of shared memory)", smem);
-  static int force = -1;  // RBG_ROLLOUT_CTAS=n: at most n CTAs per SM (experiments)
-  if (force < 0) {
-    const char *ex = getenv("RBG_ROLLOUT_CTAS");
-    force = ex ? atoi(ex) : 0;
-  }
-  if (force > 0 && force < resident) resident = force;
-  if (force <= 0 && isolated && resident > 4) resident = 4;  // more resident CTAs measure slower (5: +0.6 %, 6-8: +1.1 %)
+  if (isolated && resident > 4) resident = 4;  // more resident CTAs measure slower (5: +0.6 %, 6-8: +1.1 %)
   int64_t ctas = (int64_t)resident * device_sm_count();
   const int64_t need = (pp.ngroups + PW - 1) / PW;
   if (ctas > need) ctas = need;
@@ -1258,26 +1141,6 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   if (ce != cudaSuccess) return set_cuda_error(ce, "cudaLaunchKernelEx(rollout_persist_kernel)");
   return check_launch("rollout_persist_kernel");
 }
-
-#ifdef RBG_PERSIST_TRACE
-extern "C" int rbg_debug_persist_trace(unsigned long long *out, int n) {
-  cudaDeviceSynchronize();
-  cudaMemcpyFromSymbol(out, g_persist_trace, sizeof(unsigned long long) * n);
-  return 0;
-}
-#endif
-
-#ifdef RBG_PERSIST_STATS
-extern "C" int rbg_debug_persist_stats(unsigned long long *out16, int reset) {
-  cudaDeviceSynchronize();
-  cudaMemcpyFromSymbol(out16, g_persist_stats, sizeof(unsigned long long) * 16);
-  if (reset) {
-    unsigned long long z[16] = {0};
-    cudaMemcpyToSymbol(g_persist_stats, z, sizeof(z));
-  }
-  return 0;
-}
-#endif
 
 int launch_random_actions(const rbg_state &st, int64_t B, int G, int N, int32_t *action, cudaStream_t stream) {
   const int64_t n = B * N;

@@ -15,29 +15,14 @@
 // `key, _ = split(state.key)` first).
 #pragma once
 
+#include <string.h>
+
 #include "rbg_device.cuh"
 #include "select.cuh"
 
 namespace rbg {
 
 constexpr int GENQ_CAP = 64;  // requests in flight per queue (power of two)
-
-// -DRBG_PERSIST_STATS: counters of the generator warps / env-warp waits (tools/persist_stats.py reads them)
-// -DRBG_PERSIST_TRACE: per-warp globaltimer stamps (start, end, groups done) without atomics
-#ifdef RBG_PERSIST_TRACE
-__device__ unsigned long long g_persist_trace[3 * 8192];
-__device__ __forceinline__ unsigned long long rbg_gtime() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-#endif
-#ifdef RBG_PERSIST_STATS
-__device__ unsigned long long g_persist_stats[16];
-#define RBG_STAT(i, v) atomicAdd(&g_persist_stats[i], (unsigned long long)(v))
-#else
-#define RBG_STAT(i, v)
-#endif
 
 // multi-producer (one lane per finished env), single-consumer (one generator warp) ring
 struct GenQueue {
@@ -87,6 +72,37 @@ struct GenWarpCfg {
   int seqlock;         // readers may be running (per-step path): invalidate the entry's tag before rewriting it
   int kshift;          // log2(envs per group)
 };
+
+// The fields of a GenWarpCfg that follow from the board shape, and the bytes of one generator warp's GenWarpScratch
+// arrays in shared memory (cand, sel; the whole stride includes the boards).  The caller sets the cache pointers,
+// group_pending, kshift, seqlock and patience.
+inline GenWarpCfg gen_warp_cfg(int kind, int G, int N, int *gcand_bytes, int *gsel_bytes, int *gscr_stride) {
+  auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
+  GenWarpCfg gc;
+  memset(&gc, 0, sizeof(gc));
+  gc.kind = kind;
+  gc.G = G;
+  gc.N = N;
+  int W = 1;  // W lanes per board, N + 2 of them busy when that fits (agents + the two key-advance lanes)
+  while (W < N + 2 && W < 32) W <<= 1;
+  gc.W = W;
+  gc.S = G + 4;
+  gc.SBp = (int)up16((size_t)gc.S * gc.S);
+  gc.cells = G * G;
+  gc.nsel = kind == RBG_GEN_PRW ? N : 2 * N;
+  gc.nselp = (gc.nsel + 1) & ~1;
+  gc.cap = 4 * gc.nsel + 32;
+  {
+    const double frac = (2.0 * gc.nsel + 16.0) / (double)gc.cells;
+    gc.thresh = frac >= 1.0 ? 0xffffffffu : (uint32_t)(frac * 4294967296.0);
+  }
+  gc.divG = FastDiv::make((uint32_t)G);
+  const int gpw = 32 / W;
+  *gcand_bytes = (int)up16((size_t)gc.cap * 8);
+  *gsel_bytes = (int)up16((size_t)gpw * gc.nselp * 2);
+  *gscr_stride = (int)up16((size_t)*gcand_bytes + *gsel_bytes + (size_t)gpw * gc.SBp);
+  return gc;
+}
 
 struct GenWarpScratch {
   uint64_t *cand;        // [cap]
@@ -278,22 +294,12 @@ __device__ inline void gen_warp_loop(const GenWarpCfg &c, const GenWarpScratch &
   const int gpw = 32 / c.W;
   unsigned h = 0;
   int waited = 0;
-#ifdef RBG_PERSIST_STATS
-  long long t_done = 0;
-#endif
   for (;;) {
     const bool done = __shfl_sync(FULL, *env_warps_done, 0) >= n_env_warps;  // read BEFORE scanning: a request posted before `done` is then visible
-#ifdef RBG_PERSIST_STATS
-    if (done && t_done == 0) t_done = clock64();
-#endif
     int n = 0;
     while (n < gpw && q->seq[(h + n) & (GENQ_CAP - 1)] == h + n + 1u) ++n;
     if (n == 0) {
-#ifdef RBG_PERSIST_STATS
-      if (done && lane == 0) RBG_STAT(9, clock64() - t_done);  // cycles a generator warp ran on after its env warps had finished
-#endif
       if (done) break;
-      if (lane == 0) RBG_STAT(4, 1);  // idle polls (0.2 us)
       __nanosleep(200);
       continue;
     }
@@ -304,12 +310,6 @@ __device__ inline void gen_warp_loop(const GenWarpCfg &c, const GenWarpScratch &
       __nanosleep(500);
       ++waited;
       continue;
-    }
-    if (lane == 0) {
-      RBG_STAT(0, 1);          // batches
-      RBG_STAT(1, n);          // boards
-      RBG_STAT(2, waited);     // polls spent holding partial batches back
-      RBG_STAT(3, q->urgent);  // batches started because an env was blocked
     }
     waited = 0;
     q->urgent = 0;
@@ -324,13 +324,7 @@ __device__ inline void gen_warp_loop(const GenWarpCfg &c, const GenWarpScratch &
     __syncwarp();
     h += n;
     if (lane == 0) q->head = h;  // the slots may be reused
-#ifdef RBG_PERSIST_STATS
-    const long long t0 = clock64();
-#endif
     gen_warp_batch(c, s, n, re, rk0, rk1, lane);
-#ifdef RBG_PERSIST_STATS
-    if (lane == 0) RBG_STAT(5, clock64() - t0);  // cycles inside batches
-#endif
   }
 }
 

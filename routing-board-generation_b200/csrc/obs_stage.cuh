@@ -117,20 +117,8 @@ __device__ __forceinline__ void stage_views_fixed(uint32_t lut_s, uint32_t w, ui
 
 // Bulk asynchronous copy shared -> global (the TMA unit moves the bytes, the LSU queue does not
 // see them).  Issued by one lane; the buffer may be rewritten once its group has been READ.
-// -DRBG_BULK_L2_HINT=1 / 2: L2 eviction priority evict_first / no_allocate-like (evict_first, fraction 1.0 vs unchanged):
-// the observation is written once and read by somebody else much later.
 __device__ __forceinline__ void bulk_store(void *gdst, uint32_t ssrc, uint32_t bytes) {
-#if defined(RBG_BULK_L2_HINT)
-  uint64_t pol;
-#if RBG_BULK_L2_HINT == 1
-  asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-#else
-  asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-#endif
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(gdst), "r"(ssrc), "r"(bytes), "l"(pol) : "memory");
-#else
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(ssrc), "r"(bytes) : "memory");
-#endif
   asm volatile("cp.async.bulk.commit_group;" ::: "memory");
 }
 template <int PENDING>

@@ -418,11 +418,7 @@ __device__ __forceinline__ void prw_body(const PrwParams &p, uint8_t *smem_raw) 
   }
 }
 
-#ifdef RBG_PRW_MIN_CTAS
-__global__ void __launch_bounds__(256, RBG_PRW_MIN_CTAS) prw_kernel(const PrwParams p) {
-#else
 __global__ void __launch_bounds__(256) prw_kernel(const PrwParams p) {
-#endif
   extern __shared__ __align__(16) uint8_t smem_raw[];
   if (p.trigger_dependents) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   prw_body(p, smem_raw);
@@ -488,7 +484,7 @@ __global__ void __launch_bounds__(64) prw_pair_kernel(const PrwParams a, const R
 
 // ---------------------------------------------------------------- host side
 // derived fields of PrwParams + launch shape
-static int prw_prepare(PrwParams &p, int64_t max_boards, int force_M, int force_threads, int *threads_out, size_t *smem_out, int64_t *ctas_out) {
+static int prw_prepare(PrwParams &p, int64_t max_boards, int *threads_out, size_t *smem_out, int64_t *ctas_out) {
   const int G = p.G, N = p.N;
   p.cells = G * G;
   p.S = G + 4;
@@ -516,8 +512,6 @@ static int prw_prepare(PrwParams &p, int64_t max_boards, int force_M, int force_
     threads = 64;
     M = 2 * gpw;
   }
-  if (force_threads > 0) threads = force_threads;
-  if (force_M > 0) M = force_M;
   // keep shared memory per CTA moderate so several CTAs share an SM
   for (;;) {
     p.M = M;
@@ -536,12 +530,11 @@ static int prw_prepare(PrwParams &p, int64_t max_boards, int force_M, int force_
   return RBG_OK;
 }
 
-int launch_prw(PrwParams p, int64_t max_boards, int force_M, int force_threads,
-               cudaStream_t stream) {
+int launch_prw(PrwParams p, int64_t max_boards, cudaStream_t stream) {
   int threads = 0, rc;
   size_t smem = 0;
   int64_t ctas = 0;
-  if ((rc = prw_prepare(p, max_boards, force_M, force_threads, &threads, &smem, &ctas))) return rc;
+  if ((rc = prw_prepare(p, max_boards, &threads, &smem, &ctas))) return rc;
   if (ctas <= 0) return RBG_OK;
   if (smem > 48 * 1024) {
     cudaError_t e = cudaFuncSetAttribute(prw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -559,44 +552,21 @@ int launch_prw_pair(PrwParams a, PrwParams b, int64_t max_boards, cudaStream_t s
   int ta = 0, rc;
   size_t sa = 0;
   int64_t ca = 0;
-  if ((rc = prw_prepare(a, max_boards, 0, 64, &ta, &sa, &ca))) return rc;
+  if ((rc = prw_prepare(a, max_boards, &ta, &sa, &ca))) return rc;
   if (ta != 64 || !a.list || !b.list || !b.to_cache || !b.keys_compact) return set_error(RBG_EINVAL, "prw_pair_kernel: a 64-thread list launch and a compact-key cache refill");
   auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
-  const int G = b.G, N = b.N, kind = b.mode == PRW_MODE_UNIFORM ? RBG_GEN_UNIFORM : RBG_GEN_PRW;
-  GenWarpCfg gc;
-  memset(&gc, 0, sizeof(gc));
-  gc.kind = kind;
-  gc.G = G;
-  gc.N = N;
-  int W = 1;
-  while (W < N + 2 && W < 32) W <<= 1;
-  gc.W = W;
-  gc.S = G + 4;
-  gc.SBp = (int)up16((size_t)gc.S * gc.S);
-  gc.cells = G * G;
-  gc.nsel = kind == RBG_GEN_PRW ? N : 2 * N;
-  gc.nselp = (gc.nsel + 1) & ~1;
-  gc.cap = 4 * gc.nsel + 32;
-  {
-    const double frac = (2.0 * gc.nsel + 16.0) / (double)gc.cells;
-    gc.thresh = frac >= 1.0 ? 0xffffffffu : (uint32_t)(frac * 4294967296.0);
-  }
-  gc.divG = FastDiv::make((uint32_t)G);
-  gc.cache_tag = b.cache_tag;
-  gc.cache_key = b.cache_key;
-  gc.cache_pins = b.cache_pins;
-  gc.group_pending = nullptr;
-  gc.seqlock = 1;  // the next env kernel runs under this refill
   RefillParams rf;
   memset(&rf, 0, sizeof(rf));
   rf.list = b.list;
   rf.keys = b.keys;
   rf.list_count = const_cast<int32_t *>(b.list_count);
   rf.list_ticket = b.list_ticket;
-  const int gpw = 32 / W;
-  rf.gcand_bytes = (int)up16((size_t)gc.cap * 8);
-  rf.gsel_bytes = (int)up16((size_t)gpw * gc.nselp * 2);
-  rf.gscr_stride = (int)up16((size_t)rf.gcand_bytes + rf.gsel_bytes + (size_t)gpw * gc.SBp);
+  GenWarpCfg gc = gen_warp_cfg(b.mode == PRW_MODE_UNIFORM ? RBG_GEN_UNIFORM : RBG_GEN_PRW, b.G, b.N, &rf.gcand_bytes, &rf.gsel_bytes, &rf.gscr_stride);
+  gc.cache_tag = b.cache_tag;
+  gc.cache_key = b.cache_key;
+  gc.cache_pins = b.cache_pins;
+  gc.seqlock = 1;  // the next env kernel runs under this refill
+  const int gpw = 32 / gc.W;
   rf.tmpl_off = 0;
   rf.gscr_off = (int)up16((size_t)gc.SBp);
   const size_t sb = (size_t)rf.gscr_off + 2 * (size_t)rf.gscr_stride;  // the refill reuses the shared memory of `a`

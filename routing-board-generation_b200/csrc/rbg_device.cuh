@@ -22,21 +22,11 @@ __device__ __forceinline__ uint32_t rotl(uint32_t x, int r) {
   return __funnelshift_l(x, x, r);
 }
 
-// Pipe balance experiment (kept behind -DRBG_TF_IMAD_ADD): on sm_100 IADD3 / SHF /
-// LOP3 all issue to the ALU pipe while IMAD goes to the FMA pipe, so multiplying by a 1
-// the compiler cannot see through turns the 30 additions of a block into IMADs and
-// splits the block 40 / 30 between the pipes.  MEASURED SLOWER on B200 (r01:
-// ParallelRandomWalk 10x10/5 267 M vs 283 M boards/s, SeedExtension 14x14/7 7.26 M vs
-// 7.68 M boards/s): these kernels are bound by the dependent-issue latency of the
-// add -> rotate -> xor chain, not by ALU-pipe throughput, and the cross-pipe RAW costs
-// one extra cycle per round.  Plain additions are the default.
-static __constant__ uint32_t c_rbg_one = 1u;
-
-#ifdef RBG_TF_IMAD_ADD
-#define RBG_TF_ADD(a, b) ((b) * one + (a))
-#else
+// Plain additions: moving them to the FMA pipe as IMADs measured slower on B200 (ParallelRandomWalk 10x10/5
+// 267 M vs 283 M boards/s, SeedExtension 14x14/7 7.26 M vs 7.68 M boards/s; DESIGN.md §7).  The
+// add -> rotate -> xor chain is bound by dependent-issue latency, not by ALU-pipe throughput, and a
+// cross-pipe dependency costs one extra cycle per round.
 #define RBG_TF_ADD(a, b) ((a) + (b))
-#endif
 
 #define RBG_TF_ROUND(r)    \
   x0 = RBG_TF_ADD(x0, x1); \
@@ -47,8 +37,6 @@ static __constant__ uint32_t c_rbg_one = 1u;
 __device__ __forceinline__ void tf_block(uint32_t k0, uint32_t k1, uint32_t x0,
                                          uint32_t x1, uint32_t &o0,
                                          uint32_t &o1) {
-  const uint32_t one = c_rbg_one;
-  (void)one;
   const uint32_t ks2 = k0 ^ k1 ^ 0x1BD11BDAu;
   x0 = RBG_TF_ADD(x0, k0);
   x1 = RBG_TF_ADD(x1, k1);

@@ -59,8 +59,7 @@ struct PrwParams {
   FastDiv divG;
 };
 
-int launch_prw(PrwParams p, int64_t max_boards, int force_M, int force_threads,
-               cudaStream_t stream);
+int launch_prw(PrwParams p, int64_t max_boards, cudaStream_t stream);
 // two short-list launches in one (prw_pair_kernel): `a` then launch_dependents then `b`
 int launch_prw_pair(PrwParams a, PrwParams b, int64_t max_boards, cudaStream_t stream);
 

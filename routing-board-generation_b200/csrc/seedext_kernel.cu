@@ -48,18 +48,6 @@
 
 namespace rbg {
 
-// -DRBG_SE_STATS: counters of the extend kernel (tools/se_stats.py reads them through rbg_debug_se_stats)
-#ifdef RBG_SE_STATS
-__device__ unsigned long long g_se_stats[16];
-#define SE_STAT(i, v)                                                          \
-  do {                                                                         \
-    const unsigned long long v_ = (unsigned long long)(v); /* may hold a ballot */ \
-    if ((threadIdx.x & 31) == 0) atomicAdd(&g_se_stats[i], v_);                \
-  } while (0)
-#else
-#define SE_STAT(i, v)
-#endif
-
 struct SeScratch {
   uint8_t *board;   // [B, CB]  row-major G*G codes, CB = cells rounded up to 16
   uint32_t *keys;   // [B, 4]   loop key (2), optkey of the current iteration (2)
@@ -201,12 +189,9 @@ __device__ __forceinline__ uint32_t warp_pick(uint32_t needm, bool need, const u
   const int my_slot = __popc(needm & ((1u << lane) - 1u));
   const uint32_t my_range = (per == 32 ? FULL : ((1u << per) - 1u)) << (my_slot * per);  // the lanes that draw for me
   bool pending = need;
-  SE_STAT(3, 1);
-  SE_STAT(5, n);
   for (int t0 = 0;; t0 += per) {
     const uint32_t pendm = __ballot_sync(FULL, pending && t0 < avail);
     if (!pendm) break;
-    SE_STAT(4, 1);
     const int t = t0 + j;
     uint32_t d = 0;
     bool hit = false;
@@ -222,7 +207,6 @@ __device__ __forceinline__ uint32_t warp_pick(uint32_t needm, bool need, const u
       pending = false;
     }
   }
-  SE_STAT(6, __popc(__ballot_sync(FULL, pending)));
   if (pending) {  // outran the parked keys: the chain goes on from the key behind them (draws avail, avail + 1, ...)
     const uint2 kk = __ldcg(ring + col + (size_t)ring_n * 32);
     uint32_t k0 = kk.x, k1 = kk.y;
@@ -309,7 +293,6 @@ __global__ void __launch_bounds__(256) se_extend_kernel(const SeedExtParams p, c
     const bool fin = m >= 0 && !(again && (p.ext_steps < 0 || step_num < p.ext_steps));
     const uint32_t finm = __ballot_sync(FULL, fin);
     if (finm) {
-      SE_STAT(10, 1);
       if (fin) {
         uint32_t *dst = reinterpret_cast<uint32_t *>(sc.board + (size_t)m * sc.CB);
         int r = 0, c = 0;
@@ -360,7 +343,6 @@ __global__ void __launch_bounds__(256) se_extend_kernel(const SeedExtParams p, c
       }
     }
     if (__any_sync(FULL, fresh)) {
-      SE_STAT(9, 1);
       if (fresh) {
         // key, extkey, optkey = split(key, 3)   SE:189
         uint32_t f[6];
@@ -406,8 +388,6 @@ __global__ void __launch_bounds__(256) se_extend_kernel(const SeedExtParams p, c
     }
     if (!__syncthreads_or(m >= 0)) break;  // no board in the CTA and none left in the queue
     const bool act = m >= 0 && again && (p.ext_steps < 0 || step_num < p.ext_steps);  // false only with extension_steps == 0
-    SE_STAT(0, 1);
-    SE_STAT(8, __popc(__ballot_sync(FULL, act)));
     bool flip = false, flop = false;
     if (act) {
       ++step_num;
@@ -491,8 +471,6 @@ __global__ void __launch_bounds__(256) se_extend_kernel(const SeedExtParams p, c
     for (;;) {
       while (act && emask == 0 && rowt < G - 1) emask = trav_mask(++rowt);
       const bool have = emask != 0;
-      SE_STAT(1, 1);
-      SE_STAT(2, __popc(__ballot_sync(FULL, have)));
       if (!__any_sync(FULL, have)) break;
       const int colt = have ? (wide ? __ffsll((long long)emask) : __ffs((int)emask)) - 1 : 0;
       emask &= emask - 1;
@@ -537,7 +515,6 @@ __global__ void __launch_bounds__(256) se_extend_kernel(const SeedExtParams p, c
       // of the lanes that need one (warp_pick)
       const uint32_t needm = __ballot_sync(FULL, need);
       if (needm) pick = warp_pick(needm, need, ring, col, ring_n, pos, ok, pick, lane);
-      SE_STAT(7, __popc(__ballot_sync(FULL, ok != 0u)));
       if (ok) {
         const int delta = pick == 1u ? -sr : (pick == 2u ? -scol : (pick == 4u ? sr : scol));
         pc[delta] = (uint8_t)v;   // the head / target moves      PPU:165-167
@@ -979,7 +956,6 @@ int launch_seedext(SeedExtParams p, int64_t max_boards, cudaStream_t stream) {
       one_wave = false;
     }
   }
-  if (const char *ex = getenv("RBG_SE_OPT_WARPS")) opt_w = atoi(ex) >= 1 && atoi(ex) <= 4 ? warps_for(opt_warp, atoi(ex)) : opt_w;
   int rc = RBG_OK;
   const bool wide = G > 32;
   const void *ext_fn = wide ? reinterpret_cast<const void *>(se_extend_kernel<true>) : reinterpret_cast<const void *>(se_extend_kernel<false>);
@@ -1164,15 +1140,3 @@ int launch_board_finish(const SeedExtParams &p, const uint8_t *boards, const uin
 }
 
 }  // namespace rbg
-
-#ifdef RBG_SE_STATS
-extern "C" int rbg_debug_se_stats(unsigned long long *out16, int reset) {
-  cudaDeviceSynchronize();
-  cudaMemcpyFromSymbol(out16, rbg::g_se_stats, sizeof(unsigned long long) * 16);
-  if (reset) {
-    unsigned long long z[16] = {0};
-    cudaMemcpyToSymbol(rbg::g_se_stats, z, sizeof(z));
-  }
-  return 0;
-}
-#endif

@@ -1,5 +1,5 @@
 """Time the fused rollout (rbg_connector_rollout_random) in the stationary regime: per-kernel averages
-from the library's own event pairs.  Used for A/B builds (RBG_NVCC_EXTRA) and ncu captures.
+from the library's own event pairs.  Used for A/B builds and ncu captures.
 
     python tools/run_rollout.py [G N B T calls burnin_calls]"""
 import os, sys
