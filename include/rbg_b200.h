@@ -242,6 +242,25 @@ int rbg_connector_rollout_random(const rbg_state *state, int32_t *action_out,
                                  const rbg_timestep *ts, void *workspace,
                                  void *stream);
 
+/* per-episode metrics of rbg_connector_episodes_random (names as BenchmarkData / PickleLogger) */
+typedef struct rbg_episode_metrics {
+  float   *episode_return;     /* [B,N] per agent, summed in step order (float32, round-to-nearest) */
+  int32_t *episode_length;     /* [B]   steps taken until the first LAST step */
+  int32_t *num_connections;    /* [B]   extras of that terminal TimeStep */
+  float   *ratio_connections;  /* [B]  */
+  int32_t *total_path_length;  /* [B]  */
+} rbg_episode_metrics;
+
+/* Run every env of `start` under the random policy (rbg_random_actions' draw) until its first LAST step;
+ * Connector(time_limit, DenseRewardFn) semantics from params, params->autoreset_kind must be < 0.
+ * `start` is read only.  final_state (may be NULL): the State after each env's terminal step.
+ * The random-agent evaluation of a board generator (the reference's benchmarks / evaluators reduce each episode
+ * to these five numbers): one launch, no per-step output, and no workspace (the library takes 256 bytes of
+ * stream-ordered scratch for the call). */
+int rbg_connector_episodes_random(const rbg_state *start, int64_t B, int G, int N,
+                                  const rbg_env_params *params, const rbg_episode_metrics *out,
+                                  const rbg_state *final_state, void *stream);
+
 /* Board validity: the reference's NumPy rules (numpy_implementation/utils/
  * post_processor_utils_numpy.py:34-155 = UP, numpy_implementation/utils/board_processor.py:111-162,
  * 391-487 = BP).  flags int32[B], 0 = valid by every rule:
@@ -331,7 +350,8 @@ int64_t rbg_launch_count(int reset);
 #define RBG_K_SEEDEXT 5    /* seedext_kernel */
 #define RBG_K_ROLLOUT 6    /* rollout_persist_kernel (rollout_warp_kernel for the dataset generator): T fused steps */
 #define RBG_K_SEQRW 7      /* seqrw_walk_kernel + its finish kernel */
-#define RBG_K_COUNT 8
+#define RBG_K_EPISODES 8   /* episode_warp_kernel: random-agent episodes to their first LAST step */
+#define RBG_K_COUNT 9
 int rbg_kernel_timing(int enable);
 int rbg_kernel_time(int kernel, int64_t *launches, double *total_ms);
 

@@ -36,9 +36,13 @@ class rbg_env_params(C.Structure):
                 ("dataset_heads", C.c_void_p), ("dataset_targets", C.c_void_p), ("dataset_K", C.c_int64)]
 
 
+class rbg_episode_metrics(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("episode_return", "episode_length", "num_connections", "ratio_connections", "total_path_length")]
+
+
 # every symbol include/rbg_b200.h declares: (restype, argtypes)
 _vp, _i64, _int, _f = C.c_void_p, C.c_int64, C.c_int, C.c_float
-_SP, _TP, _EP = C.POINTER(rbg_state), C.POINTER(rbg_timestep), C.POINTER(rbg_env_params)
+_SP, _TP, _EP, _MP = C.POINTER(rbg_state), C.POINTER(rbg_timestep), C.POINTER(rbg_env_params), C.POINTER(rbg_episode_metrics)
 SYMBOLS = {
     "rbg_version": (_int, []),
     "rbg_last_error": (C.c_char_p, []),
@@ -61,6 +65,7 @@ SYMBOLS = {
     "rbg_random_actions": (_int, [_SP, _i64, _int, _int, _vp, _vp]),
     "rbg_connector_step_random": (_int, [_SP, _SP, _vp, _i64, _int, _int, _EP, _TP, _vp, _vp]),
     "rbg_connector_rollout_random": (_int, [_SP, _vp, _i64, _i64, _int, _int, _EP, _TP, _vp, _vp]),
+    "rbg_connector_episodes_random": (_int, [_SP, _i64, _int, _int, _EP, _MP, _SP, _vp]),
     "rbg_validate": (_int, [_vp, _i64, _int, _int, _vp, _vp]),
     "rbg_board_statistics": (_int, [_vp, _i64, _int, _int, _vp, _vp, _vp, _vp]),
     "rbg_prw_generate_host": (_int, [_vp, _i64, _int, _int, _vp, _vp, _vp, _int]),
@@ -107,7 +112,7 @@ def launch_count(reset: bool = False) -> int:
     return int(load().rbg_launch_count(1 if reset else 0))
 
 
-KERNELS = {"prw": 0, "env": 1, "random_actions": 2, "split": 3, "validate": 4, "seedext": 5, "rollout": 6, "seqrw": 7}
+KERNELS = {"prw": 0, "env": 1, "random_actions": 2, "split": 3, "validate": 4, "seedext": 5, "rollout": 6, "seqrw": 7, "episodes": 8}
 
 
 def kernel_timing(enable: bool) -> None:

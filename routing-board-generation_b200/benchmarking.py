@@ -1,4 +1,4 @@
-"""Batched board statistics on the CUDA engine.
+"""Batched board statistics and random-agent evaluation on the CUDA engine.
 
 Mirrors `EvaluateEmptyBoard` (routing_board_generation/benchmarking/benchmarks/empty_board_evaluation.py:31-155),
 the per-board consumer of solved boards in the reference's benchmark
@@ -11,6 +11,10 @@ wire-length / bend statistics derived from it have no deterministic result and a
 scored as given (for boards whose wires are already shortest paths the two coincide).
 """
 from __future__ import annotations
+
+from typing import Dict
+
+import torch
 
 from . import engine
 
@@ -31,3 +35,70 @@ class EvaluateEmptyBoard:
         if not count_current_wire:
             return self._detours
         return engine.board_statistics(self.filled_board, count_current_wire=True, with_scores=False)[1]
+
+
+class RandomAgentEvaluator:
+    """Scores a board generator by what the library's random policy achieves on its boards.
+
+    `eval_env` is a Connector, optionally wrapped (MultiToSingleWrapper, VmapAutoResetWrapper; the latter has no
+    effect: an evaluation episode ends at its LAST step).  A MultiToSingleWrapper's reward aggregator is applied to the
+    per-agent returns, which equals the return of the aggregated reward for torch.sum and torch.mean; another
+    (non-linear) aggregator raises ValueError.  Each episode is reduced to the five numbers the
+    reference's benchmarks and evaluators log (BenchmarkData / PickleLogger): episode_return, episode_length,
+    num_connections, ratio_connections, total_path_length.  The episodes run in one kernel launch from the reset
+    State to each env's first LAST step (engine.connector_episodes_random); nothing is written per step.
+
+    Episode i starts from the eval env's generator called on key i.  jumanji's Evaluator derives its reset keys in
+    its own way, so the board of a given key may differ from a jumanji run; the distribution of episodes is the same.
+    """
+
+    def __init__(self, eval_env, total_batch_size: int):
+        from .connector import Connector, MultiToSingleWrapper
+
+        env, agg = eval_env, None
+        while not isinstance(env, Connector):
+            if isinstance(env, MultiToSingleWrapper):
+                if agg is not None:
+                    raise TypeError("eval_env has two MultiToSingleWrappers: the second would aggregate a scalar reward")
+                # the return of an aggregated reward is the aggregate of the per-agent returns only for a linear aggregator
+                if env._ragg not in (torch.sum, torch.mean):
+                    raise ValueError(f"MultiToSingleWrapper's reward_aggregator {env._ragg!r}: episode returns are summed per agent in the kernel, "
+                                     "so only torch.sum and torch.mean (linear) can be applied to them")
+                agg = env._ragg
+            env = getattr(env, "_env", None)
+            if env is None:
+                raise TypeError("eval_env must be a Connector or a wrapper around one")
+        self.eval_env = eval_env
+        self.total_batch_size = int(total_batch_size)
+        self._env = env
+        self._reward_agg = agg
+
+    def _reset_state(self, keys):
+        """The reset State of each key (no observation): the generator's own kernel, table lookup or __call__."""
+        from .connector import _stack_states
+
+        e = self._env
+        if e._kind == "dataset":
+            return engine.dataset_state(keys, e.grid_size, e.num_agents, engine.as_tensor(e._generator.heads, torch.int32), engine.as_tensor(e._generator.targets, torch.int32))
+        if e._kind != "user":
+            return engine.generator_state(e._kind, keys, e.grid_size, e.num_agents)
+        st = e._generator(keys)
+        if st.grid.dim() == 2:  # a generator that only handles single keys
+            st = _stack_states([e._generator(k) for k in keys])
+        return engine._contig_state(st.map(engine.as_tensor))
+
+    def episode_metrics(self, keys) -> Dict[str, torch.Tensor]:
+        """Reset on `keys` (uint32[B,2], or one key of shape (2,) for unbatched results) and run every episode to
+        its LAST step.  episode_return is [B,N] per agent, or [B] aggregated over the agents with the reward aggregator
+        (torch.sum by default, or torch.mean) when the eval env has a MultiToSingleWrapper."""
+        keys, batched = engine.as_keys(keys)
+        st = self._reset_state(keys)
+        m = engine.connector_episodes_random(st, **self._env._env_args())
+        if self._reward_agg is not None:
+            m["episode_return"] = self._reward_agg(m["episode_return"], dim=-1)
+        return m if batched else {k: v[0] for k, v in m.items()}
+
+    def run_evaluation(self, key) -> Dict[str, torch.Tensor]:
+        """Means over `total_batch_size` episodes whose reset keys are split(key, total_batch_size)."""
+        m = self.episode_metrics(engine.split(key, self.total_batch_size))
+        return {k: v.to(torch.float32).mean(dim=0) for k, v in m.items()}

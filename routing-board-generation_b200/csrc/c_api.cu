@@ -960,6 +960,22 @@ int rbg_connector_rollout_random(const rbg_state *state, int32_t *action_out, in
   return RBG_OK;
 }
 
+int rbg_connector_episodes_random(const rbg_state *start, int64_t B, int G, int N, const rbg_env_params *params, const rbg_episode_metrics *out,
+                                  const rbg_state *final_state, void *stream) {
+  int rc;
+  if ((rc = check_dims(B, G, N, 1))) return rc;
+  if (B == 0) return RBG_OK;  // an empty batch has no buffers to check
+  if ((rc = check_state(start, "start", G))) return rc;
+  if (!params) return set_error(RBG_EINVAL, "params is NULL");
+  if (params->autoreset_kind >= 0)
+    return set_error(RBG_EINVAL, "episodes end at their first LAST step: params->autoreset_kind must be < 0 (got %d)", params->autoreset_kind);
+  if (!out) return set_error(RBG_EINVAL, "metrics is NULL");
+  if (!out->episode_return || !out->episode_length || !out->num_connections || !out->ratio_connections || !out->total_path_length)
+    return set_error(RBG_EINVAL, "metrics has a NULL field");
+  if (final_state && (rc = check_state(final_state, "final_state", G))) return rc;
+  return launch_episodes(*start, final_state, *out, B, G, N, *params, (cudaStream_t)stream);
+}
+
 int rbg_random_actions(const rbg_state *state, int64_t B, int G, int N, int32_t *action, void *stream) {
   int rc;
   if ((rc = check_dims(B, G, N, 1))) return rc;

@@ -1152,4 +1152,203 @@ int launch_random_actions(const rbg_state &st, int64_t B, int G, int N, int32_t 
   return check_launch("random_actions_kernel");
 }
 
+// ---------------------------------------------------------------------------
+// episode_warp_kernel: every env of a batch from its State to its FIRST LAST step under the random policy, one
+// metrics record per env (the random-agent evaluation of a board generator).  Lane layout and step body are those
+// of rollout_warp_kernel: a warp owns K = 32 / Np envs, a lane is one (env, agent), the grids are uint8 in the
+// warp's slice of shared memory.  Nothing is written per step: returns accumulate in registers and an env writes
+// ~40 bytes when its episode ends.  A group of Np lanes whose episode has ended takes the next env of the batch from
+// a global counter (episodes of one warp differ in length: without the refill a warp would run for as long as its
+// longest episode).  A group with no env left idles through the warp-wide match / ballots; the warp exits when every
+// group is idle.  The grid is persistent (resident CTAs x SMs).  The input State is never written.
+constexpr int EP_WARPS = 4;
+constexpr int kEpisodeMinCtas = 8;
+
+struct EpisodeParams {
+  rbg_state in;               // read only
+  rbg_state fin;              // State after each env's terminal step; fin.grid == NULL: not written
+  rbg_episode_metrics out;
+  long long B;
+  int G, N, cells, Np;
+  int time_limit;
+  float timestep_reward, connected_reward;
+  int ratio_off;  // smem byte offset of the n / N table
+  int wgrid;      // smem bytes of one warp's grid slice
+  int *counter;   // next env index, zeroed
+  FastDiv divG;
+};
+
+__global__ void __launch_bounds__(EP_WARPS * 32, kEpisodeMinCtas) episode_warp_kernel(const EpisodeParams p) {
+  extern __shared__ __align__(16) uint8_t smem_raw[];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int G = p.G, N = p.N, cells = p.cells, Np = p.Np;
+  float *ratio_lut = reinterpret_cast<float *>(smem_raw + p.ratio_off);  // n / N for n = 0..N (extras: ratio_connections)
+  if (tid <= N) ratio_lut[tid] = __fdiv_rn((float)tid, (float)N);
+  __syncthreads();  // the only CTA-wide barrier
+
+  const int j = lane / Np, a = lane & (Np - 1), lead = j * Np;
+  const uint32_t gmask = Np == 32 ? FULL : (((1u << Np) - 1u) << lead);
+  uint8_t *g = smem_raw + (size_t)warp * p.wgrid + (size_t)j * cells;
+  const SmemGrid sg{g, G, 0, G};
+
+  long long e = 0;
+  bool env_ok = false, agent = false, refill = true;
+  int pos = 0, tgt = 0, sc = 0, len = 0, paths = 0;
+  uint32_t k0 = 0, k1 = 0, mk3 = 0;
+  float ret = 0.0f;
+  for (;;) {
+    if (refill) {  // group-uniform: the next env of the batch, State int32 -> uint8 grid, PATH cells recounted
+      long long nx = 0;
+      if (a == 0) nx = atomicAdd(p.counter, 1);
+      nx = __shfl_sync(gmask, nx, lead);
+      env_ok = nx < p.B;
+      agent = env_ok && a < N;
+      refill = false;
+      if (env_ok) {
+        e = nx;
+        const int32_t *src = p.in.grid + e * cells;
+        int pc = 0;
+        for (int i = a; i < cells; i += Np) {
+          const uint32_t v = (uint8_t)__ldg(src + i);
+          g[i] = (uint8_t)v;
+          pc += (v % 3u == 1u) ? 1 : 0;
+        }
+        for (int off = Np >> 1; off; off >>= 1) pc += __shfl_xor_sync(gmask, pc, off);
+        paths = pc;
+        sc = __ldg(p.in.step_count + e);
+        k0 = __ldg(p.in.key + 2 * e);
+        k1 = __ldg(p.in.key + 2 * e + 1);
+        len = 0;
+        ret = 0.0f;
+        if (agent) {
+          const int2 ps = __ldg(reinterpret_cast<const int2 *>(p.in.position) + e * N + a);
+          const int2 tg = __ldg(reinterpret_cast<const int2 *>(p.in.target) + e * N + a);
+          pos = (ps.x << 8) | ps.y;
+          tgt = (tg.x << 8) | tg.y;
+        }
+        __syncwarp(gmask);  // the whole grid is in before anybody reads a neighbour
+        mk3 = agent ? move_mask(sg, pos >> 8, pos & 255, a, pos == tgt) : 0u;
+      }
+    }
+    if (__ballot_sync(FULL, env_ok) == 0u) break;
+
+    // ---- one step (rollout_warp_kernel's step body): sample action, move, collisions
+    const bool was = agent && pos == tgt;
+    const int r = pos >> 8, c = pos & 255;
+    int dest = -1;
+    if (agent) {
+      const int action = random_action(k0, k1, (uint32_t)sc, (uint32_t)a, mk3);
+      if (action != NOOP) dest = r * G + c + (action == UP ? -G : (action == DOWN ? G : (action == RIGHT ? 1 : -1)));
+    }
+    const uint32_t mval = dest >= 0 ? (((uint32_t)j << 16) | (uint32_t)dest) : (0x80000000u | (uint32_t)lane);
+    const uint32_t mm = __match_any_sync(FULL, mval);
+    const bool win = dest >= 0 && lane == 31 - __clz(mm);
+    __syncwarp();
+    if (win) {
+      g[r * G + c] = (uint8_t)(3 * a + PATH);
+      g[dest] = (uint8_t)(3 * a + POSITION);
+      uint32_t nr, nc;
+      p.divG.divmod((uint32_t)dest, nr, nc);
+      pos = (int)((nr << 8) | nc);
+    }
+    __syncwarp();
+    // ---- action mask, connected / done, reward on the new grid
+    const bool now = agent && pos == tgt;
+    mk3 = 0;
+    if (agent) mk3 = move_mask(sg, pos >> 8, pos & 255, a, now);
+    const bool done = now || mk3 == 0u;
+    const float rew = __fadd_rn(__fmul_rn(p.connected_reward, (!was && now) ? 1.0f : 0.0f), __fmul_rn(p.timestep_reward, was ? 0.0f : 1.0f));
+    const int ndone = __popc(__ballot_sync(FULL, agent && done) & gmask);
+    const int nconn = __popc(__ballot_sync(FULL, now) & gmask);
+    paths += __popc(__ballot_sync(FULL, win) & gmask);
+    sc += 1;
+    len += 1;
+    ret = __fadd_rn(ret, rew);
+    const bool terminal = env_ok && (ndone == N || sc >= p.time_limit);
+
+    // ---- the episode's record (group-uniform)
+    if (terminal) {
+      if (agent) p.out.episode_return[e * N + a] = ret;
+      if (a == 0) {
+        p.out.episode_length[e] = len;
+        p.out.num_connections[e] = nconn;
+        p.out.ratio_connections[e] = ratio_lut[nconn];
+        p.out.total_path_length[e] = paths + N;
+      }
+      if (p.fin.grid) {  // Connector.step's State: grid, position and step_count move, the rest is the input's
+        int32_t *dst = p.fin.grid + e * cells;
+        for (int i = a; i < cells; i += Np) dst[i] = g[i];
+        if (a == 0) {
+          p.fin.step_count[e] = sc;
+          p.fin.key[2 * e] = k0;
+          p.fin.key[2 * e + 1] = k1;
+        }
+        if (agent) {
+          const long long ga = e * N + a;
+          reinterpret_cast<int2 *>(p.fin.position)[ga] = make_int2(pos >> 8, pos & 255);
+          reinterpret_cast<int2 *>(p.fin.target)[ga] = make_int2(tgt >> 8, tgt & 255);
+          reinterpret_cast<int2 *>(p.fin.start)[ga] = __ldg(reinterpret_cast<const int2 *>(p.in.start) + ga);
+          p.fin.agent_id[ga] = __ldg(p.in.agent_id + ga);
+        }
+      }
+      refill = true;
+    }
+    __syncwarp();  // the next episode's grid load must not overtake this step's reads
+  }
+}
+
+int launch_episodes(const rbg_state &in, const rbg_state *fin, const rbg_episode_metrics &out, int64_t B, int G, int N,
+                    const rbg_env_params &env, cudaStream_t stream) {
+  if (B <= 0) return RBG_OK;
+  EpisodeParams p;
+  memset(&p, 0, sizeof(p));
+  p.in = in;
+  if (fin) p.fin = *fin;
+  p.out = out;
+  p.B = B;
+  p.G = G;
+  p.N = N;
+  p.cells = G * G;
+  int Np = 1;
+  while (Np < N) Np <<= 1;
+  p.Np = Np;
+  p.time_limit = env.time_limit;
+  p.timestep_reward = env.timestep_reward;
+  p.connected_reward = env.connected_reward;
+  p.divG = FastDiv::make((uint32_t)G);
+  const int K = 32 / Np;
+  p.wgrid = (int)(((size_t)K * p.cells + 15) & ~(size_t)15);
+  p.ratio_off = EP_WARPS * p.wgrid;
+  const size_t smem = (size_t)p.ratio_off + 4 * (RBG_MAX_N + 4);
+  cudaError_t ce;
+  // few agents on a big board: up to 4 warps x 32 envs x 1 600 cells = 200 KB (40x40/1), past the 48 KB default
+  if (smem > 48 * 1024 && (ce = cudaFuncSetAttribute(episode_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+    return set_cuda_error(ce, "cudaFuncSetAttribute(episode_warp_kernel)");
+  int per_sm = 0;
+  if ((ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, episode_warp_kernel, EP_WARPS * 32, smem)) != cudaSuccess)
+    return set_cuda_error(ce, "cudaOccupancyMaxActiveBlocksPerMultiprocessor(episode_warp_kernel)");
+  if (per_sm < 1) return set_error(RBG_EINVAL, "episode_warp_kernel does not fit an SM (%zu bytes of shared memory)", smem);
+  const int64_t resident = (int64_t)per_sm * device_sm_count();
+  const int64_t need = (B + (int64_t)EP_WARPS * K - 1) / ((int64_t)EP_WARPS * K);
+  const unsigned ctas = (unsigned)(need < resident ? need : resident);
+  // the env counter: stream-ordered scratch, so that the caller needs no workspace and launches on different
+  // streams never share it
+  keep_pool_cached();
+  void *scratch = nullptr;
+  if ((ce = cudaMallocAsync(&scratch, 256, stream)) != cudaSuccess) return set_cuda_error(ce, "cudaMallocAsync(episode counter)");
+  p.counter = static_cast<int *>(scratch);
+  int rc = RBG_OK;
+  if ((ce = cudaMemsetAsync(scratch, 0, 256, stream)) != cudaSuccess) {
+    rc = set_cuda_error(ce, "cudaMemsetAsync(episode counter)");
+  } else {
+    {
+      LaunchScope scope(RBG_K_EPISODES, stream);
+      episode_warp_kernel<<<ctas, EP_WARPS * 32, smem, stream>>>(p);
+    }
+    rc = check_launch("episode_warp_kernel");
+  }
+  cudaFreeAsync(scratch, stream);
+  return rc;
+}
+
 }  // namespace rbg

@@ -105,6 +105,9 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
                            int epoch, bool overlap, uint64_t *cache_tag_w, uint2 *cache_key_w, uint32_t *cache_pins_w, cudaStream_t stream);
 int launch_random_actions(const rbg_state &st, int64_t B, int G, int N,
                           int32_t *action, cudaStream_t stream);
+// every env of `in` to its first LAST step under the random policy (episode_warp_kernel); fin may be NULL
+int launch_episodes(const rbg_state &in, const rbg_state *fin, const rbg_episode_metrics &out, int64_t B, int G, int N,
+                    const rbg_env_params &env, cudaStream_t stream);
 
 // ---- misc kernels (misc_kernels.cu) --------------------------------------
 int launch_split_keys(uint32_t k0, uint32_t k1, int64_t B, int64_t offset,

@@ -16,7 +16,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import GEN_DATASET, GEN_PRW, GEN_SEEDEXT, GEN_SEQRW, GEN_UNIFORM, rbg_env_params, rbg_state, rbg_timestep
+from ._lib import GEN_DATASET, GEN_PRW, GEN_SEEDEXT, GEN_SEQRW, GEN_UNIFORM, rbg_env_params, rbg_episode_metrics, rbg_state, rbg_timestep
 from .types import Agent, Observation, State, TimeStep
 
 GENERATOR_KINDS = {"parallel_random_walk": GEN_PRW, "uniform": GEN_UNIFORM, "seed_extension": GEN_SEEDEXT, "dataset": GEN_DATASET, "sequential_random_walk": GEN_SEQRW}
@@ -383,6 +383,37 @@ def connector_rollout_random(st: State, n_steps: int, time_limit: int = 50, time
     s, t = _state_struct(st), _timestep_struct(ts)
     _lib.check(_lib.load().rbg_connector_rollout_random(C.byref(s), act.data_ptr(), n_steps, B, G, N, C.byref(params), C.byref(t), ws.data_ptr() if ws is not None else None, _stream()))
     return st, ts, act
+
+
+EPISODE_METRICS = ("episode_return", "episode_length", "num_connections", "ratio_connections", "total_path_length")
+
+
+def connector_episodes_random(st: State, time_limit: int = 50, timestep_reward: float = -0.03, connected_reward: float = 0.1, final_state: bool = False) -> Dict[str, object]:
+    """Every env of `st` under the random policy (`random_actions`' draw) until its FIRST LAST step, in one launch.
+
+    Returns per-episode tensors: episode_return float32[B,N] (per agent, summed in step order), episode_length
+    int32[B] (steps taken), and the extras of the terminal TimeStep: num_connections int32[B], ratio_connections
+    float32[B], total_path_length int32[B]; with final_state=True also "final_state", the State after each env's
+    terminal step.  `st` is not modified."""
+    st = _contig_state(st)
+    B, G, N = _dims(st)
+    dev = _device()
+    out = {
+        "episode_return": torch.empty((B, N), dtype=torch.float32, device=dev),
+        "episode_length": torch.empty((B,), dtype=torch.int32, device=dev),
+        "num_connections": torch.empty((B,), dtype=torch.int32, device=dev),
+        "ratio_connections": torch.empty((B,), dtype=torch.float32, device=dev),
+        "total_path_length": torch.empty((B,), dtype=torch.int32, device=dev),
+    }
+    m = rbg_episode_metrics(*(out[k].data_ptr() for k in EPISODE_METRICS))
+    params, _ = _env_params(time_limit, timestep_reward, connected_reward, -1)
+    fin = alloc_state(B, G, N) if final_state else None
+    s = _state_struct(st)
+    f = C.byref(_state_struct(fin)) if fin is not None else None
+    _lib.check(_lib.load().rbg_connector_episodes_random(C.byref(s), B, G, N, C.byref(params), C.byref(m), f, _stream()))
+    if fin is not None:
+        out["final_state"] = fin
+    return out
 
 
 def random_actions(st: State) -> torch.Tensor:
