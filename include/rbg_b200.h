@@ -242,7 +242,7 @@ int rbg_connector_rollout_random(const rbg_state *state, int32_t *action_out,
                                  const rbg_timestep *ts, void *workspace,
                                  void *stream);
 
-/* per-episode metrics of rbg_connector_episodes_random (names as BenchmarkData / PickleLogger) */
+/* per-episode metrics of rbg_connector_episodes_random and rbg_connector_eval_step (names as BenchmarkData / PickleLogger) */
 typedef struct rbg_episode_metrics {
   float   *episode_return;     /* [B,N] per agent, summed in step order (float32, round-to-nearest) */
   int32_t *episode_length;     /* [B]   steps taken until the first LAST step */
@@ -260,6 +260,17 @@ typedef struct rbg_episode_metrics {
 int rbg_connector_episodes_random(const rbg_state *start, int64_t B, int G, int N,
                                   const rbg_env_params *params, const rbg_episode_metrics *out,
                                   const rbg_state *final_state, void *stream);
+
+/* One plain Connector.step (params->autoreset_kind must be < 0) of the envs whose live[b] != 0, with `action` int32[B,N]
+ * given: the step of a policy evaluation, one call per policy call.  For a live env the State is stepped in place and
+ * TimeStep row b is written as rbg_connector_step writes it; the record `acc` accumulates episode_return (float32,
+ * added in step order) and episode_length, and on LAST takes the TimeStep's extras, live[b] is cleared and the device
+ * int32 *live_count is decremented.  An env with live[b] == 0 is not read (but for its live byte) nor written: not its
+ * State, TimeStep row, record or action.  The caller starts with `acc` zeroed, live 1 and *live_count = B; from a
+ * reset State every env is done after at most time_limit calls. */
+int rbg_connector_eval_step(const rbg_state *state, const int32_t *action, uint8_t *live, int32_t *live_count,
+                            int64_t B, int G, int N, const rbg_env_params *params, const rbg_timestep *ts,
+                            const rbg_episode_metrics *acc, void *stream);
 
 /* Board validity: the reference's NumPy rules (numpy_implementation/utils/
  * post_processor_utils_numpy.py:34-155 = UP, numpy_implementation/utils/board_processor.py:111-162,
@@ -351,7 +362,8 @@ int64_t rbg_launch_count(int reset);
 #define RBG_K_ROLLOUT 6    /* rollout_persist_kernel (rollout_warp_kernel for the dataset generator): T fused steps */
 #define RBG_K_SEQRW 7      /* seqrw_walk_kernel + its finish kernel */
 #define RBG_K_EPISODES 8   /* episode_warp_kernel: random-agent episodes to their first LAST step */
-#define RBG_K_COUNT 9
+#define RBG_K_EVAL_STEP 9  /* eval_step_kernel: one policy-evaluation step of the live envs */
+#define RBG_K_COUNT 10
 int rbg_kernel_timing(int enable);
 int rbg_kernel_time(int kernel, int64_t *launches, double *total_ms);
 

@@ -66,6 +66,7 @@ SYMBOLS = {
     "rbg_connector_step_random": (_int, [_SP, _SP, _vp, _i64, _int, _int, _EP, _TP, _vp, _vp]),
     "rbg_connector_rollout_random": (_int, [_SP, _vp, _i64, _i64, _int, _int, _EP, _TP, _vp, _vp]),
     "rbg_connector_episodes_random": (_int, [_SP, _i64, _int, _int, _EP, _MP, _SP, _vp]),
+    "rbg_connector_eval_step": (_int, [_SP, _vp, _vp, _vp, _i64, _int, _int, _EP, _TP, _MP, _vp]),
     "rbg_validate": (_int, [_vp, _i64, _int, _int, _vp, _vp]),
     "rbg_board_statistics": (_int, [_vp, _i64, _int, _int, _vp, _vp, _vp, _vp]),
     "rbg_prw_generate_host": (_int, [_vp, _i64, _int, _int, _vp, _vp, _vp, _int]),
@@ -112,7 +113,7 @@ def launch_count(reset: bool = False) -> int:
     return int(load().rbg_launch_count(1 if reset else 0))
 
 
-KERNELS = {"prw": 0, "env": 1, "random_actions": 2, "split": 3, "validate": 4, "seedext": 5, "rollout": 6, "seqrw": 7, "episodes": 8}
+KERNELS = {"prw": 0, "env": 1, "random_actions": 2, "split": 3, "validate": 4, "seedext": 5, "rollout": 6, "seqrw": 7, "episodes": 8, "eval_step": 9}
 
 
 def kernel_timing(enable: bool) -> None:

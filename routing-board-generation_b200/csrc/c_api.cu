@@ -122,6 +122,13 @@ static int check_timestep(const rbg_timestep *t, int G) {
   return RBG_OK;
 }
 
+static int check_metrics(const rbg_episode_metrics *m, const char *name) {
+  if (!m) return set_error(RBG_EINVAL, "%s is NULL", name);
+  if (!m->episode_return || !m->episode_length || !m->num_connections || !m->ratio_connections || !m->total_path_length)
+    return set_error(RBG_EINVAL, "%s has a NULL field", name);
+  return RBG_OK;
+}
+
 static int check_dataset(const rbg_env_params *params) {
   if (!params->dataset_heads || !params->dataset_targets)
     return set_error(RBG_EINVAL, "autoreset_kind RBG_GEN_DATASET needs params->dataset_heads / dataset_targets (device int32[K,2,N])");
@@ -969,11 +976,27 @@ int rbg_connector_episodes_random(const rbg_state *start, int64_t B, int G, int 
   if (!params) return set_error(RBG_EINVAL, "params is NULL");
   if (params->autoreset_kind >= 0)
     return set_error(RBG_EINVAL, "episodes end at their first LAST step: params->autoreset_kind must be < 0 (got %d)", params->autoreset_kind);
-  if (!out) return set_error(RBG_EINVAL, "metrics is NULL");
-  if (!out->episode_return || !out->episode_length || !out->num_connections || !out->ratio_connections || !out->total_path_length)
-    return set_error(RBG_EINVAL, "metrics has a NULL field");
+  if ((rc = check_metrics(out, "metrics"))) return rc;
   if (final_state && (rc = check_state(final_state, "final_state", G))) return rc;
   return launch_episodes(*start, final_state, *out, B, G, N, *params, (cudaStream_t)stream);
+}
+
+int rbg_connector_eval_step(const rbg_state *state, const int32_t *action, uint8_t *live, int32_t *live_count, int64_t B, int G, int N,
+                            const rbg_env_params *params, const rbg_timestep *ts, const rbg_episode_metrics *acc, void *stream) {
+  int rc;
+  if ((rc = check_dims(B, G, N, 1))) return rc;
+  if (B == 0) return RBG_OK;  // an empty batch has no buffers to check
+  if ((rc = check_state(state, "state", G))) return rc;
+  if (!action) return set_error(RBG_EINVAL, "action is NULL");
+  if (!live) return set_error(RBG_EINVAL, "live is NULL");
+  if (!live_count) return set_error(RBG_EINVAL, "live_count is NULL");
+  if (!params) return set_error(RBG_EINVAL, "params is NULL");
+  if (params->autoreset_kind >= 0)
+    return set_error(RBG_EINVAL, "an evaluation step ends an episode at its first LAST step: params->autoreset_kind must be < 0 (got %d)",
+                     params->autoreset_kind);
+  if ((rc = check_timestep(ts, G))) return rc;
+  if ((rc = check_metrics(acc, "acc"))) return rc;
+  return launch_eval_step(*state, action, live, live_count, B, G, N, *params, *ts, *acc, (cudaStream_t)stream);
 }
 
 int rbg_random_actions(const rbg_state *state, int64_t B, int G, int N, int32_t *action, void *stream) {

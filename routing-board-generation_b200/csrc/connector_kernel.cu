@@ -1351,4 +1351,236 @@ int launch_episodes(const rbg_state &in, const rbg_state *fin, const rbg_episode
   return rc;
 }
 
+// ---------------------------------------------------------------------------
+// eval_step_kernel: one plain Connector.step (actions given, no auto-reset) of the envs whose live byte is set, with
+// each env's episode record accumulated in place: the step of a policy evaluation, one launch per policy call.  Lane
+// layout, observation table and in-place grid scatter are env_warp_kernel's (a warp owns K = 32 / Np envs, a lane is
+// one (env, agent)).  An env whose live byte is 0 costs the read of that byte: its State, TimeStep row, record and
+// action are neither read nor written, so the step's traffic scales with the live envs, and a warp with no live env
+// exits after that read.  On LAST the extras go to the record, the live byte is cleared and live_count drops by the
+// warp's number of finished envs (one atomic per warp).
+struct EvalStepParams {
+  rbg_state st;  // stepped in place
+  rbg_timestep ts;
+  rbg_episode_metrics acc;
+  const int32_t *action;
+  uint8_t *live;
+  int32_t *live_count;
+  long long B;
+  int G, N, cells, Np;
+  int time_limit;
+  float timestep_reward, connected_reward;
+  int so[2];  // shared memory: [0] bytes of the observation table, [1] bytes of one warp's grid slice
+  FastDiv divG, divC4, divCells;
+};
+
+template <bool VEC>
+__global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) eval_step_kernel(const EvalStepParams p) {
+  extern __shared__ __align__(16) uint8_t smem_raw[];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int G = p.G, N = p.N, cells = p.cells;
+  const int Np = p.Np, K = 32 / Np, c4 = cells >> 2;
+  const int RS = obs_lut_stride(N);
+
+  const long long e0 = ((long long)blockIdx.x * EW_WARPS + warp) * K;
+  const int kc = e0 >= p.B ? 0 : (int)((p.B - e0) < (long long)K ? (p.B - e0) : (long long)K);
+  const int j = lane / Np, a = lane & (Np - 1);
+  const long long e = e0 + (j < kc ? j : 0);
+  const bool env_ok = j < kc && p.live[e] != 0, agent = env_ok && a < N;
+  const uint32_t livem = __ballot_sync(FULL, env_ok);  // bit j * Np (and the env's other lanes): env j is live
+  if (!__syncthreads_or(livem != 0u)) return;  // a CTA without a live env builds no table
+  uint8_t *lut = smem_raw;
+  for (int x = warp; x < N; x += EW_WARPS)
+    for (int v = lane; v < RS; v += 32) lut[x * RS + v] = v <= 3 * N ? (uint8_t)obs_value(v, 3 * x, 3 * N) : (uint8_t)0;
+  __syncthreads();  // the last CTA-wide barrier
+  if (livem == 0u) return;
+  uint8_t *wg = smem_raw + p.so[0] + (size_t)warp * p.so[1];
+  uint32_t *wg32 = reinterpret_cast<uint32_t *>(wg);
+  const uint32_t gmask = Np == 32 ? FULL : (((1u << Np) - 1u) << (j * Np));
+
+  // ---- load the live envs: State.grid int32 -> uint8, agent and env scalars
+  if (VEC) {
+    const int4 *src = reinterpret_cast<const int4 *>(p.st.grid) + e0 * c4;
+    const int nq = kc * c4;
+    for (int q0 = lane; q0 < nq; q0 += 128) {
+      int4 v[4];
+      bool ok[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const int q = q0 + 32 * u;
+        ok[u] = q < nq && ((livem >> ((int)p.divC4.div((uint32_t)q) * Np)) & 1u);
+        v[u] = ok[u] ? __ldg(src + q) : make_int4(0, 0, 0, 0);
+      }
+#pragma unroll
+      for (int u = 0; u < 4; ++u)
+        if (ok[u])
+          wg32[q0 + 32 * u] = (uint32_t)(v[u].x & 0xff) | ((uint32_t)(v[u].y & 0xff) << 8) | ((uint32_t)(v[u].z & 0xff) << 16) | ((uint32_t)(v[u].w & 0xff) << 24);
+    }
+  } else {
+    const int32_t *src = p.st.grid + e0 * cells;
+    for (int i = lane; i < kc * cells; i += 32)
+      if ((livem >> ((int)p.divCells.div((uint32_t)i) * Np)) & 1u) wg[i] = (uint8_t)__ldg(src + i);
+  }
+  int pos = 0, tgt = 0, action = 0, sc0 = 0;
+  if (agent) {
+    const int2 ps = __ldg(reinterpret_cast<const int2 *>(p.st.position) + e * N + a);
+    const int2 tg = __ldg(reinterpret_cast<const int2 *>(p.st.target) + e * N + a);
+    pos = (ps.x << 8) | ps.y;
+    tgt = (tg.x << 8) | tg.y;
+    action = __ldg(p.action + e * N + a);
+  }
+  if (env_ok) sc0 = p.st.step_count[e];
+  __syncwarp();
+
+  uint8_t *g = wg + (size_t)j * cells;
+  const SmemGrid sg{g, G, 0, G};
+  // PATH cells of the env before the move (extras: total_path_length)
+  int paths = 0;
+  if (env_ok) {
+    if (VEC) {
+      for (int q = a; q < c4; q += Np) paths += count_path_codes(wg32[j * c4 + q]);
+    } else {
+      for (int i = a; i < cells; i += Np) paths += (g[i] % 3u == 1u) ? 1 : 0;
+    }
+  }
+  for (int off = Np >> 1; off; off >>= 1) paths += __shfl_xor_sync(FULL, paths, off);
+
+  // ---- agents: move_position, is_valid_position, collisions
+  const bool was = agent && pos == tgt;
+  int r = pos >> 8, c = pos & 255, dest = -1;
+  if (agent) {
+    const int am = action < 0 ? 0 : (action > 4 ? 4 : action);  // lax.switch clamps
+    const int nr = r + (am == UP ? -1 : (am == DOWN ? 1 : 0));
+    const int nc = c + (am == RIGHT ? 1 : (am == LEFT ? -1 : 0));
+    const bool inb = (unsigned)nr < (unsigned)G && (unsigned)nc < (unsigned)G;
+    const uint32_t v = inb ? sg.at(nr, nc) : 0xFFu;
+    if (inb && (v == 0u || v == 3u * a + TARGET) && !was && action != NOOP) dest = nr * G + nc;
+  }
+  // same destination in the same env -> only the highest agent id moves
+  const uint32_t mval = dest >= 0 ? (((uint32_t)j << 16) | (uint32_t)dest) : (0x80000000u | (uint32_t)lane);
+  const uint32_t mm = __match_any_sync(FULL, mval);
+  const bool win = dest >= 0 && lane == 31 - __clz(mm);
+  __syncwarp();  // every read of the pre-move grid is done
+  if (win) {  // move_agent: old head -> PATH, new cell -> POSITION; State.grid in place: only these two cells change
+    g[r * G + c] = (uint8_t)(3 * a + PATH);
+    g[dest] = (uint8_t)(3 * a + POSITION);
+    int32_t *gg = p.st.grid + e * cells;
+    gg[r * G + c] = 3 * a + PATH;
+    gg[dest] = 3 * a + POSITION;
+    uint32_t nr, nc;
+    p.divG.divmod((uint32_t)dest, nr, nc);
+    pos = (int)((nr << 8) | nc);
+  }
+  __syncwarp();
+
+  // ---- action mask, connected / done, reward on the new grid
+  const bool now = agent && pos == tgt;
+  uint32_t mk3 = 0;
+  if (agent) mk3 = move_mask(sg, pos >> 8, pos & 255, a, now);
+  const bool done = now || mk3 == 0u;  // connected_or_blocked
+  const float rew = __fadd_rn(__fmul_rn(p.connected_reward, (!was && now) ? 1.0f : 0.0f), __fmul_rn(p.timestep_reward, was ? 0.0f : 1.0f));
+  const int ndone = __popc(__ballot_sync(FULL, agent && done) & gmask);
+  const int nconn = __popc(__ballot_sync(FULL, now) & gmask);
+  const int nmoved = __popc(__ballot_sync(FULL, win) & gmask);
+  const int sc = sc0 + 1;
+  const bool terminal = env_ok && (ndone == N || sc >= p.time_limit);
+
+  // ---- TimeStep row, State scalars and the episode record of the live envs
+  if (env_ok && a == 0) {
+    const float ratio = __fdiv_rn((float)nconn, (float)N);
+    const int tpl = paths + nmoved + N;
+    p.ts.step_type[e] = (int8_t)(terminal ? 2 : 1);
+    p.ts.num_connections[e] = nconn;
+    p.ts.ratio_connections[e] = ratio;
+    p.ts.total_path_length[e] = tpl;
+    p.ts.obs_step_count[e] = sc;
+    p.st.step_count[e] = sc;
+    p.acc.episode_length[e] += 1;
+    if (terminal) {
+      p.acc.num_connections[e] = nconn;
+      p.acc.ratio_connections[e] = ratio;
+      p.acc.total_path_length[e] = tpl;
+      p.live[e] = 0;
+    }
+  }
+  if (agent) {
+    const long long ga = e * N + a;
+    p.ts.reward[ga] = rew;
+    p.ts.discount[ga] = (terminal || done) ? 0.0f : 1.0f;
+    store_mask5(p.ts.action_mask + ga * 5, mk3);
+    reinterpret_cast<int2 *>(p.st.position)[ga] = make_int2(pos >> 8, pos & 255);
+    p.acc.episode_return[ga] = __fadd_rn(p.acc.episode_return[ga], rew);
+  }
+  const int nfinished = __popc(__ballot_sync(FULL, a == 0 && terminal));
+  if (lane == 0 && nfinished) atomicSub(p.live_count, nfinished);
+
+  // ---- observation.grid of the live envs
+  if (VEC) {
+    int4 *odst = reinterpret_cast<int4 *>(p.ts.obs_grid) + e0 * N * c4;
+    for (int q = lane; q < kc * c4; q += 32) {
+      const int m = (int)p.divC4.div((uint32_t)q);
+      if (!((livem >> (m * Np)) & 1u)) continue;
+      const uint32_t w = wg32[q];
+      const uint32_t b0 = w & 0xffu, b1 = (w >> 8) & 0xffu, b2 = (w >> 16) & 0xffu, b3 = w >> 24;
+      int4 *o = odst + (size_t)m * N * c4 + (q - m * c4);
+      const uint8_t *row = lut;
+#pragma unroll 2
+      for (int x = 0; x < N; ++x, o += c4, row += RS) *o = make_int4(row[b0], row[b1], row[b2], row[b3]);
+    }
+  } else {
+    int32_t *odst = p.ts.obs_grid + e0 * N * cells;
+    for (int i = lane; i < kc * cells; i += 32) {
+      const int m = (int)p.divCells.div((uint32_t)i);
+      if (!((livem >> (m * Np)) & 1u)) continue;
+      const uint32_t v = wg[i];
+      int32_t *o = odst + (size_t)m * N * cells + (i - m * cells);
+      for (int x = 0; x < N; ++x, o += cells) *o = lut[x * RS + v];
+    }
+  }
+}
+
+int launch_eval_step(const rbg_state &st, const int32_t *action, uint8_t *live, int32_t *live_count, int64_t B, int G, int N,
+                     const rbg_env_params &env, const rbg_timestep &ts, const rbg_episode_metrics &acc, cudaStream_t stream) {
+  if (B <= 0) return RBG_OK;
+  EvalStepParams p;
+  memset(&p, 0, sizeof(p));
+  p.st = st;
+  p.ts = ts;
+  p.acc = acc;
+  p.action = action;
+  p.live = live;
+  p.live_count = live_count;
+  p.B = B;
+  p.G = G;
+  p.N = N;
+  p.cells = G * G;
+  const bool vec = (p.cells & 3) == 0;
+  int Np = 1;
+  while (Np < N) Np <<= 1;
+  p.Np = Np;
+  p.time_limit = env.time_limit;
+  p.timestep_reward = env.timestep_reward;
+  p.connected_reward = env.connected_reward;
+  p.divG = FastDiv::make((uint32_t)G);
+  p.divC4 = FastDiv::make((uint32_t)(vec ? p.cells >> 2 : 1));
+  p.divCells = FastDiv::make((uint32_t)p.cells);
+  const int K = 32 / Np;
+  const size_t lutB = ((size_t)N * obs_lut_stride(N) + 256 + 15) & ~(size_t)15;
+  const size_t wgrid = ((size_t)K * p.cells + 15) & ~(size_t)15;
+  p.so[0] = (int)lutB;
+  p.so[1] = (int)wgrid;
+  const size_t smem = lutB + EW_WARPS * wgrid;
+  const int64_t ctas = (B + (int64_t)EW_WARPS * K - 1) / ((int64_t)EW_WARPS * K);
+  void (*fn)(const EvalStepParams) = vec ? eval_step_kernel<true> : eval_step_kernel<false>;
+  cudaError_t ce;
+  // few agents on a big board: up to 4 warps x 32 envs x 1 600 cells = 200 KB (40x40/1), past the 48 KB default
+  if (smem > 48 * 1024 && (ce = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+    return set_cuda_error(ce, "cudaFuncSetAttribute(eval_step_kernel)");
+  {
+    LaunchScope scope(RBG_K_EVAL_STEP, stream);
+    fn<<<(unsigned)ctas, EW_WARPS * 32, smem, stream>>>(p);
+  }
+  return check_launch("eval_step_kernel");
+}
+
 }  // namespace rbg

@@ -108,6 +108,9 @@ int launch_random_actions(const rbg_state &st, int64_t B, int G, int N,
 // every env of `in` to its first LAST step under the random policy (episode_warp_kernel); fin may be NULL
 int launch_episodes(const rbg_state &in, const rbg_state *fin, const rbg_episode_metrics &out, int64_t B, int G, int N,
                     const rbg_env_params &env, cudaStream_t stream);
+// one Connector.step of the envs whose live byte is set, their episode records accumulated in place (eval_step_kernel)
+int launch_eval_step(const rbg_state &st, const int32_t *action, uint8_t *live, int32_t *live_count, int64_t B, int G, int N,
+                     const rbg_env_params &env, const rbg_timestep &ts, const rbg_episode_metrics &acc, cudaStream_t stream);
 
 // ---- misc kernels (misc_kernels.cu) --------------------------------------
 int launch_split_keys(uint32_t k0, uint32_t k1, int64_t B, int64_t offset,

@@ -416,6 +416,27 @@ def connector_episodes_random(st: State, time_limit: int = 50, timestep_reward: 
     return out
 
 
+def connector_eval_step(st: State, action: torch.Tensor, live: torch.Tensor, live_count: torch.Tensor, acc: Dict[str, torch.Tensor], ts: TimeStep,
+                        time_limit: int = 50, timestep_reward: float = -0.03, connected_reward: float = 0.1) -> None:
+    """One plain Connector.step of the envs whose `live` byte (uint8[B]) is set, all buffers updated in place.
+
+    A live env's State `st` is stepped with `action` int32[B,N], TimeStep row b of `ts` is written as `connector_step`
+    writes it, and its record in `acc` (the EPISODE_METRICS tensors, as `connector_episodes_random` returns them)
+    accumulates episode_return and episode_length; on LAST the record takes the extras, the live byte is cleared and
+    `live_count` (int32[1] on the device) drops by one.  A dead env is neither read nor written.  Start with `acc`
+    zeroed, `live` ones and `live_count` = [B]."""
+    B, G, N = _dims(st)
+    if not all(t.is_contiguous() for t in (st.grid, st.step_count, st.key, st.agents.id, st.agents.start, st.agents.target, st.agents.position)):
+        raise ValueError("the evaluation step updates the State in place: its leaves must be contiguous")
+    if live.dtype != torch.uint8 or tuple(live.shape) != (B,) or live_count.dtype != torch.int32 or live_count.numel() != 1:
+        raise ValueError("live must be uint8[B] and live_count int32[1]")
+    act = as_tensor(action, torch.int32).reshape(B, N)
+    m = rbg_episode_metrics(*(acc[k].data_ptr() for k in EPISODE_METRICS))
+    params, _ = _env_params(time_limit, timestep_reward, connected_reward, -1)
+    s, t = _state_struct(st), _timestep_struct(ts)
+    _lib.check(_lib.load().rbg_connector_eval_step(C.byref(s), act.data_ptr(), live.data_ptr(), live_count.data_ptr(), B, G, N, C.byref(params), C.byref(t), C.byref(m), _stream()))
+
+
 def random_actions(st: State) -> torch.Tensor:
     st = _contig_state(st)
     B, G, N = _dims(st)
