@@ -354,7 +354,7 @@ int64_t rbg_launch_count(int reset);
  * before it, normally overlap on the stream; while timing is enabled they run one kernel at
  * a time, so that a pair of events times one kernel. */
 #define RBG_K_PRW 0        /* prw_kernel: ParallelRandomWalk / Uniform generator */
-#define RBG_K_ENV 1        /* env_kernel: Connector step / observe */
+#define RBG_K_ENV 1        /* env_warp_kernel: Connector step / observe */
 #define RBG_K_RANDACT 2    /* random_actions_kernel */
 #define RBG_K_SPLIT 3      /* split_keys_kernel */
 #define RBG_K_VALIDATE 4   /* validate_kernel */

@@ -150,7 +150,7 @@ static int debug_flags() {
 // VmapAutoResetWrapper regenerates a board whenever an env finishes.  The reset key
 // of an episode is known as soon as the episode starts (split(state.key)[0]), so the
 // NEXT episode of every env that just reset is generated ahead of time ("refill")
-// into a per-env cache; when the env finishes, env_kernel swaps the
+// into a per-env cache; when the env finishes, env_warp_kernel swaps the
 // cached episode in.  Only envs whose cache entry is not ready (first episode, or two
 // terminations in consecutive steps) take the synchronous reset kernel.  Results are
 // identical either way: a board is a pure function of its key.

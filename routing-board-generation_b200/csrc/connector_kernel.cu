@@ -53,6 +53,167 @@ __device__ __forceinline__ int random_action(uint32_t k0, uint32_t k1,
 }
 
 // ---------------------------------------------------------------------------
+// The phases of one Connector step in the warp-per-K-envs layout that every kernel below uses: a warp owns
+// K = 32 / Np envs (Np = lanes per env, the next power of two >= N), lane = (env j, agent a), and the env grids are
+// uint8 codes in the warp's slice of shared memory, env j at wg + j * cells.
+
+// observation table: row x maps a grid code v (0..3N) to agent x's view of it; rows are RS bytes apart
+__device__ __forceinline__ void build_obs_lut(uint8_t *lut, int N, int RS, int warp, int nwarps, int lane) {
+  for (int x = warp; x < N; x += nwarps)
+    for (int v = lane; v < RS; v += 32) lut[x * RS + v] = v <= 3 * N ? (uint8_t)obs_value(v, 3 * x, 3 * N) : (uint8_t)0;
+}
+
+// State.grid int32 of envs e0 .. e0 + kc - 1 -> the warp's uint8 grids (VEC: one packed word per int4)
+template <bool VEC>
+__device__ __forceinline__ void load_grids(const int32_t *grid, long long e0, int kc, int cells, int lane, uint8_t *wg) {
+  if (VEC) {
+    // four loads in flight per lane before the first one is used (a load-use pair per iteration
+    // made a warp pay one L2 round trip per 32 words: 19 % of the kernel's stall samples)
+    uint32_t *wg32 = reinterpret_cast<uint32_t *>(wg);
+    const int4 *src = reinterpret_cast<const int4 *>(grid) + e0 * (cells >> 2);
+    const int nq = kc * (cells >> 2);
+    for (int q0 = lane; q0 < nq; q0 += 128) {
+      int4 v[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) v[u] = (q0 + 32 * u < nq) ? __ldg(src + q0 + 32 * u) : make_int4(0, 0, 0, 0);
+#pragma unroll
+      for (int u = 0; u < 4; ++u)
+        if (q0 + 32 * u < nq)
+          wg32[q0 + 32 * u] = (uint32_t)(v[u].x & 0xff) | ((uint32_t)(v[u].y & 0xff) << 8) | ((uint32_t)(v[u].z & 0xff) << 16) | ((uint32_t)(v[u].w & 0xff) << 24);
+    }
+  } else {
+    const int32_t *src = grid + e0 * cells;
+    for (int i = lane; i < kc * cells; i += 32) wg[i] = (uint8_t)__ldg(src + i);
+  }
+}
+
+// PATH cells of env j (extras: total_path_length), summed over the env's Np lanes
+template <bool VEC>
+__device__ __forceinline__ int count_paths(const uint8_t *wg, int j, int a, int cells, int c4, int Np, bool env_ok) {
+  int paths = 0;
+  if (env_ok) {
+    if (VEC) {
+      const uint32_t *wg32 = reinterpret_cast<const uint32_t *>(wg);
+      for (int q = a; q < c4; q += Np) paths += count_path_codes(wg32[j * c4 + q]);
+    } else {
+      const uint8_t *g = wg + (size_t)j * cells;
+      for (int i = a; i < cells; i += Np) paths += (g[i] % 3u == 1u) ? 1 : 0;
+    }
+  }
+  for (int off = Np >> 1; off; off >>= 1) paths += __shfl_xor_sync(FULL, paths, off);
+  return paths;
+}
+
+// destination cell of a random-policy action (-1: none), the action written to out[row] if out is set.  mk is
+// is_valid_position of the four moves on this very grid (empty for a connected agent), so a non-NOOP action needs no
+// second validity test.
+__device__ __forceinline__ int random_dest(uint32_t k0, uint32_t k1, int sc, int a, uint32_t mk, int r, int c, int G, int32_t *out,
+                                           long long row) {
+  const int action = random_action(k0, k1, (uint32_t)sc, (uint32_t)a, mk);
+  if (out) out[row] = action;
+  return action != NOOP ? r * G + c + (action == UP ? -G : (action == DOWN ? G : (action == RIGHT ? 1 : -1))) : -1;
+}
+
+// the collision rule and move_agent: of the agents of one env with the same destination only the highest agent id
+// moves; a mover's old head becomes PATH and its new cell POSITION on the env grid g.  Returns the lane's position
+// after the move; win: it moved.
+__device__ __forceinline__ int resolve_moves(int dest, int j, int lane, int a, int r, int c, int G, uint8_t *g, const FastDiv &divG, int pos,
+                                             bool &win) {
+  const uint32_t mval = dest >= 0 ? (((uint32_t)j << 16) | (uint32_t)dest) : (0x80000000u | (uint32_t)lane);
+  const uint32_t mm = __match_any_sync(FULL, mval);
+  win = dest >= 0 && lane == 31 - __clz(mm);
+  __syncwarp();  // every read of the pre-move grid is done
+  if (win) {
+    g[r * G + c] = (uint8_t)(3 * a + PATH);
+    g[dest] = (uint8_t)(3 * a + POSITION);
+    uint32_t nr, nc;
+    divG.divmod((uint32_t)dest, nr, nc);
+    pos = (int)((nr << 8) | nc);
+  }
+  __syncwarp();
+  return pos;
+}
+
+// what the step leaves on the new grid: per agent, per env (group-uniform counts)
+struct StepResult {
+  uint32_t mk3;  // action mask (bit m-1: move m legal)
+  bool done;     // connected_or_blocked
+  float rew;     // DenseRewardFn
+  int ndone, nconn, nmoved;
+};
+
+// rw: anything with the env's connected_reward and timestep_reward (rbg_env_params, EpisodeParams, EvalStepParams)
+template <class Rewards>
+__device__ __forceinline__ StepResult after_move(const SmemGrid &sg, bool agent, int a, int pos, int tgt, bool was, bool win, uint32_t gmask,
+                                                 const Rewards &rw) {
+  const bool now = agent && pos == tgt;
+  uint32_t mk3 = 0;
+  if (agent) mk3 = move_mask(sg, pos >> 8, pos & 255, a, now);
+  const bool done = now || mk3 == 0u;
+  const float rew = __fadd_rn(__fmul_rn(rw.connected_reward, (!was && now) ? 1.0f : 0.0f), __fmul_rn(rw.timestep_reward, was ? 0.0f : 1.0f));
+  const int ndone = __popc(__ballot_sync(FULL, agent && done) & gmask);
+  const int nconn = __popc(__ballot_sync(FULL, now) & gmask);
+  const int nmoved = __popc(__ballot_sync(FULL, win) & gmask);
+  return StepResult{mk3, done, rew, ndone, nconn, nmoved};
+}
+
+// swap in a new episode (group-uniform): env grid g holds only the pins, heads then targets (PRWG:63-64); returns the
+// fresh action mask of agent a at pos (lanes a >= N return mk3 as it is).  cleared() runs once the grid is cleared,
+// before the pins go in.
+template <class F>
+__device__ __forceinline__ uint32_t place_episode(uint8_t *g, const SmemGrid &sg, int a, int N, int Np, int cells, int G, uint32_t gmask,
+                                                  int pos, int tgt, uint32_t mk3, F cleared) {
+  for (int i = a; i < cells; i += Np) g[i] = 0;
+  cleared();
+  __syncwarp(gmask);
+  if (a < N) g[(pos >> 8) * G + (pos & 255)] = (uint8_t)(3 * a + POSITION);
+  __syncwarp(gmask);
+  if (a < N) g[(tgt >> 8) * G + (tgt & 255)] = (uint8_t)(3 * a + TARGET);
+  __syncwarp(gmask);
+  if (a < N) mk3 = move_mask(sg, pos >> 8, pos & 255, a, pos == tgt);
+  return mk3;
+}
+
+// observation.grid of kc envs through the table, one store per cell (cells % 4 != 0); env m is skipped where bit
+// m * Np of skipm is set
+__device__ __forceinline__ void write_obs_scalar(int32_t *odst, const uint8_t *wg, const uint8_t *lut, int RS, int kc, int cells, int N, int Np,
+                                                 uint32_t skipm, const FastDiv &divCells, int lane) {
+  for (int i = lane; i < kc * cells; i += 32) {
+    const int m = (int)divCells.div((uint32_t)i);
+    if ((skipm >> (m * Np)) & 1u) continue;
+    const uint32_t v = wg[i];
+    int32_t *o = odst + (size_t)m * N * cells + (i - m * cells);
+    for (int x = 0; x < N; ++x, o += cells) *o = lut[x * RS + v];
+  }
+}
+
+// the State at the end of a rollout, written once: the warp's grids, and per env / agent what the steps moved
+template <bool VEC>
+__device__ __forceinline__ void write_state_once(const rbg_state &out, const uint8_t *wg, long long e0, int kc, int cells, int lane, long long e,
+                                                 int N, int a, bool env_ok, bool agent, int pos, int tgt, int start, int sc, uint32_t k0, uint32_t k1) {
+  if (VEC) {
+    const uint32_t *wg32 = reinterpret_cast<const uint32_t *>(wg);
+    int4 *gdst = reinterpret_cast<int4 *>(out.grid) + e0 * (cells >> 2);
+    for (int q = lane; q < kc * (cells >> 2); q += 32) gdst[q] = bytes_to_int4(wg32[q]);
+  } else {
+    int32_t *gdst = out.grid + e0 * cells;
+    for (int i = lane; i < kc * cells; i += 32) gdst[i] = wg[i];
+  }
+  if (env_ok && a == 0) {
+    out.step_count[e] = sc;
+    out.key[2 * e] = k0;
+    out.key[2 * e + 1] = k1;
+  }
+  if (agent) {
+    const long long ga = e * N + a;
+    reinterpret_cast<int2 *>(out.position)[ga] = make_int2(pos >> 8, pos & 255);
+    reinterpret_cast<int2 *>(out.target)[ga] = make_int2(tgt >> 8, tgt & 255);
+    reinterpret_cast<int2 *>(out.start)[ga] = make_int2(start >> 8, start & 255);
+    out.agent_id[ga] = a;
+  }
+}
+
+// ---------------------------------------------------------------------------
 // env_warp_kernel: one Connector step (or observe) per WARP.  A warp owns K = 32 / Np envs
 // (Np = lanes per env, the next power of two >= N; lane = (env, agent)), keeps their
 // grids in its own slice of shared memory and runs every phase with __syncwarp only,
@@ -70,8 +231,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) env_warp_kernel(co
   const int Np = p.Np, K = 32 / Np, c4 = cells >> 2;
   const int RS = obs_lut_stride(N);
   uint8_t *lut = smem_raw;
-  for (int a = warp; a < N; a += EW_WARPS)
-    for (int v = lane; v < RS; v += 32) lut[a * RS + v] = v <= 3 * N ? (uint8_t)obs_value(v, 3 * a, 3 * N) : (uint8_t)0;
+  build_obs_lut(lut, N, RS, warp, EW_WARPS, lane);
   __syncthreads();  // the only CTA-wide barrier
 
   const long long e0 = ((long long)blockIdx.x * EW_WARPS + warp) * K;
@@ -90,25 +250,8 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) env_warp_kernel(co
   const long long e = e0 + (env_ok ? j : 0);
   const uint32_t gmask = Np == 32 ? FULL : (((1u << Np) - 1u) << (j * Np));
 
-  // ---- load: State.grid int32 -> uint8 (one packed word per int4), agent and env scalars
-  if (VEC) {
-    // four loads in flight per lane before the first one is used (a load-use pair per iteration
-    // made a warp pay one L2 round trip per 32 words: 19 % of the kernel's stall samples)
-    const int4 *src = reinterpret_cast<const int4 *>(p.in.grid) + e0 * c4;
-    const int nq = kc * c4;
-    for (int q0 = lane; q0 < nq; q0 += 128) {
-      int4 v[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) v[u] = (q0 + 32 * u < nq) ? __ldg(src + q0 + 32 * u) : make_int4(0, 0, 0, 0);
-#pragma unroll
-      for (int u = 0; u < 4; ++u)
-        if (q0 + 32 * u < nq)
-          wg32[q0 + 32 * u] = (uint32_t)(v[u].x & 0xff) | ((uint32_t)(v[u].y & 0xff) << 8) | ((uint32_t)(v[u].z & 0xff) << 16) | ((uint32_t)(v[u].w & 0xff) << 24);
-    }
-  } else {
-    const int32_t *src = p.in.grid + e0 * cells;
-    for (int i = lane; i < kc * cells; i += 32) wg[i] = (uint8_t)__ldg(src + i);
-  }
+  // ---- load: State.grid int32 -> uint8, agent and env scalars
+  load_grids<VEC>(p.in.grid, e0, kc, cells, lane, wg);
   int pos = 0, tgt = 0, action = 0, sc0 = 0;
   uint32_t k0 = 0, k1 = 0;
   if (agent) {
@@ -130,19 +273,12 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) env_warp_kernel(co
   uint8_t *g = wg + (size_t)j * cells;
   const SmemGrid sg{g, G, 0, G};
   // PATH cells of the env before the move (extras: total_path_length)
-  int paths = 0;
-  if (env_ok) {
-    if (VEC) {
-      for (int q = a; q < c4; q += Np) paths += count_path_codes(wg32[j * c4 + q]);
-    } else {
-      for (int i = a; i < cells; i += Np) paths += (g[i] % 3u == 1u) ? 1 : 0;
-    }
-  }
-  for (int off = Np >> 1; off; off >>= 1) paths += __shfl_xor_sync(FULL, paths, off);
+  const int paths = count_paths<VEC>(wg, j, a, cells, c4, Np, env_ok);
 
   // ---- agents: (sample action,) move_position, is_valid_position, collisions
   const bool was = agent && pos == tgt;
-  int r = pos >> 8, c = pos & 255, dest = -1;
+  const int r = pos >> 8, c = pos & 255;
+  int dest = -1;
   if (is_step && agent) {
     if (p.random_policy) {
       const uint32_t mk = move_mask(sg, r, c, a, was);
@@ -176,18 +312,12 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) env_warp_kernel(co
   __syncwarp();
 
   // ---- action mask, connected / done, reward on the new grid
-  const bool now = agent && pos == tgt;
-  uint32_t mk3 = 0;
-  if (agent) mk3 = move_mask(sg, pos >> 8, pos & 255, a, now);
-  const bool done = now || mk3 == 0u;  // connected_or_blocked
-  const float rew = __fadd_rn(__fmul_rn(p.env.connected_reward, (!was && now) ? 1.0f : 0.0f), __fmul_rn(p.env.timestep_reward, was ? 0.0f : 1.0f));
-  const int ndone = __popc(__ballot_sync(FULL, agent && done) & gmask);
-  const int nconn = __popc(__ballot_sync(FULL, now) & gmask);
-  const int nmoved = __popc(__ballot_sync(FULL, win) & gmask);
+  const StepResult s = after_move(sg, agent, a, pos, tgt, was, win, gmask, p.env);
+  uint32_t mk3 = s.mk3;
 
   // ---- per env: termination, auto-reset bookkeeping (group-uniform values)
   const int sc = sc0 + (is_step ? 1 : 0);
-  const bool terminal = is_step && env_ok && (ndone == N || sc >= p.env.time_limit);
+  const bool terminal = is_step && env_ok && (s.ndone == N || sc >= p.env.time_limit);
   int tflag = terminal ? 1 : 0;
   // The cache entry may be REPLACED by the previous step's refill, which this kernel runs under, e.g. when a
   // State is stepped twice (functional use, inplace=False) or two batches share a workspace.  The entry is
@@ -271,9 +401,9 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) env_warp_kernel(co
   // ---- small outputs
   if (env_ok && a == 0) {
     p.ts.step_type[e] = (int8_t)(is_step ? (terminal ? 2 : 1) : 0);
-    p.ts.num_connections[e] = nconn;
-    p.ts.ratio_connections[e] = __fdiv_rn((float)nconn, (float)N);
-    p.ts.total_path_length[e] = paths + nmoved + N;
+    p.ts.num_connections[e] = s.nconn;
+    p.ts.ratio_connections[e] = __fdiv_rn((float)s.nconn, (float)N);
+    p.ts.total_path_length[e] = paths + s.nmoved + N;
     if (!(tflag & 2)) p.ts.obs_step_count[e] = (tflag & 4) ? 0 : sc;
     if (is_step) {
       p.out.step_count[e] = (tflag & 4) ? 0 : sc;
@@ -285,8 +415,8 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) env_warp_kernel(co
   }
   if (agent) {
     const long long ga = e * N + a;
-    p.ts.reward[ga] = is_step ? rew : 0.0f;
-    p.ts.discount[ga] = is_step ? ((terminal || done) ? 0.0f : 1.0f) : 1.0f;
+    p.ts.reward[ga] = is_step ? s.rew : 0.0f;
+    p.ts.discount[ga] = is_step ? ((terminal || s.done) ? 0.0f : 1.0f) : 1.0f;
     if (!(tflag & 2)) store_mask5(p.ts.action_mask + ga * 5, mk3);
     if (is_step) {
       const int2 pos2 = make_int2(pos >> 8, pos & 255);
@@ -303,7 +433,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) env_warp_kernel(co
     }
   }
 
-  // ---- bulk outputs: State.grid and observation.grid (see env_kernel phase 4)
+  // ---- bulk outputs: State.grid and observation.grid
   const uint32_t skipm = __ballot_sync(FULL, a == 0 && (tflag & 2));  // bit j*Np: env j is rewritten by the reset kernel
   const uint32_t hitm = __ballot_sync(FULL, a == 0 && (tflag & 4));
   if (VEC) {
@@ -367,8 +497,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kRolloutMinCtas) rollout_warp_k
   const int Np = p.Np, K = 32 / Np, c4 = cells >> 2;
   constexpr int RS = OBS_RS;
   uint8_t *lut = smem_raw;
-  for (int a = warp; a < N; a += EW_WARPS)
-    for (int v = lane; v < RS; v += 32) lut[a * RS + v] = v <= 3 * N ? (uint8_t)obs_value(v, 3 * a, 3 * N) : (uint8_t)0;
+  build_obs_lut(lut, N, RS, warp, EW_WARPS, lane);
   float *ratio_lut = reinterpret_cast<float *>(smem_raw + rp.ratio_off);  // n / N for n = 0..N (extras: ratio_connections)
   if (tid <= N) ratio_lut[tid] = __fdiv_rn((float)tid, (float)N);
   __syncthreads();  // the only CTA-wide barrier
@@ -385,24 +514,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kRolloutMinCtas) rollout_warp_k
   const uint32_t gmask = Np == 32 ? FULL : (((1u << Np) - 1u) << (j * Np));
 
   // ---- load the State once
-  if (VEC) {
-    // four loads in flight per lane before the first one is used (a load-use pair per iteration
-    // made a warp pay one L2 round trip per 32 words: 19 % of the kernel's stall samples)
-    const int4 *src = reinterpret_cast<const int4 *>(p.in.grid) + e0 * c4;
-    const int nq = kc * c4;
-    for (int q0 = lane; q0 < nq; q0 += 128) {
-      int4 v[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) v[u] = (q0 + 32 * u < nq) ? __ldg(src + q0 + 32 * u) : make_int4(0, 0, 0, 0);
-#pragma unroll
-      for (int u = 0; u < 4; ++u)
-        if (q0 + 32 * u < nq)
-          wg32[q0 + 32 * u] = (uint32_t)(v[u].x & 0xff) | ((uint32_t)(v[u].y & 0xff) << 8) | ((uint32_t)(v[u].z & 0xff) << 16) | ((uint32_t)(v[u].w & 0xff) << 24);
-    }
-  } else {
-    const int32_t *src = p.in.grid + e0 * cells;
-    for (int i = lane; i < kc * cells; i += 32) wg[i] = (uint8_t)__ldg(src + i);
-  }
+  load_grids<VEC>(p.in.grid, e0, kc, cells, lane, wg);
   int pos = 0, tgt = 0, start = 0, sc = 0;
   uint32_t k0 = 0, k1 = 0;
   if (agent) {
@@ -421,15 +533,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kRolloutMinCtas) rollout_warp_k
   __syncwarp();
   uint8_t *g = wg + (size_t)j * cells;
   const SmemGrid sg{g, G, 0, G};
-  int paths = 0;  // PATH cells of the env (extras: total_path_length), carried across steps
-  if (env_ok) {
-    if (VEC) {
-      for (int q = a; q < c4; q += Np) paths += count_path_codes(wg32[j * c4 + q]);
-    } else {
-      for (int i = a; i < cells; i += Np) paths += (g[i] % 3u == 1u) ? 1 : 0;
-    }
-  }
-  for (int off = Np >> 1; off; off >>= 1) paths += __shfl_xor_sync(FULL, paths, off);
+  int paths = count_paths<VEC>(wg, j, a, cells, c4, Np, env_ok);  // carried across steps
   // the action mask of the state an env is in: what step t emits is what step t+1's policy samples from
   uint32_t mk3 = 0;
   if (agent) mk3 = move_mask(sg, pos >> 8, pos & 255, a, pos == tgt);
@@ -450,37 +554,15 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kRolloutMinCtas) rollout_warp_k
     const bool was = agent && pos == tgt;
     const int r = pos >> 8, c = pos & 255;
     const long long row_e = tb + e, row_a = row_e * N + a;  // this lane's rows in the stacked per-env / per-agent outputs
-    int dest = -1;
-    if (agent) {
-      // the action comes from mk3 = is_valid_position of the four moves on this very grid (empty mask
-      // for a connected agent), so a non-NOOP action needs no second validity test
-      const int action = random_action(k0, k1, (uint32_t)sc, (uint32_t)a, mk3);
-      if (rp.action_out) rp.action_out[row_a] = action;
-      if (action != NOOP) dest = r * G + c + (action == UP ? -G : (action == DOWN ? G : (action == RIGHT ? 1 : -1)));
-    }
-    const uint32_t mval = dest >= 0 ? (((uint32_t)j << 16) | (uint32_t)dest) : (0x80000000u | (uint32_t)lane);
-    const uint32_t mm = __match_any_sync(FULL, mval);
-    const bool win = dest >= 0 && lane == 31 - __clz(mm);
-    __syncwarp();
-    if (win) {
-      g[r * G + c] = (uint8_t)(3 * a + PATH);
-      g[dest] = (uint8_t)(3 * a + POSITION);
-      uint32_t nr, nc;
-      p.divG.divmod((uint32_t)dest, nr, nc);
-      pos = (int)((nr << 8) | nc);
-    }
-    __syncwarp();
+    const int dest = agent ? random_dest(k0, k1, sc, a, mk3, r, c, G, rp.action_out, row_a) : -1;
+    bool win;
+    pos = resolve_moves(dest, j, lane, a, r, c, G, g, p.divG, pos, win);
     // ---- action mask, connected / done, reward on the new grid
-    const bool now = agent && pos == tgt;
-    mk3 = 0;
-    if (agent) mk3 = move_mask(sg, pos >> 8, pos & 255, a, now);
-    const bool done = now || mk3 == 0u;
-    const float rew = __fadd_rn(__fmul_rn(p.env.connected_reward, (!was && now) ? 1.0f : 0.0f), __fmul_rn(p.env.timestep_reward, was ? 0.0f : 1.0f));
-    const int ndone = __popc(__ballot_sync(FULL, agent && done) & gmask);
-    const int nconn = __popc(__ballot_sync(FULL, now) & gmask);
-    paths += __popc(__ballot_sync(FULL, win) & gmask);
+    const StepResult s = after_move(sg, agent, a, pos, tgt, was, win, gmask, p.env);
+    mk3 = s.mk3;
+    paths += s.nmoved;
     sc += 1;
-    const bool terminal = env_ok && (ndone == N || sc >= p.env.time_limit);
+    const bool terminal = env_ok && (s.ndone == N || sc >= p.env.time_limit);
     const int tpl = paths + N;
 
     // ---- auto-reset: the dataset board that follows
@@ -501,17 +583,16 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kRolloutMinCtas) rollout_warp_k
     // ---- small outputs of step t (terminal step's reward / discount / step_type / extras)
     if (env_ok && a == 0) {
       p.ts.step_type[row_e] = (int8_t)(terminal ? 2 : 1);
-      p.ts.num_connections[row_e] = nconn;
-      p.ts.ratio_connections[row_e] = ratio_lut[nconn];
+      p.ts.num_connections[row_e] = s.nconn;
+      p.ts.ratio_connections[row_e] = ratio_lut[s.nconn];
       p.ts.total_path_length[row_e] = tpl;
       p.ts.obs_step_count[row_e] = terminal ? 0 : sc;
     }
     if (agent) {
-      p.ts.reward[row_a] = rew;
-      p.ts.discount[row_a] = (terminal || done) ? 0.0f : 1.0f;
+      p.ts.reward[row_a] = s.rew;
+      p.ts.discount[row_a] = (terminal || s.done) ? 0.0f : 1.0f;
     }
-    if (terminal) {  // group-uniform: swap in the new episode (pins-only grid, heads then targets)
-      for (int i = a; i < cells; i += Np) g[i] = 0;
+    if (terminal) {  // group-uniform: swap in the new episode
       pos = npos;
       tgt = ntgt;
       start = npos;
@@ -519,12 +600,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kRolloutMinCtas) rollout_warp_k
       k1 = nk1;
       sc = 0;
       paths = 0;
-      __syncwarp(gmask);
-      if (a < N) g[(pos >> 8) * G + (pos & 255)] = (uint8_t)(3 * a + POSITION);
-      __syncwarp(gmask);
-      if (a < N) g[(tgt >> 8) * G + (tgt & 255)] = (uint8_t)(3 * a + TARGET);
-      __syncwarp(gmask);
-      if (a < N) mk3 = move_mask(sg, pos >> 8, pos & 255, a, pos == tgt);
+      mk3 = place_episode(g, sg, a, N, Np, cells, G, gmask, pos, tgt, mk3, [] {});
     }
     __syncwarp();
     if (agent) store_mask5(p.ts.action_mask + row_a * 5, mk3);
@@ -537,38 +613,13 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kRolloutMinCtas) rollout_warp_k
       else
         os.emit_direct(lut, wg32, kc, N, c4, lane, odst);
     } else {
-      int32_t *odst = p.ts.obs_grid + (tb + e0) * N * cells;
-      for (int i = lane; i < kc * cells; i += 32) {
-        const int m = (int)p.divCells.div((uint32_t)i);
-        const uint32_t v = wg[i];
-        int32_t *o = odst + (size_t)m * N * cells + (i - m * cells);
-        for (int x = 0; x < N; ++x, o += cells) *o = lut[x * RS + v];
-      }
+      write_obs_scalar(p.ts.obs_grid + (tb + e0) * N * cells, wg, lut, RS, kc, cells, N, Np, 0u, p.divCells, lane);
     }
     __syncwarp();  // the next step's writes must not overtake these reads
   }
 
-  // ---- write the State once
-  if (VEC) {
-    if (OBS == 2) os.drain(lane);
-    int4 *gdst = reinterpret_cast<int4 *>(p.out.grid) + e0 * c4;
-    for (int q = lane; q < kc * c4; q += 32) gdst[q] = bytes_to_int4(wg32[q]);
-  } else {
-    int32_t *gdst = p.out.grid + e0 * cells;
-    for (int i = lane; i < kc * cells; i += 32) gdst[i] = wg[i];
-  }
-  if (env_ok && a == 0) {
-    p.out.step_count[e] = sc;
-    p.out.key[2 * e] = k0;
-    p.out.key[2 * e + 1] = k1;
-  }
-  if (agent) {
-    const long long ga = e * N + a;
-    reinterpret_cast<int2 *>(p.out.position)[ga] = make_int2(pos >> 8, pos & 255);
-    reinterpret_cast<int2 *>(p.out.target)[ga] = make_int2(tgt >> 8, tgt & 255);
-    reinterpret_cast<int2 *>(p.out.start)[ga] = make_int2(start >> 8, start & 255);
-    p.out.agent_id[ga] = a;
-  }
+  if (OBS == 2) os.drain(lane);
+  write_state_once<VEC>(p.out, wg, e0, kc, cells, lane, e, N, a, env_ok, agent, pos, tgt, start, sc, k0, k1);
 }
 
 // ---------------------------------------------------------------------------
@@ -624,8 +675,7 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, kPersistMinCtas)
   constexpr int RS = OBS_RS;
   uint8_t *lut = smem_raw;
   const int nthreads = blockDim.x, nwarps = nthreads >> 5;
-  for (int a = warp; a < N; a += nwarps)
-    for (int v = lane; v < RS; v += 32) lut[a * RS + v] = v <= 3 * N ? (uint8_t)obs_value(v, 3 * a, 3 * N) : (uint8_t)0;
+  build_obs_lut(lut, N, RS, warp, nwarps, lane);
   float *ratio_lut = reinterpret_cast<float *>(smem_raw + rp.ratio_off);  // n / N for n = 0..N (extras: ratio_connections)
   if (tid <= N) ratio_lut[tid] = __fdiv_rn((float)tid, (float)N);
   uint8_t *tmpl = smem_raw + pp.tmpl_off;
@@ -689,22 +739,7 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, kPersistMinCtas)
     __syncwarp();
 
     // ---- load the State once
-    if (VEC) {
-      const int4 *src = reinterpret_cast<const int4 *>(p.in.grid) + e0 * c4;
-      const int nq = kc * c4;
-      for (int q0 = lane; q0 < nq; q0 += 128) {
-        int4 v[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) v[u] = (q0 + 32 * u < nq) ? __ldg(src + q0 + 32 * u) : make_int4(0, 0, 0, 0);
-#pragma unroll
-        for (int u = 0; u < 4; ++u)
-          if (q0 + 32 * u < nq)
-            wg32[q0 + 32 * u] = (uint32_t)(v[u].x & 0xff) | ((uint32_t)(v[u].y & 0xff) << 8) | ((uint32_t)(v[u].z & 0xff) << 16) | ((uint32_t)(v[u].w & 0xff) << 24);
-      }
-    } else {
-      const int32_t *src = p.in.grid + e0 * cells;
-      for (int i = lane; i < kc * cells; i += 32) wg[i] = (uint8_t)__ldg(src + i);
-    }
+    load_grids<VEC>(p.in.grid, e0, kc, cells, lane, wg);
     int pos = 0, tgt = 0, start = 0, sc = 0;
     uint32_t k0 = 0, k1 = 0;
     if (agent) {
@@ -726,15 +761,7 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, kPersistMinCtas)
       }
     }
     __syncwarp();
-    int paths = 0;  // PATH cells of the env (extras: total_path_length), carried across steps
-    if (env_ok) {
-      if (VEC) {
-        for (int q = a; q < c4; q += Np) paths += count_path_codes(wg32[j * c4 + q]);
-      } else {
-        for (int i = a; i < cells; i += Np) paths += (g[i] % 3u == 1u) ? 1 : 0;
-      }
-    }
-    for (int off = Np >> 1; off; off >>= 1) paths += __shfl_xor_sync(FULL, paths, off);
+    int paths = count_paths<VEC>(wg, j, a, cells, c4, Np, env_ok);  // carried across steps
     uint32_t mk3 = 0;  // the action mask of the state an env is in: what step t emits is what step t+1's policy samples from
     if (agent) mk3 = move_mask(sg, pos >> 8, pos & 255, a, pos == tgt);
     int4 *obs_t = nullptr;
@@ -750,47 +777,27 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, kPersistMinCtas)
       const bool was = agent && pos == tgt;
       const int r = pos >> 8, c = pos & 255;
       const long long row_e = tb + e, row_a = row_e * N + a;
-      int dest = -1;
-      if (agent) {
-        const int action = random_action(k0, k1, (uint32_t)sc, (uint32_t)a, mk3);
-        if (rp.action_out) rp.action_out[row_a] = action;
-        if (action != NOOP) dest = r * G + c + (action == UP ? -G : (action == DOWN ? G : (action == RIGHT ? 1 : -1)));
-      }
-      const uint32_t mval = dest >= 0 ? (((uint32_t)j << 16) | (uint32_t)dest) : (0x80000000u | (uint32_t)lane);
-      const uint32_t mm = __match_any_sync(FULL, mval);
-      const bool win = dest >= 0 && lane == 31 - __clz(mm);
-      __syncwarp();
-      if (win) {
-        g[r * G + c] = (uint8_t)(3 * a + PATH);
-        g[dest] = (uint8_t)(3 * a + POSITION);
-        uint32_t nr, nc;
-        p.divG.divmod((uint32_t)dest, nr, nc);
-        pos = (int)((nr << 8) | nc);
-      }
-      __syncwarp();
+      const int dest = agent ? random_dest(k0, k1, sc, a, mk3, r, c, G, rp.action_out, row_a) : -1;
+      bool win;
+      pos = resolve_moves(dest, j, lane, a, r, c, G, g, p.divG, pos, win);
       // ---- action mask, connected / done, reward on the new grid
-      const bool now = agent && pos == tgt;
-      mk3 = 0;
-      if (agent) mk3 = move_mask(sg, pos >> 8, pos & 255, a, now);
-      const bool done = now || mk3 == 0u;
-      const float rew = __fadd_rn(__fmul_rn(p.env.connected_reward, (!was && now) ? 1.0f : 0.0f), __fmul_rn(p.env.timestep_reward, was ? 0.0f : 1.0f));
-      const int ndone = __popc(__ballot_sync(FULL, agent && done) & gmask);
-      const int nconn = __popc(__ballot_sync(FULL, now) & gmask);
-      paths += __popc(__ballot_sync(FULL, win) & gmask);
+      const StepResult s = after_move(sg, agent, a, pos, tgt, was, win, gmask, p.env);
+      mk3 = s.mk3;
+      paths += s.nmoved;
       sc += 1;
-      const bool terminal = env_ok && (ndone == N || sc >= p.env.time_limit);
+      const bool terminal = env_ok && (s.ndone == N || sc >= p.env.time_limit);
       const int tpl = paths + N;
       // ---- small outputs of step t (the terminal step keeps its reward / discount / step_type / extras)
       if (env_ok && a == 0) {
         p.ts.step_type[row_e] = (int8_t)(terminal ? 2 : 1);
-        p.ts.num_connections[row_e] = nconn;
-        p.ts.ratio_connections[row_e] = ratio_lut[nconn];
+        p.ts.num_connections[row_e] = s.nconn;
+        p.ts.ratio_connections[row_e] = ratio_lut[s.nconn];
         p.ts.total_path_length[row_e] = tpl;
         p.ts.obs_step_count[row_e] = terminal ? 0 : sc;
       }
       if (agent) {
-        p.ts.reward[row_a] = rew;
-        p.ts.discount[row_a] = (terminal || done) ? 0.0f : 1.0f;
+        p.ts.reward[row_a] = s.rew;
+        p.ts.discount[row_a] = (terminal || s.done) ? 0.0f : 1.0f;
       }
       // ---- auto-reset: the env's cached next episode; its generator warp may still be working on it
       if (terminal) {  // group-uniform
@@ -804,7 +811,6 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, kPersistMinCtas)
         if (a != 0) (void)ld_acquire_u64(p.cache_tag + e);  // every lane orders its own reads behind the published tag
         const uint2 nk = __ldcg(p.cache_key + e);
         const uint32_t pin = a < N ? __ldcg(p.cache_pins + e * N + a) : 0u;
-        for (int i = a; i < cells; i += Np) g[i] = 0;
         pos = (int)(pin >> 16);
         tgt = (int)(pin & 0xffffu);
         start = pos;
@@ -812,16 +818,12 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, kPersistMinCtas)
         k1 = nk.y;
         sc = 0;
         paths = 0;
-        if (a == 0) {  // the episode after this one
-          atomicAdd(pp.group_pending + grp, 1);
-          genq_post(myq, (int)e, k0, k1);
-        }
-        __syncwarp(gmask);
-        if (a < N) g[(pos >> 8) * G + (pos & 255)] = (uint8_t)(3 * a + POSITION);
-        __syncwarp(gmask);
-        if (a < N) g[(tgt >> 8) * G + (tgt & 255)] = (uint8_t)(3 * a + TARGET);
-        __syncwarp(gmask);
-        if (a < N) mk3 = move_mask(sg, pos >> 8, pos & 255, a, pos == tgt);
+        mk3 = place_episode(g, sg, a, N, Np, cells, G, gmask, pos, tgt, mk3, [a, e, k0, k1, myq, pending = pp.group_pending + grp] {
+          if (a == 0) {  // the episode after this one
+            atomicAdd(pending, 1);
+            genq_post(myq, (int)e, k0, k1);
+          }
+        });
       }
       __syncwarp();
       if (agent) store_mask5(p.ts.action_mask + row_a * 5, mk3);
@@ -834,37 +836,12 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, kPersistMinCtas)
         else
           os.emit_direct(lut, wg32, kc, N, c4, lane, odst);
       } else {
-        int32_t *odst = p.ts.obs_grid + (tb + e0) * N * cells;
-        for (int i = lane; i < kc * cells; i += 32) {
-          const int m = (int)p.divCells.div((uint32_t)i);
-          const uint32_t v = wg[i];
-          int32_t *o = odst + (size_t)m * N * cells + (i - m * cells);
-          for (int x = 0; x < N; ++x, o += cells) *o = lut[x * RS + v];
-        }
+        write_obs_scalar(p.ts.obs_grid + (tb + e0) * N * cells, wg, lut, RS, kc, cells, N, Np, 0u, p.divCells, lane);
       }
       __syncwarp();  // the next step's writes must not overtake these reads
     }
 
-    // ---- write the State once
-    if (VEC) {
-      int4 *gdst = reinterpret_cast<int4 *>(p.out.grid) + e0 * c4;
-      for (int q = lane; q < kc * c4; q += 32) gdst[q] = bytes_to_int4(wg32[q]);
-    } else {
-      int32_t *gdst = p.out.grid + e0 * cells;
-      for (int i = lane; i < kc * cells; i += 32) gdst[i] = wg[i];
-    }
-    if (env_ok && a == 0) {
-      p.out.step_count[e] = sc;
-      p.out.key[2 * e] = k0;
-      p.out.key[2 * e + 1] = k1;
-    }
-    if (agent) {
-      const long long ga = e * N + a;
-      reinterpret_cast<int2 *>(p.out.position)[ga] = make_int2(pos >> 8, pos & 255);
-      reinterpret_cast<int2 *>(p.out.target)[ga] = make_int2(tgt >> 8, tgt & 255);
-      reinterpret_cast<int2 *>(p.out.start)[ga] = make_int2(start >> 8, start & 255);
-      p.out.agent_id[ga] = a;
-    }
+    write_state_once<VEC>(p.out, wg, e0, kc, cells, lane, e, N, a, env_ok, agent, pos, tgt, start, sc, k0, k1);
     // the group's State is written (the observation copies of its last steps may still be in flight: nothing
     // of a later launch depends on them); requests posted above were counted before this store
     __threadfence();
@@ -909,26 +886,61 @@ __global__ void __launch_bounds__(256) random_actions_kernel(rbg_state st, long 
   action[t] = random_action(st.key[2 * e], st.key[2 * e + 1], (uint32_t)st.step_count[e], (uint32_t)a, mk);
 }
 
-int launch_env(EnvParams p, cudaStream_t stream, bool pdl) {
-  const int G = p.G, N = p.N;
-  p.cells = G * G;
-  const bool vec = (p.cells & 3) == 0;
-  p.divN = FastDiv::make((uint32_t)N);
-  p.divG = FastDiv::make((uint32_t)G);
-  p.divC4 = FastDiv::make((uint32_t)(vec ? p.cells >> 2 : 1));
-  p.divCells = FastDiv::make((uint32_t)p.cells);
-  if (p.B <= 0) return RBG_OK;
-  int Np = 1;
-  while (Np < N) Np <<= 1;
-  p.Np = Np;
-  const int K = 32 / Np;
-  p.E = EW_WARPS * K;
-  const size_t lutB = ((size_t)N * obs_lut_stride(N) + 256 + 15) & ~(size_t)15;
-  const size_t wgrid = ((size_t)K * p.cells + 15) & ~(size_t)15;
+static size_t up16(size_t x) { return (x + 15) & ~(size_t)15; }
+
+// What every launcher of the warp-per-K-envs kernels derives from G and N: Np lanes per env (the next power of two
+// >= N), K = 32 / Np envs per warp, the bytes of one warp's grid slice and the kernels' divisors.
+struct WarpShape {
+  int cells, Np, K;
+  size_t wgrid;
+  FastDiv divG, divC4, divCells;
+  bool vec() const { return (cells & 3) == 0; }
+};
+
+static WarpShape warp_shape(int G, int N) {
+  WarpShape s;
+  s.cells = G * G;
+  s.Np = 1;
+  while (s.Np < N) s.Np <<= 1;
+  s.K = 32 / s.Np;
+  s.wgrid = up16((size_t)s.K * s.cells);
+  s.divG = FastDiv::make((uint32_t)G);
+  s.divC4 = FastDiv::make((uint32_t)(s.vec() ? s.cells >> 2 : 1));
+  s.divCells = FastDiv::make((uint32_t)s.cells);
+  return s;
+}
+
+// bytes of an observation table of N rows RS bytes apart, with 256 bytes to spare
+static size_t lut_bytes(int N, int RS) { return up16((size_t)N * RS + 256); }
+
+// EnvParams / EvalStepParams: the shape fields and the shared-memory offsets {table, grid slice}
+template <class P>
+static void set_warp_shape(P &p, const WarpShape &s, size_t lutB) {
+  p.cells = s.cells;
+  p.Np = s.Np;
+  p.divG = s.divG;
+  p.divC4 = s.divC4;
+  p.divCells = s.divCells;
   p.so[0] = (int)lutB;
-  p.so[1] = (int)wgrid;
-  const size_t smem = lutB + EW_WARPS * wgrid;
-  const int64_t ctas = (p.B + p.E - 1) / p.E;
+  p.so[1] = (int)s.wgrid;
+}
+
+// a kernel that needs more than the default 48 KB of dynamic shared memory per CTA has to opt in
+static int allow_smem(const void *fn, size_t smem, const char *what) {
+  cudaError_t ce;
+  if (smem > 48 * 1024 && (ce = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+    return set_cuda_error(ce, what);
+  return RBG_OK;
+}
+
+int launch_env(EnvParams p, cudaStream_t stream, bool pdl) {
+  if (p.B <= 0) return RBG_OK;
+  const WarpShape s = warp_shape(p.G, p.N);
+  const size_t lutB = lut_bytes(p.N, obs_lut_stride(p.N));
+  set_warp_shape(p, s, lutB);
+  const size_t smem = lutB + EW_WARPS * s.wgrid;
+  const int64_t E = EW_WARPS * s.K;  // envs per CTA
+  const int64_t ctas = (p.B + E - 1) / E;
   LaunchScope scope(RBG_K_ENV, stream);
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
@@ -941,7 +953,7 @@ int launch_env(EnvParams p, cudaStream_t stream, bool pdl) {
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = pdl ? 1 : 0;
-  cudaError_t ce = vec ? cudaLaunchKernelEx(&cfg, env_warp_kernel<true>, p) : cudaLaunchKernelEx(&cfg, env_warp_kernel<false>, p);
+  cudaError_t ce = cudaLaunchKernelEx(&cfg, s.vec() ? env_warp_kernel<true> : env_warp_kernel<false>, p);
   if (ce != cudaSuccess) return set_cuda_error(ce, "cudaLaunchKernelEx(env_warp_kernel)");
   return check_launch("env_warp_kernel");
 }
@@ -968,28 +980,17 @@ static size_t balance_waves(int64_t ctas, int cmax, int cmin, size_t smem_needed
 }
 
 int launch_rollout(EnvParams p, int T, int32_t *action_out, cudaStream_t stream) {
-  const int G = p.G, N = p.N;
-  p.cells = G * G;
-  const bool vec = (p.cells & 3) == 0;
-  p.divN = FastDiv::make((uint32_t)N);
-  p.divG = FastDiv::make((uint32_t)G);
-  p.divC4 = FastDiv::make((uint32_t)(vec ? p.cells >> 2 : 1));
-  p.divCells = FastDiv::make((uint32_t)p.cells);
   if (p.B <= 0 || T <= 0) return RBG_OK;
-  int Np = 1;
-  while (Np < N) Np <<= 1;
-  p.Np = Np;
-  const int K = 32 / Np;
-  p.E = EW_WARPS * K;
-  const size_t lutB = ((size_t)N * OBS_RS + 256 + 15) & ~(size_t)15;
-  const size_t wgrid = ((size_t)K * p.cells + 15) & ~(size_t)15;
-  p.so[0] = (int)lutB;
-  p.so[1] = (int)wgrid;
+  const WarpShape s = warp_shape(p.G, p.N);
+  const int N = p.N, K = s.K;
+  const bool vec = s.vec();
+  const size_t lutB = lut_bytes(N, OBS_RS);
+  set_warp_shape(p, s, lutB);
   RolloutParams rp;
   rp.T = T;
   rp.action_out = action_out;
-  rp.ratio_off = (int)(lutB + EW_WARPS * wgrid);
-  size_t smem = (((size_t)rp.ratio_off + 4 * (RBG_MAX_N + 4)) + 15) & ~(size_t)15;
+  rp.ratio_off = (int)(lutB + EW_WARPS * s.wgrid);
+  size_t smem = up16((size_t)rp.ratio_off + 4 * (RBG_MAX_N + 4));
   rp.stage_off = (int)smem;
   rp.stage_bytes = 0;
   rp.stage_nbuf = 1;
@@ -997,32 +998,28 @@ int launch_rollout(EnvParams p, int T, int32_t *action_out, cudaStream_t stream)
   rp.ce = 1;
   rp.cv = N;
   if (vec) {
-    const ObsStagePlan pl = obs_stage_plan(K, N, p.cells, 4096, 8192);
+    const ObsStagePlan pl = obs_stage_plan(K, N, s.cells, 4096, 8192);
     rp.stage_bytes = pl.bytes;
     rp.stage_nbuf = pl.nbuf;
     rp.ce = pl.ce;
     rp.cv = pl.cv;
-    rp.stage_warp = (rp.stage_nbuf * rp.stage_bytes + 15) & ~15;
+    rp.stage_warp = (int)up16((size_t)rp.stage_nbuf * rp.stage_bytes);
     smem += (size_t)EW_WARPS * rp.stage_warp;
   }
   if (smem > 200 * 1024) return set_error(RBG_EINVAL, "rollout: shared memory %zu too large", smem);
-  const int64_t ctas = (p.B + p.E - 1) / p.E;
+  const int64_t E = EW_WARPS * K;  // envs per CTA
+  const int64_t ctas = (p.B + E - 1) / E;
   {  // residency: registers allow kRolloutMinCtas per SM, shared memory (1 KB reserved per CTA) maybe fewer
     int cmax = (int)(device_smem_per_sm() / (smem + 1024));
     if (cmax > kRolloutMinCtas) cmax = kRolloutMinCtas;
     if (cmax >= 3) smem = balance_waves(ctas, cmax, cmax - 2, smem);
   }
-  LaunchScope scope(RBG_K_ROLLOUT, stream);
   const bool staged = vec && rp.stage_nbuf != 0;
-  if (staged) {
-    if (smem > 48 * 1024) cudaFuncSetAttribute(rollout_warp_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    rollout_warp_kernel<2><<<(unsigned)ctas, EW_WARPS * 32, smem, stream>>>(p, rp);
-  } else if (vec) {
-    if (smem > 48 * 1024) cudaFuncSetAttribute(rollout_warp_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    rollout_warp_kernel<1><<<(unsigned)ctas, EW_WARPS * 32, smem, stream>>>(p, rp);
-  } else {
-    if (smem > 48 * 1024) cudaFuncSetAttribute(rollout_warp_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    rollout_warp_kernel<0><<<(unsigned)ctas, EW_WARPS * 32, smem, stream>>>(p, rp);
+  void (*fn)(const EnvParams, const RolloutParams) = staged ? rollout_warp_kernel<2> : (vec ? rollout_warp_kernel<1> : rollout_warp_kernel<0>);
+  if (int rc = allow_smem((const void *)fn, smem, "cudaFuncSetAttribute(rollout_warp_kernel)")) return rc;
+  {
+    LaunchScope scope(RBG_K_ROLLOUT, stream);
+    fn<<<(unsigned)ctas, EW_WARPS * 32, smem, stream>>>(p, rp);
   }
   return check_launch("rollout_warp_kernel");
 }
@@ -1031,24 +1028,12 @@ int launch_rollout(EnvParams p, int T, int32_t *action_out, cudaStream_t stream)
 // `counter` points at two zeroed ints that the kernel recycles by itself.
 int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, int32_t *counter, int32_t *group_done, int32_t *group_pending,
                            int epoch, bool overlap, uint64_t *cache_tag_w, uint2 *cache_key_w, uint32_t *cache_pins_w, cudaStream_t stream) {
-  const int G = p.G, N = p.N;
-  p.cells = G * G;
-  const bool vec = (p.cells & 3) == 0;
-  p.divN = FastDiv::make((uint32_t)N);
-  p.divG = FastDiv::make((uint32_t)G);
-  p.divC4 = FastDiv::make((uint32_t)(vec ? p.cells >> 2 : 1));
-  p.divCells = FastDiv::make((uint32_t)p.cells);
   if (p.B <= 0 || T <= 0) return RBG_OK;
-  int Np = 1;
-  while (Np < N) Np <<= 1;
-  p.Np = Np;
-  const int K = 32 / Np;
-  p.E = EW_WARPS * K;
-  auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
-  const size_t lutB = up16((size_t)N * OBS_RS + 256);
-  const size_t wgrid = up16((size_t)K * p.cells);
-  p.so[0] = (int)lutB;
-  p.so[1] = (int)wgrid;
+  const WarpShape s = warp_shape(p.G, p.N);
+  const int G = p.G, N = p.N, K = s.K;
+  const bool vec = s.vec();
+  const size_t lutB = lut_bytes(N, OBS_RS);
+  set_warp_shape(p, s, lutB);
   RolloutParams rp;
   memset(&rp, 0, sizeof(rp));
   rp.T = T;
@@ -1061,7 +1046,7 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   // 20x20/10 372 / 378, 32x32/16 94.9 / 96.8 (resets are rare per byte: packed is 2 % ahead).
   const bool isolated = G >= 9 && G <= 13 && N <= 8;
   const int PW = isolated ? 3 : EW_WARPS;
-  size_t off = lutB + PW * wgrid;
+  size_t off = lutB + PW * s.wgrid;
   rp.ratio_off = (int)off;
   off = up16(off + 4 * (RBG_MAX_N + 4));
   PersistParams pp;
@@ -1095,7 +1080,7 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   rp.ce = 1;
   rp.cv = N;
   if (vec) {
-    const ObsStagePlan pl = obs_stage_plan(K, N, p.cells, 4096, 8192);
+    const ObsStagePlan pl = obs_stage_plan(K, N, s.cells, 4096, 8192);
     rp.stage_bytes = pl.bytes;
     rp.stage_nbuf = pl.nbuf;
     rp.ce = pl.ce;
@@ -1107,10 +1092,10 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   if (smem > 200 * 1024) return set_error(RBG_EINVAL, "rollout: shared memory %zu too large", smem);
   const bool staged = vec && rp.stage_nbuf != 0;
   const int threads = (PW + pp.gen_warps) * 32;
-  const void *fn = staged ? (const void *)rollout_persist_kernel<2> : (vec ? (const void *)rollout_persist_kernel<1> : (const void *)rollout_persist_kernel<0>);
+  void (*fn)(const EnvParams, const RolloutParams, const PersistParams, const GenWarpCfg) =
+      staged ? rollout_persist_kernel<2> : (vec ? rollout_persist_kernel<1> : rollout_persist_kernel<0>);
+  if (int rc = allow_smem((const void *)fn, smem, "cudaFuncSetAttribute(rollout_persist_kernel)")) return rc;
   cudaError_t ce;
-  if (smem > 48 * 1024 && (ce = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
-    return set_cuda_error(ce, "cudaFuncSetAttribute(rollout_persist_kernel)");
   int resident = 0;
   if ((ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, fn, threads, smem)) != cudaSuccess) return set_cuda_error(ce, "cudaOccupancyMaxActiveBlocksPerMultiprocessor");
   if (resident < 1) return set_error(RBG_EINVAL, "rollout_persist_kernel does not fit an SM (%zu bytes of shared memory)", smem);
@@ -1132,13 +1117,7 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = overlap ? 1 : 0;
-  if (staged)
-    ce = cudaLaunchKernelEx(&cfg, rollout_persist_kernel<2>, p, rp, pp, gc);
-  else if (vec)
-    ce = cudaLaunchKernelEx(&cfg, rollout_persist_kernel<1>, p, rp, pp, gc);
-  else
-    ce = cudaLaunchKernelEx(&cfg, rollout_persist_kernel<0>, p, rp, pp, gc);
-  if (ce != cudaSuccess) return set_cuda_error(ce, "cudaLaunchKernelEx(rollout_persist_kernel)");
+  if ((ce = cudaLaunchKernelEx(&cfg, fn, p, rp, pp, gc)) != cudaSuccess) return set_cuda_error(ce, "cudaLaunchKernelEx(rollout_persist_kernel)");
   return check_launch("rollout_persist_kernel");
 }
 
@@ -1232,47 +1211,28 @@ __global__ void __launch_bounds__(EP_WARPS * 32, kEpisodeMinCtas) episode_warp_k
     }
     if (__ballot_sync(FULL, env_ok) == 0u) break;
 
-    // ---- one step (rollout_warp_kernel's step body): sample action, move, collisions
+    // ---- one step: sample action, move, collisions
     const bool was = agent && pos == tgt;
     const int r = pos >> 8, c = pos & 255;
-    int dest = -1;
-    if (agent) {
-      const int action = random_action(k0, k1, (uint32_t)sc, (uint32_t)a, mk3);
-      if (action != NOOP) dest = r * G + c + (action == UP ? -G : (action == DOWN ? G : (action == RIGHT ? 1 : -1)));
-    }
-    const uint32_t mval = dest >= 0 ? (((uint32_t)j << 16) | (uint32_t)dest) : (0x80000000u | (uint32_t)lane);
-    const uint32_t mm = __match_any_sync(FULL, mval);
-    const bool win = dest >= 0 && lane == 31 - __clz(mm);
-    __syncwarp();
-    if (win) {
-      g[r * G + c] = (uint8_t)(3 * a + PATH);
-      g[dest] = (uint8_t)(3 * a + POSITION);
-      uint32_t nr, nc;
-      p.divG.divmod((uint32_t)dest, nr, nc);
-      pos = (int)((nr << 8) | nc);
-    }
-    __syncwarp();
+    const int dest = agent ? random_dest(k0, k1, sc, a, mk3, r, c, G, nullptr, 0) : -1;
+    bool win;
+    pos = resolve_moves(dest, j, lane, a, r, c, G, g, p.divG, pos, win);
     // ---- action mask, connected / done, reward on the new grid
-    const bool now = agent && pos == tgt;
-    mk3 = 0;
-    if (agent) mk3 = move_mask(sg, pos >> 8, pos & 255, a, now);
-    const bool done = now || mk3 == 0u;
-    const float rew = __fadd_rn(__fmul_rn(p.connected_reward, (!was && now) ? 1.0f : 0.0f), __fmul_rn(p.timestep_reward, was ? 0.0f : 1.0f));
-    const int ndone = __popc(__ballot_sync(FULL, agent && done) & gmask);
-    const int nconn = __popc(__ballot_sync(FULL, now) & gmask);
-    paths += __popc(__ballot_sync(FULL, win) & gmask);
+    const StepResult s = after_move(sg, agent, a, pos, tgt, was, win, gmask, p);
+    mk3 = s.mk3;
+    paths += s.nmoved;
     sc += 1;
     len += 1;
-    ret = __fadd_rn(ret, rew);
-    const bool terminal = env_ok && (ndone == N || sc >= p.time_limit);
+    ret = __fadd_rn(ret, s.rew);
+    const bool terminal = env_ok && (s.ndone == N || sc >= p.time_limit);
 
     // ---- the episode's record (group-uniform)
     if (terminal) {
       if (agent) p.out.episode_return[e * N + a] = ret;
       if (a == 0) {
         p.out.episode_length[e] = len;
-        p.out.num_connections[e] = nconn;
-        p.out.ratio_connections[e] = ratio_lut[nconn];
+        p.out.num_connections[e] = s.nconn;
+        p.out.ratio_connections[e] = ratio_lut[s.nconn];
         p.out.total_path_length[e] = paths + N;
       }
       if (p.fin.grid) {  // Connector.step's State: grid, position and step_count move, the rest is the input's
@@ -1308,22 +1268,20 @@ int launch_episodes(const rbg_state &in, const rbg_state *fin, const rbg_episode
   p.B = B;
   p.G = G;
   p.N = N;
-  p.cells = G * G;
-  int Np = 1;
-  while (Np < N) Np <<= 1;
-  p.Np = Np;
+  const WarpShape s = warp_shape(G, N);
+  const int K = s.K;
+  p.cells = s.cells;
+  p.Np = s.Np;
   p.time_limit = env.time_limit;
   p.timestep_reward = env.timestep_reward;
   p.connected_reward = env.connected_reward;
-  p.divG = FastDiv::make((uint32_t)G);
-  const int K = 32 / Np;
-  p.wgrid = (int)(((size_t)K * p.cells + 15) & ~(size_t)15);
+  p.divG = s.divG;
+  p.wgrid = (int)s.wgrid;
   p.ratio_off = EP_WARPS * p.wgrid;
   const size_t smem = (size_t)p.ratio_off + 4 * (RBG_MAX_N + 4);
-  cudaError_t ce;
   // few agents on a big board: up to 4 warps x 32 envs x 1 600 cells = 200 KB (40x40/1), past the 48 KB default
-  if (smem > 48 * 1024 && (ce = cudaFuncSetAttribute(episode_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
-    return set_cuda_error(ce, "cudaFuncSetAttribute(episode_warp_kernel)");
+  if (int rc = allow_smem((const void *)episode_warp_kernel, smem, "cudaFuncSetAttribute(episode_warp_kernel)")) return rc;
+  cudaError_t ce;
   int per_sm = 0;
   if ((ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, episode_warp_kernel, EP_WARPS * 32, smem)) != cudaSuccess)
     return set_cuda_error(ce, "cudaOccupancyMaxActiveBlocksPerMultiprocessor(episode_warp_kernel)");
@@ -1390,8 +1348,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) eval_step_kernel(c
   const uint32_t livem = __ballot_sync(FULL, env_ok);  // bit j * Np (and the env's other lanes): env j is live
   if (!__syncthreads_or(livem != 0u)) return;  // a CTA without a live env builds no table
   uint8_t *lut = smem_raw;
-  for (int x = warp; x < N; x += EW_WARPS)
-    for (int v = lane; v < RS; v += 32) lut[x * RS + v] = v <= 3 * N ? (uint8_t)obs_value(v, 3 * x, 3 * N) : (uint8_t)0;
+  build_obs_lut(lut, N, RS, warp, EW_WARPS, lane);
   __syncthreads();  // the last CTA-wide barrier
   if (livem == 0u) return;
   uint8_t *wg = smem_raw + p.so[0] + (size_t)warp * p.so[1];
@@ -1435,19 +1392,12 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) eval_step_kernel(c
   uint8_t *g = wg + (size_t)j * cells;
   const SmemGrid sg{g, G, 0, G};
   // PATH cells of the env before the move (extras: total_path_length)
-  int paths = 0;
-  if (env_ok) {
-    if (VEC) {
-      for (int q = a; q < c4; q += Np) paths += count_path_codes(wg32[j * c4 + q]);
-    } else {
-      for (int i = a; i < cells; i += Np) paths += (g[i] % 3u == 1u) ? 1 : 0;
-    }
-  }
-  for (int off = Np >> 1; off; off >>= 1) paths += __shfl_xor_sync(FULL, paths, off);
+  const int paths = count_paths<VEC>(wg, j, a, cells, c4, Np, env_ok);
 
-  // ---- agents: move_position, is_valid_position, collisions
+  // ---- agents: move_position, is_valid_position, collisions; State.grid in place
   const bool was = agent && pos == tgt;
-  int r = pos >> 8, c = pos & 255, dest = -1;
+  const int r = pos >> 8, c = pos & 255;
+  int dest = -1;
   if (agent) {
     const int am = action < 0 ? 0 : (action > 4 ? 4 : action);  // lax.switch clamps
     const int nr = r + (am == UP ? -1 : (am == DOWN ? 1 : 0));
@@ -1474,30 +1424,23 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) eval_step_kernel(c
   __syncwarp();
 
   // ---- action mask, connected / done, reward on the new grid
-  const bool now = agent && pos == tgt;
-  uint32_t mk3 = 0;
-  if (agent) mk3 = move_mask(sg, pos >> 8, pos & 255, a, now);
-  const bool done = now || mk3 == 0u;  // connected_or_blocked
-  const float rew = __fadd_rn(__fmul_rn(p.connected_reward, (!was && now) ? 1.0f : 0.0f), __fmul_rn(p.timestep_reward, was ? 0.0f : 1.0f));
-  const int ndone = __popc(__ballot_sync(FULL, agent && done) & gmask);
-  const int nconn = __popc(__ballot_sync(FULL, now) & gmask);
-  const int nmoved = __popc(__ballot_sync(FULL, win) & gmask);
+  const StepResult s = after_move(sg, agent, a, pos, tgt, was, win, gmask, p);
   const int sc = sc0 + 1;
-  const bool terminal = env_ok && (ndone == N || sc >= p.time_limit);
+  const bool terminal = env_ok && (s.ndone == N || sc >= p.time_limit);
 
   // ---- TimeStep row, State scalars and the episode record of the live envs
   if (env_ok && a == 0) {
-    const float ratio = __fdiv_rn((float)nconn, (float)N);
-    const int tpl = paths + nmoved + N;
+    const float ratio = __fdiv_rn((float)s.nconn, (float)N);
+    const int tpl = paths + s.nmoved + N;
     p.ts.step_type[e] = (int8_t)(terminal ? 2 : 1);
-    p.ts.num_connections[e] = nconn;
+    p.ts.num_connections[e] = s.nconn;
     p.ts.ratio_connections[e] = ratio;
     p.ts.total_path_length[e] = tpl;
     p.ts.obs_step_count[e] = sc;
     p.st.step_count[e] = sc;
     p.acc.episode_length[e] += 1;
     if (terminal) {
-      p.acc.num_connections[e] = nconn;
+      p.acc.num_connections[e] = s.nconn;
       p.acc.ratio_connections[e] = ratio;
       p.acc.total_path_length[e] = tpl;
       p.live[e] = 0;
@@ -1505,11 +1448,11 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) eval_step_kernel(c
   }
   if (agent) {
     const long long ga = e * N + a;
-    p.ts.reward[ga] = rew;
-    p.ts.discount[ga] = (terminal || done) ? 0.0f : 1.0f;
-    store_mask5(p.ts.action_mask + ga * 5, mk3);
+    p.ts.reward[ga] = s.rew;
+    p.ts.discount[ga] = (terminal || s.done) ? 0.0f : 1.0f;
+    store_mask5(p.ts.action_mask + ga * 5, s.mk3);
     reinterpret_cast<int2 *>(p.st.position)[ga] = make_int2(pos >> 8, pos & 255);
-    p.acc.episode_return[ga] = __fadd_rn(p.acc.episode_return[ga], rew);
+    p.acc.episode_return[ga] = __fadd_rn(p.acc.episode_return[ga], s.rew);
   }
   const int nfinished = __popc(__ballot_sync(FULL, a == 0 && terminal));
   if (lane == 0 && nfinished) atomicSub(p.live_count, nfinished);
@@ -1528,14 +1471,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) eval_step_kernel(c
       for (int x = 0; x < N; ++x, o += c4, row += RS) *o = make_int4(row[b0], row[b1], row[b2], row[b3]);
     }
   } else {
-    int32_t *odst = p.ts.obs_grid + e0 * N * cells;
-    for (int i = lane; i < kc * cells; i += 32) {
-      const int m = (int)p.divCells.div((uint32_t)i);
-      if (!((livem >> (m * Np)) & 1u)) continue;
-      const uint32_t v = wg[i];
-      int32_t *o = odst + (size_t)m * N * cells + (i - m * cells);
-      for (int x = 0; x < N; ++x, o += cells) *o = lut[x * RS + v];
-    }
+    write_obs_scalar(p.ts.obs_grid + e0 * N * cells, wg, lut, RS, kc, cells, N, Np, ~livem, p.divCells, lane);
   }
 }
 
@@ -1553,29 +1489,18 @@ int launch_eval_step(const rbg_state &st, const int32_t *action, uint8_t *live, 
   p.B = B;
   p.G = G;
   p.N = N;
-  p.cells = G * G;
-  const bool vec = (p.cells & 3) == 0;
-  int Np = 1;
-  while (Np < N) Np <<= 1;
-  p.Np = Np;
   p.time_limit = env.time_limit;
   p.timestep_reward = env.timestep_reward;
   p.connected_reward = env.connected_reward;
-  p.divG = FastDiv::make((uint32_t)G);
-  p.divC4 = FastDiv::make((uint32_t)(vec ? p.cells >> 2 : 1));
-  p.divCells = FastDiv::make((uint32_t)p.cells);
-  const int K = 32 / Np;
-  const size_t lutB = ((size_t)N * obs_lut_stride(N) + 256 + 15) & ~(size_t)15;
-  const size_t wgrid = ((size_t)K * p.cells + 15) & ~(size_t)15;
-  p.so[0] = (int)lutB;
-  p.so[1] = (int)wgrid;
-  const size_t smem = lutB + EW_WARPS * wgrid;
-  const int64_t ctas = (B + (int64_t)EW_WARPS * K - 1) / ((int64_t)EW_WARPS * K);
-  void (*fn)(const EvalStepParams) = vec ? eval_step_kernel<true> : eval_step_kernel<false>;
-  cudaError_t ce;
+  const WarpShape s = warp_shape(G, N);
+  const size_t lutB = lut_bytes(N, obs_lut_stride(N));
+  set_warp_shape(p, s, lutB);
+  const size_t smem = lutB + EW_WARPS * s.wgrid;
+  const int64_t E = EW_WARPS * s.K;  // envs per CTA
+  const int64_t ctas = (B + E - 1) / E;
+  void (*fn)(const EvalStepParams) = s.vec() ? eval_step_kernel<true> : eval_step_kernel<false>;
   // few agents on a big board: up to 4 warps x 32 envs x 1 600 cells = 200 KB (40x40/1), past the 48 KB default
-  if (smem > 48 * 1024 && (ce = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
-    return set_cuda_error(ce, "cudaFuncSetAttribute(eval_step_kernel)");
+  if (int rc = allow_smem((const void *)fn, smem, "cudaFuncSetAttribute(eval_step_kernel)")) return rc;
   {
     LaunchScope scope(RBG_K_EVAL_STEP, stream);
     fn<<<(unsigned)ctas, EW_WARPS * 32, smem, stream>>>(p);

@@ -86,10 +86,10 @@ struct EnvParams {
   int32_t *refill_list;    // [B]
   int32_t *refill_count;   // [1]
   uint32_t *refill_keys;   // [B,2] State.key of the episode that just started
-  // filled by launch_env
-  int cells, E, Np;  // E envs per CTA, Np lanes per env
+  // filled by the launcher
+  int cells, E, Np;  // Np lanes per env; E is unused (deleting it moves so[] onto an 8-byte boundary, which changes the kernels' code)
   int so[2];         // shared memory: [0] bytes of the observation table, [1] bytes of one warp's grid slice
-  FastDiv divN, divG, divC4, divCells;
+  FastDiv divG, divC4, divCells;
 };
 
 // pdl: launch with programmatic stream serialization (the kernel may begin while a preceding kernel that has said
