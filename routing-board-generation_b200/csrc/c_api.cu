@@ -933,7 +933,10 @@ int rbg_connector_rollout_random(const rbg_state *state, int32_t *action_out, in
   const int kind = params->autoreset_kind;
   if (kind > RBG_GEN_SEQRW) return set_error(RBG_EINVAL, "unknown autoreset generator kind %d", kind);
   if (kind < 0) return set_error(RBG_EINVAL, "rollout needs an auto-reset generator kind (params->autoreset_kind >= 0)");
-  if (kind == RBG_GEN_DATASET) {
+  // few agents on a big board: a fused CTA's grids, staging and generator scratch do not fit its shared memory; the
+  // step-wise loop below computes the same steps
+  const bool fused = (kind == RBG_GEN_DATASET || kind == RBG_GEN_PRW || kind == RBG_GEN_UNIFORM) && rollout_smem(kind, G, N) <= kRolloutMaxSmem;
+  if (fused && kind == RBG_GEN_DATASET) {
     if ((rc = check_dataset(params))) return rc;
     // resets are a table lookup inside rollout_warp_kernel: no cache, no workspace
     EnvParams p;
@@ -953,12 +956,12 @@ int rbg_connector_rollout_random(const rbg_state *state, int32_t *action_out, in
     }
     return RBG_OK;
   }
-  if (kind == RBG_GEN_PRW || kind == RBG_GEN_UNIFORM) {
+  if (fused) {
     if (!workspace) return set_error(RBG_EINVAL, "auto-reset needs a workspace (rbg_step_workspace_bytes)");
     if (!aligned16(workspace)) return set_error(RBG_EALIGN, "workspace not 16-byte aligned");
     return rollout_fused(state, action_out, T, B, G, N, params, ts, workspace, (cudaStream_t)stream);
   }
-  for (int64_t t = 0; t < T; ++t) {  // step-wise: SeedExtension / SequentialRandomWalk resets
+  for (int64_t t = 0; t < T; ++t) {  // step-wise: SeedExtension / SequentialRandomWalk resets, and shapes too big to fuse
     const rbg_timestep tt = timestep_at(*ts, t * B, G, N);
     rc = connector_step_impl(state, state, nullptr, action_out ? action_out + t * B * N : nullptr, 1, B, G, N, params, &tt, workspace,
                              (cudaStream_t)stream);

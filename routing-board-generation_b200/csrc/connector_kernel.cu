@@ -941,6 +941,8 @@ int launch_env(EnvParams p, cudaStream_t stream, bool pdl) {
   const size_t smem = lutB + EW_WARPS * s.wgrid;
   const int64_t E = EW_WARPS * s.K;  // envs per CTA
   const int64_t ctas = (p.B + E - 1) / E;
+  void (*fn)(const EnvParams) = s.vec() ? env_warp_kernel<true> : env_warp_kernel<false>;
+  if (int rc = allow_smem((const void *)fn, smem, "cudaFuncSetAttribute(env_warp_kernel)")) return rc;
   LaunchScope scope(RBG_K_ENV, stream);
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
@@ -953,7 +955,7 @@ int launch_env(EnvParams p, cudaStream_t stream, bool pdl) {
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = pdl ? 1 : 0;
-  cudaError_t ce = cudaLaunchKernelEx(&cfg, s.vec() ? env_warp_kernel<true> : env_warp_kernel<false>, p);
+  cudaError_t ce = cudaLaunchKernelEx(&cfg, fn, p);
   if (ce != cudaSuccess) return set_cuda_error(ce, "cudaLaunchKernelEx(env_warp_kernel)");
   return check_launch("env_warp_kernel");
 }
@@ -979,34 +981,89 @@ static size_t balance_waves(int64_t ctas, int cmax, int cmin, size_t smem_needed
   return pad > smem_needed ? pad : smem_needed;
 }
 
-int launch_rollout(EnvParams p, int T, int32_t *action_out, cudaStream_t stream) {
-  if (p.B <= 0 || T <= 0) return RBG_OK;
-  const WarpShape s = warp_shape(p.G, p.N);
-  const int N = p.N, K = s.K;
-  const bool vec = s.vec();
-  const size_t lutB = lut_bytes(N, OBS_RS);
-  set_warp_shape(p, s, lutB);
-  RolloutParams rp;
-  rp.T = T;
-  rp.action_out = action_out;
-  rp.ratio_off = (int)(lutB + EW_WARPS * s.wgrid);
-  size_t smem = up16((size_t)rp.ratio_off + 4 * (RBG_MAX_N + 4));
-  rp.stage_off = (int)smem;
-  rp.stage_bytes = 0;
+// The shared-memory layout of the fused rollout kernels, a function of the shape and the auto-reset generator kind
+// alone: rollout_warp_kernel for RBG_GEN_DATASET (resets are a table lookup), rollout_persist_kernel with its generator
+// warps for RBG_GEN_PRW / RBG_GEN_UNIFORM.  `smem` is the CTA's need before launch_rollout's wave-balance padding.
+struct RolloutLayout {
+  WarpShape s;
+  size_t lutB, smem;
+  bool isolated;     // rollout_persist_kernel: 3 env warps and 1 generator warp per CTA
+  int PW;            // env warps per CTA
+  RolloutParams rp;  // offsets and the observation staging plan
+  PersistParams pp;  // rollout_persist_kernel: offsets and warp counts
+  GenWarpCfg gc;     // rollout_persist_kernel: the generator warps
+};
+
+static RolloutLayout rollout_layout(int kind, int G, int N) {
+  RolloutLayout L;
+  memset(&L, 0, sizeof(L));
+  L.s = warp_shape(G, N);
+  const WarpShape &s = L.s;
+  const bool persist = kind != RBG_GEN_DATASET;
+  L.lutB = lut_bytes(N, OBS_RS);
+  RolloutParams &rp = L.rp;
+  PersistParams &pp = L.pp;
+  // CTA shape of the persistent kernel.  "Isolated": 3 env warps + 1 generator warp = 4 warps per CTA, one per SM
+  // sub-partition, so the generator warps of all resident CTAs share ONE sub-partition and never compete with env warps
+  // for issue slots, at most 4 CTAs per SM.  "Packed": 4 env + 2 generator warps, as many CTAs as fit.  Measured (65 536
+  // envs, M env-steps/s, isolated / packed): 10x10/5 2501 / 2338, 12x12/6 1649 / 1508, 10x10/4 2884 / 2850, 10x10/8 1598 /
+  // 1596; 8x8/4 2817 / 3432, 8x8/8 1477 / 1687, 6x6/3 2623 / 2989 (issue-bound: more env warps win); 14x14/7 1013 / 1034,
+  // 16x16/8 761 / 774, 20x20/10 372 / 378, 32x32/16 94.9 / 96.8 (resets are rare per byte: packed is 2 % ahead).
+  const bool isolated = persist && G >= 9 && G <= 13 && N <= 8;
+  L.isolated = isolated;
+  L.PW = isolated ? 3 : EW_WARPS;
+  size_t off = L.lutB + L.PW * s.wgrid;
+  rp.ratio_off = (int)off;
+  off = up16(off + 4 * (RBG_MAX_N + 4));
+  if (persist) {
+    GenWarpCfg &gc = L.gc;
+    gc = gen_warp_cfg(kind, G, N, &pp.gcand_bytes, &pp.gsel_bytes, &pp.gscr_stride);
+    gc.patience = 20;
+    gc.seqlock = 0;  // nobody reads an entry while it is rewritten here (see gen_warp_batch)
+    gc.kshift = 0;
+    while ((1 << gc.kshift) < s.K) ++gc.kshift;
+    pp.gen_warps = isolated ? 1 : 2;
+    pp.env_warps = L.PW;
+    pp.tmpl_off = (int)off;
+    off = up16(off + gc.SBp);
+    pp.q_off = (int)off;
+    off = up16(off + pp.gen_warps * sizeof(GenQueue));
+    pp.done_off = (int)off;
+    off += 16;
+    pp.gscr_off = (int)off;
+    off += (size_t)pp.gen_warps * pp.gscr_stride;
+  }
+  rp.stage_off = (int)off;
   rp.stage_nbuf = 1;
-  rp.stage_warp = 0;
   rp.ce = 1;
   rp.cv = N;
-  if (vec) {
-    const ObsStagePlan pl = obs_stage_plan(K, N, s.cells, 4096, 8192);
+  if (s.vec()) {
+    const ObsStagePlan pl = obs_stage_plan(s.K, N, s.cells, 4096, 8192);
     rp.stage_bytes = pl.bytes;
     rp.stage_nbuf = pl.nbuf;
     rp.ce = pl.ce;
     rp.cv = pl.cv;
     rp.stage_warp = (int)up16((size_t)rp.stage_nbuf * rp.stage_bytes);
-    smem += (size_t)EW_WARPS * rp.stage_warp;
+    off += (size_t)L.PW * rp.stage_warp;
   }
-  if (smem > 200 * 1024) return set_error(RBG_EINVAL, "rollout: shared memory %zu too large", smem);
+  L.smem = up16(off);
+  return L;
+}
+
+size_t rollout_smem(int kind, int G, int N) { return rollout_layout(kind, G, N).smem; }
+
+int launch_rollout(EnvParams p, int T, int32_t *action_out, cudaStream_t stream) {
+  if (p.B <= 0 || T <= 0) return RBG_OK;
+  const RolloutLayout L = rollout_layout(RBG_GEN_DATASET, p.G, p.N);
+  const WarpShape &s = L.s;
+  const int K = s.K;
+  const bool vec = s.vec();
+  set_warp_shape(p, s, L.lutB);
+  RolloutParams rp = L.rp;
+  rp.T = T;
+  rp.action_out = action_out;
+  size_t smem = L.smem;
+  if (smem > kRolloutMaxSmem) return set_error(RBG_EINVAL, "rollout: shared memory %zu too large", smem);
   const int64_t E = EW_WARPS * K;  // envs per CTA
   const int64_t ctas = (p.B + E - 1) / E;
   {  // residency: registers allow kRolloutMinCtas per SM, shared memory (1 KB reserved per CTA) maybe fewer
@@ -1029,67 +1086,27 @@ int launch_rollout(EnvParams p, int T, int32_t *action_out, cudaStream_t stream)
 int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, int32_t *counter, int32_t *group_done, int32_t *group_pending,
                            int epoch, bool overlap, uint64_t *cache_tag_w, uint2 *cache_key_w, uint32_t *cache_pins_w, cudaStream_t stream) {
   if (p.B <= 0 || T <= 0) return RBG_OK;
-  const WarpShape s = warp_shape(p.G, p.N);
-  const int G = p.G, N = p.N, K = s.K;
-  const bool vec = s.vec();
-  const size_t lutB = lut_bytes(N, OBS_RS);
-  set_warp_shape(p, s, lutB);
-  RolloutParams rp;
-  memset(&rp, 0, sizeof(rp));
+  const RolloutLayout L = rollout_layout(kind, p.G, p.N);
+  const WarpShape &s = L.s;
+  const int K = s.K, PW = L.PW;
+  const bool vec = s.vec(), isolated = L.isolated;
+  set_warp_shape(p, s, L.lutB);
+  RolloutParams rp = L.rp;
   rp.T = T;
   rp.action_out = action_out;
-  // CTA shape.  "Isolated": 3 env warps + 1 generator warp = 4 warps per CTA, one per SM sub-partition, so the generator
-  // warps of all resident CTAs share ONE sub-partition and never compete with env warps for issue slots, at most 4 CTAs
-  // per SM.  "Packed": 4 env + 2 generator warps, as many CTAs as fit.  Measured (65 536 envs, M env-steps/s, isolated /
-  // packed): 10x10/5 2501 / 2338, 12x12/6 1649 / 1508, 10x10/4 2884 / 2850, 10x10/8 1598 / 1596; 8x8/4 2817 / 3432,
-  // 8x8/8 1477 / 1687, 6x6/3 2623 / 2989 (issue-bound: more env warps win); 14x14/7 1013 / 1034, 16x16/8 761 / 774,
-  // 20x20/10 372 / 378, 32x32/16 94.9 / 96.8 (resets are rare per byte: packed is 2 % ahead).
-  const bool isolated = G >= 9 && G <= 13 && N <= 8;
-  const int PW = isolated ? 3 : EW_WARPS;
-  size_t off = lutB + PW * s.wgrid;
-  rp.ratio_off = (int)off;
-  off = up16(off + 4 * (RBG_MAX_N + 4));
-  PersistParams pp;
-  memset(&pp, 0, sizeof(pp));
+  PersistParams pp = L.pp;
   pp.counter = counter + (epoch % kPersistSets) * kPersistSetInts;
   pp.group_done = group_done;
   pp.group_pending = group_pending;
   pp.epoch = epoch;
   pp.ngroups = (int)((p.B + K - 1) / K);
-  GenWarpCfg gc = gen_warp_cfg(kind, G, N, &pp.gcand_bytes, &pp.gsel_bytes, &pp.gscr_stride);
-  gc.patience = 20;
+  GenWarpCfg gc = L.gc;
   gc.cache_tag = reinterpret_cast<unsigned long long *>(cache_tag_w);
   gc.cache_key = cache_key_w;
   gc.cache_pins = cache_pins_w;
   gc.group_pending = group_pending;
-  gc.seqlock = 0;  // nobody reads an entry while it is rewritten here (see gen_warp_batch)
-  gc.kshift = 0;
-  while ((1 << gc.kshift) < K) ++gc.kshift;
-  pp.gen_warps = isolated ? 1 : 2;
-  pp.env_warps = PW;
-  pp.tmpl_off = (int)off;
-  off = up16(off + gc.SBp);
-  pp.q_off = (int)off;
-  off = up16(off + pp.gen_warps * sizeof(GenQueue));
-  pp.done_off = (int)off;
-  off += 16;
-  pp.gscr_off = (int)off;
-  off += (size_t)pp.gen_warps * pp.gscr_stride;
-  rp.stage_off = (int)off;
-  rp.stage_nbuf = 1;
-  rp.ce = 1;
-  rp.cv = N;
-  if (vec) {
-    const ObsStagePlan pl = obs_stage_plan(K, N, s.cells, 4096, 8192);
-    rp.stage_bytes = pl.bytes;
-    rp.stage_nbuf = pl.nbuf;
-    rp.ce = pl.ce;
-    rp.cv = pl.cv;
-    rp.stage_warp = (int)up16((size_t)rp.stage_nbuf * rp.stage_bytes);
-    off += (size_t)PW * rp.stage_warp;
-  }
-  const size_t smem = up16(off);
-  if (smem > 200 * 1024) return set_error(RBG_EINVAL, "rollout: shared memory %zu too large", smem);
+  const size_t smem = L.smem;
+  if (smem > kRolloutMaxSmem) return set_error(RBG_EINVAL, "rollout: shared memory %zu too large", smem);
   const bool staged = vec && rp.stage_nbuf != 0;
   const int threads = (PW + pp.gen_warps) * 32;
   void (*fn)(const EnvParams, const RolloutParams, const PersistParams, const GenWarpCfg) =

@@ -103,6 +103,10 @@ int launch_rollout(EnvParams p, int T, int32_t *action_out, cudaStream_t stream)
 // epoch: 1, 2, ... per launch on those arrays; overlap: chain to the previous launch of the stream (PDL)
 int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, int32_t *counter, int32_t *group_done, int32_t *group_pending,
                            int epoch, bool overlap, uint64_t *cache_tag_w, uint2 *cache_key_w, uint32_t *cache_pins_w, cudaStream_t stream);
+// Dynamic shared memory per CTA that the fused rollout of a G x G / N batch auto-reset by `kind` needs (RBG_GEN_DATASET:
+// launch_rollout; RBG_GEN_PRW / RBG_GEN_UNIFORM: launch_rollout_persist).  Neither launches above kRolloutMaxSmem.
+constexpr size_t kRolloutMaxSmem = 200 * 1024;
+size_t rollout_smem(int kind, int G, int N);
 int launch_random_actions(const rbg_state &st, int64_t B, int G, int N,
                           int32_t *action, cudaStream_t stream);
 // every env of `in` to its first LAST step under the random policy (episode_warp_kernel); fin may be NULL

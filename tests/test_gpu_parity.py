@@ -1176,12 +1176,14 @@ print("ok", threads)
 @pytest.mark.gpu
 @pytest.mark.parametrize("env_vars,G,N,B", [({}, 5, 3, 4101), ({}, 7, 2, 70), ({"RBG_HOST_THREADS": "3"}, 10, 5, 9000),
                                             ({"RBG_HOST_THREADS": "3"}, 10, 5, 33001), ({}, 10, 5, 4500),
-                                            ({}, 5, 3, 33001), ({}, 10, 5, 4133), ({}, 8, 4, 300), ({}, 9, 6, 700), ({}, 6, 5, 131)])
+                                            ({}, 5, 3, 33001), ({}, 10, 5, 4133), ({}, 8, 4, 300), ({}, 9, 6, 700), ({}, 6, 5, 131),
+                                            ({}, 20, 1, 300), ({}, 28, 2, 150), ({}, 40, 4, 70)])
 def test_step_host_io_transports(env_vars, G, N, B):
     """rbg_connector_step_host_io moves the observation as bytes (as nibbles when the codes are <= 15: at most 5 agents and
     an even number of cells per env) and widens it on the host threads of the call: same TimeSteps as the oracle with 1, 8
     and 16 slices (B >= 32768) of either code width, ragged last slices, shapes without the vector path, unpinned and
-    odd-aligned destination, and the byte counters say what crossed."""
+    odd-aligned destination, few agents on boards whose step needs more than 48 KB of shared memory, and the byte
+    counters say what crossed."""
     import os
     import subprocess
     import sys

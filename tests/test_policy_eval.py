@@ -157,7 +157,7 @@ def _assert_metrics(got, ref, where=""):
         _eq(_np(got[k]), ref[k], f"{k} {where}")
 
 
-def oracle_policy_episodes(rbg, orc, st, keys, policy_np, time_limit):
+def oracle_policy_episodes(rbg, orc, st, keys, policy_np, time_limit, timestep_reward=-0.03, connected_reward=0.1):
     """The oracle's plain Connector.step (autoreset_kind=-1) under `policy_np` on the oracle's own observation, each env
     stepped until its first LAST step, with PolicyEvaluator's action keys (from engine.split_each, pinned against the
     oracle elsewhere); returns in float32, added in step order."""
@@ -172,7 +172,8 @@ def oracle_policy_episodes(rbg, orc, st, keys, policy_np, time_limit):
         s = rbg.engine.split_each(chain)
         chain, ak = s[:, 0], _np(s[:, 1].contiguous())
         sub = {k: v[alive] for k, v in st.items()}
-        nsub, ts = orc.connector_step_batch(sub, policy_np(mask[alive], ak[alive]), time_limit=time_limit, autoreset_kind=-1)
+        nsub, ts = orc.connector_step_batch(sub, policy_np(mask[alive], ak[alive]), time_limit=time_limit, timestep_reward=timestep_reward,
+                                            connected_reward=connected_reward, autoreset_kind=-1)
         m["episode_return"][alive] = m["episode_return"][alive] + ts["reward"]
         m["episode_length"][alive] += 1
         for k in st:
@@ -200,9 +201,8 @@ def _check_evaluator(rbg, orc, env, st_np, keys, policy, time_limit, where):
 @pytest.mark.parametrize("G,N", SHAPES + BIG_SMEM_SHAPES)
 @pytest.mark.parametrize("steps,time_limit", [(3, 50), (5, 6)])
 def test_eval_step_matches_connector_step(rbg, orc, G, N, B, steps, time_limit):
-    """Mid-episode States, a random live mask, TimeStep / record prefilled with sentinels: live rows equal the plain
-    Connector.step (the GPU library's; for the shapes whose Connector.step needs more than 48 KB of shared memory per
-    CTA, the oracle's), dead rows are untouched, and live / live_count / the record are updated as documented."""
+    """Mid-episode States, a random live mask, TimeStep / record prefilled with sentinels: live rows equal the oracle's
+    plain Connector.step, dead rows are untouched, and live / live_count / the record are updated as documented."""
     import torch
 
     seed = G * 1000 + N * 10 + B + steps
@@ -213,11 +213,7 @@ def test_eval_step_matches_connector_step(rbg, orc, G, N, B, steps, time_limit):
         s0, _ = orc.connector_step_batch(s0, orc.random_actions_batch(s0), time_limit=time_limit, autoreset_kind=-1)
     act = rng.integers(0, 5, size=(B, N)).astype(np.int32)
     live0 = (rng.random(B) < 0.7).astype(np.uint8)
-    if (G, N) in BIG_SMEM_SHAPES:
-        rs, rts = orc.connector_step_batch(s0, act, time_limit=time_limit, autoreset_kind=-1)
-    else:
-        rs, rts = rbg.engine.connector_step(_state_gpu(rbg, s0), rbg.engine.as_tensor(act), time_limit=time_limit, autoreset_kind=-1)
-        rs, rts = _state_np(rs), _ts_np(rts)
+    rs, rts = orc.connector_step_batch(s0, act, time_limit=time_limit, autoreset_kind=-1)
 
     dev = torch.device("cuda")
     st = _state_gpu(rbg, s0)
@@ -282,7 +278,7 @@ def test_eval_step_on_a_dead_batch_writes_nothing(rbg, orc):
 @pytest.mark.gpu
 @pytest.mark.parametrize("policy", list(POLICIES))
 @pytest.mark.parametrize("kind", ["parallel_random_walk", "uniform"])
-@pytest.mark.parametrize("G,N", SHAPES)
+@pytest.mark.parametrize("G,N", SHAPES + BIG_SMEM_SHAPES)
 @pytest.mark.parametrize("time_limit", [1, 7, 50])
 def test_evaluator_matches_oracle(rbg, orc, policy, kind, G, N, time_limit):
     B = 2048 if G < 32 else 512
