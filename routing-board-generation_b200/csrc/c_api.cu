@@ -209,7 +209,7 @@ static PrwParams prw_params(int kind, const uint32_t *keys, int64_t B, int G, in
 
 static int generator_state_impl(int kind, const uint32_t *keys, int64_t B, int G, int N, const rbg_state *out,
                                 const rbg_timestep *ts, int extra_split, const int32_t *list,
-                                const int32_t *list_count, cudaStream_t stream, int32_t *list_ticket = nullptr) {
+                                const int32_t *list_count, cudaStream_t stream) {
   if (kind == RBG_GEN_PRW || kind == RBG_GEN_UNIFORM) {
     PrwParams p = prw_params(kind, keys, B, G, N, extra_split);
     p.st = *out;
@@ -219,7 +219,6 @@ static int generator_state_impl(int kind, const uint32_t *keys, int64_t B, int G
     }
     p.list = list;
     p.list_count = list_count;
-    p.list_ticket = list_ticket;
     return launch_prw(p, B, stream);
   }
   if (kind == RBG_GEN_SEEDEXT) {
@@ -234,7 +233,7 @@ static int generator_state_impl(int kind, const uint32_t *keys, int64_t B, int G
     p.iterations = 1;
     p.ext_steps = -1;
     p.extra_split = 1 + extra_split;  // RSG:34 key, pos_key = split(key)
-    p.mode = 2;
+    p.mode = GEN_MODE_STATE;
     p.st = *out;
     if (ts) {
       p.ts = *ts;
@@ -252,7 +251,7 @@ static int generator_state_impl(int kind, const uint32_t *keys, int64_t B, int G
     p.G = G;
     p.N = N;
     p.extra_split = 1 + extra_split;  // sequential_random_walk_generator.py:42 key, pos_key = split(key)
-    p.mode = 2;
+    p.mode = GEN_MODE_STATE;
     p.st = *out;
     if (ts) {
       p.ts = *ts;
@@ -296,11 +295,46 @@ static int workspace_follow_stream(AutoResetCtx *ctx, cudaStream_t stream) {
   return RBG_OK;
 }
 
+// A speculative call on `ws` for another batch than the recorded one (or the first call): nothing is cached yet.  The
+// counters are zeroed, and the cache is warm-started with the next episode of EVERY env, one bulk generation keyed by
+// the current State.key `keys` (a cold cache would send each env's first reset down the synchronous path).
+static int adopt_workspace(AutoResetCtx *ctx, uint8_t *ws, int kind, const uint32_t *keys, int64_t B, int G, int N, cudaStream_t stream) {
+  if (ctx->B == B && ctx->G == G && ctx->N == N && ctx->kind == kind) return RBG_OK;
+  cudaError_t e;
+  int rc;
+  if ((e = cudaMemsetAsync(ws, 0, 256, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(counters)");
+  if ((rc = launch_prw(prw_params(kind, keys, B, G, N, 1, ws), B, stream))) return rc;
+  ctx->B = B;
+  ctx->G = G;
+  ctx->N = N;
+  ctx->kind = kind;
+  ctx->step = 0;
+  ctx->persist_epoch = 0;
+  return RBG_OK;
+}
+
+// A Connector step (ENV_MODE_STEP under `env`) or observation (ENV_MODE_OBSERVE, env NULL) of B envs from `in` into `out`
+static EnvParams env_params(int mode, const rbg_state &in, const rbg_state &out, int64_t B, int G, int N, const rbg_env_params *env) {
+  EnvParams p;
+  memset(&p, 0, sizeof(p));
+  p.in = in;
+  p.out = out;
+  p.B = B;
+  p.G = G;
+  p.N = N;
+  p.mode = mode;
+  if (env)
+    p.env = *env;
+  else
+    p.env.autoreset_kind = -1;
+  return p;
+}
+
 // Per-step auto-reset with the cache (ParallelRandomWalk / Uniform): everything runs on the caller's stream.  The
 // synchronous resets of step t and the cache refill are one kernel (prw_pair_kernel) that says launch_dependents
 // between the two, and the env kernel of step t + 1 is launched with programmatic stream serialization, so the refill
 // of step t overlaps the env kernel of step t + 1 by construction and nothing else moves.  While kernel timing is on,
-// the three run unchained: env kernel, synchronous reset kernel, refill kernel.
+// the env kernel waits for the whole of prw_pair_kernel, so that each event pair times one kernel.
 static int connector_step_impl(const rbg_state *in, const rbg_state *out, const int32_t *action, int32_t *action_out,
                                int random_policy, int64_t B, int G, int N, const rbg_env_params *params,
                                const rbg_timestep *ts, void *workspace, cudaStream_t stream) {
@@ -318,51 +352,41 @@ static int connector_step_impl(const rbg_state *in, const rbg_state *out, const 
   if (autoreset && params->autoreset_kind > RBG_GEN_SEQRW)
     return set_error(RBG_EINVAL, "unknown autoreset generator kind %d", params->autoreset_kind);
   if (dataset && (rc = check_dataset(params))) return rc;
-  if (B == 0) return RBG_OK;
-  EnvParams p;
-  memset(&p, 0, sizeof(p));
-  p.in = *in;
-  p.out = *out;
+  EnvParams p = env_params(ENV_MODE_STEP, *in, *out, B, G, N, params);
   p.ts = *ts;
   p.action = action;
   p.action_out = action_out;
   p.random_policy = random_policy;
-  p.B = B;
-  p.G = G;
-  p.N = N;
-  p.mode = ENV_MODE_STEP;
-  p.env = *params;
   if (!autoreset || dataset) return launch_env(p, stream);  // dataset resets are a lookup inside the kernel
 
   uint8_t *ws = reinterpret_cast<uint8_t *>(workspace);
   if (!aligned16(ws)) return set_error(RBG_EALIGN, "workspace not 16-byte aligned");
   const WsLayout wl = ws_layout(B, N);
   const int kind = params->autoreset_kind;
-  const bool speculative = kind == RBG_GEN_PRW || kind == RBG_GEN_UNIFORM;
   int32_t *sync_count = reinterpret_cast<int32_t *>(ws);
   int32_t *sync_list = reinterpret_cast<int32_t *>(ws + wl.sync_list);
   p.list = sync_list;
   p.list_count = sync_count;
-  cudaError_t e;
-  AutoResetCtx *ctx = nullptr;
-  if (speculative) {
+  // VmapAutoResetWrapper._auto_reset: key, _ = split(state.key); reset(key):
+  // one more leading split()[0] than a plain generator call.
+  if (kind != RBG_GEN_PRW && kind != RBG_GEN_UNIFORM) {
+    cudaError_t e;
+    if ((e = cudaMemsetAsync(ws, 0, 64, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(reset counter)");
+    // This path leaves its reset count in the counter.  If the same workspace has served (or will
+    // serve) a speculative batch, that batch must adopt it afresh: its kernels rely on counters
+    // that are zero between steps.
+    invalidate_workspace(workspace);
+    if ((rc = launch_env(p, stream))) return rc;
+    return generator_state_impl(kind, out->key, B, G, N, out, ts, 1, sync_list, sync_count, stream);
+  }
+  // speculative: the counters were zeroed once when the workspace was adopted, and the list kernels clear their own
+  // counter when they finish (prw_kernel list_ticket)
+  AutoResetCtx *ctx;
+  {
     std::lock_guard<std::mutex> lock(g_ar_mu);
     ctx = &g_ar[workspace];
     if ((rc = workspace_follow_stream(ctx, stream))) return rc;
-    if (ctx->B != B || ctx->G != G || ctx->N != N || ctx->kind != kind) {
-      // first use of this workspace (or a different batch in it): nothing cached yet
-      if ((e = cudaMemsetAsync(ws, 0, 256, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(counters)");
-      // warm start: the next episode of EVERY env, one bulk generation keyed by the
-      // current State.key (a cold cache would send each env's first reset down the
-      // synchronous path)
-      if ((rc = launch_prw(prw_params(kind, in->key, B, G, N, 1, ws), B, stream))) return rc;
-      ctx->B = B;
-      ctx->G = G;
-      ctx->N = N;
-      ctx->kind = kind;
-      ctx->step = 0;
-      ctx->persist_epoch = 0;
-    }
+    if ((rc = adopt_workspace(ctx, ws, kind, in->key, B, G, N, stream))) return rc;
     // the refill lists alternate between two buffers: this step's env kernel runs under the previous step's refill
     const int par = (int)(ctx->step & 1);
     p.cache_tag = reinterpret_cast<const unsigned long long *>(ws + wl.cache_tag);
@@ -372,48 +396,22 @@ static int connector_step_impl(const rbg_state *in, const rbg_state *out, const 
     p.refill_keys = reinterpret_cast<uint32_t *>(ws + wl.refill_keys[par]);
     p.refill_count = reinterpret_cast<int32_t *>(ws + 64 + 64 * par);
   }
-  // counters: with the speculative path the list kernels clear their own counter when
-  // they finish (prw_kernel list_ticket); they were zeroed once when the workspace was adopted
-  if (!speculative) {
-    if ((e = cudaMemsetAsync(ws, 0, 64, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(reset counter)");
-    // This path leaves its reset count in the counter.  If the same workspace has served (or will
-    // serve) a speculative batch, that batch must adopt it afresh: its kernels rely on counters
-    // that are zero between steps.
-    invalidate_workspace(workspace);
-  }
-  const bool chained = speculative && !g_timing.load(std::memory_order_relaxed);
-  if ((rc = launch_env(p, stream, chained))) return rc;
-  // VmapAutoResetWrapper._auto_reset: key, _ = split(state.key); reset(key):
-  // one more leading split()[0] than a plain generator call.
-  if (chained) {
-    // one launch: the synchronous resets (rare misses), launch_dependents, then the cache refill
-    PrwParams a = prw_params(kind, out->key, B, G, N, 1);
-    a.st = *out;
-    a.ts = *ts;
-    a.observe = 1;
-    a.list = sync_list;
-    a.list_count = sync_count;
-    a.list_ticket = sync_count + 1;
-    PrwParams q = prw_params(kind, p.refill_keys, B, G, N, 1, ws);
-    q.keys_compact = 1;
-    q.list = p.refill_list;
-    q.list_count = p.refill_count;
-    q.list_ticket = p.refill_count + 1;
-    if ((rc = launch_prw_pair(a, q, B, stream))) return rc;
-    ctx->step++;
-    return RBG_OK;
-  }
-  if ((rc = generator_state_impl(kind, out->key, B, G, N, out, ts, 1, sync_list, sync_count, stream, speculative ? sync_count + 1 : nullptr))) return rc;
-  if (speculative) {
-    PrwParams q = prw_params(kind, p.refill_keys, B, G, N, 1, ws);  // as the auto-reset call above
-    q.keys_compact = 1;
-    q.list = p.refill_list;
-    q.list_count = p.refill_count;
-    q.list_ticket = p.refill_count + 1;
-    q.trigger_dependents = 1;
-    if ((rc = launch_prw(q, B, stream))) return rc;
-    ctx->step++;
-  }
+  if ((rc = launch_env(p, stream, !kernel_timing_on()))) return rc;
+  // one launch: the synchronous resets (rare misses), launch_dependents, then the cache refill
+  PrwParams a = prw_params(kind, out->key, B, G, N, 1);
+  a.st = *out;
+  a.ts = *ts;
+  a.observe = 1;
+  a.list = sync_list;
+  a.list_count = sync_count;
+  a.list_ticket = sync_count + 1;
+  PrwParams q = prw_params(kind, p.refill_keys, B, G, N, 1, ws);
+  q.keys_compact = 1;
+  q.list = p.refill_list;
+  q.list_count = p.refill_count;
+  q.list_ticket = p.refill_count + 1;
+  if ((rc = launch_prw_pair(a, q, B, stream))) return rc;
+  ctx->step++;
   return RBG_OK;
 }
 
@@ -455,30 +453,27 @@ struct HostCtx {
 static std::atomic<long long> g_h2d_bytes{0}, g_d2h_bytes{0};
 static HostCtx g_host[kMaxDevices];
 static thread_local HostCtx *g_hc = &g_host[0];  // the device of the _host call in progress (set by use_device)
-#define g_scratch (g_hc->scratch)
-#define g_streams (g_hc->streams)
-#define g_scratch_sig (g_hc->sig)
 
 static int scratch_get(size_t bytes, int device, void **out) {
-  if (g_scratch.ptr && (g_scratch.bytes < bytes || g_scratch.device != device)) {
-    cudaFree(g_scratch.ptr);
-    g_scratch = Scratch();
+  if (g_hc->scratch.ptr && (g_hc->scratch.bytes < bytes || g_hc->scratch.device != device)) {
+    cudaFree(g_hc->scratch.ptr);
+    g_hc->scratch = Scratch();
   }
-  if (!g_scratch.ptr) {
-    cudaError_t e = cudaMalloc(&g_scratch.ptr, bytes);
+  if (!g_hc->scratch.ptr) {
+    cudaError_t e = cudaMalloc(&g_hc->scratch.ptr, bytes);
     if (e != cudaSuccess) {
-      g_scratch = Scratch();
+      g_hc->scratch = Scratch();
       return set_cuda_error(e, "cudaMalloc(host-variant scratch)");
     }
-    g_scratch.bytes = bytes;
-    g_scratch.device = device;
+    g_hc->scratch.bytes = bytes;
+    g_hc->scratch.device = device;
   }
   for (int i = 0; i < 3; ++i)
-    if (!g_streams[i]) {
-      cudaError_t e = cudaStreamCreateWithFlags(&g_streams[i], cudaStreamNonBlocking);
+    if (!g_hc->streams[i]) {
+      cudaError_t e = cudaStreamCreateWithFlags(&g_hc->streams[i], cudaStreamNonBlocking);
       if (e != cudaSuccess) return set_cuda_error(e, "cudaStreamCreate");
     }
-  *out = g_scratch.ptr;
+  *out = g_hc->scratch.ptr;
   return RBG_OK;
 }
 
@@ -486,7 +481,7 @@ static int scratch_get(size_t bytes, int device, void **out) {
 static int sync_streams() {
   int rc = RBG_OK;
   for (int i = 0; i < 3; ++i) {
-    cudaError_t e = cudaStreamSynchronize(g_streams[i]);
+    cudaError_t e = cudaStreamSynchronize(g_hc->streams[i]);
     if (e != cudaSuccess) rc = set_cuda_error(e, "cudaStreamSynchronize");
   }
   return rc;
@@ -726,7 +721,7 @@ int rbg_seedext_solved(const uint32_t *keys, int64_t B, int G, int N, float rand
   p.two_sided = two_sided;
   p.iterations = iterations;
   p.ext_steps = extension_steps;
-  p.mode = 0;
+  p.mode = GEN_MODE_BOARD;
   p.solved = solved;
   return launch_seedext(p, B, (cudaStream_t)stream);
 }
@@ -747,7 +742,7 @@ int rbg_seedext_starts_ends(const uint32_t *keys, int64_t B, int G, int N, float
   p.two_sided = two_sided;
   p.iterations = iterations;
   p.ext_steps = extension_steps;
-  p.mode = 1;
+  p.mode = GEN_MODE_STARTS_ENDS;
   p.starts = starts;
   p.ends = ends;
   return launch_seedext(p, B, (cudaStream_t)stream);
@@ -766,7 +761,7 @@ int rbg_seqrw_generate(const uint32_t *keys, int64_t B, int G, int N, void *boar
   p.B = B;
   p.G = G;
   p.N = N;
-  p.mode = 0;
+  p.mode = GEN_MODE_BOARD;
   p.float_board = as_float32 ? 1 : 0;
   p.board = reinterpret_cast<int32_t *>(board);
   p.stats = stats;
@@ -784,7 +779,7 @@ int rbg_seqrw_starts_ends(const uint32_t *keys, int64_t B, int G, int N, int32_t
   p.B = B;
   p.G = G;
   p.N = N;
-  p.mode = 1;
+  p.mode = GEN_MODE_STARTS_ENDS;
   p.starts = starts;
   p.ends = ends;
   return launch_seqrw(p, B, (cudaStream_t)stream);
@@ -796,16 +791,8 @@ int rbg_connector_observe(const rbg_state *state, int64_t B, int G, int N, const
   if (B == 0) return RBG_OK;  // an empty batch has no buffers to check
   if ((rc = check_state(state, "state", G))) return rc;
   if ((rc = check_timestep(ts, G))) return rc;
-  EnvParams p;
-  memset(&p, 0, sizeof(p));
-  p.in = *state;
-  p.out = *state;
+  EnvParams p = env_params(ENV_MODE_OBSERVE, *state, *state, B, G, N, nullptr);
   p.ts = *ts;
-  p.B = B;
-  p.G = G;
-  p.N = N;
-  p.mode = ENV_MODE_OBSERVE;
-  p.env.autoreset_kind = -1;
   return launch_env(p, (cudaStream_t)stream);
 }
 
@@ -861,56 +848,47 @@ int rbg_connector_step_random(const rbg_state *in, const rbg_state *out, int32_t
 // Steps per launch of the fused rollout kernels: the reference's n_steps (agent_training/configs/env/connector.yaml:27)
 constexpr int kRolloutChunk = 20;
 
-// Fused ParallelRandomWalk / Uniform rollout (rollout_persist_kernel): one launch per chunk of steps.  The kernel's
-// generator warps keep the next-episode cache filled; consecutive launches on the stream overlap head to tail.
+// Fused rollout, one launch per chunk of steps: rollout_warp_kernel for the dataset (resets are a table lookup inside
+// the kernel: no cache, no workspace), rollout_persist_kernel for ParallelRandomWalk / Uniform (the kernel's generator
+// warps keep the next-episode cache filled; consecutive launches on the stream overlap head to tail).
 static int rollout_fused(const rbg_state *state, int32_t *action_out, int64_t T, int64_t B, int G, int N,
                          const rbg_env_params *params, const rbg_timestep *ts, void *workspace, cudaStream_t stream) {
   uint8_t *ws = reinterpret_cast<uint8_t *>(workspace);
   const WsLayout wl = ws_layout(B, N);
   const int kind = params->autoreset_kind;
+  const bool dataset = kind == RBG_GEN_DATASET;
   cudaError_t e;
   int rc;
-  AutoResetCtx *ctx;
-  {
-    std::lock_guard<std::mutex> lock(g_ar_mu);
-    ctx = &g_ar[workspace];
-  }
-  if ((rc = workspace_follow_stream(ctx, stream))) return rc;
-  if (ctx->B != B || ctx->G != G || ctx->N != N || ctx->kind != kind) {
-    if ((e = cudaMemsetAsync(ws, 0, 256, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(counters)");
-    // warm start: the next episode of every env
-    if ((rc = launch_prw(prw_params(kind, state->key, B, G, N, 1, ws), B, stream))) return rc;
-    ctx->B = B;
-    ctx->G = G;
-    ctx->N = N;
-    ctx->kind = kind;
-    ctx->step = 0;
-    ctx->persist_epoch = 0;
-  }
-  EnvParams p;
-  memset(&p, 0, sizeof(p));
-  p.in = *state;
-  p.out = *state;
-  p.B = B;
-  p.G = G;
-  p.N = N;
-  p.mode = ENV_MODE_STEP;
+  EnvParams p = env_params(ENV_MODE_STEP, *state, *state, B, G, N, params);
   p.random_policy = 1;
-  p.env = *params;
-  p.cache_tag = reinterpret_cast<const unsigned long long *>(ws + wl.cache_tag);
-  p.cache_key = reinterpret_cast<const uint2 *>(ws + wl.cache_key);
-  p.cache_pins = reinterpret_cast<const uint32_t *>(ws + wl.cache_pins);
+  AutoResetCtx *ctx = nullptr;
+  if (!dataset) {
+    {
+      std::lock_guard<std::mutex> lock(g_ar_mu);
+      ctx = &g_ar[workspace];
+    }
+    if ((rc = workspace_follow_stream(ctx, stream))) return rc;
+    if ((rc = adopt_workspace(ctx, ws, kind, state->key, B, G, N, stream))) return rc;
+    p.cache_tag = reinterpret_cast<const unsigned long long *>(ws + wl.cache_tag);
+    p.cache_key = reinterpret_cast<const uint2 *>(ws + wl.cache_key);
+    p.cache_pins = reinterpret_cast<const uint32_t *>(ws + wl.cache_pins);
+  }
   for (int64_t t0 = 0; t0 < T; t0 += kRolloutChunk) {
     const int n = (int)((T - t0) < kRolloutChunk ? (T - t0) : kRolloutChunk);
+    int32_t *acts = action_out ? action_out + t0 * B * N : nullptr;
     p.ts = timestep_at(*ts, t0 * B, G, N);
+    if (dataset) {
+      if ((rc = launch_rollout(p, n, acts, stream))) return rc;
+      continue;
+    }
     if (ctx->persist_epoch == 0 || ctx->persist_epoch > 0x3fffffff) {  // flags start at 0 = "written by launch 0"
       if ((e = cudaMemsetAsync(ws + wl.group_done, 0, (wl.group_pending - wl.group_done) + 4 * (size_t)B, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(group flags)");
       if ((e = cudaMemsetAsync(ws + 256, 0, 256, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(persist counters)");
       ctx->persist_epoch = 0;
     }
     const int epoch = ++ctx->persist_epoch;
-    const bool overlap = epoch > 1 && !g_timing.load(std::memory_order_relaxed);  // event pairs must time one kernel at a time
-    if ((rc = launch_rollout_persist(p, kind, n, action_out ? action_out + t0 * B * N : nullptr, reinterpret_cast<int32_t *>(ws + 256),
+    const bool overlap = epoch > 1 && !kernel_timing_on();  // event pairs must time one kernel at a time
+    if ((rc = launch_rollout_persist(p, kind, n, acts, reinterpret_cast<int32_t *>(ws + 256),
                                      reinterpret_cast<int32_t *>(ws + wl.group_done), reinterpret_cast<int32_t *>(ws + wl.group_pending), epoch, overlap,
                                      reinterpret_cast<uint64_t *>(ws + wl.cache_tag), reinterpret_cast<uint2 *>(ws + wl.cache_key),
                                      reinterpret_cast<uint32_t *>(ws + wl.cache_pins), stream)))
@@ -936,29 +914,13 @@ int rbg_connector_rollout_random(const rbg_state *state, int32_t *action_out, in
   // few agents on a big board: a fused CTA's grids, staging and generator scratch do not fit its shared memory; the
   // step-wise loop below computes the same steps
   const bool fused = (kind == RBG_GEN_DATASET || kind == RBG_GEN_PRW || kind == RBG_GEN_UNIFORM) && rollout_smem(kind, G, N) <= kRolloutMaxSmem;
-  if (fused && kind == RBG_GEN_DATASET) {
-    if ((rc = check_dataset(params))) return rc;
-    // resets are a table lookup inside rollout_warp_kernel: no cache, no workspace
-    EnvParams p;
-    memset(&p, 0, sizeof(p));
-    p.in = *state;
-    p.out = *state;
-    p.B = B;
-    p.G = G;
-    p.N = N;
-    p.mode = ENV_MODE_STEP;
-    p.random_policy = 1;
-    p.env = *params;
-    for (int64_t t0 = 0; t0 < T; t0 += kRolloutChunk) {
-      const int n = (int)((T - t0) < kRolloutChunk ? (T - t0) : kRolloutChunk);
-      p.ts = timestep_at(*ts, t0 * B, G, N);
-      if ((rc = launch_rollout(p, n, action_out ? action_out + t0 * B * N : nullptr, (cudaStream_t)stream))) return rc;
-    }
-    return RBG_OK;
-  }
   if (fused) {
-    if (!workspace) return set_error(RBG_EINVAL, "auto-reset needs a workspace (rbg_step_workspace_bytes)");
-    if (!aligned16(workspace)) return set_error(RBG_EALIGN, "workspace not 16-byte aligned");
+    if (kind == RBG_GEN_DATASET) {
+      if ((rc = check_dataset(params))) return rc;
+    } else {
+      if (!workspace) return set_error(RBG_EINVAL, "auto-reset needs a workspace (rbg_step_workspace_bytes)");
+      if (!aligned16(workspace)) return set_error(RBG_EALIGN, "workspace not 16-byte aligned");
+    }
     return rollout_fused(state, action_out, T, B, G, N, params, ts, workspace, (cudaStream_t)stream);
   }
   for (int64_t t = 0; t < T; ++t) {  // step-wise: SeedExtension / SequentialRandomWalk resets, and shapes too big to fuse
@@ -1058,8 +1020,8 @@ static int use_device(int device, int *cur) {
 // used last, the auto-reset workspaces a step variant keeps in it (`nws` of them, `stride` bytes
 // apart from `ws`) hold someone else's bytes: their contexts are invalidated.
 static void scratch_claim(const ScratchSig &sig, uint8_t *ws, size_t stride, int64_t nws) {
-  if (g_scratch_sig == sig) return;
-  g_scratch_sig = sig;
+  if (g_hc->sig == sig) return;
+  g_hc->sig = sig;
   for (int64_t i = 0; i < nws; ++i) invalidate_workspace(ws + (size_t)i * stride);
 }
 
@@ -1087,7 +1049,7 @@ int rbg_prw_generate_host(const uint32_t *keys, int64_t B, int G, int N, int32_t
   int si = 0;
   for (int64_t off = 0; off < B; off += sl, ++si) {
     const int64_t n = (B - off) < sl ? (B - off) : sl;
-    cudaStream_t st = g_streams[si % 3];
+    cudaStream_t st = g_hc->streams[si % 3];
     RBG_CPY(dk + off * 2, keys + off * 2, n * 8, cudaMemcpyHostToDevice, st);
     rc = rbg_prw_generate(dk + off * 2, n, G, N, dh + off * 2 * N, dt + off * 2 * N, ds + off * G * G, nullptr, st);
     if (rc) return rc;
@@ -1122,7 +1084,7 @@ int rbg_connector_reset_host(int kind, const uint32_t *keys, int64_t B, int G, i
   int si = 0;
   for (int64_t off = 0; off < B; off += sl, ++si) {
     const int64_t n = (B - off) < sl ? (B - off) : sl;
-    cudaStream_t st = g_streams[si % 3];
+    cudaStream_t st = g_hc->streams[si % 3];
     RBG_CPY(dk + off * 2, keys + off * 2, n * 8, cudaMemcpyHostToDevice, st);
     rbg_state dss = state_at(ds, off, G, N);
     rbg_timestep dts = timestep_at(dt, off, G, N);
@@ -1161,7 +1123,7 @@ int rbg_connector_step_host(const rbg_state *in, const rbg_state *out, const int
   int si = 0;
   for (int64_t off = 0; off < B; off += sl, ++si) {
     const int64_t n = (B - off) < sl ? (B - off) : sl;
-    cudaStream_t st = g_streams[si % 3];
+    cudaStream_t st = g_hc->streams[si % 3];
     if ((rc = copy_state(&ds, in, off, n, G, N, cudaMemcpyHostToDevice, off, st))) return rc;
     RBG_CPY(da + off * N, action + off * N, n * N * 4, cudaMemcpyHostToDevice, st);
     rbg_state dss = state_at(ds, off, G, N);
@@ -1246,7 +1208,7 @@ int rbg_connector_step_host_io(const rbg_state *state, const int32_t *action, in
   // slice s into the caller's int32 buffer while slices s+1.. are in flight; the caller's observation buffer need
   // not be pinned.
   cudaEvent_t *slice_ev = g_hc->slice_ev, *copy_ev = g_hc->copy_ev;
-  cudaStream_t cs = g_streams[0];
+  cudaStream_t cs = g_hc->streams[0];
   // The State was produced by the caller on the device's default stream (or a stream that stream synchronises
   // with: every blocking stream does): our compute stream is ordered behind it by an event, the host does not wait.
   if (!g_hc->entry_ev && (e = cudaEventCreateWithFlags(&g_hc->entry_ev, cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
@@ -1269,7 +1231,7 @@ int rbg_connector_step_host_io(const rbg_state *state, const int32_t *action, in
     if ((rc = launch_narrow_codes(dts.obs_grid, obs8 + codes_off, (int64_t)((size_t)n * per_env), cs, obits))) return rc;
     if (!slice_ev[si] && (e = cudaEventCreateWithFlags(&slice_ev[si], cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
     if ((e = cudaEventRecord(slice_ev[si], cs)) != cudaSuccess) return set_cuda_error(e, "cudaEventRecord");
-    cudaStream_t xs = g_streams[1 + (si & 1)];
+    cudaStream_t xs = g_hc->streams[1 + (si & 1)];
     if ((e = cudaStreamWaitEvent(xs, slice_ev[si], 0)) != cudaSuccess) return set_cuda_error(e, "cudaStreamWaitEvent");
     RBG_CPY(g_hc->stage8 + codes_off, obs8 + codes_off, ((size_t)n * per_env) >> oshift, cudaMemcpyDeviceToHost, xs);
     if (!copy_ev[si] && (e = cudaEventCreateWithFlags(&copy_ev[si], cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");

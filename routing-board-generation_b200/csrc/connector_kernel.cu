@@ -925,14 +925,6 @@ static void set_warp_shape(P &p, const WarpShape &s, size_t lutB) {
   p.so[1] = (int)s.wgrid;
 }
 
-// a kernel that needs more than the default 48 KB of dynamic shared memory per CTA has to opt in
-static int allow_smem(const void *fn, size_t smem, const char *what) {
-  cudaError_t ce;
-  if (smem > 48 * 1024 && (ce = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
-    return set_cuda_error(ce, what);
-  return RBG_OK;
-}
-
 int launch_env(EnvParams p, cudaStream_t stream, bool pdl) {
   if (p.B <= 0) return RBG_OK;
   const WarpShape s = warp_shape(p.G, p.N);
@@ -942,22 +934,7 @@ int launch_env(EnvParams p, cudaStream_t stream, bool pdl) {
   const int64_t E = EW_WARPS * s.K;  // envs per CTA
   const int64_t ctas = (p.B + E - 1) / E;
   void (*fn)(const EnvParams) = s.vec() ? env_warp_kernel<true> : env_warp_kernel<false>;
-  if (int rc = allow_smem((const void *)fn, smem, "cudaFuncSetAttribute(env_warp_kernel)")) return rc;
-  LaunchScope scope(RBG_K_ENV, stream);
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)ctas);
-  cfg.blockDim = dim3(EW_WARPS * 32);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl ? 1 : 0;
-  cudaError_t ce = cudaLaunchKernelEx(&cfg, fn, p);
-  if (ce != cudaSuccess) return set_cuda_error(ce, "cudaLaunchKernelEx(env_warp_kernel)");
-  return check_launch("env_warp_kernel");
+  return launch_kernel(fn, (unsigned)ctas, EW_WARPS * 32, smem, stream, RBG_K_ENV, "env_warp_kernel", pdl, p);
 }
 
 // Wave balance: a launch of `ctas` CTAs runs in ceil(ctas / (148 * c)) rounds when c CTAs fit on an
@@ -1073,12 +1050,7 @@ int launch_rollout(EnvParams p, int T, int32_t *action_out, cudaStream_t stream)
   }
   const bool staged = vec && rp.stage_nbuf != 0;
   void (*fn)(const EnvParams, const RolloutParams) = staged ? rollout_warp_kernel<2> : (vec ? rollout_warp_kernel<1> : rollout_warp_kernel<0>);
-  if (int rc = allow_smem((const void *)fn, smem, "cudaFuncSetAttribute(rollout_warp_kernel)")) return rc;
-  {
-    LaunchScope scope(RBG_K_ROLLOUT, stream);
-    fn<<<(unsigned)ctas, EW_WARPS * 32, smem, stream>>>(p, rp);
-  }
-  return check_launch("rollout_warp_kernel");
+  return launch_kernel(fn, (unsigned)ctas, EW_WARPS * 32, smem, stream, RBG_K_ROLLOUT, "rollout_warp_kernel", false, p, rp);
 }
 
 // The persistent rollout with in-CTA generator warps (rollout_persist_kernel).  `cache_*` of `p` must be set;
@@ -1111,7 +1083,7 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   const int threads = (PW + pp.gen_warps) * 32;
   void (*fn)(const EnvParams, const RolloutParams, const PersistParams, const GenWarpCfg) =
       staged ? rollout_persist_kernel<2> : (vec ? rollout_persist_kernel<1> : rollout_persist_kernel<0>);
-  if (int rc = allow_smem((const void *)fn, smem, "cudaFuncSetAttribute(rollout_persist_kernel)")) return rc;
+  if (int rc = opt_in_smem(fn, smem, "rollout_persist_kernel")) return rc;
   cudaError_t ce;
   int resident = 0;
   if ((ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, fn, threads, smem)) != cudaSuccess) return set_cuda_error(ce, "cudaOccupancyMaxActiveBlocksPerMultiprocessor");
@@ -1120,32 +1092,15 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   int64_t ctas = (int64_t)resident * device_sm_count();
   const int64_t need = (pp.ngroups + PW - 1) / PW;
   if (ctas > need) ctas = need;
-  LaunchScope scope(RBG_K_ROLLOUT, stream);
-  // programmatic dependent launch: this grid may begin while the previous kernel of the stream is still
-  // running, if that kernel said so (rollout_persist_kernel does; anything else completes first)
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)ctas);
-  cfg.blockDim = dim3((unsigned)threads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = overlap ? 1 : 0;
-  if ((ce = cudaLaunchKernelEx(&cfg, fn, p, rp, pp, gc)) != cudaSuccess) return set_cuda_error(ce, "cudaLaunchKernelEx(rollout_persist_kernel)");
-  return check_launch("rollout_persist_kernel");
+  // overlap: this grid may begin under the tail of the previous rollout_persist_kernel of the stream
+  return launch_kernel(fn, (unsigned)ctas, threads, smem, stream, RBG_K_ROLLOUT, "rollout_persist_kernel", overlap, p, rp, pp, gc);
 }
 
 int launch_random_actions(const rbg_state &st, int64_t B, int G, int N, int32_t *action, cudaStream_t stream) {
   const int64_t n = B * N;
   if (n <= 0) return RBG_OK;
-  {
-    LaunchScope scope(RBG_K_RANDACT, stream);
-    random_actions_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(st, B, G, N, FastDiv::make((uint32_t)N), action);
-  }
-  return check_launch("random_actions_kernel");
+  return launch_kernel(random_actions_kernel, (unsigned)((n + 255) / 256), 256, 0, stream, RBG_K_RANDACT, "random_actions_kernel", false, st, B, G, N,
+                       FastDiv::make((uint32_t)N), action);
 }
 
 // ---------------------------------------------------------------------------
@@ -1297,7 +1252,7 @@ int launch_episodes(const rbg_state &in, const rbg_state *fin, const rbg_episode
   p.ratio_off = EP_WARPS * p.wgrid;
   const size_t smem = (size_t)p.ratio_off + 4 * (RBG_MAX_N + 4);
   // few agents on a big board: up to 4 warps x 32 envs x 1 600 cells = 200 KB (40x40/1), past the 48 KB default
-  if (int rc = allow_smem((const void *)episode_warp_kernel, smem, "cudaFuncSetAttribute(episode_warp_kernel)")) return rc;
+  if (int rc = opt_in_smem(episode_warp_kernel, smem, "episode_warp_kernel")) return rc;
   cudaError_t ce;
   int per_sm = 0;
   if ((ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, episode_warp_kernel, EP_WARPS * 32, smem)) != cudaSuccess)
@@ -1313,15 +1268,10 @@ int launch_episodes(const rbg_state &in, const rbg_state *fin, const rbg_episode
   if ((ce = cudaMallocAsync(&scratch, 256, stream)) != cudaSuccess) return set_cuda_error(ce, "cudaMallocAsync(episode counter)");
   p.counter = static_cast<int *>(scratch);
   int rc = RBG_OK;
-  if ((ce = cudaMemsetAsync(scratch, 0, 256, stream)) != cudaSuccess) {
+  if ((ce = cudaMemsetAsync(scratch, 0, 256, stream)) != cudaSuccess)
     rc = set_cuda_error(ce, "cudaMemsetAsync(episode counter)");
-  } else {
-    {
-      LaunchScope scope(RBG_K_EPISODES, stream);
-      episode_warp_kernel<<<ctas, EP_WARPS * 32, smem, stream>>>(p);
-    }
-    rc = check_launch("episode_warp_kernel");
-  }
+  else
+    rc = launch_kernel(episode_warp_kernel, ctas, EP_WARPS * 32, smem, stream, RBG_K_EPISODES, "episode_warp_kernel", false, p);
   cudaFreeAsync(scratch, stream);
   return rc;
 }
@@ -1516,13 +1466,7 @@ int launch_eval_step(const rbg_state &st, const int32_t *action, uint8_t *live, 
   const int64_t E = EW_WARPS * s.K;  // envs per CTA
   const int64_t ctas = (B + E - 1) / E;
   void (*fn)(const EvalStepParams) = s.vec() ? eval_step_kernel<true> : eval_step_kernel<false>;
-  // few agents on a big board: up to 4 warps x 32 envs x 1 600 cells = 200 KB (40x40/1), past the 48 KB default
-  if (int rc = allow_smem((const void *)fn, smem, "cudaFuncSetAttribute(eval_step_kernel)")) return rc;
-  {
-    LaunchScope scope(RBG_K_EVAL_STEP, stream);
-    fn<<<(unsigned)ctas, EW_WARPS * 32, smem, stream>>>(p);
-  }
-  return check_launch("eval_step_kernel");
+  return launch_kernel(fn, (unsigned)ctas, EW_WARPS * 32, smem, stream, RBG_K_EVAL_STEP, "eval_step_kernel", false, p);
 }
 
 }  // namespace rbg

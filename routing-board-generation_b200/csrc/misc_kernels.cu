@@ -28,11 +28,7 @@ int launch_split_keys(uint32_t k0, uint32_t k1, int64_t B, int64_t offset, int64
                       uint32_t *out, cudaStream_t stream) {
   if (count <= 0) return RBG_OK;
   const int64_t n = 2 * count;
-  {
-    LaunchScope scope(RBG_K_SPLIT, stream);
-    split_keys_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(k0, k1, B, offset, count, out);
-  }
-  return check_launch("split_keys_kernel");
+  return launch_kernel(split_keys_kernel, (unsigned)((n + 255) / 256), 256, 0, stream, RBG_K_SPLIT, "split_keys_kernel", false, k0, k1, B, offset, count, out);
 }
 
 // jax.vmap(lambda k: jax.random.split(k, num))(keys): out[b, i] = (flat[2i], flat[2i+1]) of
@@ -56,11 +52,7 @@ __global__ void __launch_bounds__(256) split_each_kernel(const uint32_t *__restr
 int launch_split_each(const uint32_t *keys, int64_t B, int num, uint32_t *out, cudaStream_t stream) {
   const int64_t n = B * 2 * num;
   if (n <= 0) return RBG_OK;
-  {
-    LaunchScope scope(RBG_K_SPLIT, stream);
-    split_each_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(keys, B, num, out);
-  }
-  return check_launch("split_each_kernel");
+  return launch_kernel(split_each_kernel, (unsigned)((n + 255) / 256), 256, 0, stream, RBG_K_SPLIT, "split_each_kernel", false, keys, B, num, out);
 }
 
 // BoardDatasetGeneratorJAX.__call__ (dataset_generator_jax.py:112-141), one warp per env:
@@ -107,11 +99,8 @@ __global__ void __launch_bounds__(DS_WARPS * 32) dataset_state_kernel(const uint
 int launch_dataset_state(const uint32_t *keys, int64_t B, int G, int N, const int32_t *heads, const int32_t *targets, int64_t K,
                          const rbg_state &st, cudaStream_t stream) {
   if (B <= 0) return RBG_OK;
-  {
-    LaunchScope scope(RBG_K_VALIDATE, stream);
-    dataset_state_kernel<<<(unsigned)((B + DS_WARPS - 1) / DS_WARPS), DS_WARPS * 32, 0, stream>>>(keys, B, G, N, heads, targets, (uint32_t)K, st);
-  }
-  return check_launch("dataset_state_kernel");
+  return launch_kernel(dataset_state_kernel, (unsigned)((B + DS_WARPS - 1) / DS_WARPS), DS_WARPS * 32, 0, stream, RBG_K_VALIDATE, "dataset_state_kernel", false,
+                       keys, B, G, N, heads, targets, (uint32_t)K, st);
 }
 
 // Board validity, one warp per board.  The rules are the reference's NumPy functions
@@ -416,11 +405,8 @@ int launch_board_stats(const int32_t *boards, int64_t B, int G, int count_curren
   const size_t smem = (size_t)STAT_WARPS * (3 * PB + STAT_SCORE_BITS / 8);
   int64_t ctas = (B + STAT_WARPS - 1) / STAT_WARPS;
   if (ctas > (int64_t)device_sm_count() * 32) ctas = (int64_t)device_sm_count() * 32;
-  {
-    LaunchScope scope(RBG_K_VALIDATE, stream);
-    board_stats_kernel<<<(unsigned)ctas, STAT_WARPS * 32, smem, stream>>>(boards, B, G, count_current_wire, scored, detours, diversity, nullptr);
-  }
-  return check_launch("board_stats_kernel");
+  return launch_kernel(board_stats_kernel, (unsigned)ctas, STAT_WARPS * 32, smem, stream, RBG_K_VALIDATE, "board_stats_kernel", false, boards, B, G,
+                       count_current_wire, scored, detours, diversity, nullptr);
 }
 
 int launch_validate(const int32_t *boards, int64_t B, int G, int N, int32_t *flags, cudaStream_t stream) {
@@ -429,11 +415,7 @@ int launch_validate(const int32_t *boards, int64_t B, int G, int N, int32_t *fla
   const size_t smem = (size_t)VAL_WARPS * (2 * cp + 5 * 4 * RBG_MAX_N);
   int64_t ctas = (B + VAL_WARPS - 1) / VAL_WARPS;
   if (ctas > (int64_t)device_sm_count() * 64) ctas = (int64_t)device_sm_count() * 64;
-  {
-    LaunchScope scope(RBG_K_VALIDATE, stream);
-    validate_kernel<<<(unsigned)ctas, VAL_WARPS * 32, smem, stream>>>(boards, B, G, N, flags);
-  }
-  return check_launch("validate_kernel");
+  return launch_kernel(validate_kernel, (unsigned)ctas, VAL_WARPS * 32, smem, stream, RBG_K_VALIDATE, "validate_kernel", false, boards, B, G, N, flags);
 }
 
 // ---- host transport of the observation (rbg_connector_step_host_io) -------------------------------------
@@ -480,21 +462,13 @@ int launch_narrow_codes(const int32_t *src, uint8_t *dst, int64_t n, cudaStream_
     const int64_t cap4 = (int64_t)device_sm_count() * 8;
     if (ctas4 > cap4) ctas4 = cap4;
     if (ctas4 < 1) ctas4 = 1;
-    {
-      LaunchScope scope(-1, stream);
-      narrow_codes4_kernel<<<(unsigned)ctas4, 256, 0, stream>>>(src, dst, (long long)n);
-    }
-    return check_launch("narrow_codes4_kernel");
+    return launch_kernel(narrow_codes4_kernel, (unsigned)ctas4, 256, 0, stream, -1, "narrow_codes4_kernel", false, src, dst, (long long)n);
   }
   int64_t ctas = ((n >> 4) + 255) / 256;
   const int64_t cap = (int64_t)device_sm_count() * 8;
   if (ctas > cap) ctas = cap;
   if (ctas < 1) ctas = 1;
-  {
-    LaunchScope scope(-1, stream);
-    narrow_codes_kernel<<<(unsigned)ctas, 256, 0, stream>>>(src, dst, (long long)n);
-  }
-  return check_launch("narrow_codes_kernel");
+  return launch_kernel(narrow_codes_kernel, (unsigned)ctas, 256, 0, stream, -1, "narrow_codes_kernel", false, src, dst, (long long)n);
 }
 
 }  // namespace rbg

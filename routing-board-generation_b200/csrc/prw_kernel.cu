@@ -420,7 +420,6 @@ __device__ __forceinline__ void prw_body(const PrwParams &p, uint8_t *smem_raw) 
 
 __global__ void __launch_bounds__(256) prw_kernel(const PrwParams p) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
-  if (p.trigger_dependents) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   prw_body(p, smem_raw);
 }
 
@@ -536,15 +535,7 @@ int launch_prw(PrwParams p, int64_t max_boards, cudaStream_t stream) {
   int64_t ctas = 0;
   if ((rc = prw_prepare(p, max_boards, &threads, &smem, &ctas))) return rc;
   if (ctas <= 0) return RBG_OK;
-  if (smem > 48 * 1024) {
-    cudaError_t e = cudaFuncSetAttribute(prw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return set_cuda_error(e, "cudaFuncSetAttribute(prw_kernel)");
-  }
-  {
-    LaunchScope scope(RBG_K_PRW, stream);
-    prw_kernel<<<(unsigned)ctas, threads, smem, stream>>>(p);
-  }
-  return check_launch("prw_kernel");
+  return launch_kernel(prw_kernel, (unsigned)ctas, threads, smem, stream, RBG_K_PRW, "prw_kernel", false, p);
 }
 
 // per-step auto-reset: synchronous list `a` and the cache refill `b` (both short lists of the same batch) in one launch
@@ -577,15 +568,7 @@ int launch_prw_pair(PrwParams a, PrwParams b, int64_t max_boards, cudaStream_t s
   if (ctas > (int64_t)sms * 4) ctas = (int64_t)sms * 4;  // per-step lists hold a few percent of the batch; both halves stride
   if (ca > ctas) ctas = ca;
   if (ctas <= 0) return RBG_OK;
-  if (smem > 48 * 1024) {
-    cudaError_t e = cudaFuncSetAttribute(prw_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return set_cuda_error(e, "cudaFuncSetAttribute(prw_pair_kernel)");
-  }
-  {
-    LaunchScope scope(RBG_K_PRW, stream);
-    prw_pair_kernel<<<(unsigned)ctas, 64, smem, stream>>>(a, rf, gc);
-  }
-  return check_launch("prw_pair_kernel");
+  return launch_kernel(prw_pair_kernel, (unsigned)ctas, 64, smem, stream, RBG_K_PRW, "prw_pair_kernel", false, a, rf, gc);
 }
 
 }  // namespace rbg

@@ -5,6 +5,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <utility>
+
 #include "../../include/rbg_b200.h"
 #include "rbg_device.cuh"
 
@@ -28,6 +30,40 @@ struct LaunchScope {
   ~LaunchScope();
 };
 
+// A kernel that takes more than the default 48 KB of dynamic shared memory per CTA has to opt in, before its launch
+// and before an occupancy query at that size (which reports 0 CTAs per SM without it).
+template <typename... KArgs>
+int opt_in_smem(void (*kernel)(KArgs...), size_t smem, const char *name) {
+  if (smem <= 48 * 1024) return RBG_OK;
+  const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  return e == cudaSuccess ? RBG_OK : set_cuda_error(e, name);
+}
+
+// Every kernel of the library is launched here: the shared-memory opt-in, one LaunchScope under kernel id `id`
+// (RBG_K_*, or -1: counted, never timed), and the launch.  pdl: programmatic stream serialization (the kernel may
+// begin while a preceding kernel that has said launch_dependents is still running; any other predecessor completes
+// first).
+template <typename... KArgs, typename... Args>
+int launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, int id, const char *name, bool pdl,
+                  Args &&...args) {
+  if (int rc = opt_in_smem(kernel, smem, name)) return rc;
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr.val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid;
+  cfg.blockDim = block;
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = stream;
+  cfg.attrs = &attr;
+  cfg.numAttrs = pdl ? 1 : 0;
+  {
+    LaunchScope scope(id, stream);
+    cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+  }
+  return check_launch(name);  // the launch's own error too: the runtime keeps it as the thread's last error
+}
+
 // ---- generator kernel (prw_kernel.cu) -----------------------------------
 enum : int { PRW_MODE_BOARD = 0, PRW_MODE_STATE = 1, PRW_MODE_UNIFORM = 2 };
 
@@ -48,8 +84,6 @@ struct PrwParams {
   // auto-reset cache refill: keys[] is indexed by list slot (not env id) and the
   // result goes to the env's cache entry instead of State / TimeStep
   int keys_compact, to_cache;
-  int trigger_dependents;  // griddepcontrol.launch_dependents at the start: the next kernel of the stream, if it was launched
-                           // with programmatic stream serialization, need not wait for this one (per-step cache refill)
   unsigned long long *cache_tag;  // [B]   state.key this entry succeeds (k0 | k1 << 32)
   uint2 *cache_key;               // [B]   State.key of the cached episode
   uint32_t *cache_pins;           // [B,N] start_r<<24 | start_c<<16 | target_r<<8 | target_c
@@ -92,8 +126,7 @@ struct EnvParams {
   FastDiv divG, divC4, divCells;
 };
 
-// pdl: launch with programmatic stream serialization (the kernel may begin while a preceding kernel that has said
-// launch_dependents is still running; any other predecessor completes first)
+// pdl: as in launch_kernel
 int launch_env(EnvParams p, cudaStream_t stream, bool pdl = false);
 // T random-policy steps in one launch, auto-reset from the board dataset of p.env; ts fields stacked [T,B,...]
 int launch_rollout(EnvParams p, int T, int32_t *action_out, cudaStream_t stream);
@@ -139,6 +172,13 @@ void host_pool_widen4(const uint8_t *src, int32_t *dst, size_t n); // the same f
 void host_pool_wait();                                            // until every enqueued piece is done
 
 // ---- seed extension (seedext_kernel.cu) ---------------------------------
+// What a SeedExtension or SequentialRandomWalk call writes
+enum GenMode : int {
+  GEN_MODE_BOARD = 0,       // the solved board
+  GEN_MODE_STARTS_ENDS = 1, // the first POSITION / TARGET cell per wire
+  GEN_MODE_STATE = 2,       // a Connector State (+ observation)
+};
+
 struct SeedExtParams {
   const uint32_t *keys;
   long long B;
@@ -147,20 +187,19 @@ struct SeedExtParams {
   int two_sided, iterations;
   long long ext_steps;  // < 0 unlimited
   int extra_split;
-  int mode;  // 0 solved board, 1 starts/ends, 2 State
+  GenMode mode;
   int32_t *solved, *starts, *ends;
   rbg_state st;
   rbg_timestep ts;
   int observe;
   const int32_t *list;
   const int32_t *list_count;
-  int solved_f32;  // mode 0: the codes as float32 (SequentialRandomWalkBoard.generate returns jnp.zeros' default dtype)
+  int solved_f32;  // GEN_MODE_BOARD: the codes as float32 (SequentialRandomWalkBoard.generate returns jnp.zeros' default dtype)
 };
 int launch_seedext(SeedExtParams p, int64_t max_boards, cudaStream_t stream);
 void keep_pool_cached();  // cudaMallocAsync's default pool keeps its memory across synchronisations (scratch of the generators)
 // se_finish_kernel on its own: boards[max_boards, CB] bytes (row-major G*G codes, CB = cells rounded up to 16) and
-// gkey[max_boards, 2] (State.key) -> the outputs of p.mode (0 board, 1 first POSITION / TARGET cell per wire, 2 State
-// (+ observation)); slot m of the scratch is board p.list[m] when p.list is set
+// gkey[max_boards, 2] (State.key) -> the outputs of p.mode; slot m of the scratch is board p.list[m] when p.list is set
 int launch_board_finish(const SeedExtParams &p, const uint8_t *boards, const uint32_t *gkey, int CB, int64_t max_boards, int kernel_id,
                         cudaStream_t stream);
 
@@ -170,8 +209,8 @@ struct SeqRwParams {
   long long B;
   int G, N;
   int extra_split;
-  int mode;         // 0 board, 1 starts/ends, 2 State
-  int float_board;  // mode 0: float32 codes
+  GenMode mode;
+  int float_board;  // GEN_MODE_BOARD: float32 codes
   int32_t *board, *starts, *ends;
   int32_t *stats;  // optional [B,2]: attempt that succeeded (0 = none), its steps
   rbg_state st;

@@ -763,7 +763,7 @@ __global__ void __launch_bounds__(SE_FIN_WARPS * 32) se_finish_kernel(const Seed
   if (lane < N) first[2 * lane] = first[2 * lane + 1] = cells;
   __syncwarp();
 
-  if (p.mode == 0) {  // return_solved_board: int32[G,G]
+  if (p.mode == GEN_MODE_BOARD) {  // return_solved_board: int32[G,G]
     int32_t *out = p.solved + e * cells;
     if (p.solved_f32) {  // SequentialRandomWalkBoard.generate: the same codes as float32
       float *fo = reinterpret_cast<float *>(out);
@@ -805,7 +805,7 @@ __global__ void __launch_bounds__(SE_FIN_WARPS * 32) se_finish_kernel(const Seed
     tr = (int)q;
     tc = (int)r;
   }
-  if (p.mode == 1) {
+  if (p.mode == GEN_MODE_STARTS_ENDS) {
     if (lane < N) {
       p.starts[e * 2 * N + lane] = sr;
       p.starts[e * 2 * N + N + lane] = scol;
@@ -861,15 +861,6 @@ __global__ void __launch_bounds__(SE_FIN_WARPS * 32) se_finish_kernel(const Seed
 
 // ---------------------------------------------------------------- host side
 static size_t round_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
-
-static int set_smem(const void *fn, size_t bytes, const char *name) {
-  if (bytes > 227 * 1024) return set_error(RBG_EINVAL, "%s needs %zu bytes of shared memory per CTA", name, bytes);
-  if (bytes > 48 * 1024) {
-    cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    if (e != cudaSuccess) return set_cuda_error(e, name);
-  }
-  return RBG_OK;
-}
 
 // second stream + fork / join events of the overlapped optimise kernel, one set per device
 struct SeOverlap {
@@ -927,8 +918,8 @@ int launch_seedext(SeedExtParams p, int64_t max_boards, cudaStream_t stream) {
   d.lane_words_ext = (d.SB2w + (G > 32 ? 2 : 1) * G) | 1;  // board + one mask of wire ends per row; odd: lanes on the same cell hit 32 different banks
   d.S1 = G + 2;
   d.SB1 = (int)round_up((size_t)d.S1 * d.S1, 4);
+  const bool byte_fifo = d.S1 * d.S1 <= 256;
   {
-    const bool byte_fifo = d.S1 * d.S1 <= 256;
     d.fifo_bytes = (int)((byte_fifo ? 1 : 2) * (size_t)((d.cells + 3) & ~1));
     size_t b = 2 * (size_t)d.SB1 + (size_t)d.fifo_bytes + 2 * (size_t)(2 * N);
     b = round_up(b, 4);
@@ -957,13 +948,13 @@ int launch_seedext(SeedExtParams p, int64_t max_boards, cudaStream_t stream) {
     }
   }
   int rc = RBG_OK;
-  const bool wide = G > 32;
-  const void *ext_fn = wide ? reinterpret_cast<const void *>(se_extend_kernel<true>) : reinterpret_cast<const void *>(se_extend_kernel<false>);
-  if ((rc = set_smem(ext_fn, ext_warp * ext_w + 32, "se_extend_kernel"))) return rc;
-  const bool byte_fifo = d.S1 * d.S1 <= 256;
-  if ((rc = set_smem(byte_fifo ? reinterpret_cast<const void *>(se_optimise_kernel<uint8_t>) : reinterpret_cast<const void *>(se_optimise_kernel<uint16_t>), opt_warp * opt_w,
-                     "se_optimise_kernel")))
-    return rc;
+  decltype(&se_extend_kernel<false>) ext_fn = G > 32 ? se_extend_kernel<true> : se_extend_kernel<false>;
+  decltype(&se_optimise_kernel<uint8_t>) opt_fn = byte_fifo ? se_optimise_kernel<uint8_t> : se_optimise_kernel<uint16_t>;
+  const size_t ext_smem = ext_warp * ext_w + 32, opt_smem = opt_warp * opt_w;
+  if (ext_smem > 227 * 1024) return set_error(RBG_EINVAL, "se_extend_kernel needs %zu bytes of shared memory per CTA", ext_smem);
+  if ((rc = opt_in_smem(ext_fn, ext_smem, "se_extend_kernel"))) return rc;
+  if (opt_smem > 227 * 1024) return set_error(RBG_EINVAL, "se_optimise_kernel needs %zu bytes of shared memory per CTA", opt_smem);
+  if ((rc = opt_in_smem(opt_fn, opt_smem, "se_optimise_kernel"))) return rc;
   {
     static int rmin = -1;
     if (rmin < 0) {
@@ -978,10 +969,9 @@ int launch_seedext(SeedExtParams p, int64_t max_boards, cudaStream_t stream) {
   unsigned ext_ctas = 1;
   {
     int per_sm = 0;
-    cudaError_t oe = wide ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, se_extend_kernel<true>, ext_w * 32, ext_warp * ext_w + 32)
-                          : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, se_extend_kernel<false>, ext_w * 32, ext_warp * ext_w + 32);
+    cudaError_t oe = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ext_fn, ext_w * 32, ext_smem);
     if (oe != cudaSuccess) return set_cuda_error(oe, "cudaOccupancyMaxActiveBlocksPerMultiprocessor(se_extend_kernel)");
-    if (per_sm < 1) return set_error(RBG_EINVAL, "se_extend_kernel: a CTA of %d warps does not fit an SM (%zu bytes of shared memory)", ext_w, ext_warp * ext_w + 32);
+    if (per_sm < 1) return set_error(RBG_EINVAL, "se_extend_kernel: a CTA of %d warps does not fit an SM (%zu bytes of shared memory)", ext_w, ext_smem);
     static int cap = -1;
     if (cap < 0) {
       const char *ex = getenv("RBG_SE_CTAS_PER_SM");
@@ -1004,8 +994,7 @@ int launch_seedext(SeedExtParams p, int64_t max_boards, cudaStream_t stream) {
   unsigned opt_resident = 1;
   {
     int per_sm = 0;
-    cudaError_t oe = byte_fifo ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, se_optimise_kernel<uint8_t>, opt_w * 32, opt_warp * opt_w)
-                               : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, se_optimise_kernel<uint16_t>, opt_w * 32, opt_warp * opt_w);
+    cudaError_t oe = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, opt_fn, opt_w * 32, opt_smem);
     if (oe != cudaSuccess) return set_cuda_error(oe, "cudaOccupancyMaxActiveBlocksPerMultiprocessor(se_optimise_kernel)");
     opt_resident = (unsigned)((per_sm < 1 ? 1 : per_sm) * device_sm_count());
   }
@@ -1044,10 +1033,8 @@ int launch_seedext(SeedExtParams p, int64_t max_boards, cudaStream_t stream) {
     {  // seeding: one warp per board
       const size_t smem = sizeof(uint64_t) * SE_SEED_WARPS * d.cap + sizeof(uint16_t) * SE_SEED_WARPS * ((N + 1) & ~1);
       const unsigned ctas = (unsigned)((max_boards + SE_SEED_WARPS - 1) / SE_SEED_WARPS);
-      LaunchScope scope(RBG_K_SEEDEXT, stream);
-      se_seed_kernel<<<ctas, SE_SEED_WARPS * 32, smem, stream>>>(p, d, sc);
+      if ((rc = launch_kernel(se_seed_kernel, ctas, SE_SEED_WARPS * 32, smem, stream, RBG_K_SEEDEXT, "se_seed_kernel", false, p, d, sc))) break;
     }
-    if ((rc = check_launch("se_seed_kernel"))) break;
     for (int it = 0; it < p.iterations && rc == RBG_OK; ++it) {  // SE:180-200 while_loop over extension_iterations
       // The optimise kernel runs WHILE the extend kernel does (on a second stream), on the boards the extend kernel
       // has finished: extension ends in a long tail (a board needs 6 .. 45 sweeps and every sweep is a sequential hash
@@ -1070,34 +1057,21 @@ int launch_seedext(SeedExtParams p, int64_t max_boards, cudaStream_t stream) {
           break;
         }
       }
-      {
-        LaunchScope scope(RBG_K_SEEDEXT, stream);
-        if (wide)
-          se_extend_kernel<true><<<ext_ctas, ext_w * 32, ext_warp * ext_w + 32, stream>>>(p, d, sc, qu);
-        else
-          se_extend_kernel<false><<<ext_ctas, ext_w * 32, ext_warp * ext_w + 32, stream>>>(p, d, sc, qu);
-      }
-      if ((rc = check_launch("se_extend_kernel"))) break;
+      if ((rc = launch_kernel(ext_fn, ext_ctas, ext_w * 32, ext_smem, stream, RBG_K_SEEDEXT, "se_extend_kernel", false, p, d, sc, qu))) break;
       if (ov) {  // beside the extend kernel: as many CTAs as the device holds; they move in as the extend CTAs leave
         unsigned ctas = (unsigned)((max_boards + opt_w * 32 - 1) / (opt_w * 32));
         if (ctas > opt_resident) ctas = opt_resident;
-        LaunchScope scope(RBG_K_SEEDEXT, ov->side);
-        if (byte_fifo)
-          se_optimise_kernel<uint8_t><<<ctas, opt_w * 32, opt_warp * opt_w, ov->side>>>(p, d, sc, done_list, queue + 128 + it, qu.resident, (int)ext_ctas);
-        else
-          se_optimise_kernel<uint16_t><<<ctas, opt_w * 32, opt_warp * opt_w, ov->side>>>(p, d, sc, done_list, queue + 128 + it, qu.resident, (int)ext_ctas);
-        if ((rc = check_launch("se_optimise_kernel"))) break;
+        if ((rc = launch_kernel(opt_fn, ctas, opt_w * 32, opt_smem, ov->side, RBG_K_SEEDEXT, "se_optimise_kernel", false, p, d, sc, done_list, queue + 128 + it,
+                                qu.resident, (int)ext_ctas)))
+          break;
       }
       {  // behind the extend kernel: everything (no overlap), or what the first launch has not taken
         unsigned ctas = (unsigned)((max_boards + opt_w * 32 - 1) / (opt_w * 32));
         if (ov && ctas > opt_resident) ctas = opt_resident;
-        LaunchScope scope(RBG_K_SEEDEXT, stream);
-        if (byte_fifo)
-          se_optimise_kernel<uint8_t><<<ctas, opt_w * 32, opt_warp * opt_w, stream>>>(p, d, sc, ov ? done_list : nullptr, queue + 128 + it, nullptr, 0);
-        else
-          se_optimise_kernel<uint16_t><<<ctas, opt_w * 32, opt_warp * opt_w, stream>>>(p, d, sc, ov ? done_list : nullptr, queue + 128 + it, nullptr, 0);
+        if ((rc = launch_kernel(opt_fn, ctas, opt_w * 32, opt_smem, stream, RBG_K_SEEDEXT, "se_optimise_kernel", false, p, d, sc, ov ? done_list : nullptr,
+                                queue + 128 + it, nullptr, 0)))
+          break;
       }
-      if ((rc = check_launch("se_optimise_kernel"))) break;
       if (ov) {
         if ((ce2 = cudaEventRecord(ov->join, ov->side)) != cudaSuccess || (ce2 = cudaStreamWaitEvent(stream, ov->join, 0)) != cudaSuccess) {
           rc = set_cuda_error(ce2, "SeedExtension: join of the optimise stream");
@@ -1109,10 +1083,8 @@ int launch_seedext(SeedExtParams p, int64_t max_boards, cudaStream_t stream) {
     {
       const size_t smem = (size_t)SE_FIN_WARPS * (2 * sc.CB + 8 * RBG_MAX_N);
       const unsigned ctas = (unsigned)((max_boards + SE_FIN_WARPS - 1) / SE_FIN_WARPS);
-      LaunchScope scope(RBG_K_SEEDEXT, stream);
-      se_finish_kernel<<<ctas, SE_FIN_WARPS * 32, smem, stream>>>(p, d, sc, FastDiv::make((uint32_t)G));
+      rc = launch_kernel(se_finish_kernel, ctas, SE_FIN_WARPS * 32, smem, stream, RBG_K_SEEDEXT, "se_finish_kernel", false, p, d, sc, FastDiv::make((uint32_t)G));
     }
-    rc = check_launch("se_finish_kernel");
   } while (0);
   cudaFreeAsync(base, stream);
   return rc;
@@ -1132,11 +1104,8 @@ int launch_board_finish(const SeedExtParams &p, const uint8_t *boards, const uin
   sc.CB = CB;
   const size_t smem = (size_t)SE_FIN_WARPS * (2 * sc.CB + 8 * RBG_MAX_N);
   const unsigned ctas = (unsigned)((max_boards + SE_FIN_WARPS - 1) / SE_FIN_WARPS);
-  {
-    LaunchScope scope(kernel_id, stream);
-    se_finish_kernel<<<ctas < 1 ? 1 : ctas, SE_FIN_WARPS * 32, smem, stream>>>(p, d, sc, FastDiv::make((uint32_t)p.G));
-  }
-  return check_launch("se_finish_kernel");
+  return launch_kernel(se_finish_kernel, ctas < 1 ? 1 : ctas, SE_FIN_WARPS * 32, smem, stream, kernel_id, "se_finish_kernel", false, p, d, sc,
+                       FastDiv::make((uint32_t)p.G));
 }
 
 }  // namespace rbg

@@ -386,7 +386,7 @@ int launch_seqrw(SeqRwParams p, int64_t max_boards, cudaStream_t stream) {
   // 32x32/16 2.48 / 2.82
   const int W = w_env ? w_env : (G <= 16 ? 6 : 8);
   const int SQ_GROUPS = W == 6 ? SqShape<6>::GROUPS : SqShape<8>::GROUPS;
-  const void *fn = W == 6 ? reinterpret_cast<const void *>(seqrw_walk_kernel<6>) : reinterpret_cast<const void *>(seqrw_walk_kernel<8>);
+  decltype(&seqrw_walk_kernel<8>) fn = W == 6 ? seqrw_walk_kernel<6> : seqrw_walk_kernel<8>;
   const size_t smem = (size_t)(SQ_GROUPS + 1) * SB + (size_t)SQ_GROUPS * 4 * RBG_MAX_N * sizeof(uint32_t);
   const size_t n = (size_t)max_boards;
   const size_t o_gkey = (n * CB + 255) & ~(size_t)255, o_queue = o_gkey + ((n * 8 + 255) & ~(size_t)255), total = o_queue + 256;
@@ -402,27 +402,18 @@ int launch_seqrw(SeqRwParams p, int64_t max_boards, cudaStream_t stream) {
       rc = set_cuda_error(ce, "cudaMemsetAsync(SequentialRandomWalk queue)");
       break;
     }
-    if (smem > 48 * 1024 && (ce = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) {
-      rc = set_cuda_error(ce, "seqrw_walk_kernel shared memory");
-      break;
-    }
+    if ((rc = opt_in_smem(fn, smem, "seqrw_walk_kernel"))) break;
     int per_sm = 0;
-    if ((ce = (W == 6 ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, seqrw_walk_kernel<6>, SQ_THREADS, smem)
-                      : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, seqrw_walk_kernel<8>, SQ_THREADS, smem))) != cudaSuccess) {
+    if ((ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, SQ_THREADS, smem)) != cudaSuccess) {
       rc = set_cuda_error(ce, "cudaOccupancyMaxActiveBlocksPerMultiprocessor(seqrw_walk_kernel)");
       break;
     }
     const long long resident = (long long)(per_sm < 1 ? 1 : per_sm) * device_sm_count();
     const long long need = (max_boards + SQ_GROUPS - 1) / SQ_GROUPS;
     const unsigned ctas = (unsigned)(need < resident ? (need < 1 ? 1 : need) : resident);
-    {
-      LaunchScope scope(RBG_K_SEQRW, stream);
-      if (W == 6)
-        seqrw_walk_kernel<6><<<ctas, SQ_THREADS, smem, stream>>>(p, base, gkey, CB, queue, FastDiv::make((uint32_t)G));
-      else
-        seqrw_walk_kernel<8><<<ctas, SQ_THREADS, smem, stream>>>(p, base, gkey, CB, queue, FastDiv::make((uint32_t)G));
-    }
-    if ((rc = check_launch("seqrw_walk_kernel"))) break;
+    if ((rc = launch_kernel(fn, ctas, SQ_THREADS, smem, stream, RBG_K_SEQRW, "seqrw_walk_kernel", false, p, base, gkey, CB, queue,
+                            FastDiv::make((uint32_t)G))))
+      break;
     SeedExtParams f;
     memset(&f, 0, sizeof(f));
     f.keys = p.keys;

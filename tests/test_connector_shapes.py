@@ -169,6 +169,38 @@ def test_autoreset_steps(rbg, orc, kind, G, N, B):
         _assert_timestep(ts, rts, f"at step {t}")
 
 
+@pytest.mark.parametrize("kind", ["parallel_random_walk", "uniform"])
+@pytest.mark.parametrize("G,N", [(10, 5), (28, 2)])
+def test_autoreset_steps_under_kernel_timing(rbg, kind, G, N):
+    """VmapAutoResetWrapper.step_random while kernel timing is on, where the env kernel is not chained to the step
+    before it.  With time_limit 2 envs finish in back-to-back steps.  State, TimeStep and actions are bit-identical to
+    the same steps with timing off, and every step is one env kernel and one generator launch (the synchronous resets
+    and the cache refill), plus the warm-start generation on the step that adopts the workspace."""
+    L, B = rbg._lib, _batch(N)
+    runs = []
+    for timing in (False, True):
+        env = rbg.VmapAutoResetWrapper(_env(rbg, kind, G, N, 2))
+        st, _ = env.reset(rbg.split(rbg.PRNGKey(G * 100 + N), B))
+        L.kernel_timing(timing)
+        try:
+            L.kernel_time("env"), L.kernel_time("prw")  # drop whatever was recorded before
+            out = []
+            for t in range(6):
+                st, ts, act = env.step_random(st)
+                o, a = ts.observation, st.agents
+                out.append([_np(x) for x in (act, st.grid, st.step_count, st.key, a.id, a.start, a.target, a.position, o.grid, o.action_mask,
+                                             o.step_count, ts.step_type, ts.reward, ts.discount, *ts.extras.values())])
+                if timing:
+                    assert L.kernel_time("env")[0] == 1, f"env launches at step {t}"
+                    assert L.kernel_time("prw")[0] == (2 if t == 0 else 1), f"generator launches at step {t}"
+        finally:
+            L.kernel_timing(False)
+        runs.append(out)
+    for t, (off, on) in enumerate(zip(*runs)):
+        for i, (x, y) in enumerate(zip(off, on)):
+            assert _same(y, x), f"leaf {i} differs at step {t} with kernel timing on"
+
+
 # ------------------------------------------------------------------ fused rollout
 def _check_rollout(rbg, orc, env, st, rst, kind, T, time_limit, ds, reward=(-0.03, 0.1), where=""):
     st, ts, act = env.rollout_random(st, T)
