@@ -129,7 +129,9 @@ static inline int32_t randint_from_bits(uint32_t hi_bits, uint32_t lo_bits,
   uint32_t span = (uint32_t)(hi - lo);
   if (hi <= lo) span = 1;
   uint32_t mult = (uint32_t)(65536u % span);
-  mult = (uint32_t)(((uint64_t)mult * mult) % span); /* mult < span <= 2^31 here */
+  /* jax squares in the span's dtype, uint32: for span > 2^16 the square 2^32
+   * wraps to 0, so the value is lo + lo_bits % span. */
+  mult = (mult * mult) % span;
   uint32_t off = (hi_bits % span) * mult + (lo_bits % span); /* uint32 wrap */
   off = off % span;
   return lo + (int32_t)off;

@@ -105,7 +105,9 @@ __device__ __forceinline__ uint32_t dataset_pick(uint32_t k0, uint32_t k1, uint3
   split2(nk0, nk1, h0, h1, l0, l1);
   const uint32_t hi = bits_scalar(h0, h1), lo = bits_scalar(l0, l1);
   uint32_t mult = 65536u % K;
-  mult = (uint32_t)(((unsigned long long)mult * mult) % K);
+  // jax squares the multiplier in the span's dtype, uint32: for K > 2^16 the square 2^32 wraps to 0 and
+  // the pick is bits(k2) % K.  A 64-bit square would pick other boards at every such K but a power of two.
+  mult = (mult * mult) % K;
   return ((hi % K) * mult + (lo % K)) % K;
 }
 

@@ -795,6 +795,9 @@ def test_connector_reference_fixtures_on_gpu(rbg):
     ("offline_parallel_rw", 5, 3, 3, 2),          # cells % 4 != 0: scalar stores
     ("offline_parallel_rw", 12, 10, 40, 5),       # two alternating staging buffers
     ("offline_parallel_rw", 32, 16, 20, 5),       # direct 128-bit stores
+    ("offline_parallel_rw", 10, 5, 100000, 7),    # more boards than 2^16: jax's pick is the low draw mod K
+    ("offline_parallel_rw", 5, 3, 65537, 2),
+    ("offline_seed_extension", 10, 5, 100000, 5),  # the reference's offline-training dataset
 ])
 def test_connector_with_dataset_generator(rbg, orc, board_name, G, N, K, time_limit):
     """Connector(generator=BoardDatasetGeneratorJAX(...)) as rl_training/setup_train.py:119-133,158 builds it:

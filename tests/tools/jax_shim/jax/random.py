@@ -96,7 +96,7 @@ def randint(key, shape, minval, maxval, dtype=_np.int32):
     span = (maxval - minval) & 0xFFFFFFFF
     if maxval <= minval:
         span = 1
-    mult = (65536 % span) ** 2 % span
+    mult = ((65536 % span) ** 2 & 0xFFFFFFFF) % span  # squared in uint32: 2**32 wraps to 0 for span > 2**16
     off = ((hi_bits % span) * mult + (lo_bits % span)) & 0xFFFFFFFF  # uint32 arithmetic wraps
     off = off % span
     return asarr((minval + off.astype(_np.int64)).astype(_np.int32).reshape(shape))
