@@ -487,6 +487,16 @@ static int sync_streams() {
   return rc;
 }
 
+// A _host call that fails after it has enqueued copies waits for its streams before it returns, so that no copy from
+// or into the caller's buffers is in flight once it has returned.  The message stays the failure's.
+static int fail_synced(int rc) {
+  char msg[sizeof(g_err)];
+  memcpy(msg, g_err, sizeof(msg));
+  sync_streams();
+  memcpy(g_err, msg, sizeof(msg));
+  return rc;
+}
+
 struct Carver {
   uint8_t *base;
   size_t off = 0;
@@ -1046,18 +1056,34 @@ int rbg_prw_generate_host(const uint32_t *keys, int64_t B, int G, int N, int32_t
   scratch_claim(ScratchSig{1, B, G, N, -1, base}, nullptr, 0, 0);
   const int nsl = B >= 4096 ? 4 : 1;
   const int64_t sl = slice_size(B, nsl);
-  int si = 0;
-  for (int64_t off = 0; off < B; off += sl, ++si) {
-    const int64_t n = (B - off) < sl ? (B - off) : sl;
-    cudaStream_t st = g_hc->streams[si % 3];
-    RBG_CPY(dk + off * 2, keys + off * 2, n * 8, cudaMemcpyHostToDevice, st);
-    rc = rbg_prw_generate(dk + off * 2, n, G, N, dh + off * 2 * N, dt + off * 2 * N, ds + off * G * G, nullptr, st);
-    if (rc) return rc;
-    RBG_CPY(heads + off * 2 * N, dh + off * 2 * N, n * 2 * N * 4, cudaMemcpyDeviceToHost, st);
-    RBG_CPY(targets + off * 2 * N, dt + off * 2 * N, n * 2 * N * 4, cudaMemcpyDeviceToHost, st);
-    RBG_CPY(solved + off * G * G, ds + off * G * G, n * G * G * 4, cudaMemcpyDeviceToHost, st);
-  }
-  return sync_streams();
+  rc = [&]() -> int {
+    int si = 0;
+    for (int64_t off = 0; off < B; off += sl, ++si) {
+      const int64_t n = (B - off) < sl ? (B - off) : sl;
+      cudaStream_t st = g_hc->streams[si % 3];
+      RBG_CPY(dk + off * 2, keys + off * 2, n * 8, cudaMemcpyHostToDevice, st);
+      int r = rbg_prw_generate(dk + off * 2, n, G, N, dh + off * 2 * N, dt + off * 2 * N, ds + off * G * G, nullptr, st);
+      if (r) return r;
+      RBG_CPY(heads + off * 2 * N, dh + off * 2 * N, n * 2 * N * 4, cudaMemcpyDeviceToHost, st);
+      RBG_CPY(targets + off * 2 * N, dt + off * 2 * N, n * 2 * N * 4, cudaMemcpyDeviceToHost, st);
+      RBG_CPY(solved + off * G * G, ds + off * G * G, n * G * G * 4, cudaMemcpyDeviceToHost, st);
+    }
+    return RBG_OK;
+  }();
+  return rc ? fail_synced(rc) : sync_streams();
+}
+
+// The generator kinds rbg_connector_reset_host can run (the dataset kind needs its boards: rbg_connector_reset_dataset),
+// and the auto-reset kinds of the step variants; checked before any CUDA call.
+static int check_host_reset_kind(int kind) {
+  if (kind == RBG_GEN_DATASET)
+    return set_error(RBG_EINVAL, "rbg_connector_reset_host: RBG_GEN_DATASET needs the dataset's boards (rbg_connector_reset_dataset)");
+  if (kind < RBG_GEN_PRW || kind > RBG_GEN_SEQRW) return set_error(RBG_EINVAL, "rbg_connector_reset_host: unknown generator kind %d", kind);
+  return RBG_OK;
+}
+static int check_host_params(const rbg_env_params *params) {
+  if (params->autoreset_kind > RBG_GEN_SEQRW) return set_error(RBG_EINVAL, "unknown autoreset generator kind %d", params->autoreset_kind);
+  return params->autoreset_kind == RBG_GEN_DATASET ? check_dataset(params) : RBG_OK;
 }
 
 int rbg_connector_reset_host(int kind, const uint32_t *keys, int64_t B, int G, int N, const rbg_state *state,
@@ -1066,6 +1092,7 @@ int rbg_connector_reset_host(int kind, const uint32_t *keys, int64_t B, int G, i
   if ((rc = check_dims(B, G, N, kind == RBG_GEN_UNIFORM ? 2 : 1))) return rc;
   if (B == 0) return RBG_OK;  // an empty batch has no buffers to check
   if (!keys || !state || !ts) return set_error(RBG_EINVAL, "rbg_connector_reset_host: NULL pointer");
+  if ((rc = check_host_reset_kind(kind))) return rc;
   if ((rc = use_device(device, &dev))) return rc;
   std::lock_guard<std::mutex> lock(g_scratch_mu);
   uint32_t *dk;
@@ -1081,18 +1108,21 @@ int rbg_connector_reset_host(int kind, const uint32_t *keys, int64_t B, int G, i
   scratch_claim(ScratchSig{2, B, G, N, kind, base}, nullptr, 0, 0);
   const int nsl = B >= 4096 ? 4 : 1;
   const int64_t sl = slice_size(B, nsl);
-  int si = 0;
-  for (int64_t off = 0; off < B; off += sl, ++si) {
-    const int64_t n = (B - off) < sl ? (B - off) : sl;
-    cudaStream_t st = g_hc->streams[si % 3];
-    RBG_CPY(dk + off * 2, keys + off * 2, n * 8, cudaMemcpyHostToDevice, st);
-    rbg_state dss = state_at(ds, off, G, N);
-    rbg_timestep dts = timestep_at(dt, off, G, N);
-    if ((rc = rbg_connector_reset(kind, dk + off * 2, n, G, N, &dss, &dts, st))) return rc;
-    if ((rc = copy_state(state, &ds, off, n, G, N, cudaMemcpyDeviceToHost, off, st))) return rc;
-    if ((rc = copy_timestep(ts, &dt, off, n, G, N, cudaMemcpyDeviceToHost, off, st))) return rc;
-  }
-  return sync_streams();
+  rc = [&]() -> int {
+    int si = 0, r;
+    for (int64_t off = 0; off < B; off += sl, ++si) {
+      const int64_t n = (B - off) < sl ? (B - off) : sl;
+      cudaStream_t st = g_hc->streams[si % 3];
+      RBG_CPY(dk + off * 2, keys + off * 2, n * 8, cudaMemcpyHostToDevice, st);
+      rbg_state dss = state_at(ds, off, G, N);
+      rbg_timestep dts = timestep_at(dt, off, G, N);
+      if ((r = rbg_connector_reset(kind, dk + off * 2, n, G, N, &dss, &dts, st))) return r;
+      if ((r = copy_state(state, &ds, off, n, G, N, cudaMemcpyDeviceToHost, off, st))) return r;
+      if ((r = copy_timestep(ts, &dt, off, n, G, N, cudaMemcpyDeviceToHost, off, st))) return r;
+    }
+    return RBG_OK;
+  }();
+  return rc ? fail_synced(rc) : sync_streams();
 }
 
 int rbg_connector_step_host(const rbg_state *in, const rbg_state *out, const int32_t *action, int64_t B, int G,
@@ -1101,6 +1131,7 @@ int rbg_connector_step_host(const rbg_state *in, const rbg_state *out, const int
   if ((rc = check_dims(B, G, N, 1))) return rc;
   if (B == 0) return RBG_OK;  // an empty batch has no buffers to check
   if (!in || !out || !action || !params || !ts) return set_error(RBG_EINVAL, "rbg_connector_step_host: NULL pointer");
+  if ((rc = check_host_params(params))) return rc;
   if ((rc = use_device(device, &dev))) return rc;
   std::lock_guard<std::mutex> lock(g_scratch_mu);
   const int nsl = B >= 4096 ? 8 : 1;
@@ -1120,20 +1151,22 @@ int rbg_connector_step_host(const rbg_state *in, const rbg_state *out, const int
   });
   if (rc) return rc;
   scratch_claim(ScratchSig{3, B, G, N, params->autoreset_kind, base}, ws, ws_bytes, nslices);
-  int si = 0;
-  for (int64_t off = 0; off < B; off += sl, ++si) {
-    const int64_t n = (B - off) < sl ? (B - off) : sl;
-    cudaStream_t st = g_hc->streams[si % 3];
-    if ((rc = copy_state(&ds, in, off, n, G, N, cudaMemcpyHostToDevice, off, st))) return rc;
-    RBG_CPY(da + off * N, action + off * N, n * N * 4, cudaMemcpyHostToDevice, st);
-    rbg_state dss = state_at(ds, off, G, N);
-    rbg_timestep dts = timestep_at(dt, off, G, N);
-    if ((rc = rbg_connector_step(&dss, &dss, da + off * N, n, G, N, params, &dts, ws + (size_t)si * ws_bytes, st)))
-      return rc;
-    if ((rc = copy_state(out, &ds, off, n, G, N, cudaMemcpyDeviceToHost, off, st))) return rc;
-    if ((rc = copy_timestep(ts, &dt, off, n, G, N, cudaMemcpyDeviceToHost, off, st))) return rc;
-  }
-  return sync_streams();
+  rc = [&]() -> int {
+    int si = 0, r;
+    for (int64_t off = 0; off < B; off += sl, ++si) {
+      const int64_t n = (B - off) < sl ? (B - off) : sl;
+      cudaStream_t st = g_hc->streams[si % 3];
+      if ((r = copy_state(&ds, in, off, n, G, N, cudaMemcpyHostToDevice, off, st))) return r;
+      RBG_CPY(da + off * N, action + off * N, n * N * 4, cudaMemcpyHostToDevice, st);
+      rbg_state dss = state_at(ds, off, G, N);
+      rbg_timestep dts = timestep_at(dt, off, G, N);
+      if ((r = rbg_connector_step(&dss, &dss, da + off * N, n, G, N, params, &dts, ws + (size_t)si * ws_bytes, st))) return r;
+      if ((r = copy_state(out, &ds, off, n, G, N, cudaMemcpyDeviceToHost, off, st))) return r;
+      if ((r = copy_timestep(ts, &dt, off, n, G, N, cudaMemcpyDeviceToHost, off, st))) return r;
+    }
+    return RBG_OK;
+  }();
+  return rc ? fail_synced(rc) : sync_streams();
 }
 
 // Env-pool style step: the State stays on the device (updated in place), the actions come from and
@@ -1145,6 +1178,7 @@ int rbg_connector_step_host_io(const rbg_state *state, const int32_t *action, in
   if (B == 0) return RBG_OK;  // an empty batch has no buffers to check
   if (!action || !params || !ts) return set_error(RBG_EINVAL, "rbg_connector_step_host_io: NULL pointer");
   if ((rc = check_state(state, "state", G))) return rc;
+  if ((rc = check_host_params(params))) return rc;
   if ((rc = use_device(device, &dev))) return rc;
   std::lock_guard<std::mutex> lock(g_scratch_mu);
   cudaError_t e;
@@ -1221,25 +1255,28 @@ int rbg_connector_step_host_io(const rbg_state *state, const int32_t *action, in
   // multiple of 64 envs, so every slice starts on a whole, 16-byte aligned byte when an env has an even number of cells).
   const int obits = (3 * N <= 15 && (per_env & 1u) == 0) ? 4 : 8;
   const int oshift = obits == 4 ? 1 : 0;
-  int si = 0;
-  for (int64_t off = 0; off < B; off += sl, ++si) {
-    const int64_t n = (B - off) < sl ? (B - off) : sl;
-    const size_t codes_off = ((size_t)off * per_env) >> oshift;
-    rbg_state dss = state_at(*state, off, G, N);
-    rbg_timestep dts = timestep_at(dt, off, G, N);
-    if ((rc = rbg_connector_step(&dss, &dss, da + off * N, n, G, N, params, &dts, ws + (size_t)si * ws_bytes, cs))) return rc;
-    if ((rc = launch_narrow_codes(dts.obs_grid, obs8 + codes_off, (int64_t)((size_t)n * per_env), cs, obits))) return rc;
-    if (!slice_ev[si] && (e = cudaEventCreateWithFlags(&slice_ev[si], cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
-    if ((e = cudaEventRecord(slice_ev[si], cs)) != cudaSuccess) return set_cuda_error(e, "cudaEventRecord");
-    cudaStream_t xs = g_hc->streams[1 + (si & 1)];
-    if ((e = cudaStreamWaitEvent(xs, slice_ev[si], 0)) != cudaSuccess) return set_cuda_error(e, "cudaStreamWaitEvent");
-    RBG_CPY(g_hc->stage8 + codes_off, obs8 + codes_off, ((size_t)n * per_env) >> oshift, cudaMemcpyDeviceToHost, xs);
-    if (!copy_ev[si] && (e = cudaEventCreateWithFlags(&copy_ev[si], cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
-    if ((e = cudaEventRecord(copy_ev[si], xs)) != cudaSuccess) return set_cuda_error(e, "cudaEventRecord(copy)");
-  }
-  if ((rc = copy_timestep(ts, &dt, 0, B, G, N, cudaMemcpyDeviceToHost, 0, cs, false))) return rc;
+  rc = [&]() -> int {
+    int si = 0, r;
+    for (int64_t off = 0; off < B; off += sl, ++si) {
+      const int64_t n = (B - off) < sl ? (B - off) : sl;
+      const size_t codes_off = ((size_t)off * per_env) >> oshift;
+      rbg_state dss = state_at(*state, off, G, N);
+      rbg_timestep dts = timestep_at(dt, off, G, N);
+      if ((r = rbg_connector_step(&dss, &dss, da + off * N, n, G, N, params, &dts, ws + (size_t)si * ws_bytes, cs))) return r;
+      if ((r = launch_narrow_codes(dts.obs_grid, obs8 + codes_off, (int64_t)((size_t)n * per_env), cs, obits))) return r;
+      if (!slice_ev[si] && (e = cudaEventCreateWithFlags(&slice_ev[si], cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
+      if ((e = cudaEventRecord(slice_ev[si], cs)) != cudaSuccess) return set_cuda_error(e, "cudaEventRecord");
+      cudaStream_t xs = g_hc->streams[1 + (si & 1)];
+      if ((e = cudaStreamWaitEvent(xs, slice_ev[si], 0)) != cudaSuccess) return set_cuda_error(e, "cudaStreamWaitEvent");
+      RBG_CPY(g_hc->stage8 + codes_off, obs8 + codes_off, ((size_t)n * per_env) >> oshift, cudaMemcpyDeviceToHost, xs);
+      if (!copy_ev[si] && (e = cudaEventCreateWithFlags(&copy_ev[si], cudaEventDisableTiming)) != cudaSuccess) return set_cuda_error(e, "cudaEventCreate");
+      if ((e = cudaEventRecord(copy_ev[si], xs)) != cudaSuccess) return set_cuda_error(e, "cudaEventRecord(copy)");
+    }
+    return copy_timestep(ts, &dt, 0, B, G, N, cudaMemcpyDeviceToHost, 0, cs, false);
+  }();
+  if (rc) return fail_synced(rc);
   g_d2h_bytes.fetch_add((long long)(obs_n >> oshift) + (long long)B * (N * 5 + 4 + N * 8 + 1 + 12), std::memory_order_relaxed);
-  si = 0;
+  int si = 0;
   for (int64_t off = 0; off < B; off += sl, ++si) {
     const int64_t n = (B - off) < sl ? (B - off) : sl;
     if ((e = cudaEventSynchronize(copy_ev[si])) != cudaSuccess) {
