@@ -272,6 +272,24 @@ int rbg_connector_eval_step(const rbg_state *state, const int32_t *action, uint8
                             int64_t B, int G, int N, const rbg_env_params *params, const rbg_timestep *ts,
                             const rbg_episode_metrics *acc, void *stream);
 
+/* rbg_connector_eval_step over a list of live envs, with the list and the observation compacted in the same pass: the
+ * step of a policy evaluation whose policy sees only the live envs.  Replaces a call of rbg_connector_eval_step
+ * whose batch still holds finished envs.
+ * Reads the envs order_in[0, L) and action int32[L,N], whose row i belongs to env order_in[i]; steps each of them as
+ * rbg_connector_eval_step steps a live env (State in place, record `acc` accumulated, extras into the record on LAST).
+ * Writes, for the envs that did not reach LAST, in their order in order_in: order_out[r] = env, and row r of the
+ * observation (ts->obs_grid [.,N,G,G], ts->action_mask [.,N,5], ts->obs_step_count [.]); *count_out (a device int32)
+ * = the number of those rows.  No other TimeStep field is read or written: ts->reward, discount, step_type and the
+ * extras may be NULL.  Envs not in the list are neither read nor written, nor are action rows >= L.
+ * The order_in entries must be distinct and in [0, B): this is the caller's duty, the library does not check it (a
+ * duplicate is a data race, an entry outside [0, B) an access out of bounds).  order_in and order_out must not overlap;
+ * a caller ping-pongs two buffers.  0 <= L <= B; L == 0 returns at once, before any pointer check, and writes nothing
+ * (not even *count_out).  The library takes 8 bytes per tile of stream-ordered scratch for the call. */
+int rbg_connector_eval_step_live(const rbg_state *state, const int32_t *action, const int32_t *order_in, int64_t L,
+                                 int32_t *order_out, int32_t *count_out, int64_t B, int G, int N,
+                                 const rbg_env_params *params, const rbg_timestep *ts,
+                                 const rbg_episode_metrics *acc, void *stream);
+
 /* Board validity: the reference's NumPy rules (numpy_implementation/utils/
  * post_processor_utils_numpy.py:34-155 = UP, numpy_implementation/utils/board_processor.py:111-162,
  * 391-487 = BP).  flags int32[B], 0 = valid by every rule:
@@ -362,7 +380,7 @@ int64_t rbg_launch_count(int reset);
 #define RBG_K_ROLLOUT 6    /* rollout_persist_kernel (rollout_warp_kernel for the dataset generator): T fused steps */
 #define RBG_K_SEQRW 7      /* seqrw_walk_kernel + its finish kernel */
 #define RBG_K_EPISODES 8   /* episode_warp_kernel: random-agent episodes to their first LAST step */
-#define RBG_K_EVAL_STEP 9  /* eval_step_kernel: one policy-evaluation step of the live envs */
+#define RBG_K_EVAL_STEP 9  /* eval_step_kernel: one policy-evaluation step of the live envs (both entry points) */
 #define RBG_K_COUNT 10
 int rbg_kernel_timing(int enable);
 int rbg_kernel_time(int kernel, int64_t *launches, double *total_ms);

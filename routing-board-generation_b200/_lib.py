@@ -67,6 +67,7 @@ SYMBOLS = {
     "rbg_connector_rollout_random": (_int, [_SP, _vp, _i64, _i64, _int, _int, _EP, _TP, _vp, _vp]),
     "rbg_connector_episodes_random": (_int, [_SP, _i64, _int, _int, _EP, _MP, _SP, _vp]),
     "rbg_connector_eval_step": (_int, [_SP, _vp, _vp, _vp, _i64, _int, _int, _EP, _TP, _MP, _vp]),
+    "rbg_connector_eval_step_live": (_int, [_SP, _vp, _vp, _i64, _vp, _vp, _i64, _int, _int, _EP, _TP, _MP, _vp]),
     "rbg_validate": (_int, [_vp, _i64, _int, _int, _vp, _vp]),
     "rbg_board_statistics": (_int, [_vp, _i64, _int, _int, _vp, _vp, _vp, _vp]),
     "rbg_prw_generate_host": (_int, [_vp, _i64, _int, _int, _vp, _vp, _vp, _int]),

@@ -17,6 +17,7 @@ from typing import Dict
 import torch
 
 from . import engine
+from .types import Observation
 
 
 class EvaluateEmptyBoard:
@@ -123,12 +124,23 @@ class PolicyEvaluator:
     Episode i resets with the unwrapped Connector.reset on key i, so for the same keys it scores the same boards as
     RandomAgentEvaluator.  The action keys are this library's convention, modelled on jumanji's Evaluator but not its
     derivation: chain = split_each(keys)[:, 1], then at every step chain, action_key = split_each(chain).
+
+    live_only=True runs the policy on the live envs only (engine.connector_eval_step_live): each call receives the
+    Observation rows of the envs still in their first episode, in ascending env order, and their action keys, so the
+    batch dimension L shrinks from call to call, and the policy must return int32[L,N].  The step compacts the live
+    envs' observation as it steps them.  For a policy that computes each row from that row alone the metrics are those
+    of the default mode, bit for bit.  Reading L costs one host wait per step; the default mode keeps a static batch
+    shape (what torch.compile or a CUDA graph of the policy needs) and waits on a count read one step late.  The gain
+    is the policy work on finished envs; with a cheap policy, or episodes that nearly all run to time_limit, the wait
+    and the list step cost more than that: on a B200 live_only measured 0.67x to 0.96x the default mode's speed for a
+    cheap policy and a small MLP (DESIGN.md K7, tools/bench_policy_eval.py --live-only).
     """
 
-    def __init__(self, eval_env, policy, total_batch_size: int):
+    def __init__(self, eval_env, policy, total_batch_size: int, live_only: bool = False):
         self.eval_env = eval_env
         self.policy = policy
         self.total_batch_size = int(total_batch_size)
+        self.live_only = bool(live_only)
         self._env, self._reward_agg = _unwrap_eval_env(eval_env)
 
     def episode_metrics(self, keys) -> Dict[str, torch.Tensor]:
@@ -141,12 +153,23 @@ class PolicyEvaluator:
         dev = st.grid.device
         m = {k: torch.zeros((B, N) if k == "episode_return" else (B,), dtype=torch.float32 if k in ("episode_return", "ratio_connections") else torch.int32, device=dev)
              for k in engine.EPISODE_METRICS}
+        chain = engine.split_each(keys)[:, 1]
+        if self.live_only:
+            self._run_live(st, ts.observation, m, chain)
+        else:
+            self._run_masked(st, ts, m, chain)
+        if self._reward_agg is not None:
+            m["episode_return"] = self._reward_agg(m["episode_return"], dim=-1)
+        return m if batched else {k: v[0] for k, v in m.items()}
+
+    def _run_masked(self, st, ts, m, chain) -> None:
+        """The whole batch to every policy call; a live byte per env selects the envs the step advances."""
+        B, dev = st.grid.shape[0], st.grid.device
         live = torch.ones(B, dtype=torch.uint8, device=dev)
         live_count = torch.full((1,), B, dtype=torch.int32, device=dev)
         # the count is read one step late (a step over an all-dead batch changes nothing): at most one host wait per step
         seen = torch.empty(2, dtype=torch.int32, pin_memory=True)
         done = [torch.cuda.Event(), torch.cuda.Event()]
-        chain = engine.split_each(keys)[:, 1]
         t = 0
         while True:
             s = engine.split_each(chain)
@@ -159,9 +182,27 @@ class PolicyEvaluator:
                 if int(seen[(t - 1) % 2]) == 0:
                     break
             t += 1
-        if self._reward_agg is not None:
-            m["episode_return"] = self._reward_agg(m["episode_return"], dim=-1)
-        return m if batched else {k: v[0] for k, v in m.items()}
+
+    def _run_live(self, st, obs, m, chain) -> None:
+        """The live envs only: rows [0, L) of `obs` are the envs order[0][:L]; the step compacts both for the next call."""
+        B, dev = st.grid.shape[0], st.grid.device
+        order = [torch.arange(B, dtype=torch.int32, device=dev), torch.empty(B, dtype=torch.int32, device=dev)]
+        count = torch.empty(1, dtype=torch.int32, device=dev)
+        seen = torch.empty(1, dtype=torch.int32, pin_memory=True)
+        done = torch.cuda.Event()
+        L = B
+        while L > 0:
+            s = engine.split_each(chain)
+            chain, action_key = s[:, 0], s[:, 1]
+            idx = order[0][:L]
+            view = Observation(grid=obs.grid[:L], action_mask=obs.action_mask[:L], step_count=obs.step_count[:L])
+            action = self.policy(view, action_key.contiguous() if L == B else action_key.view(torch.int32)[idx.long()].view(torch.uint32))
+            engine.connector_eval_step_live(st, action, order[0], L, order[1], count, m, obs, **self._env._env_args())
+            seen.copy_(count, non_blocking=True)
+            done.record()
+            done.synchronize()  # the next call's batch size
+            L = int(seen[0])
+            order.reverse()
 
     def run_evaluation(self, key) -> Dict[str, torch.Tensor]:
         """Means over `total_batch_size` episodes whose reset keys are split(key, total_batch_size)."""

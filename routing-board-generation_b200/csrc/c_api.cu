@@ -974,6 +974,30 @@ int rbg_connector_eval_step(const rbg_state *state, const int32_t *action, uint8
   return launch_eval_step(*state, action, live, live_count, B, G, N, *params, *ts, *acc, (cudaStream_t)stream);
 }
 
+int rbg_connector_eval_step_live(const rbg_state *state, const int32_t *action, const int32_t *order_in, int64_t L, int32_t *order_out,
+                                 int32_t *count_out, int64_t B, int G, int N, const rbg_env_params *params, const rbg_timestep *ts,
+                                 const rbg_episode_metrics *acc, void *stream) {
+  int rc;
+  if ((rc = check_dims(B, G, N, 1))) return rc;
+  if (L < 0 || L > B) return set_error(RBG_EINVAL, "list length L=%lld outside [0, B=%lld]", (long long)L, (long long)B);
+  if (L == 0) return RBG_OK;  // an empty list has no buffers to check
+  if ((rc = check_state(state, "state", G))) return rc;
+  if (!action) return set_error(RBG_EINVAL, "action is NULL");
+  if (!order_in) return set_error(RBG_EINVAL, "order_in is NULL");
+  if (!order_out) return set_error(RBG_EINVAL, "order_out is NULL");
+  if (!count_out) return set_error(RBG_EINVAL, "count_out is NULL");
+  if (order_in < order_out + L && order_out < order_in + L) return set_error(RBG_EINVAL, "order_in and order_out overlap");
+  if (!params) return set_error(RBG_EINVAL, "params is NULL");
+  if (params->autoreset_kind >= 0)
+    return set_error(RBG_EINVAL, "an evaluation step ends an episode at its first LAST step: params->autoreset_kind must be < 0 (got %d)",
+                     params->autoreset_kind);
+  if (!ts) return set_error(RBG_EINVAL, "timestep is NULL");
+  if (!ts->obs_grid || !ts->action_mask || !ts->obs_step_count) return set_error(RBG_EINVAL, "timestep has a NULL observation field");
+  if ((G * G) % 4 == 0 && !aligned16(ts->obs_grid)) return set_error(RBG_EALIGN, "timestep.obs_grid not 16-byte aligned");
+  if ((rc = check_metrics(acc, "acc"))) return rc;
+  return launch_eval_step_live(*state, action, order_in, L, order_out, count_out, B, G, N, *params, *ts, *acc, (cudaStream_t)stream);
+}
+
 int rbg_random_actions(const rbg_state *state, int64_t B, int G, int N, int32_t *action, void *stream) {
   int rc;
   if ((rc = check_dims(B, G, N, 1))) return rc;

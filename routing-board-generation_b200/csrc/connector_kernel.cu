@@ -15,6 +15,8 @@
 // kernel reads the State once (int32 -> uint8 into shared memory) and writes State +
 // observation [N,G,G] int32 exactly once; the fused rollout kernel keeps the State on
 // chip for a whole chunk of steps.  All bulk traffic is 128-bit coalesced.
+#include <cuda/atomic>
+
 #include "connector_device.cuh"
 #include "gen_warp.cuh"
 #include "obs_stage.cuh"
@@ -175,14 +177,14 @@ __device__ __forceinline__ uint32_t place_episode(uint8_t *g, const SmemGrid &sg
 }
 
 // observation.grid of kc envs through the table, one store per cell (cells % 4 != 0); env m is skipped where bit
-// m * Np of skipm is set
+// m * Np of skipm is set.  Env m goes to row m of odst, or to row rows[m] when a row table is given.
 __device__ __forceinline__ void write_obs_scalar(int32_t *odst, const uint8_t *wg, const uint8_t *lut, int RS, int kc, int cells, int N, int Np,
-                                                 uint32_t skipm, const FastDiv &divCells, int lane) {
+                                                 uint32_t skipm, const FastDiv &divCells, int lane, const int *rows = nullptr) {
   for (int i = lane; i < kc * cells; i += 32) {
     const int m = (int)divCells.div((uint32_t)i);
     if ((skipm >> (m * Np)) & 1u) continue;
     const uint32_t v = wg[i];
-    int32_t *o = odst + (size_t)m * N * cells + (i - m * cells);
+    int32_t *o = odst + (size_t)(rows ? rows[m] : m) * N * cells + (i - m * cells);
     for (int x = 0; x < N; ++x, o += cells) *o = lut[x * RS + v];
   }
 }
@@ -1284,6 +1286,14 @@ int launch_episodes(const rbg_state &in, const rbg_state *fin, const rbg_episode
 // action are neither read nor written, so the step's traffic scales with the live envs, and a warp with no live env
 // exits after that read.  On LAST the extras go to the record, the live byte is cleared and live_count drops by the
 // warp's number of finished envs (one atomic per warp).
+//
+// LIST (rbg_connector_eval_step_live): the same step of the envs order_in[0, L), all of them live, with action row i
+// belonging to env order_in[i].  The step also compacts the list: an env that did not reach LAST gets output row r =
+// the number of such envs before it in order_in, order_out[r] = env, and its observation (grid, action mask, step
+// count) goes to row r of ts; *count_out = the number of them.  Nothing else of the TimeStep is written.  A CTA is
+// a tile of EW_WARPS * K consecutive list entries; r comes from a warp ballot, a scan of the CTA's warp counts and a
+// single-pass decoupled look-back over the tiles before it (tile_status), with tiles numbered by a ticket counter
+// so that a CTA waits only on CTAs that are already running.  The grids stay in shared memory until r is known.
 struct EvalStepParams {
   rbg_state st;  // stepped in place
   rbg_timestep ts;
@@ -1297,32 +1307,82 @@ struct EvalStepParams {
   float timestep_reward, connected_reward;
   int so[2];  // shared memory: [0] bytes of the observation table, [1] bytes of one warp's grid slice
   FastDiv divG, divC4, divCells;
+  // LIST only
+  const int32_t *order_in;
+  int32_t *order_out, *count_out;
+  unsigned long long *tile_status;  // [tiles]: flag << 32 | count, zeroed; flag 1: the tile's own count, 2: inclusive prefix
+  int *ticket;                      // zeroed
+  long long L, tiles;
+  int so_list;  // smem byte offset of the LIST scratch (LS_*)
 };
 
-template <bool VEC>
+// LIST scratch in shared memory, in ints: per warp 32 slots (env index of slot j, then its output row or -1), the
+// warp counts of survivors, their exclusive prefixes over the list, the tile
+enum : int { LS_SLOTS = 0, LS_WCOUNT = EW_WARPS * 32, LS_WBASE = LS_WCOUNT + EW_WARPS, LS_TILE = LS_WBASE + EW_WARPS, LS_INTS = LS_TILE + 1 };
+
+// decoupled look-back, warp-wide: publish this tile's count, wait for the tiles before it in windows of 32 until one
+// with an inclusive prefix is found, publish the inclusive prefix; returns the exclusive prefix (every lane)
+__device__ __forceinline__ int tile_prefix(unsigned long long *status, long long tile, int agg, int lane) {
+  using ref = cuda::atomic_ref<unsigned long long, cuda::thread_scope_device>;
+  if (tile == 0) {
+    if (lane == 0) ref(status[0]).store((2ull << 32) | (uint32_t)agg, cuda::memory_order_relaxed);
+    return 0;
+  }
+  if (lane == 0) ref(status[tile]).store((1ull << 32) | (uint32_t)agg, cuda::memory_order_relaxed);
+  int excl = 0;
+  for (long long top = tile - 1;; top -= 32) {
+    const long long t = top - lane;
+    unsigned long long w = 2ull << 32;  // before tile 0: an inclusive prefix of 0
+    if (t >= 0) {
+      ref s(status[t]);
+      do w = s.load(cuda::memory_order_relaxed);
+      while ((w >> 32) == 0);
+    }
+    const uint32_t incl = __ballot_sync(FULL, (w >> 32) == 2);
+    const int stop = incl ? __ffs((int)incl) - 1 : 31;  // the nearest tile with an inclusive prefix
+    int v = lane <= stop ? (int)(uint32_t)w : 0;
+    for (int off = 16; off; off >>= 1) v += __shfl_xor_sync(FULL, v, off);
+    excl += v;
+    if (incl) break;
+  }
+  if (lane == 0) ref(status[tile]).store((2ull << 32) | (uint32_t)(excl + agg), cuda::memory_order_relaxed);
+  return excl;
+}
+
+template <bool VEC, bool LIST>
 __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) eval_step_kernel(const EvalStepParams p) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int G = p.G, N = p.N, cells = p.cells;
   const int Np = p.Np, K = 32 / Np, c4 = cells >> 2;
   const int RS = obs_lut_stride(N);
+  int *ls = reinterpret_cast<int *>(smem_raw + p.so_list);  // LIST scratch
+  int *slots = ls + LS_SLOTS + warp * 32;
 
-  const long long e0 = ((long long)blockIdx.x * EW_WARPS + warp) * K;
-  const int kc = e0 >= p.B ? 0 : (int)((p.B - e0) < (long long)K ? (p.B - e0) : (long long)K);
+  long long tile = blockIdx.x;
+  if (LIST) {
+    if (tid == 0) ls[LS_TILE] = atomicAdd(p.ticket, 1);
+    __syncthreads();
+    tile = ls[LS_TILE];
+  }
+  // e0: the warp's first env (LIST: its first list entry)
+  const long long e0 = (tile * EW_WARPS + warp) * K, n = LIST ? p.L : p.B;
+  const int kc = e0 >= n ? 0 : (int)((n - e0) < (long long)K ? (n - e0) : (long long)K);
   const int j = lane / Np, a = lane & (Np - 1);
-  const long long e = e0 + (j < kc ? j : 0);
-  const bool env_ok = j < kc && p.live[e] != 0, agent = env_ok && a < N;
+  const long long e = LIST ? (j < kc ? (long long)__ldg(p.order_in + e0 + j) : 0) : e0 + (j < kc ? j : 0);
+  const bool env_ok = j < kc && (LIST || p.live[e] != 0), agent = env_ok && a < N;
   const uint32_t livem = __ballot_sync(FULL, env_ok);  // bit j * Np (and the env's other lanes): env j is live
-  if (!__syncthreads_or(livem != 0u)) return;  // a CTA without a live env builds no table
+  if (!LIST && !__syncthreads_or(livem != 0u)) return;  // a CTA without a live env builds no table
   uint8_t *lut = smem_raw;
   build_obs_lut(lut, N, RS, warp, EW_WARPS, lane);
-  __syncthreads();  // the last CTA-wide barrier
-  if (livem == 0u) return;
+  if (LIST && env_ok && a == 0) slots[j] = (int)e;
+  __syncthreads();  // LIST: the last CTA-wide barrier but the two of the row scan
+  if (!LIST && livem == 0u) return;
   uint8_t *wg = smem_raw + p.so[0] + (size_t)warp * p.so[1];
   uint32_t *wg32 = reinterpret_cast<uint32_t *>(wg);
   const uint32_t gmask = Np == 32 ? FULL : (((1u << Np) - 1u) << (j * Np));
 
-  // ---- load the live envs: State.grid int32 -> uint8, agent and env scalars
+  // ---- load the live envs: State.grid int32 -> uint8, agent and env scalars (LIST: env m of the warp is slots[m])
   if (VEC) {
     const int4 *src = reinterpret_cast<const int4 *>(p.st.grid) + e0 * c4;
     const int nq = kc * c4;
@@ -1333,7 +1393,14 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) eval_step_kernel(c
       for (int u = 0; u < 4; ++u) {
         const int q = q0 + 32 * u;
         ok[u] = q < nq && ((livem >> ((int)p.divC4.div((uint32_t)q) * Np)) & 1u);
-        v[u] = ok[u] ? __ldg(src + q) : make_int4(0, 0, 0, 0);
+        if (!ok[u]) {
+          v[u] = make_int4(0, 0, 0, 0);
+        } else if (LIST) {
+          const int m = (int)p.divC4.div((uint32_t)q);
+          v[u] = __ldg(reinterpret_cast<const int4 *>(p.st.grid) + (size_t)slots[m] * c4 + (q - m * c4));
+        } else {
+          v[u] = __ldg(src + q);
+        }
       }
 #pragma unroll
       for (int u = 0; u < 4; ++u)
@@ -1342,8 +1409,10 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) eval_step_kernel(c
     }
   } else {
     const int32_t *src = p.st.grid + e0 * cells;
-    for (int i = lane; i < kc * cells; i += 32)
-      if ((livem >> ((int)p.divCells.div((uint32_t)i) * Np)) & 1u) wg[i] = (uint8_t)__ldg(src + i);
+    for (int i = lane; i < kc * cells; i += 32) {
+      const int m = (int)p.divCells.div((uint32_t)i);
+      if ((livem >> (m * Np)) & 1u) wg[i] = (uint8_t)__ldg(LIST ? p.st.grid + (size_t)slots[m] * cells + (i - m * cells) : src + i);
+    }
   }
   int pos = 0, tgt = 0, action = 0, sc0 = 0;
   if (agent) {
@@ -1351,7 +1420,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) eval_step_kernel(c
     const int2 tg = __ldg(reinterpret_cast<const int2 *>(p.st.target) + e * N + a);
     pos = (ps.x << 8) | ps.y;
     tgt = (tg.x << 8) | tg.y;
-    action = __ldg(p.action + e * N + a);
+    action = __ldg(p.action + (LIST ? e0 + j : e) * N + a);
   }
   if (env_ok) sc0 = p.st.step_count[e];
   __syncwarp();
@@ -1399,60 +1468,96 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kEnvMinCtas) eval_step_kernel(c
   if (env_ok && a == 0) {
     const float ratio = __fdiv_rn((float)s.nconn, (float)N);
     const int tpl = paths + s.nmoved + N;
-    p.ts.step_type[e] = (int8_t)(terminal ? 2 : 1);
-    p.ts.num_connections[e] = s.nconn;
-    p.ts.ratio_connections[e] = ratio;
-    p.ts.total_path_length[e] = tpl;
-    p.ts.obs_step_count[e] = sc;
+    if (!LIST) {
+      p.ts.step_type[e] = (int8_t)(terminal ? 2 : 1);
+      p.ts.num_connections[e] = s.nconn;
+      p.ts.ratio_connections[e] = ratio;
+      p.ts.total_path_length[e] = tpl;
+      p.ts.obs_step_count[e] = sc;
+    }
     p.st.step_count[e] = sc;
     p.acc.episode_length[e] += 1;
     if (terminal) {
       p.acc.num_connections[e] = s.nconn;
       p.acc.ratio_connections[e] = ratio;
       p.acc.total_path_length[e] = tpl;
-      p.live[e] = 0;
+      if (!LIST) p.live[e] = 0;
     }
   }
   if (agent) {
     const long long ga = e * N + a;
-    p.ts.reward[ga] = s.rew;
-    p.ts.discount[ga] = (terminal || s.done) ? 0.0f : 1.0f;
-    store_mask5(p.ts.action_mask + ga * 5, s.mk3);
+    if (!LIST) {
+      p.ts.reward[ga] = s.rew;
+      p.ts.discount[ga] = (terminal || s.done) ? 0.0f : 1.0f;
+      store_mask5(p.ts.action_mask + ga * 5, s.mk3);
+    }
     reinterpret_cast<int2 *>(p.st.position)[ga] = make_int2(pos >> 8, pos & 255);
     p.acc.episode_return[ga] = __fadd_rn(p.acc.episode_return[ga], s.rew);
   }
-  const int nfinished = __popc(__ballot_sync(FULL, a == 0 && terminal));
-  if (lane == 0 && nfinished) atomicSub(p.live_count, nfinished);
+  uint32_t obsm = livem;  // bit m * Np: env m of the warp writes an observation row
+  if (!LIST) {
+    const int nfinished = __popc(__ballot_sync(FULL, a == 0 && terminal));
+    if (lane == 0 && nfinished) atomicSub(p.live_count, nfinished);
+  } else {
+    // ---- the output rows of the survivors: rank in the warp (ballot), in the CTA (scan of the warp counts), in the
+    // list (look-back over the tiles before this one)
+    obsm = __ballot_sync(FULL, a == 0 && env_ok && !terminal);
+    if (lane == 0) ls[LS_WCOUNT + warp] = __popc(obsm);
+    __syncthreads();
+    if (warp == 0) {
+      const int own = lane < EW_WARPS ? ls[LS_WCOUNT + lane] : 0;
+      int incl = own;
+      for (int off = 1; off < EW_WARPS; off <<= 1) {
+        const int t = __shfl_up_sync(FULL, incl, off);
+        if (lane >= off) incl += t;
+      }
+      const int agg = __shfl_sync(FULL, incl, EW_WARPS - 1);
+      const int before = tile_prefix(p.tile_status, tile, agg, lane);
+      if (lane < EW_WARPS) ls[LS_WBASE + lane] = before + incl - own;
+      if (lane == 0 && tile == p.tiles - 1) *p.count_out = before + agg;
+    }
+    __syncthreads();
+    const bool keep = (obsm >> (j * Np)) & 1u;
+    const int row = ls[LS_WBASE + warp] + __popc(obsm & ((1u << (j * Np)) - 1u));
+    if (keep) {
+      if (a == 0) {
+        p.order_out[row] = (int32_t)e;
+        p.ts.obs_step_count[row] = sc;
+      }
+      if (a < N) store_mask5(p.ts.action_mask + ((long long)row * N + a) * 5, s.mk3);
+    }
+    if (j < kc && a == 0) slots[j] = keep ? row : -1;
+    __syncwarp();
+  }
 
-  // ---- observation.grid of the live envs
+  // ---- observation.grid of the live envs (LIST: of the survivors, env m of the warp to row slots[m])
   if (VEC) {
     int4 *odst = reinterpret_cast<int4 *>(p.ts.obs_grid) + e0 * N * c4;
     for (int q = lane; q < kc * c4; q += 32) {
       const int m = (int)p.divC4.div((uint32_t)q);
-      if (!((livem >> (m * Np)) & 1u)) continue;
+      if (!((obsm >> (m * Np)) & 1u)) continue;
       const uint32_t w = wg32[q];
       const uint32_t b0 = w & 0xffu, b1 = (w >> 8) & 0xffu, b2 = (w >> 16) & 0xffu, b3 = w >> 24;
-      int4 *o = odst + (size_t)m * N * c4 + (q - m * c4);
+      int4 *o = (LIST ? reinterpret_cast<int4 *>(p.ts.obs_grid) + (size_t)slots[m] * N * c4 : odst + (size_t)m * N * c4) + (q - m * c4);
       const uint8_t *row = lut;
 #pragma unroll 2
       for (int x = 0; x < N; ++x, o += c4, row += RS) *o = make_int4(row[b0], row[b1], row[b2], row[b3]);
     }
+  } else if (LIST) {
+    write_obs_scalar(p.ts.obs_grid, wg, lut, RS, kc, cells, N, Np, ~obsm, p.divCells, lane, slots);
   } else {
     write_obs_scalar(p.ts.obs_grid + e0 * N * cells, wg, lut, RS, kc, cells, N, Np, ~livem, p.divCells, lane);
   }
 }
 
-int launch_eval_step(const rbg_state &st, const int32_t *action, uint8_t *live, int32_t *live_count, int64_t B, int G, int N,
-                     const rbg_env_params &env, const rbg_timestep &ts, const rbg_episode_metrics &acc, cudaStream_t stream) {
-  if (B <= 0) return RBG_OK;
+static EvalStepParams eval_step_params(const rbg_state &st, const int32_t *action, int64_t B, int G, int N, const rbg_env_params &env,
+                                       const rbg_timestep &ts, const rbg_episode_metrics &acc, size_t &smem, int64_t &envs_per_cta, bool &vec) {
   EvalStepParams p;
   memset(&p, 0, sizeof(p));
   p.st = st;
   p.ts = ts;
   p.acc = acc;
   p.action = action;
-  p.live = live;
-  p.live_count = live_count;
   p.B = B;
   p.G = G;
   p.N = N;
@@ -1462,11 +1567,59 @@ int launch_eval_step(const rbg_state &st, const int32_t *action, uint8_t *live, 
   const WarpShape s = warp_shape(G, N);
   const size_t lutB = lut_bytes(N, obs_lut_stride(N));
   set_warp_shape(p, s, lutB);
-  const size_t smem = lutB + EW_WARPS * s.wgrid;
-  const int64_t E = EW_WARPS * s.K;  // envs per CTA
+  smem = lutB + EW_WARPS * s.wgrid;
+  envs_per_cta = EW_WARPS * s.K;
+  vec = s.vec();
+  return p;
+}
+
+int launch_eval_step(const rbg_state &st, const int32_t *action, uint8_t *live, int32_t *live_count, int64_t B, int G, int N,
+                     const rbg_env_params &env, const rbg_timestep &ts, const rbg_episode_metrics &acc, cudaStream_t stream) {
+  if (B <= 0) return RBG_OK;
+  size_t smem;
+  int64_t E;
+  bool vec;
+  EvalStepParams p = eval_step_params(st, action, B, G, N, env, ts, acc, smem, E, vec);
+  p.live = live;
+  p.live_count = live_count;
   const int64_t ctas = (B + E - 1) / E;
-  void (*fn)(const EvalStepParams) = s.vec() ? eval_step_kernel<true> : eval_step_kernel<false>;
+  void (*fn)(const EvalStepParams) = vec ? eval_step_kernel<true, false> : eval_step_kernel<false, false>;
   return launch_kernel(fn, (unsigned)ctas, EW_WARPS * 32, smem, stream, RBG_K_EVAL_STEP, "eval_step_kernel", false, p);
+}
+
+int launch_eval_step_live(const rbg_state &st, const int32_t *action, const int32_t *order_in, int64_t L, int32_t *order_out, int32_t *count_out,
+                          int64_t B, int G, int N, const rbg_env_params &env, const rbg_timestep &ts, const rbg_episode_metrics &acc,
+                          cudaStream_t stream) {
+  if (L <= 0) return RBG_OK;
+  size_t smem;
+  int64_t E;
+  bool vec;
+  EvalStepParams p = eval_step_params(st, action, B, G, N, env, ts, acc, smem, E, vec);
+  p.so_list = (int)smem;
+  smem += up16(sizeof(int) * LS_INTS);
+  p.order_in = order_in;
+  p.order_out = order_out;
+  p.count_out = count_out;
+  p.L = L;
+  p.tiles = (L + E - 1) / E;
+  // the tile status words and the ticket: stream-ordered scratch, cleared before the launch, so that the caller needs
+  // no workspace and launches on different streams never share it
+  const size_t bytes = 8 * (size_t)p.tiles + 16;
+  keep_pool_cached();
+  void *scratch = nullptr;
+  cudaError_t ce;
+  if ((ce = cudaMallocAsync(&scratch, bytes, stream)) != cudaSuccess) return set_cuda_error(ce, "cudaMallocAsync(eval step tile status)");
+  p.tile_status = static_cast<unsigned long long *>(scratch);
+  p.ticket = reinterpret_cast<int *>(static_cast<char *>(scratch) + 8 * (size_t)p.tiles);
+  int rc = RBG_OK;
+  if ((ce = cudaMemsetAsync(scratch, 0, bytes, stream)) != cudaSuccess) {
+    rc = set_cuda_error(ce, "cudaMemsetAsync(eval step tile status)");
+  } else {
+    void (*fn)(const EvalStepParams) = vec ? eval_step_kernel<true, true> : eval_step_kernel<false, true>;
+    rc = launch_kernel(fn, (unsigned)p.tiles, EW_WARPS * 32, smem, stream, RBG_K_EVAL_STEP, "eval_step_kernel<LIST>", false, p);
+  }
+  cudaFreeAsync(scratch, stream);
+  return rc;
 }
 
 }  // namespace rbg

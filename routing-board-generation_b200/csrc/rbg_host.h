@@ -148,6 +148,11 @@ int launch_episodes(const rbg_state &in, const rbg_state *fin, const rbg_episode
 // one Connector.step of the envs whose live byte is set, their episode records accumulated in place (eval_step_kernel)
 int launch_eval_step(const rbg_state &st, const int32_t *action, uint8_t *live, int32_t *live_count, int64_t B, int G, int N,
                      const rbg_env_params &env, const rbg_timestep &ts, const rbg_episode_metrics &acc, cudaStream_t stream);
+// the same step of the envs order_in[0, L), the survivors compacted to order_out / ts rows [0, *count_out)
+// (eval_step_kernel<LIST>)
+int launch_eval_step_live(const rbg_state &st, const int32_t *action, const int32_t *order_in, int64_t L, int32_t *order_out, int32_t *count_out,
+                          int64_t B, int G, int N, const rbg_env_params &env, const rbg_timestep &ts, const rbg_episode_metrics &acc,
+                          cudaStream_t stream);
 
 // ---- misc kernels (misc_kernels.cu) --------------------------------------
 int launch_split_keys(uint32_t k0, uint32_t k1, int64_t B, int64_t offset,

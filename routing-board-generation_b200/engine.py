@@ -437,6 +437,34 @@ def connector_eval_step(st: State, action: torch.Tensor, live: torch.Tensor, liv
     _lib.check(_lib.load().rbg_connector_eval_step(C.byref(s), act.data_ptr(), live.data_ptr(), live_count.data_ptr(), B, G, N, C.byref(params), C.byref(t), C.byref(m), _stream()))
 
 
+def connector_eval_step_live(st: State, action: torch.Tensor, order_in: torch.Tensor, L: int, order_out: torch.Tensor, count: torch.Tensor,
+                             acc: Dict[str, torch.Tensor], obs: Observation, time_limit: int = 50, timestep_reward: float = -0.03,
+                             connected_reward: float = 0.1) -> None:
+    """`connector_eval_step` of the envs order_in[:L] (int32, distinct, in [0, B)), with `action` int32[L,N] in list
+    order, compacting the list as it steps.  The envs that did not reach LAST keep their order: the r-th of them goes
+    to order_out[r] and its observation to row r of `obs` (an Observation of at least L rows: grid, action_mask,
+    step_count), and `count` (int32[1] on the device) receives their number.  Nothing else of a TimeStep is written.
+    order_in and order_out must be different buffers; the distinctness and range of the entries are not checked."""
+    B, G, N = _dims(st)
+    if not all(t.is_contiguous() for t in (st.grid, st.step_count, st.key, st.agents.id, st.agents.start, st.agents.target, st.agents.position)):
+        raise ValueError("the evaluation step updates the State in place: its leaves must be contiguous")
+    L = int(L)
+    for name, o in (("order_in", order_in), ("order_out", order_out)):
+        if o.dtype != torch.int32 or o.dim() != 1 or not o.is_contiguous() or o.numel() < L:
+            raise ValueError(f"{name} must be a contiguous int32 vector of at least L={L} entries")
+    if count.dtype != torch.int32 or count.numel() != 1:
+        raise ValueError("count must be int32[1]")
+    if not all(t.is_contiguous() and t.shape[0] >= L for t in (obs.grid, obs.action_mask, obs.step_count)):
+        raise ValueError(f"the observation buffers must be contiguous with at least L={L} rows")
+    act = as_tensor(action, torch.int32).reshape(L, N)
+    m = rbg_episode_metrics(*(acc[k].data_ptr() for k in EPISODE_METRICS))
+    params, _ = _env_params(time_limit, timestep_reward, connected_reward, -1)
+    s = _state_struct(st)
+    t = rbg_timestep(obs.grid.data_ptr(), obs.action_mask.data_ptr(), obs.step_count.data_ptr(), None, None, None, None, None, None)
+    _lib.check(_lib.load().rbg_connector_eval_step_live(C.byref(s), act.data_ptr(), order_in.data_ptr(), L, order_out.data_ptr(), count.data_ptr(), B, G, N,
+                                                        C.byref(params), C.byref(t), C.byref(m), _stream()))
+
+
 def random_actions(st: State) -> torch.Tensor:
     st = _contig_state(st)
     B, G, N = _dims(st)

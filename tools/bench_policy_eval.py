@@ -1,15 +1,24 @@
-"""Policy evaluation throughput: PolicyEvaluator (one eval-step launch per policy call) against a Connector.step loop.
+"""Policy evaluation throughput: PolicyEvaluator (one eval-step launch per policy call) against a Connector.step loop,
+and with --live-only its two modes against each other.
 
 The policy is "keyed", a pure torch function of the action mask and the action key (agent a takes the
-((key0 ^ a * 0x9E3779B9) mod n)-th of its n legal actions), so that every arm computes the same episodes.  For each
-workload (ParallelRandomWalk boards, time_limit 50) it first checks that the arms give the same per-episode metrics,
-then times them with CUDA events, alternating the arms in the same run, each window >= --min-ms:
+((key0 ^ a * 0x9E3779B9) mod n)-th of its n legal actions), so that every arm computes the same episodes, or "mlp", a
+seeded two-layer float32 MLP (G*G -> 128 -> 5) over each agent's observation.grid with an argmax over the legal
+actions: a policy whose cost grows with the rows it is given.  For each workload (ParallelRandomWalk boards,
+time_limit 50) it first checks that the arms give the same per-episode metrics (for "mlp" it reports whether they do:
+a matrix product may round a row differently at another batch size), then times them with CUDA events, alternating
+the arms in the same run, each window >= --min-ms:
   (a) PolicyEvaluator.episode_metrics: Connector.reset, then policy -> eval step until no env is live, one host wait
       per step on a count read one step late;
   (b) Connector.reset, then `time_limit` plain Connector.step calls driven by the same policy and action keys, with
       the metrics accumulated in torch from each env's first LAST step (as tools/bench_episodes.py step_loop);
   (c) eval_step_kernel alone: its device time summed over the steps of (a), from the library's kernel timing
       (rbg_kernel_time(RBG_K_EVAL_STEP)), which brackets each launch with an event pair.
+With --live-only, (b) is replaced by
+  (d) PolicyEvaluator(live_only=True).episode_metrics: the policy sees only the live envs, one host wait per step to
+      read their number;
+  (e) the live step kernel alone (eval_step_kernel<LIST>), timed as (c) over the steps of (d).
+Policy rows per evaluation (the rows the policy was handed, summed over its calls) are counted for (a) and (d).
 Rates: episodes/s = B / time, env-steps/s = sum(episode_length) / time (the same numerator for every arm).
 Kernel bandwidth: the bytes one live env-step moves (computed from the shape below) times sum(episode_length), over the
 kernel time of (c); a dead env costs its live byte.  DESIGN K2's count for a full Connector.step (3 206 B at 10x10/5,
@@ -17,7 +26,7 @@ kernel time of (c); a dead env costs its live byte.  DESIGN K2's count for a ful
 Prints one JSON line per workload (and writes them to --out when given) with the card name, power limit and max SM
 clock read in the same run.
 
-    python tools/bench_policy_eval.py [--shapes 10x10/5x65536,32x32/16x8192] [--rounds 7] [--out FILE]
+    python tools/bench_policy_eval.py [--shapes 10x10/5x65536,32x32/16x8192] [--policy keyed|mlp] [--live-only] [--rounds 7] [--out FILE]
 """
 from __future__ import annotations
 
@@ -67,6 +76,38 @@ def keyed_policy(obs, key):
     for i in range(1, c.shape[-1]):
         c[..., i] += c[..., i - 1]
     return (mask & (c == (k + 1)[..., None])).to(torch.int8).argmax(-1).to(torch.int32)
+
+
+class MlpPolicy:
+    """A seeded two-layer MLP over each agent's observation.grid (float32), argmax of its logits over the legal actions."""
+
+    def __init__(self, G: int, hidden: int = 128, seed: int = 0):
+        import torch
+
+        g = torch.Generator().manual_seed(seed)
+        self.w1 = (torch.randn(G * G, hidden, generator=g) / G).cuda()
+        self.b1 = (torch.randn(hidden, generator=g) * 0.1).cuda()
+        self.w2 = (torch.randn(hidden, 5, generator=g) / hidden ** 0.5).cuda()
+
+    def __call__(self, obs, key):
+        import torch
+
+        L, N = obs.grid.shape[:2]
+        h = torch.relu(obs.grid.reshape(L * N, -1).to(torch.float32) @ self.w1 + self.b1)
+        logits = (h @ self.w2).reshape(L, N, 5).masked_fill(~obs.action_mask, float("-inf"))
+        return logits.argmax(-1).to(torch.int32)
+
+
+class RowCounter:
+    """Counts the rows a policy is handed (a host-side shape: no device sync)."""
+
+    def __init__(self, policy):
+        self.policy, self.rows, self.calls = policy, 0, 0
+
+    def __call__(self, obs, key):
+        self.rows += obs.grid.shape[0]
+        self.calls += 1
+        return self.policy(obs, key)
 
 
 def step_loop(rbg, env, policy, keys, time_limit):
@@ -135,24 +176,46 @@ def kernel_window(rbg, ev, keys, reps: int):
     return ms / reps, n / reps
 
 
-def run_shape(rbg, G: int, N: int, B: int, time_limit: int, rounds: int, min_ms: float, seed: int) -> dict:
+def _same(a: dict, b: dict) -> bool:
     import torch
 
+    return all(torch.equal(x.view(torch.int32) if x.dtype == torch.float32 else x, y.view(torch.int32) if y.dtype == torch.float32 else y)
+               for x, y in ((a[k], b[k]) for k in METRICS))
+
+
+def run_shape(rbg, G: int, N: int, B: int, time_limit: int, rounds: int, min_ms: float, seed: int, policy_name: str, live_only: bool) -> dict:
+    import torch
+
+    policy = keyed_policy if policy_name == "keyed" else MlpPolicy(G, seed=seed)
     env = rbg.Connector(generator=rbg.ParallelRandomWalkGenerator(G, N), time_limit=time_limit)
-    ev = rbg.PolicyEvaluator(env, keyed_policy, B)
+    ev = rbg.PolicyEvaluator(env, policy, B)
+    ev_live = rbg.PolicyEvaluator(env, policy, B, live_only=True)
     keys = rbg.split(rbg.PRNGKey(seed), B)
 
-    # ---- the arms must agree before they are timed
-    a = ev.episode_metrics(keys)
-    b, done = step_loop(rbg, env, keyed_policy, keys, time_limit)
-    assert bool(done.all()), "an env had no LAST step within time_limit steps of its reset"
-    for k in METRICS:
-        x, y = a[k], b[k]
-        if x.dtype == torch.float32:
-            x, y = x.view(torch.int32), y.view(torch.int32)
-        assert torch.equal(x, y), f"{k}: PolicyEvaluator and the Connector.step loop disagree"
+    # ---- the arms must agree before they are timed (a keyed policy: bit for bit)
+    count = RowCounter(policy)
+    a = rbg.PolicyEvaluator(env, count, B).episode_metrics(keys)
+    rows = {"evaluator": count.rows}
     env_steps = int(a["episode_length"].to(torch.int64).sum())
     max_length = int(a["episode_length"].max())
+    res = {"workload": f"PRW {G}x{G}/{N}", "policy": policy_name, "B": B, "time_limit": time_limit, "env_steps": env_steps, "mean_episode_length": env_steps / B,
+           "max_episode_length": max_length}
+    if live_only:
+        count = RowCounter(policy)
+        b = rbg.PolicyEvaluator(env, count, B, live_only=True).episode_metrics(keys)
+        rows["evaluator_live"] = count.rows
+        res["env_steps_live"] = int(b["episode_length"].to(torch.int64).sum())
+        res["modes_agree_bit_for_bit"] = _same(a, b)
+        if policy_name == "keyed":
+            assert res["modes_agree_bit_for_bit"], "PolicyEvaluator's two modes disagree"
+            assert rows["evaluator_live"] == env_steps, "the live mode handed the policy a row that is not a live env-step"
+    else:
+        b, done = step_loop(rbg, env, policy, keys, time_limit)
+        assert bool(done.all()), "an env had no LAST step within time_limit steps of its reset"
+        res["modes_agree_bit_for_bit"] = _same(a, b)
+        if policy_name == "keyed":
+            assert res["modes_agree_bit_for_bit"], "PolicyEvaluator and the Connector.step loop disagree"
+    res["policy_rows_per_evaluation"] = rows
 
     # ---- library launches: the evaluator's, less those of its reset, per step
     torch.cuda.synchronize()
@@ -162,21 +225,26 @@ def run_shape(rbg, G: int, N: int, B: int, time_limit: int, rounds: int, min_ms:
     ev.episode_metrics(keys)
     eval_launches = rbg.launch_count(reset=True)
     _, steps = kernel_window(rbg, ev, keys, 1)
+    steps_live = kernel_window(rbg, ev_live, keys, 1)[1] if live_only else None
 
-    arms = {
-        "evaluator": lambda: ev.episode_metrics(keys),
-        "step_loop": lambda: step_loop(rbg, env, keyed_policy, keys, time_limit),
-    }
+    arms = {"evaluator": lambda: ev.episode_metrics(keys)}
+    if live_only:
+        arms["evaluator_live"] = lambda: ev_live.episode_metrics(keys)
+    else:
+        arms["step_loop"] = lambda: step_loop(rbg, env, policy, keys, time_limit)
+    kernels = {"kernel": ev, "kernel_live": ev_live} if live_only else {"kernel": ev}
     reps = {k: calibrate(f, min_ms) for k, f in arms.items()}
-    ms = {k: [] for k in list(arms) + ["kernel"]}
+    ms = {k: [] for k in list(arms) + list(kernels)}
     for _ in range(rounds):  # alternate the arms so that drift and neighbours hit them alike
         for k, f in arms.items():
             ms[k].append(window_ms(f, reps[k]))
-        ms["kernel"].append(kernel_window(rbg, ev, keys, reps["evaluator"])[0])
+        for k, e in kernels.items():
+            ms[k].append(kernel_window(rbg, e, keys, reps["evaluator"])[0])
     nbytes = eval_step_bytes(G, N)
-    res = {"workload": f"PRW {G}x{G}/{N}", "policy": "keyed", "B": B, "time_limit": time_limit, "env_steps": env_steps, "mean_episode_length": env_steps / B,
-           "max_episode_length": max_length, "eval_steps_per_evaluation": steps, "library_launches_per_step": (eval_launches - reset_launches) / steps,
-           "reset_launches": reset_launches, "rounds": rounds, "min_window_ms": min_ms}
+    res.update({"eval_steps_per_evaluation": steps, "library_launches_per_step": (eval_launches - reset_launches) / steps,
+                "reset_launches": reset_launches, "rounds": rounds, "min_window_ms": min_ms})
+    if live_only:
+        res["live_steps_per_evaluation"] = steps_live
     for k in ms:
         med = statistics.median(ms[k])
         res[k] = {"ms_median": med, "ms_min": min(ms[k]), "ms_max": max(ms[k]), "episodes_per_s": B / (med * 1e-3), "env_steps_per_s": env_steps / (med * 1e-3)}
@@ -188,7 +256,11 @@ def run_shape(rbg, G: int, N: int, B: int, time_limit: int, rounds: int, min_ms:
     if (G, N) in K2_BYTES:
         kb = K2_BYTES[(G, N)]
         res["kernel"].update({"k2_bytes_per_env_step": kb, "hbm_fraction_at_k2_bytes": kb * env_steps / (kms * 1e-3) / HBM_BYTES_PER_S})
-    res["speedup_evaluator_vs_step_loop"] = res["step_loop"]["ms_median"] / res["evaluator"]["ms_median"]
+    if live_only:
+        res["kernel_live"]["us_per_step"] = res["kernel_live"]["ms_median"] * 1e3 / steps_live
+        res["speedup_live_vs_default"] = res["evaluator"]["ms_median"] / res["evaluator_live"]["ms_median"]
+    else:
+        res["speedup_evaluator_vs_step_loop"] = res["step_loop"]["ms_median"] / res["evaluator"]["ms_median"]
     return res
 
 
@@ -199,6 +271,8 @@ def main() -> None:
     ap.add_argument("--rounds", type=int, default=7)
     ap.add_argument("--min-ms", type=float, default=60.0)
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--policy", choices=("keyed", "mlp"), default="keyed")
+    ap.add_argument("--live-only", action="store_true", help="time PolicyEvaluator(live_only=True) against the default mode instead of the step loop")
     ap.add_argument("--out", default=None, help="also write the JSON lines here")
     args = ap.parse_args()
 
@@ -217,7 +291,7 @@ def main() -> None:
         gg, rest = spec.split("/")
         G = int(gg.split("x")[0])
         N, B = (int(x) for x in rest.split("x"))
-        res = run_shape(rbg, G, N, B, args.time_limit, args.rounds, args.min_ms, args.seed)
+        res = run_shape(rbg, G, N, B, args.time_limit, args.rounds, args.min_ms, args.seed, args.policy, args.live_only)
         res.update(info)
         lines.append(json.dumps(res))
         print(lines[-1], flush=True)
