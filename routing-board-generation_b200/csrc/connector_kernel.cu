@@ -116,6 +116,10 @@ __device__ __forceinline__ int random_dest(uint32_t k0, uint32_t k1, int sc, int
   return action != NOOP ? r * G + c + (action == UP ? -G : (action == DOWN ? G : (action == RIGHT ? 1 : -1))) : -1;
 }
 
+// two cells of a G x G grid in one register (ObsStager::emit_delta); pin_cell: the cell of a packed (row << 8 | col)
+__device__ __forceinline__ uint32_t cell_pair(int c0, int c1) { return (uint32_t)c0 | ((uint32_t)c1 << 16); }
+__device__ __forceinline__ int pin_cell(int rc, int G) { return (rc >> 8) * G + (rc & 255); }
+
 // the collision rule and move_agent: of the agents of one env with the same destination only the highest agent id
 // moves; a mover's old head becomes PATH and its new cell POSITION on the env grid g.  Returns the lane's position
 // after the move; win: it moved.
@@ -486,6 +490,8 @@ struct RolloutParams {
   int stage_nbuf;        // 1: one chunk per step (a whole step passes before it is refilled); 2: alternate
   int stage_warp;        // bytes per warp (>= stage_nbuf * stage_bytes)
   int ce, cv;            // a staged chunk = ce whole envs (cv == N) or cv views of one env (ce == 1)
+  int delta;             // 1: the one buffer holds the warp's whole observation range (nbuf == 1, ce == K), so after the
+                         // first step of a group only the cells that changed are restaged (ObsStager::emit_delta)
 };
 
 constexpr int kRolloutMinCtas = 6;
@@ -559,6 +565,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kRolloutMinCtas) rollout_warp_k
     const int dest = agent ? random_dest(k0, k1, sc, a, mk3, r, c, G, rp.action_out, row_a) : -1;
     bool win;
     pos = resolve_moves(dest, j, lane, a, r, c, G, g, p.divG, pos, win);
+    uint32_t dirty = win ? cell_pair(r * G + c, dest) : OBS_CLEAN;  // the cells of g this step changed
     // ---- action mask, connected / done, reward on the new grid
     const StepResult s = after_move(sg, agent, a, pos, tgt, was, win, gmask, p.env);
     mk3 = s.mk3;
@@ -603,6 +610,7 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kRolloutMinCtas) rollout_warp_k
       sc = 0;
       paths = 0;
       mk3 = place_episode(g, sg, a, N, Np, cells, G, gmask, pos, tgt, mk3, [] {});
+      dirty = a < N ? cell_pair(pin_cell(pos, G), pin_cell(tgt, G)) : OBS_CLEAN;
     }
     __syncwarp();
     if (agent) store_mask5(p.ts.action_mask + row_a * 5, mk3);
@@ -610,7 +618,9 @@ __global__ void __launch_bounds__(EW_WARPS * 32, kRolloutMinCtas) rollout_warp_k
     if (VEC) {
       int4 *odst = obs_t;
       obs_t += obs_step;
-      if (OBS == 2)
+      if (OBS == 2 && rp.delta && t > 0)
+        os.emit_delta(kc, N, lane, j, __ffs(Np) - 1, (uint32_t)__cvta_generic_to_shared(g), dirty, terminal && a == 0, odst);
+      else if (OBS == 2)
         os.emit(kc, N, c4, lane, odst);
       else
         os.emit_direct(lut, wg32, kc, N, c4, lane, odst);
@@ -782,6 +792,7 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, kPersistMinCtas)
       const int dest = agent ? random_dest(k0, k1, sc, a, mk3, r, c, G, rp.action_out, row_a) : -1;
       bool win;
       pos = resolve_moves(dest, j, lane, a, r, c, G, g, p.divG, pos, win);
+      uint32_t dirty = win ? cell_pair(r * G + c, dest) : OBS_CLEAN;  // the cells of g this step changed
       // ---- action mask, connected / done, reward on the new grid
       const StepResult s = after_move(sg, agent, a, pos, tgt, was, win, gmask, p.env);
       mk3 = s.mk3;
@@ -826,6 +837,7 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, kPersistMinCtas)
             genq_post(myq, (int)e, k0, k1);
           }
         });
+        dirty = a < N ? cell_pair(pin_cell(pos, G), pin_cell(tgt, G)) : OBS_CLEAN;
       }
       __syncwarp();
       if (agent) store_mask5(p.ts.action_mask + row_a * 5, mk3);
@@ -833,7 +845,9 @@ __global__ void __launch_bounds__((EW_WARPS + 2) * 32, kPersistMinCtas)
       if (VEC) {
         int4 *odst = obs_t;
         obs_t += obs_step;
-        if (OBS == 2)
+        if (OBS == 2 && rp.delta && t > 0)
+          os.emit_delta(kc, N, lane, j, __ffs(Np) - 1, (uint32_t)__cvta_generic_to_shared(g), dirty, terminal && a == 0, odst);
+        else if (OBS == 2)
           os.emit(kc, N, c4, lane, odst);
         else
           os.emit_direct(lut, wg32, kc, N, c4, lane, odst);
@@ -1022,6 +1036,7 @@ static RolloutLayout rollout_layout(int kind, int G, int N) {
     rp.stage_nbuf = pl.nbuf;
     rp.ce = pl.ce;
     rp.cv = pl.cv;
+    rp.delta = pl.nbuf == 1 && pl.ce == s.K;
     rp.stage_warp = (int)up16((size_t)rp.stage_nbuf * rp.stage_bytes);
     off += (size_t)L.PW * rp.stage_warp;
   }
@@ -1090,7 +1105,7 @@ int launch_rollout_persist(EnvParams p, int kind, int T, int32_t *action_out, in
   int resident = 0;
   if ((ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, fn, threads, smem)) != cudaSuccess) return set_cuda_error(ce, "cudaOccupancyMaxActiveBlocksPerMultiprocessor");
   if (resident < 1) return set_error(RBG_EINVAL, "rollout_persist_kernel does not fit an SM (%zu bytes of shared memory)", smem);
-  if (isolated && resident > 4) resident = 4;  // more resident CTAs measure slower (5: +0.6 %, 6-8: +1.1 %)
+  if (isolated && resident > 4) resident = 4;  // more resident CTAs measure slower (10x10/5 on B200: 5 -0.4 %, 6 -0.8 %)
   int64_t ctas = (int64_t)resident * device_sm_count();
   const int64_t need = (pp.ngroups + PW - 1) / PW;
   if (ctas > need) ctas = need;

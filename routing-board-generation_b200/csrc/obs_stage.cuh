@@ -16,6 +16,8 @@ namespace rbg {
 // The fused rollout kernel uses ONE stride for every N (codes 0..96), so that the per-agent
 // table rows sit at compile-time offsets from the four cell addresses of a packed word.
 constexpr int OBS_RS = 100;
+// ObsStager::emit_delta: a lane with no changed cell
+constexpr uint32_t OBS_CLEAN = 0xffffffffu;
 
 // four cells (one packed word) -> the same four cells in every agent's view: per agent four
 // table bytes and one 128-bit store, nothing else (views are c4 int4 apart).
@@ -64,6 +66,9 @@ __device__ __forceinline__ uint32_t lds_u8(uint32_t a) {
 }
 __device__ __forceinline__ void sts_v4(uint32_t a, uint32_t x, uint32_t y, uint32_t z, uint32_t w) {
   asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(x), "r"(y), "r"(z), "r"(w) : "memory");
+}
+__device__ __forceinline__ void sts_u32(uint32_t a, uint32_t x) {
+  asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(x) : "memory");
 }
 __device__ __forceinline__ uint32_t opaque(uint32_t v) {  // the compiler may not re-derive v
   asm volatile("" : "+r"(v));
@@ -243,6 +248,43 @@ struct ObsStager {
         buf ^= nbuf - 1;
       }
     }
+  }
+
+  // cell i of an env's grid (shared address g_s) -> the same cell of the env's N views, staged from shared address o
+  __device__ __forceinline__ void stage_cell(uint32_t o, uint32_t g_s, uint32_t i, int N) const {
+    uint32_t l = lut_s + lds_u8<0>(g_s + i);
+    o += 4u * i;
+    for (int x = 0; x < N; ++x, l += OBS_RS, o += view_b) sts_u32(o, lds_u8<0>(l));
+  }
+
+  // all 32 lanes, when the one buffer holds the warp's whole observation range (nbuf == 1, ce == K) and still holds
+  // the views that the previous emit of the same envs sent: restage only the cells that changed since, send it all.
+  // A step changes two cells per agent that moved (old head, destination); an env that reset is pins only, so its
+  // views are cleared (EMPTY is 0 in every view) and its agents restage their two pin cells.  dirty: this lane's two
+  // changed cells (cell | cell << 16) or OBS_CLEAN; reset_lead: the lane is the first of an env that reset; g_s:
+  // shared address of the lane's env grid (env j, lanes j << np_shift ..).  Every cell is looked up on the final
+  // grid, so the views are those a full fill would stage.
+  __device__ __forceinline__ void emit_delta(int kc, int N, int lane, int j, int np_shift, uint32_t g_s, uint32_t dirty, bool reset_lead,
+                                             int4 *odst) const {
+    const uint32_t env_b = view_b * (uint32_t)N;
+    if (lane == 0) bulk_wait_read<0>();  // the buffer has been read
+    __syncwarp();
+    uint32_t rm = __ballot_sync(FULL, reset_lead);
+    if (rm) {
+      for (; rm; rm &= rm - 1) {
+        const uint32_t o = stage_s + ((uint32_t)(__ffs(rm) - 1) >> np_shift) * env_b;
+        for (uint32_t b = 16u * (uint32_t)lane; b < env_b; b += 512u) sts_v4(o + b, 0u, 0u, 0u, 0u);
+      }
+      __syncwarp();  // cleared before the pins go in
+    }
+    if (dirty != OBS_CLEAN) {
+      const uint32_t o = stage_s + (uint32_t)j * env_b;
+      stage_cell(o, g_s, dirty & 0xffffu, N);
+      stage_cell(o, g_s, dirty >> 16, N);
+    }
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    __syncwarp();
+    if (lane == 0) bulk_store(odst, stage_s, (uint32_t)kc * env_b);
   }
 
   // the same views by direct 128-bit stores: for boards whose views are so large that a staged chunk

@@ -1,7 +1,7 @@
 """Time the fused rollout (rbg_connector_rollout_random) in the stationary regime: per-kernel averages
 from the library's own event pairs.  Used for A/B builds and ncu captures.
 
-    python tools/run_rollout.py [G N B T calls burnin_calls]"""
+    [KIND=uniform|dataset] python tools/run_rollout.py [G N B T calls burnin_calls]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -9,7 +9,11 @@ import routing_board_generation_b200 as rbg
 
 a = [int(x) for x in sys.argv[1:]]
 G, N, B, T, calls, burn = (a + [10, 5, 65536, 20, 25, 8][len(a):])[:6]
-gen = (rbg.UniformRandomGenerator if os.environ.get('KIND') == 'uniform' else rbg.ParallelRandomWalkGenerator)(grid_size=G, num_agents=N)
+kind = os.environ.get('KIND')
+if kind == 'dataset':  # rollout_warp_kernel: resets are picks from a stored board set
+    gen = rbg.BoardDatasetGeneratorJAX(G, N, board_name="offline_parallel_rw", number_of_boards=int(os.environ.get('BOARDS', '4096')))
+else:  # rollout_persist_kernel with its generator warps
+    gen = (rbg.UniformRandomGenerator if kind == 'uniform' else rbg.ParallelRandomWalkGenerator)(grid_size=G, num_agents=N)
 env = rbg.VmapAutoResetWrapper(rbg.Connector(generator=gen, time_limit=int(os.environ.get('TL', '50'))))
 keys = rbg.split(rbg.PRNGKey(0), B)
 st, _ = env.reset(keys)
