@@ -290,6 +290,37 @@ int rbg_connector_eval_step_live(const rbg_state *state, const int32_t *action, 
                                  const rbg_env_params *params, const rbg_timestep *ts,
                                  const rbg_episode_metrics *acc, void *stream);
 
+/* ---- CUDA graphs ----------------------------------------------------------------------------------------------------
+ * Capture: a call can be made while its `stream` is being captured into a CUDA graph (cudaStreamBeginCapture,
+ * torch.cuda.graph), and a replay computes, bit for bit, what the call computes eagerly, for rbg_split_keys,
+ * rbg_split_each, rbg_random_actions, rbg_generator_state, rbg_connector_observe, rbg_connector_reset,
+ * rbg_connector_step and rbg_connector_step_random (every auto-reset kind), rbg_connector_eval_step,
+ * rbg_connector_eval_step_live and rbg_connector_episodes_random.  While capturing, an auto-reset workspace is only
+ * recorded against the capture stream, never waited for: ordering a replay against other streams is the caller's job.
+ * SeedExtension's optimise kernel, which overlaps the extend kernel on a side stream when called eagerly, runs behind it
+ * on the captured stream.  Refused with RBG_EINVAL before anything is enqueued: any launch while kernel timing is on,
+ * rbg_connector_rollout_random (its persistent kernel takes host-side epochs that every replay would reuse), and the
+ * first use, or re-adoption, of an auto-reset workspace (step it once outside the capture).  The _host variants
+ * synchronise and are not capturable.
+ *
+ * Device-side evaluation loop: one graph launch runs a captured body (a policy-evaluation step) for as long as a
+ * device count says, with no host round trip.  The body's last node is rbg_eval_loop_condition.
+ *   rbg_eval_loop_create    a graph and the conditional handle `cond` of its WHILE node (default value 1, reapplied at
+ *                           every launch: the body runs at least once)
+ *   rbg_eval_loop_condition captured into the body: ++*steps, then the loop goes on while *live_count > 0 and
+ *                           *steps < max_steps (device int32 pointers; max_steps >= 1 bounds the loop whatever the count)
+ *   rbg_eval_loop_finalize  adds the WHILE node whose body is a copy of `body_graph` (a cudaGraph_t, e.g. torch's
+ *                           CUDAGraph(keep_graph=True).raw_cuda_graph()) and instantiates the loop; once per loop.
+ *                           The body may hold kernel, memset, memcpy and child-graph nodes only (no memory allocation:
+ *                           rbg_connector_eval_step_live's stream-ordered scratch cannot go in it)
+ *   rbg_eval_loop_launch    one launch of the finalized loop on `stream`
+ *   rbg_eval_loop_destroy   frees the loop (the caller first waits for its launches) */
+int rbg_eval_loop_create(void **loop, uint64_t *cond);
+int rbg_eval_loop_condition(uint64_t cond, const int32_t *live_count, int32_t *steps, int max_steps, void *stream);
+int rbg_eval_loop_finalize(void *loop, void *body_graph);
+int rbg_eval_loop_launch(void *loop, void *stream);
+int rbg_eval_loop_destroy(void *loop);
+
 /* Board validity: the reference's NumPy rules (numpy_implementation/utils/
  * post_processor_utils_numpy.py:34-155 = UP, numpy_implementation/utils/board_processor.py:111-162,
  * 391-487 = BP).  flags int32[B], 0 = valid by every rule:
@@ -381,7 +412,8 @@ int64_t rbg_launch_count(int reset);
 #define RBG_K_SEQRW 7      /* seqrw_walk_kernel + its finish kernel */
 #define RBG_K_EPISODES 8   /* episode_warp_kernel: random-agent episodes to their first LAST step */
 #define RBG_K_EVAL_STEP 9  /* eval_step_kernel: one policy-evaluation step of the live envs (both entry points) */
-#define RBG_K_COUNT 10
+#define RBG_K_EVAL_LOOP 10 /* eval_loop_cond_kernel: the condition of a device-side evaluation loop */
+#define RBG_K_COUNT 11
 int rbg_kernel_timing(int enable);
 int rbg_kernel_time(int kernel, int64_t *launches, double *total_ms);
 

@@ -68,6 +68,11 @@ SYMBOLS = {
     "rbg_connector_episodes_random": (_int, [_SP, _i64, _int, _int, _EP, _MP, _SP, _vp]),
     "rbg_connector_eval_step": (_int, [_SP, _vp, _vp, _vp, _i64, _int, _int, _EP, _TP, _MP, _vp]),
     "rbg_connector_eval_step_live": (_int, [_SP, _vp, _vp, _i64, _vp, _vp, _i64, _int, _int, _EP, _TP, _MP, _vp]),
+    "rbg_eval_loop_create": (_int, [C.POINTER(_vp), C.POINTER(C.c_uint64)]),
+    "rbg_eval_loop_condition": (_int, [C.c_uint64, _vp, _vp, _int, _vp]),
+    "rbg_eval_loop_finalize": (_int, [_vp, _vp]),
+    "rbg_eval_loop_launch": (_int, [_vp, _vp]),
+    "rbg_eval_loop_destroy": (_int, [_vp]),
     "rbg_validate": (_int, [_vp, _i64, _int, _int, _vp, _vp]),
     "rbg_board_statistics": (_int, [_vp, _i64, _int, _int, _vp, _vp, _vp, _vp]),
     "rbg_prw_generate_host": (_int, [_vp, _i64, _int, _int, _vp, _vp, _vp, _int]),
@@ -114,7 +119,7 @@ def launch_count(reset: bool = False) -> int:
     return int(load().rbg_launch_count(1 if reset else 0))
 
 
-KERNELS = {"prw": 0, "env": 1, "random_actions": 2, "split": 3, "validate": 4, "seedext": 5, "rollout": 6, "seqrw": 7, "episodes": 8, "eval_step": 9}
+KERNELS = {"prw": 0, "env": 1, "random_actions": 2, "split": 3, "validate": 4, "seedext": 5, "rollout": 6, "seqrw": 7, "episodes": 8, "eval_step": 9, "eval_loop": 10}
 
 
 def kernel_timing(enable: bool) -> None:

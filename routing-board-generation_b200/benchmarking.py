@@ -134,14 +134,27 @@ class PolicyEvaluator:
     is the policy work on finished envs; with a cheap policy, or episodes that nearly all run to time_limit, the wait
     and the list step cost more than that: on a B200 live_only measured 0.67x to 0.96x the default mode's speed for a
     cheap policy and a small MLP (DESIGN.md K7, tools/bench_policy_eval.py --live-only).
+
+    cuda_graph=True runs every evaluation as one CUDA graph launch: the policy call, the key split and the evaluation
+    step are captured once per batch size B (torch.cuda.CUDAGraph) and repeated on the device by a WHILE node until no
+    env is live (engine.EvalLoop), with no host wait per step and no step past the last episode.  The reset stays
+    eager (any generator, user Generators included) and is copied into the graph's static buffers.  The policy must be
+    capturable: static shapes, no host sync, no allocation outside torch's caching allocator.  The loop does not advance
+    torch's RNG from one iteration to the next: a stochastic policy must draw from the action keys it is given.  For a
+    policy that computes each row from that row alone the metrics are the default mode's, bit for bit.  A capture costs
+    a policy warm-up and a device synchronisation; the graph is kept until B changes or `close()`.  Not with live_only.
     """
 
-    def __init__(self, eval_env, policy, total_batch_size: int, live_only: bool = False):
+    def __init__(self, eval_env, policy, total_batch_size: int, live_only: bool = False, cuda_graph: bool = False):
         self.eval_env = eval_env
         self.policy = policy
         self.total_batch_size = int(total_batch_size)
         self.live_only = bool(live_only)
+        self.cuda_graph = bool(cuda_graph)
+        if self.live_only and self.cuda_graph:
+            raise ValueError("cuda_graph=True needs a static batch shape, and live_only=True changes it from step to step")
         self._env, self._reward_agg = _unwrap_eval_env(eval_env)
+        self._captured = None  # _CapturedEvaluation of the last batch size (cuda_graph=True)
 
     def episode_metrics(self, keys) -> Dict[str, torch.Tensor]:
         """Reset on `keys` (uint32[B,2], or one key of shape (2,) for unbatched results) and run the policy until
@@ -151,13 +164,16 @@ class PolicyEvaluator:
         B, N = keys.shape[0], self._env.num_agents
         st, ts = self._env.reset(keys)
         dev = st.grid.device
-        m = {k: torch.zeros((B, N) if k == "episode_return" else (B,), dtype=torch.float32 if k in ("episode_return", "ratio_connections") else torch.int32, device=dev)
-             for k in engine.EPISODE_METRICS}
-        chain = engine.split_each(keys)[:, 1]
-        if self.live_only:
-            self._run_live(st, ts.observation, m, chain)
+        if self.cuda_graph:
+            m = self._run_graph(st, ts, keys)
         else:
-            self._run_masked(st, ts, m, chain)
+            m = {k: torch.zeros((B, N) if k == "episode_return" else (B,), dtype=torch.float32 if k in ("episode_return", "ratio_connections") else torch.int32, device=dev)
+                 for k in engine.EPISODE_METRICS}
+            chain = engine.split_each(keys)[:, 1]
+            if self.live_only:
+                self._run_live(st, ts.observation, m, chain)
+            else:
+                self._run_masked(st, ts, m, chain)
         if self._reward_agg is not None:
             m["episode_return"] = self._reward_agg(m["episode_return"], dim=-1)
         return m if batched else {k: v[0] for k, v in m.items()}
@@ -204,7 +220,109 @@ class PolicyEvaluator:
             L = int(seen[0])
             order.reverse()
 
+    def _run_graph(self, st, ts, keys) -> Dict[str, torch.Tensor]:
+        """One launch of the captured loop (captured first when the batch size is new); the metrics cloned out."""
+        B = keys.shape[0]
+        if self._captured is not None and self._captured.B != B:
+            self.close()
+        first = self._captured is None
+        if first:
+            self._captured = _CapturedEvaluation(self._env, self.policy, B)
+        c = self._captured
+        c.load(st, ts, keys)
+        if first:
+            try:
+                c.capture()
+            except BaseException:
+                self.close()
+                raise
+        c.loop.launch()
+        return {k: v.clone() for k, v in c.m.items()}
+
+    @property
+    def loop_steps(self) -> int:
+        """Iterations of the device-side loop in the last cuda_graph=True evaluation: the longest episode's length
+        (reads the device)."""
+        if self._captured is None:
+            raise RuntimeError("no cuda_graph=True evaluation has run")
+        return int(self._captured.steps.item())
+
+    def close(self) -> None:
+        """Frees the captured graph and its static buffers (cuda_graph=True); the next evaluation captures again."""
+        if self._captured is not None:
+            if self._captured.loop is not None:
+                self._captured.loop.close()
+            self._captured = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
     def run_evaluation(self, key) -> Dict[str, torch.Tensor]:
         """Means over `total_batch_size` episodes whose reset keys are split(key, total_batch_size)."""
         m = self.episode_metrics(engine.split(key, self.total_batch_size))
         return {k: v.to(torch.float32).mean(dim=0) for k, v in m.items()}
+
+
+def _i32(t: torch.Tensor) -> torch.Tensor:
+    return t.view(torch.int32) if t.dtype == torch.uint32 else t
+
+
+class _CapturedEvaluation:
+    """PolicyEvaluator(cuda_graph=True) at one batch size: the static buffers and the device-side loop over them.
+
+    Loop body (captured once): chain, action_key = split_each(chain); action = policy(observation, action_key); the
+    evaluation step of the live envs; the loop condition (steps += 1, go on while an env is live and steps <= time_limit).
+    `graph` owns the memory of the body's intermediate tensors, so it lives as long as the loop."""
+
+    def __init__(self, env, policy, B: int):
+        G, N = env.grid_size, env.num_agents
+        dev = engine._device()
+        self.B, self._env, self._policy = B, env, policy
+        self.st, self.ts = engine.alloc_state(B, G, N), engine.alloc_timestep(B, G, N)
+        self.live = torch.empty(B, dtype=torch.uint8, device=dev)
+        self.live_count = torch.empty(1, dtype=torch.int32, device=dev)
+        self.steps = torch.empty(1, dtype=torch.int32, device=dev)
+        self.m = {k: torch.empty((B, N) if k == "episode_return" else (B,), dtype=torch.float32 if k in ("episode_return", "ratio_connections") else torch.int32, device=dev)
+                  for k in engine.EPISODE_METRICS}
+        self.chain = torch.empty((B, 2), dtype=torch.uint32, device=dev)
+        self.action_key = torch.empty((B, 2), dtype=torch.uint32, device=dev)
+        self.action = torch.empty((B, N), dtype=torch.int32, device=dev)
+        self.graph = self.loop = None
+
+    def load(self, st, ts, keys) -> None:
+        """The per-evaluation start: the reset State and observation, every env live, the counters and metrics zeroed,
+        chain = split_each(keys)[:, 1]."""
+        for dst, src in zip((self.st.grid, self.st.step_count, self.st.key, self.st.agents.id, self.st.agents.start, self.st.agents.target, self.st.agents.position),
+                            (st.grid, st.step_count, st.key, st.agents.id, st.agents.start, st.agents.target, st.agents.position)):
+            _i32(dst).copy_(_i32(src))
+        o, so = self.ts.observation, ts.observation
+        o.grid.copy_(so.grid)
+        o.action_mask.copy_(so.action_mask)
+        o.step_count.copy_(so.step_count)
+        self.live.fill_(1)
+        self.live_count.fill_(self.B)
+        self.steps.zero_()
+        for v in self.m.values():
+            v.zero_()
+        _i32(self.chain).copy_(_i32(engine.split_each(keys)[:, 1]))
+
+    def capture(self) -> None:
+        side = torch.cuda.Stream()
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side):  # torch's warm-up before a capture: the policy once, eagerly, on a side stream
+            self._policy(self.ts.observation, engine.split_each(self.chain)[:, 1].contiguous())
+        torch.cuda.current_stream().wait_stream(side)
+        args = self._env._env_args()
+        self.loop = engine.EvalLoop()
+        self.graph = torch.cuda.CUDAGraph(keep_graph=True)
+        with torch.cuda.graph(self.graph):
+            s = engine.split_each(self.chain)
+            _i32(self.chain).copy_(_i32(s[:, 0]))
+            _i32(self.action_key).copy_(_i32(s[:, 1]))
+            self.action.copy_(self._policy(self.ts.observation, self.action_key))
+            engine.connector_eval_step(self.st, self.action, self.live, self.live_count, self.m, self.ts, **args)
+            self.loop.condition(self.live_count, self.steps, args["time_limit"] + 1)
+        self.loop.finalize(self.graph)

@@ -204,6 +204,9 @@ def _generic_autoreset_step(env: Connector, state: State, action, inplace: bool)
     """VmapAutoResetWrapper.step for ANY Generator: plain Connector.step in the kernel, then for the envs whose
     step_type is LAST: `key, _ = split(state.key)`, `generator(key)`, the observation half of reset from the
     kernel, scattered over the batch (jumanji wrappers.py `_auto_reset` / `_maybe_reset`)."""
+    if torch.cuda.is_current_stream_capturing():
+        raise RuntimeError("auto-reset with a user Generator selects the finished envs on the host (a data-dependent index), "
+                           "which a CUDA graph cannot capture: step it eagerly, or use one of this package's generators")
     st, ts = engine.connector_step(state, action, **env._env_args(), inplace=inplace)
     idx = torch.nonzero(ts.step_type == LAST).flatten()
     if idx.numel() == 0:

@@ -56,6 +56,15 @@ static const DevProps &dev_props() {
 int device_sm_count() { return dev_props().sms; }
 size_t device_smem_per_sm() { return dev_props().smem_per_sm; }
 
+bool stream_capturing(cudaStream_t stream) {
+  cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
+  if (cudaStreamGetCaptureInfo(stream, &st) != cudaSuccess) {
+    cudaGetLastError();  // (the legacy stream beside a capturing blocking stream): not ours to report here
+    return false;
+  }
+  return st == cudaStreamCaptureStatusActive;
+}
+
 // ---- per-kernel event timing (rbg_kernel_timing / rbg_kernel_time) --------
 struct EventPair {
   cudaEvent_t a, b;
@@ -284,9 +293,10 @@ static void invalidate_workspace(void *workspace) {
 }
 
 // The workspace moves to another stream (rare): its work on the old stream is awaited on the host.  Events per call
-// would do, but an event record between two launches stops the second from starting under the first's tail.
+// would do, but an event record between two launches stops the second from starting under the first's tail.  A stream
+// that is being captured is only recorded: a graph's replays are ordered against other streams by whoever launches them.
 static int workspace_follow_stream(AutoResetCtx *ctx, cudaStream_t stream) {
-  if (ctx->tail_valid && ctx->last_stream != stream) {
+  if (ctx->tail_valid && ctx->last_stream != stream && !stream_capturing(stream)) {
     cudaStreamSynchronize(ctx->last_stream);
     cudaGetLastError();  // (the old stream may be gone)
   }
@@ -298,8 +308,11 @@ static int workspace_follow_stream(AutoResetCtx *ctx, cudaStream_t stream) {
 // A speculative call on `ws` for another batch than the recorded one (or the first call): nothing is cached yet.  The
 // counters are zeroed, and the cache is warm-started with the next episode of EVERY env, one bulk generation keyed by
 // the current State.key `keys` (a cold cache would send each env's first reset down the synchronous path).
+// Adoption is host-side bookkeeping that a replay would not redo, so it is refused while `stream` is capturing.
 static int adopt_workspace(AutoResetCtx *ctx, uint8_t *ws, int kind, const uint32_t *keys, int64_t B, int G, int N, cudaStream_t stream) {
   if (ctx->B == B && ctx->G == G && ctx->N == N && ctx->kind == kind) return RBG_OK;
+  if (stream_capturing(stream))
+    return set_error(RBG_EINVAL, "the auto-reset workspace is new to this batch (or was re-initialised): step once outside the capture before capturing a step");
   cudaError_t e;
   int rc;
   if ((e = cudaMemsetAsync(ws, 0, 256, stream)) != cudaSuccess) return set_cuda_error(e, "cudaMemsetAsync(counters)");
@@ -913,6 +926,9 @@ int rbg_connector_rollout_random(const rbg_state *state, int32_t *action_out, in
   if (T < 0) return set_error(RBG_EINVAL, "rollout length T=%lld", (long long)T);
   if ((rc = check_dims(B, G, N, 1))) return rc;
   if (B == 0 || T == 0) return RBG_OK;  // an empty batch has no buffers to check
+  if (stream_capturing((cudaStream_t)stream))
+    return set_error(RBG_EINVAL, "rbg_connector_rollout_random cannot be captured into a CUDA graph: its persistent kernel takes host-side "
+                                 "epochs that every replay would reuse (capture rbg_connector_step_random instead)");
   // (when G*G % 4 == 0 every step slice of the stacked arrays keeps the 16-byte alignment the
   // vector path needs; otherwise the kernels use scalar accesses)
   if ((rc = check_state(state, "state", G))) return rc;
@@ -996,6 +1012,76 @@ int rbg_connector_eval_step_live(const rbg_state *state, const int32_t *action, 
   if ((G * G) % 4 == 0 && !aligned16(ts->obs_grid)) return set_error(RBG_EALIGN, "timestep.obs_grid not 16-byte aligned");
   if ((rc = check_metrics(acc, "acc"))) return rc;
   return launch_eval_step_live(*state, action, order_in, L, order_out, count_out, B, G, N, *params, *ts, *acc, (cudaStream_t)stream);
+}
+
+// ---- device-side evaluation loop: a graph whose one node is a WHILE loop around a captured body
+struct EvalLoop {
+  cudaGraph_t graph = nullptr;
+  cudaGraphExec_t exec = nullptr;
+  cudaGraphConditionalHandle cond = 0;
+};
+
+int rbg_eval_loop_create(void **loop, uint64_t *cond) {
+  if (!loop || !cond) return set_error(RBG_EINVAL, "rbg_eval_loop_create: NULL pointer");
+  *loop = nullptr;
+  EvalLoop *l = new EvalLoop;
+  cudaError_t e = cudaGraphCreate(&l->graph, 0);
+  if (e == cudaSuccess) e = cudaGraphConditionalHandleCreate(&l->cond, l->graph, 1, cudaGraphCondAssignDefault);
+  if (e != cudaSuccess) {
+    if (l->graph) cudaGraphDestroy(l->graph);
+    delete l;
+    return set_cuda_error(e, "rbg_eval_loop_create");
+  }
+  *loop = l;
+  *cond = (uint64_t)l->cond;
+  return RBG_OK;
+}
+
+int rbg_eval_loop_condition(uint64_t cond, const int32_t *live_count, int32_t *steps, int max_steps, void *stream) {
+  if (!live_count || !steps) return set_error(RBG_EINVAL, "rbg_eval_loop_condition: NULL pointer");
+  if (max_steps < 1) return set_error(RBG_EINVAL, "rbg_eval_loop_condition: max_steps=%d must be >= 1", max_steps);
+  return launch_eval_loop_cond((unsigned long long)cond, live_count, steps, max_steps, (cudaStream_t)stream);
+}
+
+int rbg_eval_loop_finalize(void *loop, void *body_graph) {
+  if (!loop || !body_graph) return set_error(RBG_EINVAL, "rbg_eval_loop_finalize: NULL pointer");
+  EvalLoop *l = static_cast<EvalLoop *>(loop);
+  if (l->exec) return set_error(RBG_EINVAL, "rbg_eval_loop_finalize: the loop is already finalized");
+  cudaGraphNodeParams np = {};
+  np.type = cudaGraphNodeTypeConditional;
+  np.conditional.handle = l->cond;
+  np.conditional.type = cudaGraphCondTypeWhile;
+  np.conditional.size = 1;
+  cudaGraphNode_t node, child;
+  cudaError_t e = cudaGraphAddNode(&node, l->graph, nullptr, 0, &np);
+  if (e != cudaSuccess) return set_cuda_error(e, "rbg_eval_loop_finalize: WHILE node");
+  if ((e = cudaGraphAddChildGraphNode(&child, np.conditional.phGraph_out[0], nullptr, 0, static_cast<cudaGraph_t>(body_graph))) != cudaSuccess) {
+    cudaGraphDestroyNode(node);
+    return set_cuda_error(e, "rbg_eval_loop_finalize: body");
+  }
+  if ((e = cudaGraphInstantiate(&l->exec, l->graph, 0)) != cudaSuccess) {
+    l->exec = nullptr;
+    cudaGraphDestroyNode(node);
+    return set_cuda_error(e, "rbg_eval_loop_finalize: cudaGraphInstantiate");
+  }
+  return RBG_OK;
+}
+
+int rbg_eval_loop_launch(void *loop, void *stream) {
+  if (!loop) return set_error(RBG_EINVAL, "rbg_eval_loop_launch: NULL loop");
+  EvalLoop *l = static_cast<EvalLoop *>(loop);
+  if (!l->exec) return set_error(RBG_EINVAL, "rbg_eval_loop_launch: the loop has not been finalized (rbg_eval_loop_finalize)");
+  const cudaError_t e = cudaGraphLaunch(l->exec, (cudaStream_t)stream);
+  return e == cudaSuccess ? RBG_OK : set_cuda_error(e, "rbg_eval_loop_launch: cudaGraphLaunch");
+}
+
+int rbg_eval_loop_destroy(void *loop) {
+  if (!loop) return set_error(RBG_EINVAL, "rbg_eval_loop_destroy: NULL loop");
+  EvalLoop *l = static_cast<EvalLoop *>(loop);
+  if (l->exec) cudaGraphExecDestroy(l->exec);
+  if (l->graph) cudaGraphDestroy(l->graph);
+  delete l;
+  return RBG_OK;
 }
 
 int rbg_random_actions(const rbg_state *state, int64_t B, int G, int N, int32_t *action, void *stream) {

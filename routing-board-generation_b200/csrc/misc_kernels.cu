@@ -471,4 +471,17 @@ int launch_narrow_codes(const int32_t *src, uint8_t *dst, int64_t n, cudaStream_
   return launch_kernel(narrow_codes_kernel, (unsigned)ctas, 256, 0, stream, -1, "narrow_codes_kernel", false, src, dst, (long long)n);
 }
 
+// The last node of a device-side evaluation loop's body: counts the iteration and sets the WHILE node's condition.
+// max_steps bounds the loop whatever the count says.
+__global__ void __launch_bounds__(1) eval_loop_cond_kernel(cudaGraphConditionalHandle cond, const int32_t *__restrict__ live_count,
+                                                           int32_t *__restrict__ steps, int max_steps) {
+  const int s = ++*steps;
+  cudaGraphSetConditional(cond, (*live_count > 0 && s < max_steps) ? 1u : 0u);
+}
+
+int launch_eval_loop_cond(unsigned long long cond, const int32_t *live_count, int32_t *steps, int max_steps, cudaStream_t stream) {
+  return launch_kernel(eval_loop_cond_kernel, 1, 1, 0, stream, RBG_K_EVAL_LOOP, "eval_loop_cond_kernel", false, (cudaGraphConditionalHandle)cond,
+                       live_count, steps, max_steps);
+}
+
 }  // namespace rbg

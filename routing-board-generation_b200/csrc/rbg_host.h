@@ -19,6 +19,8 @@ int check_launch(const char *what);
 // properties of the current device (cached per device): SM count, shared memory per SM in bytes
 int device_sm_count();
 size_t device_smem_per_sm();
+// `stream` is being captured into a CUDA graph (cudaStreamGetCaptureInfo)
+bool stream_capturing(cudaStream_t stream);
 // Brackets one kernel launch: counts it (rbg_launch_count) and, while
 // rbg_kernel_timing is on, records a CUDA event pair on `stream` around it.
 bool kernel_timing_on();  // rbg_kernel_timing(1) is in effect
@@ -42,10 +44,13 @@ int opt_in_smem(void (*kernel)(KArgs...), size_t smem, const char *name) {
 // Every kernel of the library is launched here: the shared-memory opt-in, one LaunchScope under kernel id `id`
 // (RBG_K_*, or -1: counted, never timed), and the launch.  pdl: programmatic stream serialization (the kernel may
 // begin while a preceding kernel that has said launch_dependents is still running; any other predecessor completes
-// first).
+// first).  While kernel timing is on, a launch into a stream capture is refused: the event pairs would become graph
+// nodes that no host ever reads.
 template <typename... KArgs, typename... Args>
 int launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, int id, const char *name, bool pdl,
                   Args &&...args) {
+  if (kernel_timing_on() && stream_capturing(stream))
+    return set_error(RBG_EINVAL, "%s: kernel timing is on (rbg_kernel_timing(1)); a timed launch cannot be captured into a CUDA graph", name);
   if (int rc = opt_in_smem(kernel, smem, name)) return rc;
   cudaLaunchAttribute attr;
   attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -158,6 +163,9 @@ int launch_eval_step_live(const rbg_state &st, const int32_t *action, const int3
 int launch_split_keys(uint32_t k0, uint32_t k1, int64_t B, int64_t offset,
                       int64_t count, uint32_t *out, cudaStream_t stream);
 int launch_split_each(const uint32_t *keys, int64_t B, int num, uint32_t *out, cudaStream_t stream);
+// the condition of a device-side evaluation loop (eval_loop_cond_kernel): ++*steps, continue while *live_count > 0 and
+// *steps < max_steps
+int launch_eval_loop_cond(unsigned long long cond, const int32_t *live_count, int32_t *steps, int max_steps, cudaStream_t stream);
 int launch_dataset_state(const uint32_t *keys, int64_t B, int G, int N, const int32_t *heads, const int32_t *targets, int64_t K,
                          const rbg_state &st, cudaStream_t stream);
 int launch_board_stats(const int32_t *boards, int64_t B, int G, int count_current_wire, int32_t *scored, int32_t *detours, int32_t *diversity,

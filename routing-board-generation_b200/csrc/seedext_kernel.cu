@@ -990,7 +990,9 @@ int launch_seedext(SeedExtParams p, int64_t max_boards, cudaStream_t stream) {
     const char *ex = getenv("RBG_SE_OVERLAP");
     overlap_env = ex ? (atoi(ex) != 0 ? 1 : 0) : 1;
   }
-  const bool overlap = overlap_env == 1 && !kernel_timing_on();  // per-kernel timing wants one kernel at a time
+  // per-kernel timing wants one kernel at a time; a capture takes the serialized order too (DESIGN K7: the side stream
+  // and its events are shared by every caller of the device, and two graph branches are not promised to run at once)
+  const bool overlap = overlap_env == 1 && !kernel_timing_on() && !stream_capturing(stream);
   unsigned opt_resident = 1;
   {
     int per_sm = 0;

@@ -325,6 +325,8 @@ def _workspace(B: int, G: int, N: int, owner=None) -> torch.Tensor:
                 token = ("id", id(owner))
     k = (dev.index, B, G, N, token)
     if k not in _workspaces:
+        if torch.cuda.is_current_stream_capturing():  # (the allocation would come from the graph's private pool)
+            raise RuntimeError("the auto-reset workspace of this env batch does not exist yet: step once outside the capture before capturing a step")
         nbytes = int(_lib.load().rbg_step_workspace_bytes(B, G, N))
         _workspaces[k] = torch.empty((nbytes + 15) // 16 * 16, dtype=torch.uint8, device=dev)
         if owner is not None and not isinstance(token, tuple):
@@ -463,6 +465,44 @@ def connector_eval_step_live(st: State, action: torch.Tensor, order_in: torch.Te
     t = rbg_timestep(obs.grid.data_ptr(), obs.action_mask.data_ptr(), obs.step_count.data_ptr(), None, None, None, None, None, None)
     _lib.check(_lib.load().rbg_connector_eval_step_live(C.byref(s), act.data_ptr(), order_in.data_ptr(), L, order_out.data_ptr(), count.data_ptr(), B, G, N,
                                                         C.byref(params), C.byref(t), C.byref(m), _stream()))
+
+
+class EvalLoop:
+    """A device-side loop: one CUDA graph launch runs a captured body until a device count says stop (rbg_eval_loop_*).
+
+    Capture the body on a torch.cuda.CUDAGraph(keep_graph=True) and end it with `condition(live_count, steps,
+    max_steps)`; then `finalize(graph)` and `launch()` as often as needed.  The body is copied into the loop, but the
+    torch graph keeps owning the memory the body's tensors live in: keep it alive as long as the loop."""
+
+    def __init__(self):
+        h, c = C.c_void_p(), C.c_uint64()
+        _lib.check(_lib.load().rbg_eval_loop_create(C.byref(h), C.byref(c)))
+        self._h, self.cond = h.value, c.value
+
+    def condition(self, live_count: torch.Tensor, steps: torch.Tensor, max_steps: int) -> None:
+        """(captured) ++steps[0]; the loop goes on while live_count[0] > 0 and steps[0] < max_steps (int32[1] tensors)."""
+        if live_count.dtype != torch.int32 or steps.dtype != torch.int32 or live_count.numel() != 1 or steps.numel() != 1:
+            raise ValueError("live_count and steps must be int32[1]")
+        _lib.check(_lib.load().rbg_eval_loop_condition(self.cond, live_count.data_ptr(), steps.data_ptr(), int(max_steps), _stream()))
+
+    def finalize(self, body: "torch.cuda.CUDAGraph") -> None:
+        _lib.check(_lib.load().rbg_eval_loop_finalize(self._h, body.raw_cuda_graph()))
+
+    def launch(self) -> None:
+        _lib.check(_lib.load().rbg_eval_loop_launch(self._h, _stream()))
+
+    def close(self) -> None:
+        """Waits for the device and frees the loop."""
+        if self._h:
+            torch.cuda.synchronize()
+            _lib.load().rbg_eval_loop_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def random_actions(st: State) -> torch.Tensor:

@@ -1,5 +1,5 @@
 """Policy evaluation throughput: PolicyEvaluator (one eval-step launch per policy call) against a Connector.step loop,
-and with --live-only its two modes against each other.
+with --live-only its two modes against each other, and with --cuda-graph its default mode against its CUDA-graph mode.
 
 The policy is "keyed", a pure torch function of the action mask and the action key (agent a takes the
 ((key0 ^ a * 0x9E3779B9) mod n)-th of its n legal actions), so that every arm computes the same episodes, or "mlp", a
@@ -18,6 +18,10 @@ With --live-only, (b) is replaced by
   (d) PolicyEvaluator(live_only=True).episode_metrics: the policy sees only the live envs, one host wait per step to
       read their number;
   (e) the live step kernel alone (eval_step_kernel<LIST>), timed as (c) over the steps of (d).
+With --cuda-graph, (b) is replaced by
+  (f) PolicyEvaluator(cuda_graph=True).episode_metrics: the eager reset copied into static buffers, then one launch of
+      the captured loop (split, policy, eval step, loop condition) that runs on the device until no env is live; the
+      capture happens in the agreement check, before any timed window.  Its loop iterations are reported.
 Policy rows per evaluation (the rows the policy was handed, summed over its calls) are counted for (a) and (d).
 Rates: episodes/s = B / time, env-steps/s = sum(episode_length) / time (the same numerator for every arm).
 Kernel bandwidth: the bytes one live env-step moves (computed from the shape below) times sum(episode_length), over the
@@ -26,7 +30,7 @@ kernel time of (c); a dead env costs its live byte.  DESIGN K2's count for a ful
 Prints one JSON line per workload (and writes them to --out when given) with the card name, power limit and max SM
 clock read in the same run.
 
-    python tools/bench_policy_eval.py [--shapes 10x10/5x65536,32x32/16x8192] [--policy keyed|mlp] [--live-only] [--rounds 7] [--out FILE]
+    python tools/bench_policy_eval.py [--shapes 10x10/5x65536,32x32/16x8192] [--policy keyed|mlp] [--live-only | --cuda-graph] [--rounds 7] [--out FILE]
 """
 from __future__ import annotations
 
@@ -183,13 +187,15 @@ def _same(a: dict, b: dict) -> bool:
                for x, y in ((a[k], b[k]) for k in METRICS))
 
 
-def run_shape(rbg, G: int, N: int, B: int, time_limit: int, rounds: int, min_ms: float, seed: int, policy_name: str, live_only: bool) -> dict:
+def run_shape(rbg, G: int, N: int, B: int, time_limit: int, rounds: int, min_ms: float, seed: int, policy_name: str, live_only: bool,
+              cuda_graph: bool = False) -> dict:
     import torch
 
     policy = keyed_policy if policy_name == "keyed" else MlpPolicy(G, seed=seed)
     env = rbg.Connector(generator=rbg.ParallelRandomWalkGenerator(G, N), time_limit=time_limit)
     ev = rbg.PolicyEvaluator(env, policy, B)
     ev_live = rbg.PolicyEvaluator(env, policy, B, live_only=True)
+    ev_graph = rbg.PolicyEvaluator(env, policy, B, cuda_graph=True) if cuda_graph else None
     keys = rbg.split(rbg.PRNGKey(seed), B)
 
     # ---- the arms must agree before they are timed (a keyed policy: bit for bit)
@@ -209,6 +215,13 @@ def run_shape(rbg, G: int, N: int, B: int, time_limit: int, rounds: int, min_ms:
         if policy_name == "keyed":
             assert res["modes_agree_bit_for_bit"], "PolicyEvaluator's two modes disagree"
             assert rows["evaluator_live"] == env_steps, "the live mode handed the policy a row that is not a live env-step"
+    elif cuda_graph:
+        b = ev_graph.episode_metrics(keys)  # (captures the loop)
+        res["loop_iterations"] = ev_graph.loop_steps
+        res["modes_agree_bit_for_bit"] = _same(a, b)
+        if policy_name == "keyed":
+            assert res["modes_agree_bit_for_bit"], "PolicyEvaluator's default and CUDA-graph modes disagree"
+            assert res["loop_iterations"] == max_length, "the device-side loop did not stop after the longest episode"
     else:
         b, done = step_loop(rbg, env, policy, keys, time_limit)
         assert bool(done.all()), "an env had no LAST step within time_limit steps of its reset"
@@ -230,6 +243,8 @@ def run_shape(rbg, G: int, N: int, B: int, time_limit: int, rounds: int, min_ms:
     arms = {"evaluator": lambda: ev.episode_metrics(keys)}
     if live_only:
         arms["evaluator_live"] = lambda: ev_live.episode_metrics(keys)
+    elif cuda_graph:
+        arms["evaluator_graph"] = lambda: ev_graph.episode_metrics(keys)
     else:
         arms["step_loop"] = lambda: step_loop(rbg, env, policy, keys, time_limit)
     kernels = {"kernel": ev, "kernel_live": ev_live} if live_only else {"kernel": ev}
@@ -259,6 +274,8 @@ def run_shape(rbg, G: int, N: int, B: int, time_limit: int, rounds: int, min_ms:
     if live_only:
         res["kernel_live"]["us_per_step"] = res["kernel_live"]["ms_median"] * 1e3 / steps_live
         res["speedup_live_vs_default"] = res["evaluator"]["ms_median"] / res["evaluator_live"]["ms_median"]
+    elif cuda_graph:
+        res["speedup_graph_vs_default"] = res["evaluator"]["ms_median"] / res["evaluator_graph"]["ms_median"]
     else:
         res["speedup_evaluator_vs_step_loop"] = res["step_loop"]["ms_median"] / res["evaluator"]["ms_median"]
     return res
@@ -273,8 +290,11 @@ def main() -> None:
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--policy", choices=("keyed", "mlp"), default="keyed")
     ap.add_argument("--live-only", action="store_true", help="time PolicyEvaluator(live_only=True) against the default mode instead of the step loop")
+    ap.add_argument("--cuda-graph", action="store_true", help="time PolicyEvaluator(cuda_graph=True) against the default mode instead of the step loop")
     ap.add_argument("--out", default=None, help="also write the JSON lines here")
     args = ap.parse_args()
+    if args.live_only and args.cuda_graph:
+        raise SystemExit("--live-only and --cuda-graph are two different comparisons: pick one")
 
     import torch
 
@@ -291,7 +311,7 @@ def main() -> None:
         gg, rest = spec.split("/")
         G = int(gg.split("x")[0])
         N, B = (int(x) for x in rest.split("x"))
-        res = run_shape(rbg, G, N, B, args.time_limit, args.rounds, args.min_ms, args.seed, args.policy, args.live_only)
+        res = run_shape(rbg, G, N, B, args.time_limit, args.rounds, args.min_ms, args.seed, args.policy, args.live_only, args.cuda_graph)
         res.update(info)
         lines.append(json.dumps(res))
         print(lines[-1], flush=True)
